@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: 768x512 images/s of forward + likelihood + rate-distortion terms (BASELINE.json).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--precision bf16x3|bf16|fp32|mixed]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--precision bf16x3|bf16|fp32|mixed] [--dump-outputs DIR]
 
 The default arm is precision="bf16x3": every transform on the tcgen05 tensor cores with hi/lo-split bf16 operands (fp32 grade) -
 the arm that meets the parity bar of BASELINE.json (symbols, likelihoods 1e-4, bpp / PSNR 1e-3; tests/test_gpu_model.py).  The
@@ -29,6 +29,9 @@ One "step" = model(x, training=False) + the rd terms on one batch.
             host cores beside it (rank 0, bounded sample)
 
 --impl reference runs only that CPU arm (rank 0) and prints the same line shape with "impl": "reference".
+
+--dump-outputs DIR writes what the last timed step returned on rank 0 (the model's output dict and the rd terms) as DIR/<name>.npy,
+float32, so that two builds can be compared output for output on the same seeded inputs (see dump_outputs).
 """
 from __future__ import annotations
 
@@ -44,6 +47,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the source tree as it found it (it may be read-only)
 
 M, K, LAMBDA = 128, 3, 0.005
 H_IMG, W_IMG, B_PER_GPU = 512, 768, 16
@@ -98,6 +102,37 @@ def seeded_input(shape, seed=1):
     import torch
     g = torch.Generator(device="cpu"); g.manual_seed(seed)
     return torch.rand(*shape, generator=g)
+
+
+DUMP_MAX_ELEMS = 1 << 20        # per array: the outputs of one 16-image step then come to ~35 MB, inside the 64 MB budget
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(arrays: dict, out_dir: str) -> None:
+    """Write every floating-point tensor of `arrays` as out_dir/<name>.npy in float32 (float64 stays float64); other entries (flags,
+    None) are skipped.  An array of more than DUMP_MAX_ELEMS elements is reduced to a fixed sample of its flattened elements:
+    DUMP_MAX_ELEMS distinct indices in ascending order, drawn from a generator seeded with 0, so arrays of equal size share one index
+    set, from run to run and from build to build."""
+    import numpy as np
+    import torch
+    picked, index = {}, {}
+    for name, t in arrays.items():
+        if not isinstance(t, torch.Tensor) or not t.is_floating_point():
+            continue
+        t = t.detach().double() if t.dtype == torch.float64 else t.detach().float()
+        n = t.numel()
+        if n > DUMP_MAX_ELEMS:
+            if n not in index:
+                g = torch.Generator(device="cpu"); g.manual_seed(0)
+                index[n] = torch.randperm(n, generator=g)[:DUMP_MAX_ELEMS].sort().values
+            t = t.reshape(-1)[index[n].to(t.device)]
+        picked[name] = t.cpu().numpy()
+    total = sum(a.nbytes for a in picked.values())
+    if total > DUMP_MAX_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES}-byte budget")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in picked.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def load_peaks():
@@ -200,7 +235,11 @@ def main():
     ap.add_argument("--no-scalable", action="store_true", help="skip the scalable-coding line item (BASELINE.json configs[4])")
     ap.add_argument("--no-train-step", action="store_true", help="skip the training-step line item (BASELINE.json configs[3])")
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel from Python instead of replaying a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step (rank 0) as DIR/<name>.npy, float32; "
+                                                          "arrays over 2^20 elements as a fixed seeded sample (dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -257,8 +296,7 @@ def main():
     evaluator = parallel.ShardedEvaluator(model, LAMBDA, lean=False, graph=use_graph)
 
     def step(i):
-        _, terms = evaluator.step(dev_batches[i % nbuf])
-        return terms
+        return evaluator.step(dev_batches[i % nbuf])
 
     def sync_all():
         torch.cuda.synchronize()
@@ -267,14 +305,14 @@ def main():
             torch.cuda.synchronize()
 
     for i in range(args.warmup):
-        terms = step(i)
+        step(i)
     sync_all()
     sampler = ClockSampler(local_rank); sampler.start()
     l0 = lib.nic_launch_count()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(args.steps):
-        terms = step(i)
+        out, terms = step(i)
     e1.record()
     sync_all()
     launches = lib.nic_launch_count() - l0
@@ -287,6 +325,9 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_total = float(t.item())
     value = B * world * args.steps / (ms_total / 1e3)
+    if args.dump_outputs and rank == 0:
+        # now, before later steps overwrite them: a graphed step returns the static buffers of its CUDA graph
+        dump_outputs({**out, **{k: v for k, v in terms.items() if k != "scalars"}}, args.dump_outputs)
 
     # ---- e2e: pinned host input -> H2D -> forward -> rd_loss floats (D2H) every step -----------------
     # public API: ShardedEvaluator.evaluate_host_batches - per batch: pinned-host -> device copy (on a copy stream, overlapping

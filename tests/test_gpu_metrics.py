@@ -12,13 +12,13 @@ pytestmark = pytest.mark.gpu
 
 
 @pytest.mark.parametrize("shape", [(1, 3, 512, 768), (2, 3, 203, 181), (1, 3, 161, 400)])
-def test_compute_metrics_matches_the_oracle(shape):
+def test_compute_metrics_matches_the_oracle(shape, tmp_path):
     from neural_image_compression_b200.Evaluator import CompressionEvaluator, ms_ssim
     torch.manual_seed(sum(shape))
     orig = torch.rand(*shape)
     raw = orig + 0.08 * torch.randn_like(orig)                  # leaves [0, 1]: the evaluator clamps (Evaluator.py:73)
     ref = OM.compute_metrics(orig, raw.clamp(0, 1))
-    ev = CompressionEvaluator(None, None, "cuda", 0.005, save_dir="/tmp/nic_eval_test")
+    ev = CompressionEvaluator(None, None, "cuda", 0.005, save_dir=str(tmp_path))
     got = ev.compute_metrics(orig.cuda(), raw.cuda(), clamp=True)
     got2 = ev.compute_metrics(orig.cuda(), raw.clamp(0, 1).cuda())          # the reference's own call pattern
     assert set(got) == set(ref) == {"MSE(255)", "PSNR(RGB)", "MS-SSIM(RGB)", "PSNR(Y)", "MS-SSIM(Y)"}
@@ -40,13 +40,13 @@ def test_ms_ssim_rejects_small_images_like_the_reference_package():
         ms_ssim(torch.rand(1, 3, 160, 300).cuda(), torch.rand(1, 3, 160, 300).cuda())
 
 
-def test_evaluate_loop_keeps_the_reference_report_and_its_bpp_quirk():
+def test_evaluate_loop_keeps_the_reference_report_and_its_bpp_quirk(tmp_path):
     """Evaluator.py:55-92 on two synthetic 'Kodak' images; 'BPP' is the mean of bpp_y as in the reference (:81) unless fix_bpp."""
     from neural_image_compression_b200.Evaluator import CompressionEvaluator
     from neural_image_compression_b200.RateDistortionLoss import rd_loss
     model = H.seeded_model(128, 3, "calib", precision="bf16x3").cuda()
     loader = [H.seeded_input((1, 3, 256, 192)), H.seeded_input((1, 3, 192, 256)) * 0.5]
-    ev = CompressionEvaluator(model, loader, "cuda", 0.005, save_dir="/tmp/nic_eval_test")
+    ev = CompressionEvaluator(model, loader, "cuda", 0.005, save_dir=str(tmp_path))
     avg, imgs, recons = ev.evaluate(rd_loss)
     assert set(avg) == {"MSE(255)", "PSNR(RGB)", "MS-SSIM(RGB)", "PSNR(Y)", "MS-SSIM(Y)", "BPP", "BPP(y)", "BPP(z)"}
     assert avg["BPP"] == avg["BPP(y)"] and len(imgs) == len(recons) == 2 and float(recons[0].max()) <= 1.0
