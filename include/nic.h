@@ -450,6 +450,51 @@ size_t nic_ms_ssim_workspace_bytes(int32_t planes, int32_t h, int32_t w);
 int nic_ms_ssim_levels(const float* x, const float* y, int32_t planes, int32_t h, int32_t w, float data_range, int32_t clamp_y,
                        float* level_means, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- entropy coder (DESIGN.md section 9): byte strings for JointAutoregressiveHierarchical ------------------------------------
+ * rANS with a 32-bit state in [2^16, 2^32), 16-bit renormalisation words and 16-bit probabilities.  A table row of one element is
+ * a window of n <= NIC_CODEC_WINDOW consecutive integers starting at lo plus an escape bin (index n) for any other value; an
+ * escaped value v follows the escape bin as two raw 16-bit words of zigzag(v) (low half first).  Row layout: cdf[0] = 0,
+ * cdf[i + 1] = cdf[i] + freq_i (freq_i >= 1), cdf[n + 1] = 2^16; NIC_CODEC_WINDOW + 2 uint32 entries per row.
+ * y elements are coded in wavefront order: pixel (i, j) belongs to step t = 3 i + j (3 h + w - 3 steps; the masked 5x5 context of
+ * a pixel only reads pixels of earlier steps), pixels of a step with i ascending, lane l holds channels c = l (mod lanes)
+ * ascending.  z elements: pixels in raster order, the same channel-to-lane rule.
+ */
+#define NIC_CODEC_PREC_BITS 16
+#define NIC_CODEC_WINDOW 128
+enum { NIC_CODEC_GM = 0, NIC_CODEC_FACTORIZED = 1 };   /* y: Gaussian mixture (K = 1: Gaussian); z: factorized prior */
+enum { NIC_CODEC_TABLES = 0, NIC_CODEC_SYMBOL = 1 };
+
+/*
+ * The quantised tables, the one function both coder directions use (a single compiled kernel with a runtime mode, so the
+ * float -> integer step is the same instructions for both).
+ *   kind GM:         params = raw entropy parameters [b, (3K | 2) m, h, w] (nic_ctx_ep_fwd's raw), k = K
+ *   kind FACTORIZED: params = nic_pack_factorized's [m, 43] (k ignored)
+ *   mode TABLES:     GM: the elements of wavefront step t, e = (img * cnt + p) * m + c (p-th pixel of the step) -> cdf [e][W + 2],
+ *                    lo [e], nbins [e];  FACTORIZED: one row per channel (e = c; b, h, w only checked)
+ *   mode SYMBOL:     every element e of the NCHW latent sym [b, m, h, w] -> code [e] = start | freq << 16 | escape << 32 of its symbol
+ */
+int nic_codec_tables(int32_t kind, int32_t mode, const float* params, const float* sym, int32_t b, int32_t m, int32_t k, int32_t h,
+                     int32_t w, int32_t t, uint32_t* cdf, int32_t* lo, int32_t* nbins, uint64_t* code, void* stream);
+/*
+ * rANS encode, one thread per (image, lane): code / sym as nic_codec_tables(SYMBOL) saw them.  Lane g = img * lanes + l writes its
+ * segment - the final state (2 words, low first) followed by the words in decode order - at the END of words[g * cap, (g + 1) * cap)
+ * and its length in words (state included) to count[g].  cap >= 3 * ceil(m / lanes) * h * w + 2.
+ */
+int nic_codec_encode(int32_t kind, const uint64_t* code, const float* sym, int32_t b, int32_t m, int32_t h, int32_t w, int32_t lanes,
+                     int64_t cap, uint16_t* words, int32_t* count, void* stream);
+/*
+ * rANS decode, one thread per (image, lane).  kind GM: wavefront step t with the step's tables; kind FACTORIZED: all of z with the
+ * per-channel tables.  blob holds the byte strings; lane g's segment starts at byte lane_off[g] (4 state bytes, then lane_words[g]
+ * words; reads past them return 0).  state / pos [b * lanes] carry each lane's cursor from one step to the next (init = 1: start
+ * from the segment).  Symbols go to out, NHWC f32 [b, h, w, m].
+ */
+int nic_codec_decode(int32_t kind, const uint8_t* blob, const int64_t* lane_off, const int32_t* lane_words, uint32_t* state, int32_t* pos,
+                     int32_t init, const uint32_t* cdf, const int32_t* lo, const int32_t* nbins, int32_t b, int32_t m, int32_t h, int32_t w,
+                     int32_t lanes, int32_t t, float* out, void* stream);
+/* out [b] = per image sum over the symbols (y [b, y_per_image] then z [b, z_per_image], NCHW f32) of a 32-bit mix of (index, value),
+ * mod 2^32 */
+int nic_codec_checksum(const float* y, int64_t y_per_image, const float* z, int64_t z_per_image, int32_t b, uint32_t* out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

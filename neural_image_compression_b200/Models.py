@@ -278,6 +278,19 @@ class JointAutoregressiveHierarchical(nn.Module):
                 out.update({"weights": ly["weights"], "mus": ly["mus"], "sigmas": ly["sigmas"]})
         return out
 
+    def compress(self, x: torch.Tensor) -> dict:
+        """x [B, 3, H, W] (H, W multiples of 64) -> {"strings": [y_strings, z_strings], "shape": (hz, wz)}: one bytes object per
+        image in each list, coded with the eval-mode symbols (the forward's y_in / z_in).  Format: DESIGN.md section 9."""
+        from . import codec
+        return codec.compress(self, x)
+
+    def decompress(self, strings, shape) -> dict:
+        """strings / shape as compress returned them (any subset of the images, in any order) -> {"x_hat", "y_hat", "z_hat"},
+        NCHW f32; x_hat = g_s(y_hat), not clamped.  Raises ValueError on a string of another precision arm / M / K, on a malformed
+        string, or when an image's symbol checksum does not match (corrupted bytes, other weights)."""
+        from . import codec
+        return codec.decompress(self, strings, shape)
+
 
 class HierarchicalMixtureResidual(nn.Module):
     """``HierarchicalMixtureResidual`` of /root/reference/Models.py:109-205: the same entropy side and output dict as

@@ -99,7 +99,17 @@ SIGNATURES = {
     "nic_gdn_bwd_finish_workspace_bytes": (_sz, [_i64, _i32]),
     "nic_gdn_bwd_finish": (C.c_int, [_vp, _vp, _vp, _i64, _i32, _f32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "nic_adam_step": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _f32, _f32, _f32, _f32, _i32, _vp]),
+    # entropy coder
+    "nic_codec_tables": (C.c_int, [_i32, _i32, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp]),
+    "nic_codec_encode": (C.c_int, [_i32, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i64, _vp, _vp, _vp]),
+    "nic_codec_decode": (C.c_int, [_i32, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp]),
+    "nic_codec_checksum": (C.c_int, [_vp, _i64, _vp, _i64, _i32, _vp, _vp]),
 }
+
+# entropy coder constants of include/nic.h
+CODEC_GM, CODEC_FACTORIZED = 0, 1
+CODEC_TABLES, CODEC_SYMBOL = 0, 1
+CODEC_PREC_BITS, CODEC_WINDOW = 16, 128
 
 _lib = None
 
