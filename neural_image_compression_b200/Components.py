@@ -4,7 +4,8 @@ Same class names, constructor arguments and ``net.<i>`` parameter names as the r
 (Encoder5x5 :6-18, Decoder5x5 :35-47, HyperEncoder5x5 :65-75, HyperDecoder5x5 :94-105), so
 ``state_dict`` round-trips.  ``forward`` does not execute the ``nn.Sequential``: each
 conv (+ the GDN / IGDN / LeakyReLU after it) is one ``nic_conv_fwd`` call with the activation fused
-into the epilogue, activations staying NHWC between layers.
+into the epilogue, activations staying NHWC between layers.  ``run_nhwc`` is the layer-by-layer form
+the training step records on a ``training.Tape`` (GDN / IGDN as ops of their own).
 
 The 3x3 residual family (Encoder3x3 / Decoder3x3 / HyperEncoder3x3 / HyperDecoder3x3, Components.py:20-32, 49-62, 77-91,
 107-122; blocks in Layers.py) runs layer by layer on the same engine (SURVEY.md section 8 row f4).
@@ -14,8 +15,9 @@ from __future__ import annotations
 import torch
 import torch.nn as nn
 
+from . import Layers as L
 from . import engine
-from ._lib import EPI_BIAS, EPI_GDN, EPI_IGDN, EPI_LRELU
+from ._lib import EPI_BIAS, EPI_GDN, EPI_IGDN, EPI_LRELU, LAYOUT_NCHW, LAYOUT_NHWC
 from .gdn import GDN
 
 
@@ -43,6 +45,19 @@ class _Transform(nn.Module):
     @property
     def ops(self):
         return self._ops
+
+    def run_nhwc(self, x, n, h, w, arm, in_layout=None, tape=None, final_kw=None):
+        """The chain layer by layer on f32 NHWC tensors (the calls of _Chain.run_nhwc): a conv followed by a GDN / IGDN keeps the
+        bias epilogue and the GDN runs as its own op (the training forward keeps the pre-GDN tensor for the GDN backward)."""
+        layout = LAYOUT_NHWC if in_layout is None else in_layout
+        for i, op in enumerate(self._ops):
+            kw = final_kw if (final_kw and i == len(self._ops) - 1) else {}
+            x, h, w = L._conv(arm, op.conv, EPI_BIAS if op.gdn is not None else op.epilogue, x, n, h, w, in_layout=layout, tape=tape,
+                              **kw)
+            if op.gdn is not None:
+                x = L._gdn(arm, op.gdn, x, n, h, w, tape=tape)
+            layout = LAYOUT_NHWC
+        return x, h, w
 
     def forward(self, x: torch.Tensor) -> torch.Tensor:
         # stand-alone call of one transform: the fp32 arm unless the owner asked for a tensor-core arm explicitly
@@ -122,8 +137,6 @@ class _Chain(nn.Module):
     def run_nhwc(self, x, n, h, w, arm, in_layout=None, tape=None, final_kw=None):
         """tape: training.Tape that records every op for the backward (training forward); final_kw: `out=` window arguments of
         the LAST conv (h_s writes psi straight into the concat buffer of the entropy-parameter stack)."""
-        from . import Layers as L
-        from ._lib import LAYOUT_NHWC
         layout = LAYOUT_NHWC if in_layout is None else in_layout
         mods, i = list(self.net), 0
         while i < len(mods):
@@ -148,8 +161,6 @@ class _Chain(nn.Module):
         return x, h, w
 
     def forward(self, x: torch.Tensor) -> torch.Tensor:
-        from . import Layers as L
-        from ._lib import LAYOUT_NCHW
         engine.require_cuda(x, "x")
         n, c, h, w = x.shape
         arm = L._arm(self.precision, c if c >= 64 else 64)

@@ -33,17 +33,78 @@ from .EntropyModels import FactorizedEntropyBottleneck, GaussianConditional, Gau
 from .ParametersModels import EntropyParameters
 
 
-def _pair_noise(model, x, training, noise):
-    B, _, H, W = x.shape
-    if not training:
-        return None, None
+def check_channels(latent_channels, K):
+    """The constructor arguments every model shares."""
+    if not isinstance(latent_channels, int) or latent_channels < 1:
+        raise ValueError(f"latent_channels must be int >= 1, got {latent_channels}")
+    if not isinstance(K, int) or K < 1:
+        raise ValueError(f"K must be int >= 1, got {K}")
+
+
+def check_input(x: torch.Tensor):
+    """x must be a CUDA tensor [B, 3, H, W] with H and W multiples of 64."""
+    engine.require_cuda(x, "x")
+    if x.dim() != 4 or x.shape[1] != 3:
+        raise ValueError(f"expected x of shape [B, 3, H, W], got {tuple(x.shape)}")
+    H, W = x.shape[2:]
+    if H % 64 or W % 64:
+        raise ValueError(f"H and W must be multiples of 64 (four stride-2 stages in g_a, two in h_a); got {H}x{W}")
+
+
+def draw_noise(M: int, x: torch.Tensor, noise=None):
+    """(noise_z, noise_y) of a training forward: `noise` when given, else U(-0.5, 0.5) drawn z first, then y, as the reference
+    does (Models.py:57-58), so seeded runs draw the same noise on every path."""
     if noise is not None:
         return noise
-    M = model.M
+    B, _, H, W = x.shape
     return (torch.rand((B, M, H // 64, W // 64), device=x.device) - 0.5, torch.rand((B, M, H // 16, W // 16), device=x.device) - 0.5)
 
 
-def _pair_g_a(model, x, training, noise_y, prec_up, prec):
+def precision_arms(precision: str) -> Tuple[str, str]:
+    """Model precision -> (arm of g_a and h_a, arm of h_s, the context model, the entropy parameters and g_s): "mixed" keeps
+    everything that decides the symbols in fp32."""
+    return ("fp32" if precision == "mixed" else precision), ("bf16" if precision == "mixed" else precision)
+
+
+def _param_names(K: int):
+    return ("mu", "sigma") if K == 1 else ("weights", "mus", "sigmas")
+
+
+def mixture_params(ly: dict, K: int, lean: bool = False) -> list:
+    """The distribution parameters of a gm_likelihood result in output order: (mu, sigma) for K == 1, else (weights, mus,
+    sigmas); none when lean."""
+    return [] if lean else [ly[k] for k in _param_names(K)]
+
+
+def single_head_outputs(x_hat, logp_y, logp_z, y, y_in, z, z_in, p_z, p_y, parts_y, parts_z, *params, K: int, training: bool) -> dict:
+    """The output dict of JointAutoregressiveHierarchical and HierarchicalMixtureResidual (Models.py:92-104, same key order)
+    from the values in the order training._forward_impl returns them; params = mixture_params(...).  The per-image sums of
+    logp ride along on logp_y / logp_z for rd_loss (RateDistortionLoss.py:13-14)."""
+    engine.attach_partials(logp_y, parts_y)
+    engine.attach_partials(logp_z, parts_z)
+    out = {"x_hat": x_hat, "y": y, "y_in": y_in, "z": z, "z_in": z_in, "p_z": p_z, "logp_z": logp_z, "p_y": p_y, "logp_y": logp_y,
+           "training": training}
+    out.update(zip(_param_names(K), params))
+    return out
+
+
+def two_head_outputs(x_hat, logp_y1, logp_y2, logp_z, y, y_in, z, z_in, p_z, p_y1, p_y2, parts_y1, parts_y2, parts_z, *params,
+                     M1: int, K: int, training: bool) -> dict:
+    """The output dict of ScalableImageCoding (Models.py:321-338 without 'F_tilde') from the values in the order
+    training_scalable's autograd node returns them; params = mixture_params of head 1, then of head 2."""
+    for logp, parts in ((logp_y1, parts_y1), (logp_y2, parts_y2), (logp_z, parts_z)):
+        engine.attach_partials(logp, parts)
+    y1, y2 = torch.split(y_in, [M1, y_in.shape[1] - M1], dim=1)            # Models.py:279 (views, as in the reference)
+    out = {"x_hat": x_hat, "y": y, "y_in": y_in, "y1": y1, "y2": y2, "z": z, "z_in": z_in, "p_z": p_z, "logp_z": logp_z,
+           "p_y1": p_y1, "logp_y1": logp_y1, "p_y2": p_y2, "logp_y2": logp_y2, "training": training}
+    names = _param_names(K)
+    out.update(zip([k + "1" for k in names] + [k + "2" for k in names], params))
+    return out
+
+
+# ---- stages of the fused pair-tensor pipeline (JointAutoregressiveHierarchical, ScalableImageCoding's bf16x3 arm, the codec) ----
+
+def fused_g_a(model, x, training, noise_y, prec_up, prec):
     """g_a -> y hand-off of the fused pipeline (Models.py:52, 57-64): activations NHWC between layers (bf16 hi/lo pairs in the bf16x3
     arm).  Returns (y, y_in, y_in_nhwc, y_src) with y_src = the unquantised y in the engine's layout for h_a (Models.py:53)."""
     B, _, H, W = x.shape
@@ -63,7 +124,7 @@ def _pair_g_a(model, x, training, noise_y, prec_up, prec):
     return y, y_in, y_in_nhwc, (y_lowp if lowp else y_nhwc)
 
 
-def _pair_h_a(model, y_src, B, hy, wy, training, noise_z, prec_up, prec):
+def fused_h_a(model, y_src, B, hy, wy, training, noise_z, prec_up, prec):
     """h_a -> z hand-off (Models.py:53, 57-64).  Returns (z, z_in, z_in_nhwc)."""
     adt = engine.act_dtype(prec)
     a, h, w = y_src, hy, wy
@@ -75,16 +136,16 @@ def _pair_h_a(model, y_src, B, hy, wy, training, noise_z, prec_up, prec):
     return z, z_in, z_in_nhwc
 
 
-def _pair_h_s_into(model, z_in_nhwc, B, hz, wz, prec, combined, c_total, c_offset):
-    """h_s (Models.py:69) with its last conv writing psi into channels [c_offset, c_offset + 2M) of `combined`."""
-    z_flag = getattr(z_in_nhwc, "_nic_lo_flag", None)
+def fused_h_s_into(model, z_in_nhwc, B, hz, wz, prec, combined, c_total, c_offset, lo_flag):
+    """h_s (Models.py:69) with its last conv writing psi into channels [c_offset, c_offset + 2M) of `combined`.  lo_flag: the
+    `_nic_lo_flag` of z_in_nhwc (its first conv skips the MMA pass of an all-zero lo half), or None for all three passes."""
     a, h, w = z_in_nhwc, hz, wz
     hs = model.hyper_decoder.ops
     for i, op in enumerate(hs):
         if i == len(hs) - 1:
             op.run(a, B, h, w, prec, out=combined, out_c_total=c_total, out_c_offset=c_offset)
         else:
-            a = op.run(a, B, h, w, prec, in_lo_flag=z_flag if i == 0 else None)
+            a = op.run(a, B, h, w, prec, in_lo_flag=lo_flag if i == 0 else None)
         h, w = engine.conv_out_hw(op.conv, h, w)
 
 
@@ -104,7 +165,7 @@ def _branch_stream(device, index: int = 0):
     return _SIDE_STREAMS[key]
 
 
-def _pair_g_s(model, y_in_nhwc, B, hy, wy, prec):
+def fused_g_s(model, y_in_nhwc, B, hy, wy, prec):
     """g_s (Models.py:90): NHWC symbols -> x_hat NCHW f32."""
     y_flag = getattr(y_in_nhwc, "_nic_lo_flag", None)
     a, h, w = y_in_nhwc, hy, wy
@@ -135,10 +196,7 @@ class JointAutoregressiveHierarchical(nn.Module):
 
     def __init__(self, latent_channels: int = 192, K: int = 1, *, precision: Optional[str] = None):
         super().__init__()
-        if not isinstance(latent_channels, int) or latent_channels < 1:
-            raise ValueError(f"latent_channels must be int >= 1, got {latent_channels}")
-        if not isinstance(K, int) or K < 1:
-            raise ValueError(f"K must be int >= 1, got {K}")
+        check_channels(latent_channels, K)
         self.M = latent_channels
         self.K = K
         self.H = latent_channels
@@ -164,12 +222,8 @@ class JointAutoregressiveHierarchical(nn.Module):
                 (training=True only; the reference draws z's noise first, Models.py:57-58).
         lean  : skip materialising weights/mus/sigmas (mu/sigma); those keys are then absent.
         """
-        engine.require_cuda(x, "x")
-        if x.dim() != 4 or x.shape[1] != 3:
-            raise ValueError(f"expected x of shape [B, 3, H, W], got {tuple(x.shape)}")
+        check_input(x)
         B, _, H, W = x.shape
-        if H % 64 or W % 64:
-            raise ValueError(f"H and W must be multiples of 64 (four stride-2 stages in g_a, two in h_a); got {H}x{W}")
         if training and torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
             # the reference's training call (Trainer.py:82): autograd is on, so the step must be differentiable.  One autograd
             # node over the fp32 arm with hand-written backward kernels (training.py); under torch.no_grad() the call below
@@ -183,25 +237,14 @@ class JointAutoregressiveHierarchical(nn.Module):
             if self.M % 64:
                 raise ValueError(f"precision='bf16x3' needs latent_channels % 64 == 0, got {self.M}")
             from . import training as _training
-            from ._lib import Q_NOISE as _QN, Q_ROUND as _QR
             with torch.no_grad():
-                nz = ny = None
-                if training:
-                    nz, ny = noise if noise is not None else (torch.rand((B, self.M, H // 64, W // 64), device=x.device) - 0.5,
-                                                              torch.rand((B, self.M, H // 16, W // 16), device=x.device) - 0.5)
+                nz, ny = draw_noise(self.M, x, noise) if training else (None, None)
                 _training.forget_pairs()
-                res, _ = _training._forward_impl(self, x.contiguous().float(), nz, ny, lean, qmode=_QN if training else _QR, arm="bf16x3")
+                res, _ = _training._forward_impl(self, x.contiguous().float(), nz, ny, lean, qmode=Q_NOISE if training else Q_ROUND,
+                                                 arm="bf16x3")
                 _training.forget_pairs()
-            x_hat, logp_y, logp_z, y, y_in, z, z_in, p_z, p_y, parts_y, parts_z = res[:11]
-            engine.attach_partials(logp_y, parts_y)
-            engine.attach_partials(logp_z, parts_z)
-            out = {"x_hat": x_hat, "y": y, "y_in": y_in, "z": z, "z_in": z_in, "p_z": p_z, "logp_z": logp_z, "p_y": p_y,
-                   "logp_y": logp_y, "training": training}
-            if not lean:
-                out.update(dict(zip(("mu", "sigma") if self.K == 1 else ("weights", "mus", "sigmas"), res[11:])))
-            return out
-        prec_up = {"fp32": "fp32", "mixed": "fp32", "bf16x3": "bf16x3", "bf16": "bf16"}[self.precision]   # g_a, h_a
-        prec = {"fp32": "fp32", "mixed": "bf16", "bf16x3": "bf16x3", "bf16": "bf16"}[self.precision]    # h_s, context, entropy parameters, g_s
+            return single_head_outputs(*res, K=self.K, training=training)
+        prec_up, prec = precision_arms(self.precision)
         adt = engine.act_dtype(prec)
         pair = prec == "bf16x3"                      # activations are bf16 hi/lo pairs: [hi(c) | lo(c)] channels
         cw = 2 if pair else 1
@@ -209,8 +252,8 @@ class JointAutoregressiveHierarchical(nn.Module):
         x = x.contiguous().float()
         hy, wy, hz, wz = H // 16, W // 16, H // 64, W // 64
         with torch.cuda.device(x.device), torch.no_grad():
-            noise_z, noise_y = _pair_noise(self, x, training, noise)
-            y, y_in, y_in_nhwc, y_src = _pair_g_a(self, x, training, noise_y, prec_up, prec)
+            noise_z, noise_y = draw_noise(M, x, noise) if training else (None, None)
+            y, y_in, y_in_nhwc, y_src = fused_g_a(self, x, training, noise_y, prec_up, prec)
 
             # ---- two parallel branches while the pass is captured in a CUDA graph: g_s (needs y_in only) and the context conv
             # (y_in only) run beside h_a -> h_s; the context conv joins before the 1x1 stack, g_s at the end
@@ -218,7 +261,7 @@ class JointAutoregressiveHierarchical(nn.Module):
             if branch is not None:
                 branch.wait_stream(main_stream)
                 with torch.cuda.stream(branch):
-                    x_hat = _pair_g_s(self, y_in_nhwc, B, hy, wy, prec)
+                    x_hat = fused_g_s(self, y_in_nhwc, B, hy, wy, prec)
             # phi = combined[..., 0:2M] (context), psi = combined[..., 2M:4M] (h_s): torch.cat([phi, psi]) never happens.
             # (the quantised symbols split into bf16 pairs with an all-zero lo half - the hand-off kernel checks and flags it on the
             #  device: their first consumers - h_s layer 1, the context conv, g_s layer 1 - run 2 of the 3 MMA passes)
@@ -235,8 +278,8 @@ class JointAutoregressiveHierarchical(nn.Module):
                 with (torch.cuda.stream(branch2) if branch2 is not None else contextlib.nullcontext()):
                     self.context_model.masked._op.run(y_in_nhwc, B, hy, wy, prec, out=combined, out_c_total=4 * M, out_c_offset=0,
                                                       in_lo_flag=y_flag)
-            z, z_in, z_in_nhwc = _pair_h_a(self, y_src, B, hy, wy, training, noise_z, prec_up, prec)
-            _pair_h_s_into(self, z_in_nhwc, B, hz, wz, prec, combined, 4 * M, 2 * M)
+            z, z_in, z_in_nhwc = fused_h_a(self, y_src, B, hy, wy, training, noise_z, prec_up, prec)
+            fused_h_s_into(self, z_in_nhwc, B, hz, wz, prec, combined, 4 * M, 2 * M, getattr(z_in_nhwc, "_nic_lo_flag", None))
             if branch2 is not None:
                 main_stream.wait_stream(branch2)
 
@@ -256,27 +299,14 @@ class JointAutoregressiveHierarchical(nn.Module):
                 # ---- likelihoods -------------------------------------------------------------------------
                 ly = gm_likelihood(y_in, raw, M, K, Q_PASSTHRU, full=not lean, want_y_in=False)
             _, p_z, logp_z, parts_z = self.factorized_entropy_model.likelihood(z_in, Q_PASSTHRU)
-            p_y, logp_y = ly["p"], ly["logp"]
 
             # ---- g_s -----------------------------------------------------------------------------------
             if branch is not None:
                 main_stream.wait_stream(branch)                 # join
             else:
-                x_hat = _pair_g_s(self, y_in_nhwc, B, hy, wy, prec)
-
-        # per-image partial sums of logp ride along for rd_loss (RateDistortionLoss.py:13-14)
-        engine.attach_partials(logp_y, ly["partials"])
-        engine.attach_partials(logp_z, parts_z)
-        out = {
-            "x_hat": x_hat, "y": y, "y_in": y_in, "z": z, "z_in": z_in,
-            "p_z": p_z, "logp_z": logp_z, "p_y": p_y, "logp_y": logp_y, "training": training,
-        }
-        if not lean:
-            if K == 1:
-                out.update({"mu": ly["mu"], "sigma": ly["sigma"]})
-            else:
-                out.update({"weights": ly["weights"], "mus": ly["mus"], "sigmas": ly["sigmas"]})
-        return out
+                x_hat = fused_g_s(self, y_in_nhwc, B, hy, wy, prec)
+        return single_head_outputs(x_hat, ly["logp"], logp_z, y, y_in, z, z_in, p_z, ly["p"], ly["partials"], parts_z,
+                                   *mixture_params(ly, K, lean), K=K, training=training)
 
     def compress(self, x: torch.Tensor) -> dict:
         """x [B, 3, H, W] (H, W multiples of 64) -> {"strings": [y_strings, z_strings], "shape": (hz, wz)}: one bytes object per
@@ -305,10 +335,7 @@ class HierarchicalMixtureResidual(nn.Module):
 
     def __init__(self, latent_channels: int = 192, K: int = 1, *, precision: Optional[str] = None):
         super().__init__()
-        if not isinstance(latent_channels, int) or latent_channels < 1:
-            raise ValueError(f"latent_channels must be int >= 1, got {latent_channels}")
-        if not isinstance(K, int) or K < 1:
-            raise ValueError(f"K must be int >= 1, got {K}")
+        check_channels(latent_channels, K)
         from .Components import Decoder3x3, Encoder3x3, HyperDecoder3x3, HyperEncoder3x3
         self.M = latent_channels
         self.K = K
@@ -330,12 +357,8 @@ class HierarchicalMixtureResidual(nn.Module):
 
     def forward(self, x: torch.Tensor, training: bool = True, *, noise: Optional[Tuple[torch.Tensor, torch.Tensor]] = None,
                 lean: bool = False):
-        engine.require_cuda(x, "x")
-        if x.dim() != 4 or x.shape[1] != 3:
-            raise ValueError(f"expected x of shape [B, 3, H, W], got {tuple(x.shape)}")
+        check_input(x)
         B, _, H, W = x.shape
-        if H % 64 or W % 64:
-            raise ValueError(f"H and W must be multiples of 64; got {H}x{W}")
         from . import training as T
         if training and torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
             # the training step: ONE autograd node over the hand-written backward (training.Tape walks the residual graphs)
@@ -344,10 +367,7 @@ class HierarchicalMixtureResidual(nn.Module):
         hy, wy, hz, wz = H // 16, W // 16, H // 64, W // 64
         x = x.contiguous().float()
         with torch.cuda.device(x.device), torch.no_grad():
-            noise_z = noise_y = None
-            if training:
-                noise_z, noise_y = noise if noise is not None else (torch.rand((B, M, hz, wz), device=x.device) - 0.5,
-                                                                    torch.rand((B, M, hy, wy), device=x.device) - 0.5)
+            noise_z, noise_y = draw_noise(M, x, noise) if training else (None, None)
             qmode = Q_NOISE if training else Q_ROUND
             y_nhwc, _, _ = self.encoder.run_nhwc(x, B, H, W, arm, in_layout=LAYOUT_NCHW)
             y, y_in, y_in_nhwc, _ = engine.latent_handoff(y_nhwc, qmode, noise_y, torch.float32)
@@ -369,15 +389,8 @@ class HierarchicalMixtureResidual(nn.Module):
             _, p_z, logp_z, parts_z = self.factorized_entropy_model.likelihood(z_in, Q_PASSTHRU)
             x_nhwc, _, _ = self.decoder.run_nhwc(y_in_nhwc, B, hy, wy, arm)
             x_hat = x_nhwc.permute(0, 3, 1, 2).contiguous()
-        p_y, logp_y = ly["p"], ly["logp"]
-        engine.attach_partials(logp_y, ly["partials"])
-        engine.attach_partials(logp_z, parts_z)
-        out = {"x_hat": x_hat, "y": y, "y_in": y_in, "z": z, "z_in": z_in, "p_z": p_z, "logp_z": logp_z, "p_y": p_y, "logp_y": logp_y,
-               "training": training}
-        if not lean:
-            out.update({"mu": ly["mu"], "sigma": ly["sigma"]} if K == 1 else
-                       {"weights": ly["weights"], "mus": ly["mus"], "sigmas": ly["sigmas"]})
-        return out
+        return single_head_outputs(x_hat, ly["logp"], logp_z, y, y_in, z, z_in, p_z, ly["p"], ly["partials"], parts_z,
+                                   *mixture_params(ly, K, lean), K=K, training=training)
 
 
 class ScalableImageCoding(nn.Module):
@@ -400,10 +413,7 @@ class ScalableImageCoding(nn.Module):
 
     def __init__(self, latent_channels: int = 192, base_channels: int = 128, K: int = 1, *, precision: Optional[str] = None):
         super().__init__()
-        if not isinstance(latent_channels, int) or latent_channels < 1:
-            raise ValueError(f"latent_channels must be int >= 1, got {latent_channels}")
-        if not isinstance(K, int) or K < 1:
-            raise ValueError(f"K must be int >= 1, got {K}")
+        check_channels(latent_channels, K)
         if not isinstance(base_channels, int) or not 0 < base_channels < latent_channels:
             raise ValueError(f"base_channels must be an int in (0, latent_channels), got {base_channels}")
         self.M, self.M1, self.M2 = latent_channels, base_channels, latent_channels - base_channels
@@ -442,19 +452,20 @@ class ScalableImageCoding(nn.Module):
         x = x.contiguous().float()
         hy, wy, hz, wz = H // 16, W // 16, H // 64, W // 64
         with torch.cuda.device(x.device), torch.no_grad():
-            noise_z, noise_y = _pair_noise(self, x, training, noise)
-            y, y_in, y_in_nhwc, y_src = _pair_g_a(self, x, training, noise_y, prec, prec)
+            noise_z, noise_y = draw_noise(M, x, noise) if training else (None, None)
+            y, y_in, y_in_nhwc, y_src = fused_g_a(self, x, training, noise_y, prec, prec)
             branch, main_stream = _branch_stream(x.device), torch.cuda.current_stream(x.device)
             if branch is not None:                                        # g_s as a parallel branch of a captured graph
                 branch.wait_stream(main_stream)
                 with torch.cuda.stream(branch):
-                    x_hat = _pair_g_s(self, y_in_nhwc, B, hy, wy, prec)
-            z, z_in, z_in_nhwc = _pair_h_a(self, y_src, B, hy, wy, training, noise_z, prec, prec)
+                    x_hat = fused_g_s(self, y_in_nhwc, B, hy, wy, prec)
+            z, z_in, z_in_nhwc = fused_h_a(self, y_src, B, hy, wy, training, noise_z, prec, prec)
             y_flag = getattr(y_in_nhwc, "_nic_lo_flag", None)
             c1, c2 = 2 * M1 + 2 * M, 2 * M2 + 2 * M                       # [phi_i (2 M_i) | psi (2 M)] channels of the two heads
             comb1 = torch.empty((B, hy, wy, 2 * c1), dtype=torch.bfloat16, device=x.device)      # pair tensors: [hi(c) | lo(c)]
             comb2 = torch.empty((B, hy, wy, 2 * c2), dtype=torch.bfloat16, device=x.device)
-            _pair_h_s_into(self, z_in_nhwc, B, hz, wz, prec, comb1, c1, 2 * M1)                  # psi once, into head 1's buffer
+            fused_h_s_into(self, z_in_nhwc, B, hz, wz, prec, comb1, c1, 2 * M1,                  # psi once, into head 1's buffer
+                           getattr(z_in_nhwc, "_nic_lo_flag", None))
             comb2[..., 2 * M2:c2] = comb1[..., 2 * M1:c1]                                        # ... head 2 gets a copy: hi half,
             comb2[..., c2 + 2 * M2:] = comb1[..., c1 + 2 * M1:]                                  # lo half
             y1, y2 = torch.split(y_in, [M1, M2], dim=1)                   # Models.py:279 (views, as in the reference)
@@ -473,30 +484,15 @@ class ScalableImageCoding(nn.Module):
             if branch is not None:
                 main_stream.wait_stream(branch)
             else:
-                x_hat = _pair_g_s(self, y_in_nhwc, B, hy, wy, prec)
+                x_hat = fused_g_s(self, y_in_nhwc, B, hy, wy, prec)
         l1, l2 = heads
-        engine.attach_partials(l1["logp"], l1["partials"])
-        engine.attach_partials(l2["logp"], l2["partials"])
-        engine.attach_partials(logp_z, parts_z)
-        out = {
-            "x_hat": x_hat, "y": y, "y_in": y_in, "y1": y1, "y2": y2, "z": z, "z_in": z_in, "p_z": p_z, "logp_z": logp_z,
-            "p_y1": l1["p"], "logp_y1": l1["logp"], "p_y2": l2["p"], "logp_y2": l2["logp"], "training": training,
-        }
-        if K == 1:
-            out.update({"mu1": l1["mu"], "sigma1": l1["sigma"], "mu2": l2["mu"], "sigma2": l2["sigma"]})
-        else:
-            out.update({"weights1": l1["weights"], "mus1": l1["mus"], "sigmas1": l1["sigmas"],
-                        "weights2": l2["weights"], "mus2": l2["mus"], "sigmas2": l2["sigmas"]})
-        return out
+        return two_head_outputs(x_hat, l1["logp"], l2["logp"], logp_z, y, y_in, z, z_in, p_z, l1["p"], l2["p"], l1["partials"],
+                                l2["partials"], parts_z, *mixture_params(l1, K), *mixture_params(l2, K), M1=M1, K=K, training=training)
 
     def forward(self, x: torch.Tensor, training: bool = True, debug=False, *,
                 noise: Optional[Tuple[torch.Tensor, torch.Tensor]] = None):
-        engine.require_cuda(x, "x")
-        if x.dim() != 4 or x.shape[1] != 3:
-            raise ValueError(f"expected x of shape [B, 3, H, W], got {tuple(x.shape)}")
+        check_input(x)
         B, _, H, W = x.shape
-        if H % 64 or W % 64:
-            raise ValueError(f"H and W must be multiples of 64; got {H}x{W}")
         if training and torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
             # the training call with autograd on: one autograd node over the layer-by-layer forward (training_scalable.py)
             from . import training_scalable as _ts
@@ -520,10 +516,7 @@ class ScalableImageCoding(nn.Module):
         x = x.contiguous().float()
         hy, wy, hz, wz = H // 16, W // 16, H // 64, W // 64
         with torch.cuda.device(x.device), torch.no_grad():
-            noise_z = noise_y = None
-            if training:
-                noise_z, noise_y = noise if noise is not None else (torch.rand((B, M, hz, wz), device=x.device) - 0.5,
-                                                                    torch.rand((B, M, hy, wy), device=x.device) - 0.5)
+            noise_z, noise_y = draw_noise(M, x, noise) if training else (None, None)
             qmode = Q_NOISE if training else Q_ROUND
             a, h, w, layout = x, H, W, LAYOUT_NCHW
             for op in self.encoder.ops:
@@ -571,16 +564,5 @@ class ScalableImageCoding(nn.Module):
                 h, w = engine.conv_out_hw(op.conv, h, w)
             x_hat = a
         l1, l2 = heads
-        engine.attach_partials(l1["logp"], l1["partials"])
-        engine.attach_partials(l2["logp"], l2["partials"])
-        engine.attach_partials(logp_z, parts_z)
-        out = {
-            "x_hat": x_hat, "y": y, "y_in": y_in, "y1": y1, "y2": y2, "z": z, "z_in": z_in, "p_z": p_z, "logp_z": logp_z,
-            "p_y1": l1["p"], "logp_y1": l1["logp"], "p_y2": l2["p"], "logp_y2": l2["logp"], "training": training,
-        }
-        if K == 1:
-            out.update({"mu1": l1["mu"], "sigma1": l1["sigma"], "mu2": l2["mu"], "sigma2": l2["sigma"]})
-        else:
-            out.update({"weights1": l1["weights"], "mus1": l1["mus"], "sigmas1": l1["sigmas"],
-                        "weights2": l2["weights"], "mus2": l2["mus"], "sigmas2": l2["sigmas"]})
-        return out
+        return two_head_outputs(x_hat, l1["logp"], l2["logp"], logp_z, y, y_in, z, z_in, p_z, l1["p"], l2["p"], l1["partials"],
+                                l2["partials"], parts_z, *mixture_params(l1, K), *mixture_params(l2, K), M1=M1, K=K, training=training)

@@ -17,6 +17,7 @@ import torch
 from . import _lib, engine
 from ._lib import (CODEC_FACTORIZED, CODEC_GM, CODEC_SYMBOL, CODEC_TABLES, CODEC_WINDOW, Q_PASSTHRU, check, current_stream,
                    ptr)
+from .Models import check_input, fused_g_a, fused_g_s, fused_h_a, fused_h_s_into, precision_arms
 
 FORMAT_VERSION = 1
 ARMS = ("fp32", "bf16", "mixed", "bf16x3")          # header byte 1
@@ -87,13 +88,6 @@ def parse_string(data: bytes, n_lanes: int, with_header: bool):
 
 # ---- the shared parameter path ---------------------------------------------------------------------------------------
 
-def _arms(model):
-    prec_up = {"fp32": "fp32", "mixed": "fp32", "bf16x3": "bf16x3", "bf16": "bf16"}[model.precision]   # g_a, h_a
-    prec = {"fp32": "fp32", "mixed": "bf16", "bf16x3": "bf16x3", "bf16": "bf16"}[model.precision]      # the rest
-    hdt = "bf16x2" if prec == "bf16x3" else engine.act_dtype(prec)   # engine-layout copies of the symbols (as the forward's)
-    return prec_up, prec, hdt
-
-
 def check_supported(model):
     if model.precision != "fp32" and model.M not in (128, 192):
         raise ValueError(f"compress/decompress: precision={model.precision!r} is built for latent_channels 128 and 192 "
@@ -109,7 +103,8 @@ class ParamPath:
 
     def __init__(self, model, B: int, hy: int, wy: int, device):
         self.model, self.B, self.hy, self.wy, self.device = model, B, hy, wy, device
-        _, self.prec, self.hdt = _arms(model)
+        _, self.prec = precision_arms(model.precision)
+        self.hdt = "bf16x2" if self.prec == "bf16x3" else engine.act_dtype(self.prec)     # engine-layout symbols, as the forward's
         M, K = model.M, model.K
         model.context_model.masked.apply_mask_()
         self.plan = engine.CtxEpPlan(model.context_model.masked._op, model.entropy_parameters.ops, B, hy, wy, self.prec, M, K, device,
@@ -120,16 +115,9 @@ class ParamPath:
         M, B, prec = self.model.M, self.B, self.prec
         hz, wz = z_nhwc.shape[1:3]
         _, z_hat, z_eng, _ = engine.latent_handoff(z_nhwc, Q_PASSTHRU, None, self.hdt)
-        adt = engine.act_dtype(prec)
-        combined = torch.empty((B, self.hy, self.wy, (2 if prec == "bf16x3" else 1) * 4 * M), dtype=adt, device=self.device)
-        hs = self.model.hyper_decoder.ops
-        a, h, w = z_eng, hz, wz
-        for i, op in enumerate(hs):
-            if i == len(hs) - 1:
-                op.run(a, B, h, w, prec, out=combined, out_c_total=4 * M, out_c_offset=2 * M)
-            else:
-                a = op.run(a, B, h, w, prec)
-            h, w = engine.conv_out_hw(op.conv, h, w)
+        combined = torch.empty((B, self.hy, self.wy, (2 if prec == "bf16x3" else 1) * 4 * M), dtype=engine.act_dtype(prec),
+                               device=self.device)
+        fused_h_s_into(self.model, z_eng, B, hz, wz, prec, combined, 4 * M, 2 * M, None)          # no lo-half hint (module docstring)
         return z_hat, combined
 
     def raw(self, y_nhwc: torch.Tensor, combined: torch.Tensor) -> torch.Tensor:
@@ -201,22 +189,17 @@ def checksums(y: torch.Tensor, z: torch.Tensor) -> torch.Tensor:
 # ---- compress / decompress -------------------------------------------------------------------------------------------
 
 def compress(model, x: torch.Tensor) -> dict:
-    engine.require_cuda(x, "x")
-    if x.dim() != 4 or x.shape[1] != 3:
-        raise ValueError(f"expected x of shape [B, 3, H, W], got {tuple(x.shape)}")
+    check_input(x)
     B, _, H, W = x.shape
-    if H % 64 or W % 64:
-        raise ValueError(f"H and W must be multiples of 64 (four stride-2 stages in g_a, two in h_a); got {H}x{W}")
     check_supported(model)
-    from .Models import _pair_g_a, _pair_h_a
     M, K = model.M, model.K
-    prec_up, prec, _ = _arms(model)
+    prec_up, prec = precision_arms(model.precision)
     hy, wy, hz, wz = H // 16, W // 16, H // 64, W // 64
     ly, lz = lanes(Y_LANES, M), lanes(Z_LANES, M)
     with torch.cuda.device(x.device), torch.no_grad():
         x = x.contiguous().float()
-        _, y_in, _, y_src = _pair_g_a(model, x, False, None, prec_up, prec)
-        _, z_in, _ = _pair_h_a(model, y_src, B, hy, wy, False, None, prec_up, prec)
+        _, y_in, _, y_src = fused_g_a(model, x, False, None, prec_up, prec)
+        _, z_in, _ = fused_h_a(model, y_src, B, hy, wy, False, None, prec_up, prec)
         big = torch.maximum(y_in.abs().amax(), z_in.abs().amax())
         if not bool(big < SYMBOL_LIMIT):
             raise ValueError(f"a latent symbol has magnitude {float(big)} >= 2^20: the stream format cannot carry it")
@@ -278,7 +261,6 @@ def decompress(model, strings, shape) -> dict:
     hz, wz = int(shape[0]), int(shape[1])
     hy, wy = 4 * hz, 4 * wz
     ly, lz = lanes(Y_LANES, M), lanes(Z_LANES, M)
-    _, prec, hdt = _arms(model)
     dev = w0.device
     # one blob: z strings, then y strings; lane tables as absolute byte offsets into it
     blob = b"".join(z_strings) + b"".join(y_strings)
@@ -311,9 +293,8 @@ def decompress(model, strings, shape) -> dict:
             check(lib.nic_codec_decode(CODEC_GM, ptr(blob_d), ptr(y_off_d), ptr(y_nw_d), ptr(ys_state), ptr(ys_pos), int(t == 0),
                                        ptr(tabs[0]), ptr(tabs[1]), ptr(tabs[2]), B, M, hy, wy, ly, t, ptr(y_nhwc), st), "nic_codec_decode")
         # g_s reads the symbols through the same hand-off as the forward's (same engine copy, same lo-half flag)
-        _, y_hat, y_eng, _ = engine.latent_handoff(y_nhwc, Q_PASSTHRU, None, hdt)
-        from .Models import _pair_g_s
-        x_hat = _pair_g_s(model, y_eng, B, hy, wy, prec)
+        _, y_hat, y_eng, _ = engine.latent_handoff(y_nhwc, Q_PASSTHRU, None, path.hdt)
+        x_hat = fused_g_s(model, y_eng, B, hy, wy, path.prec)
         bad = (checksums(y_hat, z_hat) != want).cpu().numpy()
     if bad.any():
         raise ValueError(f"checksum mismatch in image(s) {np.flatnonzero(bad).tolist()}: the strings are corrupted or were written "

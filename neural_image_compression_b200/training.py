@@ -3,8 +3,10 @@ on the sm_100a kernels.
 
 The reference has no backward code of its own: its gradients are what torch autograd derives from Models.py:49-106 and
 RateDistortionLoss.py:5-49.  Here the whole model is ONE autograd node (``_TrainForward``): its forward (``_forward_impl``) runs
-layer by layer with fp32 NHWC tensors in between and keeps the layer inputs, its backward (``_backward_impl``) is a hand-scheduled
-chain of C-ABI calls (include/nic.h, "training step" section):
+layer by layer with fp32 NHWC tensors in between, every transform (g_a, g_s, h_a, h_s; the 5x5 chains and the 3x3 residual
+graphs alike) recording its ops and their tensors on a ``Tape``; its backward (``_backward_impl``) walks each transform's tape in
+reverse (``Tape.backward``) around the hand-written entropy side, a hand-scheduled chain of C-ABI calls (include/nic.h,
+"training step" section):
 
     data gradient of a conv      nic_conv_fwd with the mirrored descriptor (Conv2d <-> ConvTranspose2d, same weight tensor)
     weight / bias gradients      nic_conv_wgrad_tc (tcgen05, MN-major operands) / nic_conv_wgrad (fp32) - all 25 taps of the masked
@@ -42,6 +44,7 @@ import torch.nn as nn
 
 from . import _lib, engine
 from ._lib import (ConvDesc, DT_F32, EPI_BIAS, EPI_LRELU, LAYOUT_NCHW, LAYOUT_NHWC, PREC_FP32, Q_NOISE, Q_PASSTHRU, Q_ROUND, check, current_stream, ptr)
+from .Models import draw_noise, mixture_params, single_head_outputs
 
 PREC = "fp32"
 WGRAD_TC = os.environ.get("NIC_WGRAD_TC", "1") != "0"      # tensor-core weight gradients in the bf16x3 arm (0: fp32 kernel everywhere)
@@ -403,11 +406,11 @@ def add_(dst: torch.Tensor, src: torch.Tensor) -> torch.Tensor:
 
 
 class Tape:
-    """Record of a transform whose graph is not a plain chain (the 3x3 residual family, Layers.py / Components.py:20-122): every
-    conv (+ bias / LeakyReLU), GDN / IGDN and residual sum of the forward is appended with its input and output tensors;
-    `backward` walks the record in reverse, keeps one gradient per tensor (summed where a tensor feeds two consumers: the block
-    input of a residual block) and returns the gradient of the transform's input.  Kernels: the same C-ABI calls as the 5x5
-    chains (conv_wgrad, conv_dgrad, gdn_bwd, nic_lrelu_bwd, nic_add_inplace)."""
+    """Record of one transform's training forward (the 5x5 chains and the 3x3 residual graphs alike, `run_nhwc(..., tape=)`):
+    every conv (+ bias / LeakyReLU), GDN / IGDN and residual sum is appended with its input and output tensors; `backward` walks
+    the record in reverse, keeps one gradient per tensor (summed where a tensor feeds two consumers: the block input of a residual
+    block) and returns the gradient of the transform's input.  Kernels: conv_wgrad, conv_dgrad, gdn_bwd, nic_lrelu_bwd,
+    nic_add_inplace."""
 
     def __init__(self, arm: str, n: int):
         self.arm, self.n, self.recs = arm, n, []
@@ -434,7 +437,7 @@ class Tape:
     def backward(self, g_out, g_layout, put, wgrad, root=None, side=None, keep=None):
         """g_out: gradient of `output` (in g_layout).  root: the transform's input tensor; its gradient is returned (None when
         root is None: the image needs none).  put(param, grad) collects parameter gradients, wgrad = conv_wgrad or its
-        side-stream form."""
+        side-stream form; keep holds what the side stream reads until the caller's join."""
         n, arm = self.n, self.arm
         grads = {id(self.output): (g_out, g_layout)}
         internal = {id(r[-1]) for r in self.recs}
@@ -449,35 +452,29 @@ class Tape:
                 grads[id(t)] = (g, LAYOUT_NHWC)
 
         for rec in reversed(self.recs):
-            got = grads.pop(id(rec[-1]), None)
-            if got is None:
+            if id(rec[-1]) not in grads:
                 continue
-            g, gl = got
+            g, gl = grads.pop(id(rec[-1]))                  # popped: freed as soon as this op's backward has consumed it
             if rec[0] == "conv":
                 _, conv, epi, x, h, w, in_layout, out_layout, y = rec
                 if epi == EPI_LRELU:
                     g = lrelu_bwd_(g, y)
                 dw, db = wgrad(conv, x, g, n, h, w, in_layout, gl, arm=arm)
                 put(conv.weight, dw); put(conv.bias, db)
-                if keep is not None:
+                if keep is not None and side is not None:
                     keep.append(g)
                 if id(x) in internal or (root is not None and x is root):
                     give(x, conv_dgrad(conv, g, n, h, w, gl, arm=arm))
             elif rec[0] == "gdn":
                 _, gdn, u, nrm, h, w, y = rec
-                du, dbeta, dgamma = gdn_bwd(gdn, u, g, n, h, w, norm=nrm, side=side, keep=keep)
+                g, dbeta, dgamma = gdn_bwd(gdn, u, g, n, h, w, norm=nrm, side=side, keep=keep)
                 put(gdn.beta, dbeta); put(gdn.gamma, dgamma)
-                give(u, du)
+                give(u, g)
             else:
                 _, a, b, y = rec
                 give(a, g)
                 give(b, g.clone())                                  # the two consumers may modify their gradient in place
         return grads.pop(id(root), (None, None))[0] if root is not None else None
-
-
-def _is_chain(transform) -> bool:
-    """5x5 transforms expose `.ops` (a plain chain of conv [+ GDN]); the 3x3 residual family records a Tape."""
-    return hasattr(transform, "ops")
 
 
 _FACT_SLICES = (("matrices", 0, 0, 3), ("biases", 0, 3, 6), ("factors", 0, 6, 9), ("matrices", 1, 9, 18), ("biases", 1, 18, 21),
@@ -492,53 +489,18 @@ def _forward_impl(model, x, noise_z, noise_y, lean, qmode: int = Q_NOISE, arm: O
     qmode = Q_NOISE is the training forward; Q_ROUND the evaluation forward of a model whose channel count the fused
     pair-tensor pipeline is not built for (Models.py uses it for M != 128 on the bf16x3 arm)."""
     engine.require_cuda(x, "x")
-    lib = _lib.load()
     dev = x.device
     B, _, H, W = x.shape
     M, K = model.M, model.K
     hy, wy, hz, wz = H // 16, W // 16, H // 64, W // 64
-    S = {}
     arm = arm or train_precision(model)
+    S = {t: Tape(arm, B) for t in ("g_a", "g_s", "h_a", "h_s")}       # each transform's ops with the tensors its backward reads
     with torch.cuda.device(dev):
-        # g_a: conv (+ bias) -> u, kept for the GDN backward; GDN -> the next layer's input, kept for its weight gradient
-        a, h, w, layout = x, H, W, LAYOUT_NCHW
-        enc = model.encoder.ops if _is_chain(model.encoder) else ()
-        S["enc_in"], S["enc_u"] = [], []
-        if not _is_chain(model.encoder):
-            S["enc_tape"] = Tape(arm, B)
-            a, h, w = model.encoder.run_nhwc(x, B, H, W, arm, in_layout=LAYOUT_NCHW, tape=S["enc_tape"])
-        for op in enc:
-            S["enc_in"].append((a, h, w, layout))
-            a = conv_forward(arm, op.conv, EPI_BIAS, a, B, h, w, in_layout=layout)
-            h, w = engine.conv_out_hw(op.conv, h, w)
-            if op.gdn is not None:
-                u = a
-                a, nrm = gdn_forward(arm, op.gdn, u, B, h, w)
-                S["enc_u"].append((u, nrm))
-            else:
-                S["enc_u"].append(None)
-            layout = LAYOUT_NHWC
-        y_nhwc = a
+        y_nhwc, _, _ = model.encoder.run_nhwc(x, B, H, W, arm, in_layout=LAYOUT_NCHW, tape=S["g_a"])
         y, y_in, y_in_nhwc, _ = engine.latent_handoff(y_nhwc, qmode, noise_y, torch.float32)
+
         def synthesis():
-            a, h, w = y_in_nhwc, hy, wy
-            if not _is_chain(model.decoder):
-                S["dec_tape"] = Tape(arm, B)
-                return model.decoder.run_nhwc(a, B, h, w, arm, tape=S["dec_tape"])[0]        # the RGB layer writes NCHW
-            dec = model.decoder.ops
-            S["dec_in"], S["dec_u"] = [], []
-            for i, op in enumerate(dec):
-                last = i == len(dec) - 1
-                S["dec_in"].append((a, h, w))
-                a = conv_forward(arm, op.conv, EPI_BIAS, a, B, h, w, out_layout=LAYOUT_NCHW if last else LAYOUT_NHWC)
-                h, w = engine.conv_out_hw(op.conv, h, w)
-                if op.gdn is not None:
-                    u = a
-                    a, nrm = gdn_forward(arm, op.gdn, u, B, h, w)
-                    S["dec_u"].append((u, nrm))
-                else:
-                    S["dec_u"].append(None)
-            return a
+            return model.decoder.run_nhwc(y_in_nhwc, B, hy, wy, arm, tape=S["g_s"])[0]        # the RGB layer writes NCHW
         # g_s reads only y_in: it runs as its own branch (a second stream; a parallel branch of a captured graph) beside the
         # entropy path h_a -> h_s -> context -> entropy parameters -> likelihoods
         main = torch.cuda.current_stream(dev)
@@ -550,31 +512,12 @@ def _forward_impl(model, x, noise_z, noise_y, lean, qmode: int = Q_NOISE, arm: O
             with torch.cuda.stream(branch):
                 x_hat = synthesis()
         # h_a (reads the unquantised y)
-        a, h, w = y_nhwc, hy, wy
-        S["ha_in"] = []
-        if not _is_chain(model.hyper_encoder):
-            S["ha_tape"] = Tape(arm, B)
-            a, h, w = model.hyper_encoder.run_nhwc(a, B, h, w, arm, tape=S["ha_tape"])
-        for op in (model.hyper_encoder.ops if _is_chain(model.hyper_encoder) else ()):
-            S["ha_in"].append((a, h, w))
-            a = conv_forward(arm, op.conv, op.epilogue, a, B, h, w)
-            h, w = engine.conv_out_hw(op.conv, h, w)
-        z, z_in, z_in_nhwc, _ = engine.latent_handoff(a, qmode, noise_z, torch.float32)
+        z_nhwc, _, _ = model.hyper_encoder.run_nhwc(y_nhwc, B, hy, wy, arm, tape=S["h_a"])
+        z, z_in, z_in_nhwc, _ = engine.latent_handoff(z_nhwc, qmode, noise_z, torch.float32)
         # h_s -> psi, context -> phi, both windows of `combined`
         combined = _f32((B, hy, wy, 4 * M), dev)
-        a, h, w = z_in_nhwc, hz, wz
-        hs = model.hyper_decoder.ops if _is_chain(model.hyper_decoder) else ()
-        S["hs_in"] = []
-        if not _is_chain(model.hyper_decoder):
-            S["hs_tape"] = Tape(arm, B)
-            model.hyper_decoder.run_nhwc(a, B, h, w, arm, tape=S["hs_tape"], final_kw=dict(out=combined, out_c_total=4 * M, out_c_offset=2 * M))
-        for i, op in enumerate(hs):
-            S["hs_in"].append((a, h, w))
-            if i == len(hs) - 1:
-                conv_forward(arm, op.conv, op.epilogue, a, B, h, w, out=combined, out_c_total=4 * M, out_c_offset=2 * M)
-            else:
-                a = conv_forward(arm, op.conv, op.epilogue, a, B, h, w)
-            h, w = engine.conv_out_hw(op.conv, h, w)
+        model.hyper_decoder.run_nhwc(z_in_nhwc, B, hz, wz, arm, tape=S["h_s"],
+                                     final_kw=dict(out=combined, out_c_total=4 * M, out_c_offset=2 * M))
         masked = model.context_model.masked
         masked.apply_mask_()
         conv_forward(arm, masked, EPI_BIAS, y_in_nhwc, B, hy, wy, out=combined, out_c_total=4 * M, out_c_offset=0, mask_a=True)
@@ -592,10 +535,8 @@ def _forward_impl(model, x, noise_z, noise_y, lean, qmode: int = Q_NOISE, arm: O
     S["arm"] = arm
     S.update(combined=combined, e1=e1, e2=e2, raw=raw, y_in=y_in, y_in_nhwc=y_in_nhwc, z_in=z_in, z_in_nhwc=z_in_nhwc, y_nhwc=y_nhwc,
              fparams=model.factorized_entropy_model.packed(), shape=(B, H, W))
-    logp_y = ly["logp"]
-    extra = [] if lean else ([ly["mu"], ly["sigma"]] if K == 1 else [ly["weights"], ly["mus"], ly["sigmas"]])
-    nd = [y, y_in, z, z_in, p_z, ly["p"], ly["partials"], parts_z] + extra
-    return (x_hat, logp_y, logp_z, *nd), S
+    nd = [y, y_in, z, z_in, p_z, ly["p"], ly["partials"], parts_z] + mixture_params(ly, K, lean)
+    return (x_hat, ly["logp"], logp_z, *nd), S
 
 
 def _backward_impl(model, S, g_xhat, g_logp_y, g_logp_z, partial_hook=None) -> Dict[int, torch.Tensor]:
@@ -640,23 +581,8 @@ def _backward_impl(model, S, g_xhat, g_logp_y, g_logp_z, partial_hook=None) -> D
             if branch is not None:
                 branch.wait_stream(main)
             with (torch.cuda.stream(branch) if branch is not None else contextlib.nullcontext()):
-                g, g_layout = g_xhat.contiguous().float(), LAYOUT_NCHW
-                dec = model.decoder.ops if _is_chain(model.decoder) else ()
-                if not _is_chain(model.decoder):
-                    g = S["dec_tape"].backward(g, g_layout, put, conv_wgrad_async, root=S["y_in_nhwc"], side=side, keep=keep)
-                for i in range(len(dec) - 1, -1, -1):
-                    op = dec[i]
-                    a, h, w = S["dec_in"][i]
-                    ho, wo = engine.conv_out_hw(op.conv, h, w)
-                    if op.gdn is not None:
-                        g, dbeta, dgamma = gdn_bwd(op.gdn, S["dec_u"][i][0], g, B, ho, wo, norm=S["dec_u"][i][1], side=side, keep=keep)
-                        put(op.gdn.beta, dbeta); put(op.gdn.gamma, dgamma)
-                    dw, db = conv_wgrad_async(op.conv, a, g, B, h, w, LAYOUT_NHWC, g_layout, arm=arm)
-                    put(op.conv.weight, dw); put(op.conv.bias, db)
-                    keep.append(g)
-                    g = conv_dgrad(op.conv, g, B, h, w, g_layout, arm=arm)
-                    g_layout = LAYOUT_NHWC
-                d_yin_gs = g
+                d_yin_gs = S["g_s"].backward(g_xhat.contiguous().float(), LAYOUT_NCHW, put, conv_wgrad_async, root=S["y_in_nhwc"],
+                                             side=side, keep=keep)
         # ---- p_y: likelihood, entropy parameters, context model, h_s --------------------------------------------
         d_zin = None
         if g_logp_y is not None:
@@ -680,19 +606,8 @@ def _backward_impl(model, S, g_xhat, g_logp_y, g_logp_z, partial_hook=None) -> D
             dw, db = conv_wgrad_async(masked, S["y_in_nhwc"], d_phi, B, hy, wy, LAYOUT_NHWC, LAYOUT_NHWC, arm=arm)
             put(masked.weight, dw); put(masked.bias, db)
             d_yin = add_(d_yin, conv_dgrad(masked, d_phi, B, hy, wy, arm=arm))
-            g = d_psi
-            hs = model.hyper_decoder.ops if _is_chain(model.hyper_decoder) else ()
-            if not _is_chain(model.hyper_decoder):
-                g = S["hs_tape"].backward(g, LAYOUT_NHWC, put, conv_wgrad_async, root=S["z_in_nhwc"], side=side, keep=keep)
-            for i in range(len(hs) - 1, -1, -1):
-                op = hs[i]
-                a, h, w = S["hs_in"][i]
-                dw, db = conv_wgrad_async(op.conv, a, g, B, h, w, LAYOUT_NHWC, LAYOUT_NHWC, arm=arm)
-                put(op.conv.weight, dw); put(op.conv.bias, db)
-                g = conv_dgrad(op.conv, g, B, h, w, arm=arm)
-                if i > 0:
-                    g = lrelu_bwd_(g, a)                         # a = LeakyReLU output of layer i - 1
-            d_zin = g
+            del g                                                # the concat buffer's gradient is consumed: free it before h_s's backward
+            d_zin = S["h_s"].backward(d_psi, LAYOUT_NHWC, put, conv_wgrad_async, root=S["z_in_nhwc"], side=side, keep=keep)
         # ---- p_z ----------------------------------------------------------------------------------------------------
         if g_logp_z is not None:
             gl = g_logp_z.contiguous().float()
@@ -708,19 +623,9 @@ def _backward_impl(model, S, g_xhat, g_logp_y, g_logp_z, partial_hook=None) -> D
         # ---- h_a (z_in = z + noise: the gradient passes unchanged) --------------------------------------------------
         dy = d_yin
         if d_zin is not None:
-            g = d_zin
-            ha = model.hyper_encoder.ops if _is_chain(model.hyper_encoder) else ()
-            if not _is_chain(model.hyper_encoder):
-                g = S["ha_tape"].backward(g, LAYOUT_NHWC, put, conv_wgrad_async, root=S["y_nhwc"], side=side, keep=keep)
-            for i in range(len(ha) - 1, -1, -1):
-                op = ha[i]
-                a, h, w = S["ha_in"][i]
-                dw, db = conv_wgrad_async(op.conv, a, g, B, h, w, LAYOUT_NHWC, LAYOUT_NHWC, arm=arm)
-                put(op.conv.weight, dw); put(op.conv.bias, db)
-                g = conv_dgrad(op.conv, g, B, h, w, arm=arm)
-                if i > 0:
-                    g = lrelu_bwd_(g, a)
+            g = S["h_a"].backward(d_zin, LAYOUT_NHWC, put, conv_wgrad_async, root=S["y_nhwc"], side=side, keep=keep)
             dy = g if dy is None else add_(dy, g)
+            del g                                                # summed into dy: free it before g_a's backward
         # ---- merge the branches: dy = d(entropy path) + d(h_a) + d(g_s) ---------------------------------------------------------
         if branch is not None:
             main.wait_stream(branch)
@@ -730,21 +635,7 @@ def _backward_impl(model, S, g_xhat, g_logp_y, g_logp_z, partial_hook=None) -> D
             partial_hook(grads, [st for st in (main, side) if st is not None])
         # ---- g_a (y_in = y + noise) ---------------------------------------------------------------------------------
         if dy is not None:
-            g = dy
-            enc = model.encoder.ops if _is_chain(model.encoder) else ()
-            if not _is_chain(model.encoder):
-                S["enc_tape"].backward(g, LAYOUT_NHWC, put, conv_wgrad_async, root=None, side=side, keep=keep)
-            for i in range(len(enc) - 1, -1, -1):
-                op = enc[i]
-                a, h, w, layout = S["enc_in"][i]
-                ho, wo = engine.conv_out_hw(op.conv, h, w)
-                if op.gdn is not None:
-                    g, dbeta, dgamma = gdn_bwd(op.gdn, S["enc_u"][i][0], g, B, ho, wo, norm=S["enc_u"][i][1], side=side, keep=keep)
-                    put(op.gdn.beta, dbeta); put(op.gdn.gamma, dgamma)
-                dw, db = conv_wgrad_async(op.conv, a, g, B, h, w, layout, LAYOUT_NHWC, arm=arm)
-                put(op.conv.weight, dw); put(op.conv.bias, db)
-                if i > 0:
-                    g = conv_dgrad(op.conv, g, B, h, w, arm=arm)
+            S["g_a"].backward(dy, LAYOUT_NHWC, put, conv_wgrad_async, root=None, side=side, keep=keep)
     if side is not None:
         main.wait_stream(side)     # join: every weight gradient is complete before the caller (optimizer, all-reduce) reads it
     keep.clear()
@@ -781,12 +672,7 @@ def step_gradients(model, x: torch.Tensor, lambda_rd: float, noise=None, partial
     (loss [device scalar], per_image [3, B], scalars [8])."""
     from .RateDistortionLoss import rd_terms
     B, _, H, W = x.shape
-    M = model.M
-    if noise is not None:
-        noise_z, noise_y = noise
-    else:
-        noise_z = torch.rand((B, M, H // 64, W // 64), device=x.device) - 0.5
-        noise_y = torch.rand((B, M, H // 16, W // 16), device=x.device) - 0.5
+    noise_z, noise_y = draw_noise(model.M, x, noise)
     forget_pairs()
     x = x.contiguous().float()
     outs, S = _forward_impl(model, x, noise_z, noise_y, True)
@@ -810,27 +696,11 @@ def step_gradients(model, x: torch.Tensor, lambda_rd: float, noise=None, partial
 
 def train_forward(model, x: torch.Tensor, noise=None, lean: bool = False) -> dict:
     """``model(x, training=True)`` as a differentiable call (used by JointAutoregressiveHierarchical.forward when autograd is on)."""
-    B, _, H, W = x.shape
-    M, K = model.M, model.K
-    if noise is not None:
-        noise_z, noise_y = noise
-    else:                                                    # the reference draws z's noise first (Models.py:57-58)
-        noise_z = torch.rand((B, M, H // 64, W // 64), device=x.device) - 0.5
-        noise_y = torch.rand((B, M, H // 16, W // 16), device=x.device) - 0.5
+    noise_z, noise_y = draw_noise(model.M, x, noise)
     forget_pairs()
     params = [p for _, p in model.named_parameters()]
     res = _TrainForward.apply(model, x.contiguous().float(), noise_z, noise_y, lean, *params)
-    x_hat, logp_y, logp_z, y, y_in, z, z_in, p_z, p_y, parts_y, parts_z = res[:11]
-    engine.attach_partials(logp_y, parts_y)
-    engine.attach_partials(logp_z, parts_z)      # per-image sums of logp ride along for rd_loss
-    out = {"x_hat": x_hat, "y": y, "y_in": y_in, "z": z, "z_in": z_in, "p_z": p_z, "logp_z": logp_z, "p_y": p_y, "logp_y": logp_y,
-           "training": True}
-    if not lean:
-        if K == 1:
-            out["mu"], out["sigma"] = res[11:13]
-        else:
-            out["weights"], out["mus"], out["sigmas"] = res[11:14]
-    return out
+    return single_head_outputs(*res, K=model.K, training=True)
 
 
 class _RDLoss(torch.autograd.Function):

@@ -1,9 +1,10 @@
 """Training step of ``ScalableImageCoding`` (reference Models.py:208-338 with the repairs of SURVEY.md section 2.4, loss
 ``vision_rd_loss`` of RateDistortionLoss.py:52-121 with V = None): forward with noise, loss, hand-written backward.
 
-Same kernels and helpers as training.py; what differs from the single-head model is the split of y into a base part (M1 channels)
-and an enhancement part (M - M1), each with its own (context model, entropy-parameter net) over the SHARED hyper features psi:
-the psi gradient is the sum over the two heads, the y gradient of the entropy path is the channel concatenation of the heads'.
+Same kernels and helpers as training.py, the transforms recorded on and walked back by the same ``training.Tape``; what differs
+from the single-head model is the split of y into a base part (M1 channels) and an enhancement part (M - M1), each with its own
+(context model, entropy-parameter net) over the SHARED hyper features psi: the psi gradient is the sum over the two heads, the y
+gradient of the entropy path is the channel concatenation of the heads'.
 ``train_forward`` makes ``model(x)`` ONE autograd node (with ``_VisionRDLoss`` for the loss, so the reference-style
 ``vision_rd_loss(...)['loss'].backward()`` works); ``step_gradients`` runs the same forward + loss + backward on the calling thread
 without the autograd engine (what ``parallel.ShardedTrainer`` uses and captures).  Oracle: torch autograd over
@@ -20,6 +21,7 @@ import torch
 from . import _lib, engine
 from . import training as T
 from ._lib import EPI_BIAS, LAYOUT_NCHW, LAYOUT_NHWC, Q_NOISE, Q_PASSTHRU, check, current_stream, ptr
+from .Models import draw_noise, mixture_params, two_head_outputs
 
 
 def _heads(model):
@@ -35,41 +37,15 @@ def _forward_impl(model, x, noise_z, noise_y):
     hy, wy, hz, wz = H // 16, W // 16, H // 64, W // 64
     arm = T.train_precision(model)
     heads = _heads(model)
+    S = {t: T.Tape(arm, B) for t in ("g_a", "g_s", "h_a", "h_s")}
     with torch.cuda.device(dev):
-        # ---------------------------------------------------------------- forward ----------------------------------------------
-        a, h, w, layout = x, H, W, LAYOUT_NCHW
-        enc_in, enc_u = [], []
-        for op in model.encoder.ops:
-            enc_in.append((a, h, w, layout))
-            a = T.conv_forward(arm, op.conv, EPI_BIAS, a, B, h, w, in_layout=layout)
-            h, w = engine.conv_out_hw(op.conv, h, w)
-            if op.gdn is not None:
-                u = a
-                a, nrm = T.gdn_forward(arm, op.gdn, u, B, h, w)
-                enc_u.append((u, nrm))
-            else:
-                enc_u.append(None)
-            layout = LAYOUT_NHWC
-        y_nhwc = a
+        y_nhwc, _, _ = model.encoder.run_nhwc(x, B, H, W, arm, in_layout=LAYOUT_NCHW, tape=S["g_a"])
         y, y_in, y_in_nhwc, _ = engine.latent_handoff(y_nhwc, Q_NOISE, noise_y, torch.float32)
-        a, h, w = y_nhwc, hy, wy
-        ha_in = []
-        for op in model.hyper_encoder.ops:
-            ha_in.append((a, h, w))
-            a = T.conv_forward(arm, op.conv, op.epilogue, a, B, h, w)
-            h, w = engine.conv_out_hw(op.conv, h, w)
-        z, z_in, z_in_nhwc, _ = engine.latent_handoff(a, Q_NOISE, noise_z, torch.float32)
+        z_nhwc, _, _ = model.hyper_encoder.run_nhwc(y_nhwc, B, hy, wy, arm, tape=S["h_a"])
+        z, z_in, z_in_nhwc, _ = engine.latent_handoff(z_nhwc, Q_NOISE, noise_z, torch.float32)
         combs = [T._f32((B, hy, wy, 2 * (c1 - c0) + 2 * M), dev) for _, _, c0, c1 in heads]
-        a, h, w = z_in_nhwc, hz, wz
-        hs_in = []
-        hs = model.hyper_decoder.ops
-        for i, op in enumerate(hs):
-            hs_in.append((a, h, w))
-            if i == len(hs) - 1:
-                T.conv_forward(arm, op.conv, op.epilogue, a, B, h, w, out=combs[0], out_c_total=combs[0].shape[-1], out_c_offset=2 * M1)
-            else:
-                a = T.conv_forward(arm, op.conv, op.epilogue, a, B, h, w)
-            h, w = engine.conv_out_hw(op.conv, h, w)
+        model.hyper_decoder.run_nhwc(z_in_nhwc, B, hz, wz, arm, tape=S["h_s"],
+                                     final_kw=dict(out=combs[0], out_c_total=combs[0].shape[-1], out_c_offset=2 * M1))
         combs[1][..., 2 * M2:] = combs[0][..., 2 * M1:]                       # the second head reads the same psi
         head_state = []
         for (ctx, ep, c0, c1), comb in zip(heads, combs):
@@ -85,23 +61,9 @@ def _forward_impl(model, x, noise_z, noise_y):
             head_state.append(dict(yi=yi, yi_nhwc=yi_nhwc, comb=comb, e1=e1, e2=e2, raw=raw, parts=ly["partials"], ly=ly))
         fe = model.factorized_entropy_model
         _, p_z, logp_z, parts_z = fe.likelihood(z_in, Q_PASSTHRU)
-        a, h, w = y_in_nhwc, hy, wy
-        dec_in, dec_u = [], []
-        dec = model.decoder.ops
-        for i, op in enumerate(dec):
-            last = i == len(dec) - 1
-            dec_in.append((a, h, w))
-            a = T.conv_forward(arm, op.conv, EPI_BIAS, a, B, h, w, out_layout=LAYOUT_NCHW if last else LAYOUT_NHWC)
-            h, w = engine.conv_out_hw(op.conv, h, w)
-            if op.gdn is not None:
-                u = a
-                a, nrm = T.gdn_forward(arm, op.gdn, u, B, h, w)
-                dec_u.append((u, nrm))
-            else:
-                dec_u.append(None)
-        x_hat = a
-    S = dict(arm=arm, shape=(B, H, W), enc_in=enc_in, enc_u=enc_u, ha_in=ha_in, hs_in=hs_in, dec_in=dec_in, dec_u=dec_u, head_state=head_state,
-             z_in=z_in, fparams=fe.packed())
+        x_hat, _, _ = model.decoder.run_nhwc(y_in_nhwc, B, hy, wy, arm, tape=S["g_s"])         # the RGB layer writes NCHW
+    S.update(arm=arm, shape=(B, H, W), head_state=head_state, y_nhwc=y_nhwc, y_in_nhwc=y_in_nhwc, z_in=z_in, z_in_nhwc=z_in_nhwc,
+             fparams=fe.packed())
     return (x_hat, head_state, p_z, logp_z, parts_z, y, y_in, z, z_in), S
 
 
@@ -112,28 +74,15 @@ def _backward_impl(model, S, g, g_logp_heads, g_logp_z) -> Dict[int, torch.Tenso
     B, H, W = S["shape"]
     M, K = model.M, model.K
     hy, wy, hz, wz = H // 16, W // 16, H // 64, W // 64
-    arm, heads, head_state = S["arm"], _heads(model), S["head_state"]
-    enc_in, enc_u, ha_in, hs_in, dec_in, dec_u, z_in = (S[k] for k in ("enc_in", "enc_u", "ha_in", "hs_in", "dec_in", "dec_u", "z_in"))
-    dec, hs, fe = model.decoder.ops, model.hyper_decoder.ops, model.factorized_entropy_model
+    arm, heads, head_state, z_in = S["arm"], _heads(model), S["head_state"], S["z_in"]
+    fe = model.factorized_entropy_model
     grads: Dict[int, torch.Tensor] = {}
 
     def put(param, gr):
         grads[id(param)] = gr if id(param) not in grads else grads[id(param)] + gr
 
     with torch.cuda.device(dev):
-        g_layout = LAYOUT_NCHW
-        for i in range(len(dec) - 1, -1, -1):                                  # g_s
-            op = dec[i]
-            a, h, w = dec_in[i]
-            ho, wo = engine.conv_out_hw(op.conv, h, w)
-            if op.gdn is not None:
-                g, dbeta, dgamma = T.gdn_bwd(op.gdn, dec_u[i][0], g, B, ho, wo, norm=dec_u[i][1])
-                put(op.gdn.beta, dbeta); put(op.gdn.gamma, dgamma)
-            dw, db = T.conv_wgrad(op.conv, a, g, B, h, w, LAYOUT_NHWC, g_layout, arm=arm)
-            put(op.conv.weight, dw); put(op.conv.bias, db)
-            g = T.conv_dgrad(op.conv, g, B, h, w, g_layout, arm=arm)
-            g_layout = LAYOUT_NHWC
-        d_yin_gs = g
+        d_yin_gs = S["g_s"].backward(g, LAYOUT_NCHW, put, T.conv_wgrad, root=S["y_in_nhwc"])
         d_psi, d_yin_parts = None, []
         for (ctx, ep, c0, c1), hsd in zip(heads, head_state):                  # the two entropy heads
             mi = c1 - c0
@@ -156,16 +105,8 @@ def _backward_impl(model, S, g, g_logp_heads, g_logp_z) -> Dict[int, torch.Tenso
             dw, db = T.conv_wgrad(ctx.masked, hsd["yi_nhwc"], d_phi, B, hy, wy, LAYOUT_NHWC, LAYOUT_NHWC, arm=arm)
             put(ctx.masked.weight, dw); put(ctx.masked.bias, db)
             d_yin_parts.append(T.add_(d_yi, T.conv_dgrad(ctx.masked, d_phi, B, hy, wy, arm=arm)))
-        g = d_psi                                                              # h_s
-        for i in range(len(hs) - 1, -1, -1):
-            op = hs[i]
-            a, h, w = hs_in[i]
-            dw, db = T.conv_wgrad(op.conv, a, g, B, h, w, LAYOUT_NHWC, LAYOUT_NHWC, arm=arm)
-            put(op.conv.weight, dw); put(op.conv.bias, db)
-            g = T.conv_dgrad(op.conv, g, B, h, w, arm=arm)
-            if i > 0:
-                g = T.lrelu_bwd_(g, a)
-        d_zin = g
+        del g                                                                  # the last head's concat gradient: free it before h_s
+        d_zin = S["h_s"].backward(d_psi, LAYOUT_NHWC, put, T.conv_wgrad, root=S["z_in_nhwc"])
         glz = g_logp_z.contiguous().float()                                    # factorized prior
         dz_fac = torch.empty_like(z_in)
         dpar = T._f32((M, 43), dev)
@@ -175,30 +116,9 @@ def _backward_impl(model, S, g, g_logp_heads, g_logp_z) -> Dict[int, torch.Tenso
             prm = getattr(fe, name)[idx]
             put(prm, dpar[:, lo:hi].reshape(prm.shape).contiguous())
         d_zin = T.to_nhwc(dz_fac, accumulate_into=d_zin)
-        g = d_zin                                                              # h_a
-        ha = model.hyper_encoder.ops
-        for i in range(len(ha) - 1, -1, -1):
-            op = ha[i]
-            a, h, w = ha_in[i]
-            dw, db = T.conv_wgrad(op.conv, a, g, B, h, w, LAYOUT_NHWC, LAYOUT_NHWC, arm=arm)
-            put(op.conv.weight, dw); put(op.conv.bias, db)
-            g = T.conv_dgrad(op.conv, g, B, h, w, arm=arm)
-            if i > 0:
-                g = T.lrelu_bwd_(g, a)
+        g = S["h_a"].backward(d_zin, LAYOUT_NHWC, put, T.conv_wgrad, root=S["y_nhwc"])
         dy = T.add_(T.add_(g, torch.cat(d_yin_parts, dim=-1).contiguous()), d_yin_gs)
-        g = dy                                                                 # g_a
-        enc = model.encoder.ops
-        for i in range(len(enc) - 1, -1, -1):
-            op = enc[i]
-            a, h, w, layout = enc_in[i]
-            ho, wo = engine.conv_out_hw(op.conv, h, w)
-            if op.gdn is not None:
-                g, dbeta, dgamma = T.gdn_bwd(op.gdn, enc_u[i][0], g, B, ho, wo, norm=enc_u[i][1])
-                put(op.gdn.beta, dbeta); put(op.gdn.gamma, dgamma)
-            dw, db = T.conv_wgrad(op.conv, a, g, B, h, w, layout, LAYOUT_NHWC, arm=arm)
-            put(op.conv.weight, dw); put(op.conv.bias, db)
-            if i > 0:
-                g = T.conv_dgrad(op.conv, g, B, h, w, arm=arm)
+        S["g_a"].backward(dy, LAYOUT_NHWC, put, T.conv_wgrad, root=None)
     T.forget_pairs()
     return grads
 
@@ -211,12 +131,7 @@ def step_gradients(model, x: torch.Tensor, lambda_rd: float, noise=None):
     dev = x.device
     x = x.contiguous().float()
     B, _, H, W = x.shape
-    M = model.M
-    if noise is not None:
-        noise_z, noise_y = noise
-    else:
-        noise_z = torch.rand((B, M, H // 64, W // 64), device=dev) - 0.5
-        noise_y = torch.rand((B, M, H // 16, W // 16), device=dev) - 0.5
+    noise_z, noise_y = draw_noise(model.M, x, noise)
     T.forget_pairs()
     (x_hat, head_state, p_z, logp_z, parts_z, y, y_in, z, z_in), S = _forward_impl(model, x, noise_z, noise_y)
     with torch.cuda.device(dev):
@@ -253,8 +168,8 @@ class _ScalableTrainForward(torch.autograd.Function):
         (x_hat, head_state, p_z, logp_z, parts_z, y, y_in, z, z_in), S = _forward_impl(model, x, noise_z, noise_y)
         ctx.model, ctx.S = model, S
         l1, l2 = head_state[0]["ly"], head_state[1]["ly"]
-        names = ("mu", "sigma") if model.K == 1 else ("weights", "mus", "sigmas")
-        nd = [y, y_in, z, z_in, p_z, l1["p"], l2["p"], l1["partials"], l2["partials"], parts_z] + [l1[n] for n in names] + [l2[n] for n in names]
+        nd = [y, y_in, z, z_in, p_z, l1["p"], l2["p"], l1["partials"], l2["partials"], parts_z] + mixture_params(l1, model.K) + \
+            mixture_params(l2, model.K)
         ctx.mark_non_differentiable(*nd)
         return (x_hat, l1["logp"], l2["logp"], logp_z, *nd)
 
@@ -271,28 +186,11 @@ class _ScalableTrainForward(torch.autograd.Function):
 
 def train_forward(model, x: torch.Tensor, noise=None) -> dict:
     """``model(x, training=True)`` of ScalableImageCoding as a differentiable call (reference dict keys, Models.py:321-338 minus F_tilde)."""
-    B, _, H, W = x.shape
-    M, M1, K = model.M, model.M1, model.K
-    if noise is not None:
-        noise_z, noise_y = noise
-    else:
-        noise_z = torch.rand((B, M, H // 64, W // 64), device=x.device) - 0.5
-        noise_y = torch.rand((B, M, H // 16, W // 16), device=x.device) - 0.5
+    noise_z, noise_y = draw_noise(model.M, x, noise)
     T.forget_pairs()
     params = [p for _, p in model.named_parameters()]
     res = _ScalableTrainForward.apply(model, x.contiguous().float(), noise_z, noise_y, *params)
-    x_hat, logp_y1, logp_y2, logp_z, y, y_in, z, z_in, p_z, p_y1, p_y2, parts1, parts2, parts_z = res[:14]
-    engine.attach_partials(logp_y1, parts1)
-    engine.attach_partials(logp_y2, parts2)
-    engine.attach_partials(logp_z, parts_z)
-    y1, y2 = torch.split(y_in, [M1, M - M1], dim=1)
-    out = {"x_hat": x_hat, "y": y, "y_in": y_in, "y1": y1, "y2": y2, "z": z, "z_in": z_in, "p_z": p_z, "logp_z": logp_z,
-           "p_y1": p_y1, "logp_y1": logp_y1, "p_y2": p_y2, "logp_y2": logp_y2, "training": True}
-    names = ("mu", "sigma") if K == 1 else ("weights", "mus", "sigmas")
-    rest = res[14:]
-    for i, n in enumerate(names):
-        out[f"{n}1"], out[f"{n}2"] = rest[i], rest[len(names) + i]
-    return out
+    return two_head_outputs(*res, M1=model.M1, K=model.K, training=True)
 
 
 class _VisionRDLoss(torch.autograd.Function):

@@ -1,10 +1,10 @@
-"""CPU (no GPU): the host logic of the residual family's training step - ``training.Tape`` and the ``tape=`` plumbing of
-Layers.py / Components._Chain - with torch stand-ins for the C-ABI calls (conv forward / weight gradient / adjoint conv, GDN forward /
-backward, LeakyReLU backward, add).  What is checked is the BOOKKEEPING: every op of the 3x3 transforms is recorded once, gradients of
-tensors with two consumers (the block input feeding the main path and the skip) are summed, the gradient of the transform's input
-comes back, and every parameter gets its gradient - against torch autograd over the oracle's restatement of the same transforms
-(oracle/forward.py: analysis_3x3 / synthesis_3x3 / hyper_*_3x3, pinned to the reference's own classes by tests/test_oracle.py).
-The kernels themselves are checked on the GPU (tests/test_gpu_residual.py)."""
+"""CPU (no GPU): the host logic of the training step's transforms - ``training.Tape`` and the ``tape=`` plumbing of Layers.py /
+Components._Transform (5x5) / Components._Chain (3x3) - with torch stand-ins for the C-ABI calls (conv forward / weight gradient /
+adjoint conv, GDN forward / backward, LeakyReLU backward, add).  What is checked is the BOOKKEEPING: every op of the transforms is
+recorded once, gradients of tensors with two consumers (the block input feeding the main path and the skip) are summed, the gradient
+of the transform's input comes back, and every parameter gets its gradient - against torch autograd over the oracle's restatement
+of the same transforms (oracle/forward.py: analysis / synthesis / hyper_* and their _3x3 forms, pinned to the reference's own
+classes by tests/test_oracle.py).  The kernels themselves are checked on the GPU (tests/test_gpu_train.py, test_gpu_residual.py)."""
 import pytest
 import torch
 import torch.nn as nn
@@ -96,14 +96,18 @@ def _perturb(mod, seed):
     return mod
 
 
+_CLASSES = {"encoder": "Encoder", "decoder": "Decoder", "hyper_encoder": "HyperEncoder", "hyper_decoder": "HyperDecoder"}
+_ORACLE = {"encoder": "analysis", "decoder": "synthesis", "hyper_encoder": "hyper_analysis", "hyper_decoder": "hyper_synthesis"}
+
+
 @pytest.mark.parametrize("which", ["encoder", "decoder", "hyper_encoder", "hyper_decoder"])
-def test_tape_routes_gradients_through_the_3x3_transforms(torch_backend, which):
+@pytest.mark.parametrize("family", ["3x3", "5x5"])
+def test_tape_routes_gradients_through_the_transforms(torch_backend, family, which):
     from neural_image_compression_b200 import Components as Cm
     T = torch_backend
     M = 8
     torch.manual_seed(3)
-    mod = _perturb({"encoder": Cm.Encoder3x3, "decoder": Cm.Decoder3x3, "hyper_encoder": Cm.HyperEncoder3x3,
-                    "hyper_decoder": Cm.HyperDecoder3x3}[which](latent_channels=M), 4)
+    mod = _perturb(getattr(Cm, _CLASSES[which] + family)(latent_channels=M), 4)
     n, h, w = 2, (32 if which == "encoder" else 4), (48 if which == "encoder" else 6)
     x_nchw = (torch.rand(n, 3, h, w) if which == "encoder" else torch.randn(n, M, h, w)).double()
     # oracle: autograd over the restated transform
@@ -112,8 +116,7 @@ def test_tape_routes_gradients_through_the_3x3_transforms(torch_backend, which):
     xr = x_nchw.clone().requires_grad_()
     prev, O.DIFFERENTIABLE = O.DIFFERENTIABLE, True
     try:
-        fn = {"encoder": O.analysis_3x3, "decoder": O.synthesis_3x3, "hyper_encoder": O.hyper_analysis_3x3,
-              "hyper_decoder": O.hyper_synthesis_3x3}[which]
+        fn = getattr(O, _ORACLE[which] + ("_3x3" if family == "3x3" else ""))
         y_ref = fn(sd, xr, torch.float64)
         g_out = torch.randn(y_ref.shape, generator=torch.Generator().manual_seed(5), dtype=torch.float64)
         y_ref.backward(g_out)
@@ -148,20 +151,22 @@ def test_tape_routes_gradients_through_the_3x3_transforms(torch_backend, which):
 
 
 def test_chain_writes_its_last_conv_into_a_channel_window(torch_backend):
-    """h_s of the training forward writes psi straight into its window of the entropy-parameter stack's concat buffer
-    (`final_kw`): same values as the plain call, the other window untouched, and the backward starts from the window's gradient."""
+    """h_s of the training forward (the 3x3 and the 5x5 family) writes psi straight into its window of the entropy-parameter
+    stack's concat buffer (`final_kw`): same values as the plain call, the other window untouched, and the backward starts from the
+    window's gradient."""
     from neural_image_compression_b200 import Components as Cm
     T = torch_backend
     M, n, h, w = 8, 1, 2, 3
-    torch.manual_seed(7)
-    mod = Cm.HyperDecoder3x3(latent_channels=M)
-    x = torch.randn(n, h, w, M).double()
-    plain, ho, wo = mod.run_nhwc(x, n, h, w, "fp32", tape=T.Tape("fp32", n))
-    combined = torch.full((n, ho, wo, 4 * M), 7.0, dtype=torch.float64)
-    tape = T.Tape("fp32", n)
-    mod.run_nhwc(x, n, h, w, "fp32", tape=tape, final_kw=dict(out=combined, out_c_total=4 * M, out_c_offset=2 * M))
-    assert tape.output is combined and torch.equal(combined[..., 2 * M:], plain) and bool((combined[..., :2 * M] == 7.0).all())
-    grads = {}
-    g = torch.randn(n, ho, wo, 2 * M, dtype=torch.float64)
-    gx = tape.backward(g, NHWC, lambda p, v: grads.__setitem__(id(p), v), T.conv_wgrad, root=x)
-    assert gx.shape == x.shape and len(grads) == len(list(mod.parameters()))
+    for cls in (Cm.HyperDecoder3x3, Cm.HyperDecoder5x5):
+        torch.manual_seed(7)
+        mod = cls(latent_channels=M)
+        x = torch.randn(n, h, w, M).double()
+        plain, ho, wo = mod.run_nhwc(x, n, h, w, "fp32", tape=T.Tape("fp32", n))
+        combined = torch.full((n, ho, wo, 4 * M), 7.0, dtype=torch.float64)
+        tape = T.Tape("fp32", n)
+        mod.run_nhwc(x, n, h, w, "fp32", tape=tape, final_kw=dict(out=combined, out_c_total=4 * M, out_c_offset=2 * M))
+        assert tape.output is combined and torch.equal(combined[..., 2 * M:], plain) and bool((combined[..., :2 * M] == 7.0).all())
+        grads = {}
+        g = torch.randn(n, ho, wo, 2 * M, dtype=torch.float64)
+        gx = tape.backward(g, NHWC, lambda p, v: grads.__setitem__(id(p), v), T.conv_wgrad, root=x)
+        assert gx.shape == x.shape and len(grads) == len(list(mod.parameters())), cls.__name__
