@@ -495,6 +495,37 @@ int nic_codec_decode(int32_t kind, const uint8_t* blob, const int64_t* lane_off,
  * mod 2^32 */
 int nic_codec_checksum(const float* y, int64_t y_per_image, const float* z, int64_t z_per_image, int32_t b, uint32_t* out, void* stream);
 
+/*
+ * Step-local entropy parameters (DESIGN.md section 10; ScalableImageCoding's coder): the masked 5x5 context conv 'A' of a head on
+ * m channels -> 2m, then the 1x1 stack (2m + 2M) -> 640 -> 640 -> (2m | 3Km) with LeakyReLU(0.01) after the first two, computed
+ * only at the pixels of one launch - every pixel (t = -1) or those of wavefront step t.  fp32 CUDA cores: every output element is
+ * one thread's fixed-order __fmaf_rn chain (bias first, then the inputs in the order of the packed weights, zeros at the borders),
+ * so a pixel's value is the same bits whichever launch, batch or pixel count computed it.
+ * Per head (n_heads = 1 or 2, one launch per layer serves both):
+ *   sym     the head's symbols, NHWC f32 [b, h, w, m]; psi = NHWC f32 [b, h, w, 2 M] (shared by the heads)
+ *   w_ctx   [12 m][2 m]: live tap s (rows i - 2, i - 1 at columns j - 2 .. j + 2, then row i at j - 2, j - 1), channel c -> row
+ *           s m + c; w1 [2 m + 2 M][640] (rows: phi, then psi), w2 [640][640], w3 [640][np m]; biases f32; np = 2 (k = 1) or 3 k
+ *   raw     NCHW f32 [b, np m, h, w] (nic_codec_tables' GM params), written at the launch's pixels only
+ *   work    n (2 m + 1280) floats, n = b h w (t = -1) or b * (pixels of step t)
+ */
+typedef struct nic_codec_head {
+  const float* sym;
+  const float* w_ctx;
+  const float* b_ctx;
+  const float* w1;
+  const float* b1;
+  const float* w2;
+  const float* b2;
+  const float* w3;
+  const float* b3;
+  float* raw;
+  float* work;
+  int64_t work_floats;
+  int32_t m, reserved;
+} nic_codec_head;
+int nic_codec_params(const nic_codec_head* heads, int32_t n_heads, const float* psi, int32_t b, int32_t M, int32_t k, int32_t h,
+                     int32_t w, int32_t t, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

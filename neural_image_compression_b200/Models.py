@@ -19,6 +19,7 @@ the host):
 from __future__ import annotations
 
 import contextlib
+import functools
 import os
 from typing import Optional, Tuple
 
@@ -497,50 +498,19 @@ class ScalableImageCoding(nn.Module):
             # the training call with autograd on: one autograd node over the layer-by-layer forward (training_scalable.py)
             from . import training_scalable as _ts
             return _ts.train_forward(self, x, noise=noise)
-        arm, M, M1, M2, K = self.precision, self.M, self.M1, self.M2, self.K
-        if arm == "bf16x3" and M in (128, 192) and M1 % 64 == 0 and M2 % 64 == 0:
+        M, M1, M2, K = self.M, self.M1, self.M2, self.K
+        if self.fused_pipeline:
             return self._forward_pairs(x, training, noise)
-        from . import training as T
-
-        def layer(op, a, h, w, **kw):
-            """One conv (+ GDN / LeakyReLU) with f32 tensors at both ends."""
-            if arm == "fp32":
-                return op.run(a, B, h, w, "fp32", **kw)
-            u = T.conv_forward(arm, op.conv, engine.EPI_BIAS if op.gdn is not None else op.epilogue, a, B, h, w,
-                               mask_a=op.mask_a, **kw)
-            if op.gdn is not None:
-                ho, wo = engine.conv_out_hw(op.conv, h, w)
-                u = T.gdn_forward(arm, op.gdn, u, B, ho, wo)[0]
-            T.forget_pairs()                     # the split copies are per layer here (the training step keeps them for its backward)
-            return u
+        layer = functools.partial(self._layer, B=B)
         x = x.contiguous().float()
         hy, wy, hz, wz = H // 16, W // 16, H // 64, W // 64
         with torch.cuda.device(x.device), torch.no_grad():
             noise_z, noise_y = draw_noise(M, x, noise) if training else (None, None)
-            qmode = Q_NOISE if training else Q_ROUND
-            a, h, w, layout = x, H, W, LAYOUT_NCHW
-            for op in self.encoder.ops:
-                a = layer(op, a, h, w, in_layout=layout, out_layout=LAYOUT_NHWC)
-                h, w = engine.conv_out_hw(op.conv, h, w)
-                layout = LAYOUT_NHWC
-            y_nhwc = a
-            y, y_in, y_in_nhwc, _ = engine.latent_handoff(y_nhwc, qmode, noise_y, torch.float32)
-            a, h, w = y_nhwc, hy, wy
-            for op in self.hyper_encoder.ops:
-                a = layer(op, a, h, w)
-                h, w = engine.conv_out_hw(op.conv, h, w)
-            z, z_in, z_in_nhwc, _ = engine.latent_handoff(a, qmode, noise_z, torch.float32)
+            y, y_in, y_in_nhwc, z, z_in, z_in_nhwc = self._layer_analysis(x, Q_NOISE if training else Q_ROUND, noise_y, noise_z)
             # psi once, into head 1's concat buffer [phi1 (2 M1) | psi (2 M)]; head 2's buffer gets a copy of the window
             comb1 = torch.empty((B, hy, wy, 2 * M1 + 2 * M), dtype=torch.float32, device=x.device)
             comb2 = torch.empty((B, hy, wy, 2 * M2 + 2 * M), dtype=torch.float32, device=x.device)
-            a, h, w = z_in_nhwc, hz, wz
-            hs = self.hyper_decoder.ops
-            for i, op in enumerate(hs):
-                if i == len(hs) - 1:
-                    layer(op, a, h, w, out=comb1, out_c_total=2 * M1 + 2 * M, out_c_offset=2 * M1)
-                else:
-                    a = layer(op, a, h, w)
-                h, w = engine.conv_out_hw(op.conv, h, w)
+            self._layer_h_s_into(z_in_nhwc, B, hz, wz, comb1, 2 * M1 + 2 * M, 2 * M1)
             comb2[..., 2 * M2:] = comb1[..., 2 * M1:]
             y1, y2 = torch.split(y_in, [M1, M2], dim=1)                   # Models.py:279 (views, as in the reference)
             y1c, y2c = y1.contiguous(), y2.contiguous()
@@ -556,13 +526,79 @@ class ScalableImageCoding(nn.Module):
                 raw = layer(ep.ops[2], a, hy, wy, out_layout=LAYOUT_NCHW)
                 heads.append(gm_likelihood(yi, raw, mi, K, Q_PASSTHRU, full=True, want_y_in=False))
             _, p_z, logp_z, parts_z = self.factorized_entropy_model.likelihood(z_in, Q_PASSTHRU)
-            a, h, w = y_in_nhwc, hy, wy
-            dec = self.decoder.ops
-            for i, op in enumerate(dec):
-                last = i == len(dec) - 1
-                a = layer(op, a, h, w, out_layout=LAYOUT_NCHW if last else LAYOUT_NHWC)
-                h, w = engine.conv_out_hw(op.conv, h, w)
-            x_hat = a
+            x_hat = self._layer_g_s(y_in_nhwc, B, hy, wy)
         l1, l2 = heads
         return two_head_outputs(x_hat, l1["logp"], l2["logp"], logp_z, y, y_in, z, z_in, p_z, l1["p"], l2["p"], l1["partials"],
                                 l2["partials"], parts_z, *mixture_params(l1, K), *mixture_params(l2, K), M1=M1, K=K, training=training)
+
+    # ---- the layer-by-layer path (fp32, and bf16x3 outside the fused pipeline's channel counts); the coder calls the same stages
+
+    @property
+    def fused_pipeline(self) -> bool:
+        """True when the eval forward runs _forward_pairs (bf16x3 at M = 128 / 192), else the layer-by-layer stages below."""
+        return self.precision == "bf16x3" and self.M in (128, 192) and self.M1 % 64 == 0 and self.M2 % 64 == 0
+
+    def _layer(self, op, a, h, w, B, **kw):
+        """One conv (+ GDN / LeakyReLU) with f32 tensors at both ends."""
+        arm = self.precision
+        if arm == "fp32":
+            return op.run(a, B, h, w, "fp32", **kw)
+        from . import training as T
+        u = T.conv_forward(arm, op.conv, engine.EPI_BIAS if op.gdn is not None else op.epilogue, a, B, h, w, mask_a=op.mask_a, **kw)
+        if op.gdn is not None:
+            ho, wo = engine.conv_out_hw(op.conv, h, w)
+            u = T.gdn_forward(arm, op.gdn, u, B, ho, wo)[0]
+        T.forget_pairs()                     # the split copies are per layer here (the training step keeps them for its backward)
+        return u
+
+    def _layer_analysis(self, x, qmode, noise_y, noise_z):
+        """g_a -> y hand-off -> h_a -> z hand-off: (y, y_in, y_in_nhwc, z, z_in, z_in_nhwc), the engine copies NHWC f32."""
+        B, _, H, W = x.shape
+        a, h, w, layout = x, H, W, LAYOUT_NCHW
+        for op in self.encoder.ops:
+            a = self._layer(op, a, h, w, B, in_layout=layout, out_layout=LAYOUT_NHWC)
+            h, w = engine.conv_out_hw(op.conv, h, w)
+            layout = LAYOUT_NHWC
+        y_nhwc = a
+        y, y_in, y_in_nhwc, _ = engine.latent_handoff(y_nhwc, qmode, noise_y, torch.float32)
+        for op in self.hyper_encoder.ops:
+            a = self._layer(op, a, h, w, B)
+            h, w = engine.conv_out_hw(op.conv, h, w)
+        z, z_in, z_in_nhwc, _ = engine.latent_handoff(a, qmode, noise_z, torch.float32)
+        return y, y_in, y_in_nhwc, z, z_in, z_in_nhwc
+
+    def _layer_h_s_into(self, z_in_nhwc, B, hz, wz, out, c_total, c_offset):
+        """h_s with its last conv writing psi into channels [c_offset, c_offset + 2M) of `out` (NHWC f32, c_total channels)."""
+        a, h, w = z_in_nhwc, hz, wz
+        hs = self.hyper_decoder.ops
+        for i, op in enumerate(hs):
+            if i == len(hs) - 1:
+                self._layer(op, a, h, w, B, out=out, out_c_total=c_total, out_c_offset=c_offset)
+            else:
+                a = self._layer(op, a, h, w, B)
+            h, w = engine.conv_out_hw(op.conv, h, w)
+
+    def _layer_g_s(self, y_in_nhwc, B, hy, wy):
+        """g_s: NHWC f32 symbols -> x_hat NCHW f32."""
+        a, h, w = y_in_nhwc, hy, wy
+        dec = self.decoder.ops
+        for i, op in enumerate(dec):
+            last = i == len(dec) - 1
+            a = self._layer(op, a, h, w, B, out_layout=LAYOUT_NCHW if last else LAYOUT_NHWC)
+            h, w = engine.conv_out_hw(op.conv, h, w)
+        return a
+
+    def compress(self, x: torch.Tensor) -> dict:
+        """x [B, 3, H, W] (H, W multiples of 64) -> {"strings": [y1_strings, y2_strings, z_strings], "shape": (hz, wz)}: one bytes
+        object per image in each list, coded with the eval-mode symbols.  The base layer (y1 + z) decodes without the y2 strings.
+        Format: DESIGN.md section 10."""
+        from . import scalable_codec
+        return scalable_codec.compress(self, x)
+
+    def decompress(self, strings, shape, base_only: bool = False) -> dict:
+        """strings / shape as compress returned them (any subset of the images, in any order) -> {"x_hat", "y_hat", "y1_hat",
+        "y2_hat", "z_hat"}, NCHW f32; x_hat = g_s(y_hat), not clamped.  base_only=True decodes z and y1 alone (strings[1] may be
+        None) and returns {"y1_hat", "z_hat"}.  Raises ValueError on a malformed string, a string of another model configuration,
+        or a checksum mismatch of a decoded layer (corrupted bytes, other weights)."""
+        from . import scalable_codec
+        return scalable_codec.decompress(self, strings, shape, base_only=base_only)

@@ -42,6 +42,12 @@ class CtxEpArgs(C.Structure):
                 ("workspace", _vp), ("workspace_bytes", _sz)]
 
 
+class CodecHead(C.Structure):
+    """struct nic_codec_head (include/nic.h): one entropy head of nic_codec_params."""
+    _fields_ = [(n, _vp) for n in ("sym", "w_ctx", "b_ctx", "w1", "b1", "w2", "b2", "w3", "b3", "raw", "work")] + \
+               [("work_floats", _i64), ("m", _i32), ("reserved", _i32)]
+
+
 # name -> (restype, argtypes); must list every function include/nic.h declares (tests check this)
 SIGNATURES = {
     "nic_version": (C.c_int, []),
@@ -104,6 +110,7 @@ SIGNATURES = {
     "nic_codec_encode": (C.c_int, [_i32, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i64, _vp, _vp, _vp]),
     "nic_codec_decode": (C.c_int, [_i32, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp]),
     "nic_codec_checksum": (C.c_int, [_vp, _i64, _vp, _i64, _i32, _vp, _vp]),
+    "nic_codec_params": (C.c_int, [C.POINTER(CodecHead), _i32, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _vp]),
 }
 
 # entropy coder constants of include/nic.h

@@ -8,6 +8,7 @@
 // rANS: 32-bit state in [2^16, 2^32), 16-bit renormalisation words, 16-bit probability precision.  A table row of one
 // element is a window of n <= NIC_CODEC_WINDOW consecutive integers starting at `lo`, plus one escape bin (index n) that
 // carries any other value; an escaped value follows the escape bin as two raw 16-bit words (zigzag value, low half first).
+#include "codec_step.cuh"
 #include "common.cuh"
 #include "entropy_math.cuh"
 
@@ -21,13 +22,6 @@ constexpr int kRow = NIC_CODEC_WINDOW + 2;                 // cdf entries of one
 constexpr float kTail = 6.0f;                              // window = [min mu_k - 6 sigma_k, max mu_k + 6 sigma_k]
 constexpr float kSymLimit = 1048576.0f;                    // 2^20: compress() rejects larger magnitudes
 constexpr int kNoSymbol = -2147483647 - 1;
-
-// Pixel rows of wavefront step t (pixel (i, j) is decoded at step 3 i + j): i in [i0, i0 + cnt), j = t - 3 i.
-__host__ __device__ __forceinline__ void step_rows(int t, int h, int w, int& i0, int& cnt) {
-  const int i1 = min(h - 1, t / 3);
-  i0 = t - w + 1 > 0 ? (t - w + 3) / 3 : 0;
-  cnt = i1 - i0 + 1;
-}
 
 __device__ __forceinline__ uint32_t zigzag(int v) { return v >= 0 ? 2u * static_cast<uint32_t>(v) : 2u * static_cast<uint32_t>(-v) - 1u; }
 __device__ __forceinline__ float unzigzag(uint32_t z) {
