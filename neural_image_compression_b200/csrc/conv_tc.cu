@@ -162,14 +162,15 @@ int encode_2d_c32(CUtensorMap* m, const void* base, uint64_t inner, uint64_t row
   return NIC_OK;
 }
 
-// NHWC bf16 tensor, boxes of 32 channels (64-byte rows, SWIZZLE_64B: 16-byte chunk ^= (row >> 1) & 3) x box_w x box_h pixels
-int encode_nhwc_c32(CUtensorMap* m, const void* base, int n, int h, int w, int c, int box_w, int box_h) {
+// NHWC bf16 tensor, boxes of 32 channels (64-byte rows, SWIZZLE_64B: 16-byte chunk ^= (row >> 1) & 3) x box_w x box_h pixels,
+// every stride-th pixel in w and h (the output phases of a transposed conv)
+int encode_nhwc_c32(CUtensorMap* m, const void* base, int n, int h, int w, int c, int box_w, int box_h, int stride) {
   EncodeTiledFn enc = get_encode();
   if (!enc) return fail(NIC_E_CUDA, "cuTensorMapEncodeTiled entry point not available");
   cuuint64_t dims[4] = {(cuuint64_t)c, (cuuint64_t)w, (cuuint64_t)h, (cuuint64_t)n};
   cuuint64_t strides[3] = {(cuuint64_t)c * 2, (cuuint64_t)w * c * 2, (cuuint64_t)h * w * c * 2};
-  cuuint32_t box[4] = {32, (cuuint32_t)box_w, (cuuint32_t)box_h, 1};
-  cuuint32_t es[4] = {1, 1, 1, 1};
+  cuuint32_t box[4] = {32, (cuuint32_t)(box_w * stride), (cuuint32_t)(box_h * stride), 1};
+  cuuint32_t es[4] = {1, (cuuint32_t)stride, (cuuint32_t)stride, 1};
   CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(base), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
                    CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) return fail(NIC_E_CUDA, "cuTensorMapEncodeTiled(nhwc %dx%dx%dx%d, 32-channel box %dx%d) failed: %d", n, h, w, c, box_w, box_h, (int)r);
@@ -232,6 +233,8 @@ struct TcParams {
   int flat_hw;                                 // > 0: 1x1 conv over a flattened pixel list; pixel p -> image p / flat_hw
   int stage2;                                  // bf16-pair output with TWO staging tiles (hi tile, lo tile): no store is waited for
                                                // right after it was issued (layers whose mainloop is as short as their epilogue)
+  int epi_slices;                              // bf16-pair output, normal orientation: per-warp staging slices and stores
+                                               // (epilogue_block_slices) instead of the CTA-wide rounds of epilogue_block
   int tma_out;                                 // NHWC output leaves through shared memory + TMA tensor stores: 1 = bf16 (two
                                                // [128 px][64 ch] panels), 2 = f32 (four [128 px][32 ch] panels)
   int out_c_offset;                            // channel window start inside the output tensor (TMA coordinates)
@@ -274,6 +277,11 @@ __device__ __forceinline__ void trace(const TcParams& p, uint32_t tile_iter, int
       p.dbg_times[(static_cast<long>(blockIdx.x) * 32 + tile_iter) * 16 + 15] = static_cast<long long>(ns);
     }
   }
+}
+
+// a value (not a clock) into the same trace record: the phase of the tile, for tools/trace_layer.py's per-phase summary
+__device__ __forceinline__ void trace_value(const TcParams& p, uint32_t tile_iter, int slot, long long value) {
+  if (p.dbg_times && tile_iter < 16) p.dbg_times[(static_cast<long>(blockIdx.x) * 32 + tile_iter) * 16 + slot] = value;
 }
 
 // Tile order.  Default: x, y, image, phase, N tile (phase-major: consecutive tiles cost the same, the static round robin over
@@ -637,6 +645,71 @@ __device__ __forceinline__ bool epilogue_block(const TcParams& p, TcBarriers* sb
   return true;
 }
 
+// bf16-pair output of one M = 128 block, normal orientation, bias / LeakyReLU (TcParams::epi_slices).  epilogue_block stages
+// hi and lo in turn through the one CTA-wide 32 KB tile and waits for each store right after issuing it, inside CTA-wide
+// barriers - on layers whose mainloop is short (g_s layer 3: ~300 MMAs per tile) that epilogue is longer than the mainloop.
+// Here each of the 8 warps owns 4 KB of that tile: two 2 KB slices of 32 pixels (4 rows x 8) x 32 channels in the 64-byte
+// swizzle layout, each stored by the warp's own TMA box.  The warp reads its two 32-column groups of the accumulator once,
+// forms hi and lo together in registers, and sends hi / lo / hi / lo through the two slices in rotation, one bulk group per
+// store: a slice is rewritten only after the store two groups back (its previous use) has read it, never the one just issued.
+// No barrier between warps.  The caller's `release` runs right after the block's TMEM reads when `last` is set, so the MMAs of
+// the next tile but one may start while the stores are still draining.
+template <typename Release>
+__device__ __forceinline__ void epilogue_block_slices(const TcParams& p, const float* s_bias, uint8_t* sq, const CUtensorMap* map_o_ptr,
+                                                      uint32_t acc_tmem, int q, int lane, int wi, int img, int oy0, int ox0, int py, int px,
+                                                      int cbase, bool last, Release&& release, uint32_t trace_tile) {
+  const bool leader = wi == 0 && lane == 0;
+  if (leader) trace(p, trace_tile, 8 + 0);
+  const int cg0 = (wi >> 2) * 2;                                 // warpgroup hs takes channel groups 2 hs, 2 hs + 1
+  const bool live = cbase + cg0 * 32 < p.cout;                   // c_out % 64 == 0: both groups exist or neither
+  uint32_t hi[32], lo[32];                                       // 64 channels of this thread's pixel, packed in pairs
+  if (live) {
+    const uint32_t addr = acc_tmem + (static_cast<uint32_t>(q * 32) << 16) + cg0 * 32;
+#pragma unroll
+    for (int g = 0; g < 2; ++g) {
+      float v[32];
+      tmem_ld_32x32(addr + g * 32, v);
+      tmem_ld_wait();
+#pragma unroll
+      for (int j = 0; j < 32; j += 2) {
+        const int c = cbase + (cg0 + g) * 32 + j;
+        float a = v[j] + s_bias[c], b = v[j + 1] + s_bias[c + 1];
+        if (p.epilogue == NIC_EPI_LRELU) { a = a > 0.f ? a : 0.01f * a; b = b > 0.f ? b : 0.01f * b; }
+        const uint32_t h = pack_bf16x2(a, b);
+        hi[g * 16 + (j >> 1)] = h;
+        lo[g * 16 + (j >> 1)] = pack_bf16x2(a - __uint_as_float(h << 16), b - __uint_as_float(h & 0xffff0000u));   // lo = x - bf16(x)
+      }
+    }
+  }
+  if (last) release();
+  if (leader) trace(p, trace_tile, 8 + 4);
+  if (!live) return;
+  uint8_t* slices = sq + wi * 4096;
+  uint8_t* mine = slices + lane * 64;                            // box row = lane: pixel (q * 4 + lane / 8, lane % 8) of the block
+  const uint32_t swz = static_cast<uint32_t>(lane >> 1) & 3u;
+  const int wc = ox0 * p.out_stride + px, hc = (oy0 + q * 4) * p.out_stride + py;
+#pragma unroll
+  for (int k = 0; k < 4; ++k) {
+    const int g = k >> 1, half = k & 1;                          // hi of group 0, lo of group 0, hi of group 1, lo of group 1
+    if (lane == 0) tma_store_wait_read_1();
+    __syncwarp();
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      uint32_t w[4];
+#pragma unroll
+      for (int e = 0; e < 4; ++e) w[e] = half ? lo[g * 16 + j * 4 + e] : hi[g * 16 + j * 4 + e];
+      *reinterpret_cast<uint4*>(mine + half * 2048 + ((static_cast<uint32_t>(j) ^ swz) << 4)) = make_uint4(w[0], w[1], w[2], w[3]);
+    }
+    fence_proxy_async_smem();
+    __syncwarp();
+    if (lane == 0 && !(p.dbg & 2)) {
+      tma_store_4d(map_o_ptr, slices + half * 2048, p.out_c_offset + (half ? p.split_lo_off : 0) + cbase + (cg0 + g) * 32, wc, hc, img);
+      tma_store_commit();
+    }
+  }
+  if (leader) trace(p, trace_tile, 8 + 5);
+}
+
 // Epilogue of one tile in the swapped orientation (TcParams::swap): TMEM lane = output channel, column = pixel (block h of the
 // tile owns columns [128 h, 128 h + 128)).  Bias / LeakyReLU per lane, then the tile is TRANSPOSED into the same [pixel][64 ch]
 // 128-byte-swizzled staging panels the TMA stores of the normal orientation use: lane c writes bf16 (pixel p, channel c) with
@@ -998,7 +1071,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
           const int nplanes = ph.nplanes;
           const uint32_t buf = tcount & 1;
           if (!wait_or_abort(&sb.acc_empty[buf], ((tcount >> 1) & 1) ^ 1, &sb, p.status)) break;
-          if (lane == 0 && mw == 0) trace(p, tcount, 0);
+          if (lane == 0 && mw == 0) { trace(p, tcount, 0); trace_value(p, tcount, 7, phase); }
           tcgen05_fence_after();
           // swapped orientation: issuer 0 alone issues N = 256 MMAs (weights first, the pixels of both blocks second) into the
           // whole 256-column buffer; issuer 1 walks the rings and only commits
@@ -1116,6 +1189,38 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
       }
       __syncwarp();
     }
+  } else if (p.epi_slices) {
+    // ===================== epilogue (8 warps): bf16-pair output through per-warp slices =====================
+    // (a loop of its own: inlined into the generic loop below, epilogue_block_slices pushes the fused-GDN path of epilogue_block
+    // into register spills)
+    const int q = warp & 3, wi = warp - kFirstEpiWarp;
+    uint8_t* sq = smem + p.off_sq;
+    uint32_t tcount = 0;
+    for (int tile = first_tile; tile < p.total_tiles; tile += tile_step, ++tcount) {
+      int ntile, phase, img, ty, tx;
+      if (!decode_tile(p, tile, ntile, phase, img, ty, tx)) break;
+      const TcPhase& ph = p.phases[phase];
+      const int nblk = live_blocks(p, ty, tx);
+      const uint32_t buf = tcount & 1;
+      if (!__all_sync(0xffffffffu, wait_or_abort(&sb.acc_full[buf], (tcount >> 1) & 1, &sb, p.status))) break;
+      tcgen05_fence_after();
+      auto release = [&]() {
+        tcgen05_fence_before();
+        __syncwarp();
+        if (lane == 0) {
+          if (PAIR && rank != 0) mbar_arrive_cluster(mapa_u32(smem_u32(&sb.acc_empty[buf]), 0));   // the leader's issuers wait for both CTAs
+          else mbar_arrive(&sb.acc_empty[buf]);
+        }
+      };
+      int b0 = 0, b1 = (p.dbg & 8) ? 0 : nblk;                     // the blocks of this slot (tail_block: one of them)
+      if (const int only = tail_block(p, tile); only >= 0) { b0 = only; b1 = only < b1 ? only + 1 : b0; }
+      for (int b = b0; b < b1; ++b)      // the last block releases the accumulator right after its TMEM reads
+        epilogue_block_slices(p, s_bias, sq, &map_o, tmem + buf * 256 + b * 128, q, lane, wi, img, ty * p.tile_h + p.blk_roff[b],
+                              tx * p.tile_w + p.blk_coff[b], ph.py, ph.px, ntile * p.nb, b == b1 - 1, release, b == b0 ? tcount : 0xffffffffu);
+      if (wi == 0 && lane == 0) trace(p, tcount, 4);
+      if (b0 >= b1) release();
+    }
+    if (lane == 0) tma_store_wait_all();     // bulk groups belong to the thread that committed them: every warp has its own
   } else {
     // ===================== epilogue (8 warps) =====================
     const int q = warp & 3;                       // TMEM lane quadrant this warp may read
@@ -1761,6 +1866,12 @@ static int launch_tc(const nic_conv_desc* d, const TapTable& tt, const void* x, 
   if (!p.tma_out && !shuffle && !gdn && d->out_layout == NIC_LAYOUT_NHWC && p.out_dtype == NIC_DT_F32 && p.nb == 128 && d->c_out % 32 == 0 &&
       ctot % 4 == 0 && (reinterpret_cast<uintptr_t>(y) & 15) == 0 && !getenv("NIC_TC_NO_F32_TMA"))
     p.tma_out = 2;      // (y and z, the f32 tensors the latent hand-off reads: small layers, the ring depth does not matter there)
+  // bf16-pair outputs in the normal orientation leave through per-warp staging slices (epilogue_block_slices): bit-identical,
+  // and the epilogue no longer serialises on its own stores.  NIC_TC_EPI_SLICES=0 keeps the CTA-wide rounds as a cross-check.
+  {
+    const char* e = getenv("NIC_TC_EPI_SLICES");
+    p.epi_slices = (p.split_out && p.tma_out == 1 && !gdn && !p.swap && !(e && atoi(e) == 0)) ? 1 : 0;
+  }
   // gamma (32 KB, GDN only) + one tile (32 KB; 64 KB for f32 outputs) that holds the squares for the gamma contraction and
   // then stages the output
   // bf16-pair outputs of layers with a short mainloop (<= 96 tap-chunks per tile: the 1x1 stack, the 3x3 layers, the masked
@@ -1777,7 +1888,7 @@ static int launch_tc(const nic_conv_desc* d, const TapTable& tt, const void* x, 
   const char* st2 = getenv("NIC_TC_STAGE2");
   const bool st2_fits = 2 * p.slot_bytes + 4 * 128 * 128 + 4 * 128 * 128 + 1024 <= kMaxDynSmem;
   const bool st2_auto = p.swap && tapchunks <= 96 && tt.ntaps > tt.nphases;
-  p.stage2 = (p.split_out && p.tma_out == 1 && !gdn && st2_fits &&
+  p.stage2 = (p.split_out && p.tma_out == 1 && !gdn && !p.epi_slices && st2_fits &&
               (st2 ? (atoi(st2) != 0 && (p.swap || tapchunks <= 96)) : st2_auto)) ? 1 : 0;
   const int stage_bytes = p.tma_out == 2 ? 4 * 128 * 128 : ((gdn || p.tma_out) ? (p.stage2 ? 4 : 2) * 128 * 128 : 0);
   const int gdn_bytes = (gdn ? 2 * 128 * 128 : 0) + stage_bytes;
@@ -1843,7 +1954,9 @@ static int launch_tc(const nic_conv_desc* d, const TapTable& tt, const void* x, 
   if (p.tma_out) {
     // the output tensor (all ctot channels), walked with the output stride of the phase decomposition
     const int on = flat ? 1 : d->n, oh = flat ? gh : d->h_out, ow = flat ? gw : d->w_out;
-    if (int rc = encode_nhwc(&map_o, y, on, oh, ow, ctot, kTileW, kTileH, tt.out_stride, p.tma_out == 2 ? 4 : 2)) return rc;
+    if (p.epi_slices) {       // one warp's slice: 32 channels x 8 x 4 pixels
+      if (int rc = encode_nhwc_c32(&map_o, y, on, oh, ow, ctot, kTileW, 4, tt.out_stride)) return rc;
+    } else if (int rc = encode_nhwc(&map_o, y, on, oh, ow, ctot, kTileW, kTileH, tt.out_stride, p.tma_out == 2 ? 4 : 2)) return rc;
   } else map_o = map_w;
 
   if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(conv_tc_kernel<false>), kMaxDynSmem)) return rc;

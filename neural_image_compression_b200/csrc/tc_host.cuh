@@ -16,7 +16,7 @@ int encode_2d(CUtensorMap* m, const void* base, uint64_t inner, uint64_t rows, u
 int encode_2d_ex(CUtensorMap* m, const void* base, int elem_bytes, uint64_t inner, uint64_t rows, uint32_t box_inner, uint32_t box_rows);
 int encode_nhwc(CUtensorMap* m, const void* base, int n, int h, int w, int c, int box_w, int box_h, int stride, int elem_bytes);   // bf16 / f32
 int encode_2d_c32(CUtensorMap* m, const void* base, uint64_t inner, uint64_t rows, uint32_t box_rows);   // bf16, 32-column SWIZZLE_64B boxes
-int encode_nhwc_c32(CUtensorMap* m, const void* base, int n, int h, int w, int c, int box_w, int box_h);   // bf16, SWIZZLE_64B
+int encode_nhwc_c32(CUtensorMap* m, const void* base, int n, int h, int w, int c, int box_w, int box_h, int stride = 1);   // bf16, SWIZZLE_64B
 int encode_image_patch(CUtensorMap* m, const void* base, int n, int c, int h, int w, int box_w, int box_h);              // f32 NCHW
 // one device int per process: the kernels' "a bounded wait expired" flag (nic_pipeline_status)
 int* status_word();

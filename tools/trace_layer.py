@@ -1,5 +1,8 @@
-"""Pipeline trace of conv_tc_kernel for one layer (GPU box):  python tools/trace_layer.py k2|d2|d3|k3|ep3|k2c|d2c [bf16|bf16x3]
-(k2c / d2c: the conv alone with a bias epilogue and f32 NHWC output, as the bf16x3 arm runs it before gdn_x3_kernel)"""
+"""Pipeline trace of conv_tc_kernel for one layer (GPU box):  python tools/trace_layer.py k2|d2|d3|k3|ep3|k2c|d2c|gs3 [bf16|bf16x3]
+(k2c / d2c: the conv alone with a bias epilogue and f32 NHWC output, as the bf16x3 arm runs it before gdn_x3_kernel;
+gs3: g_s layer 3's conv as the bf16x3 arm runs it before its IGDN - bias epilogue, bf16-pair output, CTA-pair form)
+Ends with a per-phase summary over every CTA that issues MMAs: mainloop (first A slot ready -> last MMA issued) against
+epilogue (accumulator ready -> last store issued) per tile, in SM clocks."""
 import ctypes as C, os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -30,6 +33,7 @@ cfg = {
     "k2p": (nn.Conv2d(128, 128, 5, 2, 2), EPI_BIAS, (256, 384), {}),      # pair (bf16x3) or bf16 output: the swapped orientation
     "d2p": (nn.ConvTranspose2d(128, 128, 5, 2, 2, output_padding=1), EPI_BIAS, (128, 192), {}),
     "d2c": (nn.ConvTranspose2d(128, 128, 5, 2, 2, output_padding=1), EPI_BIAS, (128, 192), dict(out_dtype=torch.float32)),
+    "gs3": (nn.ConvTranspose2d(128, 128, 5, 2, 2, output_padding=1), EPI_BIAS, (128, 192), {}),
 }[which]
 conv, epi, (h, w), kw = cfg
 conv = conv.to(dev)
@@ -69,3 +73,16 @@ for cta in (0, 77):
         a, b = live[1], live[-1]
         dclk, dns = int(t[cta, b][0]) - int(t[cta, a][0]), int(t[cta, b][15]) - int(t[cta, a][15])
         print(f"  SM clock during the kernel: {dclk / dns * 1000:.0f} MHz ({dclk} clk in {dns} ns, tiles {a}..{b})")
+if which != "l1":
+    # slot 7: the tile's phase (stamped by the MMA issuer); tile 0 of each CTA is left out (it starts on an idle pipeline)
+    import collections
+    acc = collections.defaultdict(lambda: [0, 0, 0])
+    for cta in range(148):
+        for i in range(1, 16):
+            row = t[cta, i]
+            if int(row[1]) and int(row[2]) and int(row[8]) and int(row[4]):
+                a = acc[int(row[7])]
+                a[0] += 1; a[1] += int(row[2]) - int(row[1]); a[2] += int(row[4]) - int(row[8])
+    for ph in sorted(acc):
+        n, ml, ep = acc[ph]
+        print(f"phase {ph}: {n:4d} tiles  mainloop {ml / n:8.0f} clk  epilogue {ep / n:8.0f} clk per tile")
