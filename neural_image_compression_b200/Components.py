@@ -135,8 +135,9 @@ class _Chain(nn.Module):
     precision = None
 
     def run_nhwc(self, x, n, h, w, arm, in_layout=None, tape=None, final_kw=None):
-        """tape: training.Tape that records every op for the backward (training forward); final_kw: `out=` window arguments of
-        the LAST conv (h_s writes psi straight into the concat buffer of the entropy-parameter stack)."""
+        """tape: training.Tape that records every op for the backward (training forward); final_kw: output arguments of the LAST
+        conv (`out=` window: h_s writes psi straight into the concat buffer of the entropy-parameter stack; out_layout: g_s writes
+        x_hat NCHW)."""
         layout = LAYOUT_NHWC if in_layout is None else in_layout
         mods, i = list(self.net), 0
         while i < len(mods):
@@ -148,7 +149,8 @@ class _Chain(nn.Module):
             # evaluation: a conv whose only consumer is the next conv hands its result over as a bf16 hi/lo pair (bf16x3 arm)
             pair = tape is None and isinstance(after, (nn.Conv2d, nn.ConvTranspose2d, L.TransposedDeconv3x3))
             if isinstance(m, L.TransposedDeconv3x3):
-                x, h, w = m.run_nhwc(x, n, h, w, arm, in_layout=layout, epilogue=EPI_LRELU if fuse else EPI_BIAS, tape=tape, pair_out=pair)
+                x, h, w = m.run_nhwc(x, n, h, w, arm, in_layout=layout, epilogue=EPI_LRELU if fuse else EPI_BIAS, tape=tape, pair_out=pair,
+                                    **kw)
             elif isinstance(m, L._Block):
                 x, h, w = m.run_nhwc(x, n, h, w, arm, in_layout=layout, tape=tape)
                 fuse = False

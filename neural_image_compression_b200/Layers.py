@@ -103,8 +103,8 @@ class TransposedDeconv3x3(_Block):
         super().__init__()
         self.deconv = nn.ConvTranspose2d(in_ch, out_ch, kernel_size=3, stride=upsample, padding=1, output_padding=upsample - 1)
 
-    def run_nhwc(self, x, n, h, w, arm, in_layout=LAYOUT_NHWC, epilogue=EPI_BIAS, tape=None, pair_out=False):
-        return _conv(arm, self.deconv, epilogue, x, n, h, w, in_layout=in_layout, tape=tape, pair_out=pair_out)
+    def run_nhwc(self, x, n, h, w, arm, in_layout=LAYOUT_NHWC, epilogue=EPI_BIAS, tape=None, pair_out=False, **out_kw):
+        return _conv(arm, self.deconv, epilogue, x, n, h, w, in_layout=in_layout, tape=tape, pair_out=pair_out, **out_kw)
 
 
 class ResidualBlockWithStride(_Block):

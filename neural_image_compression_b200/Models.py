@@ -19,7 +19,6 @@ the host):
 from __future__ import annotations
 
 import contextlib
-import functools
 import os
 from typing import Optional, Tuple
 
@@ -359,39 +358,16 @@ class HierarchicalMixtureResidual(nn.Module):
     def forward(self, x: torch.Tensor, training: bool = True, *, noise: Optional[Tuple[torch.Tensor, torch.Tensor]] = None,
                 lean: bool = False):
         check_input(x)
-        B, _, H, W = x.shape
         from . import training as T
         if training and torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
             # the training step: ONE autograd node over the hand-written backward (training.Tape walks the residual graphs)
             return T.train_forward(self, x, noise=noise, lean=lean)
-        arm, M, K = self.precision, self.M, self.K
-        hy, wy, hz, wz = H // 16, W // 16, H // 64, W // 64
-        x = x.contiguous().float()
-        with torch.cuda.device(x.device), torch.no_grad():
-            noise_z, noise_y = draw_noise(M, x, noise) if training else (None, None)
-            qmode = Q_NOISE if training else Q_ROUND
-            y_nhwc, _, _ = self.encoder.run_nhwc(x, B, H, W, arm, in_layout=LAYOUT_NCHW)
-            y, y_in, y_in_nhwc, _ = engine.latent_handoff(y_nhwc, qmode, noise_y, torch.float32)
-            z_nhwc, _, _ = self.hyper_encoder.run_nhwc(y_nhwc, B, hy, wy, arm)
-            z, z_in, z_in_nhwc, _ = engine.latent_handoff(z_nhwc, qmode, noise_z, torch.float32)
-            psi, _, _ = self.hyper_decoder.run_nhwc(z_in_nhwc, B, hz, wz, arm)
-            combined = torch.empty((B, hy, wy, 4 * M), dtype=torch.float32, device=x.device)
-            combined[..., 2 * M:] = psi                      # torch.cat([phi, psi]) of Models.py:171: phi is written in place below
-            masked = self.context_model.masked
-            masked.apply_mask_()
-            T.conv_forward(arm, masked, engine.EPI_BIAS, y_in_nhwc, B, hy, wy, out=combined, out_c_total=4 * M, out_c_offset=0,
-                           mask_a=masked._op.mask_a)
-            ep = self.entropy_parameters.ops
-            a = T.conv_forward(arm, ep[0].conv, ep[0].epilogue, combined, B, hy, wy)
-            a = T.conv_forward(arm, ep[1].conv, ep[1].epilogue, a, B, hy, wy)
-            raw = T.conv_forward(arm, ep[2].conv, ep[2].epilogue, a, B, hy, wy, out_layout=LAYOUT_NCHW)
-            T.forget_pairs()
-            ly = gm_likelihood(y_in, raw, M, K, Q_PASSTHRU, full=not lean, want_y_in=False)
-            _, p_z, logp_z, parts_z = self.factorized_entropy_model.likelihood(z_in, Q_PASSTHRU)
-            x_nhwc, _, _ = self.decoder.run_nhwc(y_in_nhwc, B, hy, wy, arm)
-            x_hat = x_nhwc.permute(0, 3, 1, 2).contiguous()
-        return single_head_outputs(x_hat, ly["logp"], logp_z, y, y_in, z, z_in, p_z, ly["p"], ly["partials"], parts_z,
-                                   *mixture_params(ly, K, lean), K=K, training=training)
+        # evaluation: the training forward's layer-by-layer form without tapes (training._forward_impl, record=False)
+        with torch.no_grad():
+            noise_z, noise_y = draw_noise(self.M, x, noise) if training else (None, None)
+            outs, _ = T._forward_impl(self, x.contiguous().float(), noise_z, noise_y, lean, qmode=Q_NOISE if training else Q_ROUND,
+                                      arm=self.precision, record=False)
+        return single_head_outputs(*outs, K=self.K, training=training)
 
 
 class ScalableImageCoding(nn.Module):
@@ -493,100 +469,24 @@ class ScalableImageCoding(nn.Module):
     def forward(self, x: torch.Tensor, training: bool = True, debug=False, *,
                 noise: Optional[Tuple[torch.Tensor, torch.Tensor]] = None):
         check_input(x)
-        B, _, H, W = x.shape
         if training and torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
             # the training call with autograd on: one autograd node over the layer-by-layer forward (training_scalable.py)
             from . import training_scalable as _ts
             return _ts.train_forward(self, x, noise=noise)
-        M, M1, M2, K = self.M, self.M1, self.M2, self.K
         if self.fused_pipeline:
             return self._forward_pairs(x, training, noise)
-        layer = functools.partial(self._layer, B=B)
-        x = x.contiguous().float()
-        hy, wy, hz, wz = H // 16, W // 16, H // 64, W // 64
-        with torch.cuda.device(x.device), torch.no_grad():
-            noise_z, noise_y = draw_noise(M, x, noise) if training else (None, None)
-            y, y_in, y_in_nhwc, z, z_in, z_in_nhwc = self._layer_analysis(x, Q_NOISE if training else Q_ROUND, noise_y, noise_z)
-            # psi once, into head 1's concat buffer [phi1 (2 M1) | psi (2 M)]; head 2's buffer gets a copy of the window
-            comb1 = torch.empty((B, hy, wy, 2 * M1 + 2 * M), dtype=torch.float32, device=x.device)
-            comb2 = torch.empty((B, hy, wy, 2 * M2 + 2 * M), dtype=torch.float32, device=x.device)
-            self._layer_h_s_into(z_in_nhwc, B, hz, wz, comb1, 2 * M1 + 2 * M, 2 * M1)
-            comb2[..., 2 * M2:] = comb1[..., 2 * M1:]
-            y1, y2 = torch.split(y_in, [M1, M2], dim=1)                   # Models.py:279 (views, as in the reference)
-            y1c, y2c = y1.contiguous(), y2.contiguous()
-            heads = []
-            for ctx, ep, comb, mi, yi_nhwc, yi in ((self.context_model_1, self.entropy_parameters_1, comb1, M1,
-                                                    y_in_nhwc[..., :M1].contiguous(), y1c),
-                                                   (self.context_model_2, self.entropy_parameters_2, comb2, M2,
-                                                    y_in_nhwc[..., M1:].contiguous(), y2c)):
-                ctx.masked.apply_mask_()
-                layer(ctx.masked._op, yi_nhwc, hy, wy, out=comb, out_c_total=comb.shape[-1], out_c_offset=0)
-                a = layer(ep.ops[0], comb, hy, wy)
-                a = layer(ep.ops[1], a, hy, wy)
-                raw = layer(ep.ops[2], a, hy, wy, out_layout=LAYOUT_NCHW)
-                heads.append(gm_likelihood(yi, raw, mi, K, Q_PASSTHRU, full=True, want_y_in=False))
-            _, p_z, logp_z, parts_z = self.factorized_entropy_model.likelihood(z_in, Q_PASSTHRU)
-            x_hat = self._layer_g_s(y_in_nhwc, B, hy, wy)
-        l1, l2 = heads
-        return two_head_outputs(x_hat, l1["logp"], l2["logp"], logp_z, y, y_in, z, z_in, p_z, l1["p"], l2["p"], l1["partials"],
-                                l2["partials"], parts_z, *mixture_params(l1, K), *mixture_params(l2, K), M1=M1, K=K, training=training)
-
-    # ---- the layer-by-layer path (fp32, and bf16x3 outside the fused pipeline's channel counts); the coder calls the same stages
+        # fp32, and bf16x3 outside the fused pipeline's channel counts: the training forward's layer-by-layer form without tapes
+        from . import training as T
+        with torch.no_grad():
+            noise_z, noise_y = draw_noise(self.M, x, noise) if training else (None, None)
+            outs, _ = T._forward_impl(self, x.contiguous().float(), noise_z, noise_y, False, qmode=Q_NOISE if training else Q_ROUND,
+                                      arm=self.precision, record=False)
+        return two_head_outputs(*outs, M1=self.M1, K=self.K, training=training)
 
     @property
     def fused_pipeline(self) -> bool:
-        """True when the eval forward runs _forward_pairs (bf16x3 at M = 128 / 192), else the layer-by-layer stages below."""
+        """True when the eval forward runs _forward_pairs (bf16x3 at M = 128 / 192), else training._forward_impl (record=False)."""
         return self.precision == "bf16x3" and self.M in (128, 192) and self.M1 % 64 == 0 and self.M2 % 64 == 0
-
-    def _layer(self, op, a, h, w, B, **kw):
-        """One conv (+ GDN / LeakyReLU) with f32 tensors at both ends."""
-        arm = self.precision
-        if arm == "fp32":
-            return op.run(a, B, h, w, "fp32", **kw)
-        from . import training as T
-        u = T.conv_forward(arm, op.conv, engine.EPI_BIAS if op.gdn is not None else op.epilogue, a, B, h, w, mask_a=op.mask_a, **kw)
-        if op.gdn is not None:
-            ho, wo = engine.conv_out_hw(op.conv, h, w)
-            u = T.gdn_forward(arm, op.gdn, u, B, ho, wo)[0]
-        T.forget_pairs()                     # the split copies are per layer here (the training step keeps them for its backward)
-        return u
-
-    def _layer_analysis(self, x, qmode, noise_y, noise_z):
-        """g_a -> y hand-off -> h_a -> z hand-off: (y, y_in, y_in_nhwc, z, z_in, z_in_nhwc), the engine copies NHWC f32."""
-        B, _, H, W = x.shape
-        a, h, w, layout = x, H, W, LAYOUT_NCHW
-        for op in self.encoder.ops:
-            a = self._layer(op, a, h, w, B, in_layout=layout, out_layout=LAYOUT_NHWC)
-            h, w = engine.conv_out_hw(op.conv, h, w)
-            layout = LAYOUT_NHWC
-        y_nhwc = a
-        y, y_in, y_in_nhwc, _ = engine.latent_handoff(y_nhwc, qmode, noise_y, torch.float32)
-        for op in self.hyper_encoder.ops:
-            a = self._layer(op, a, h, w, B)
-            h, w = engine.conv_out_hw(op.conv, h, w)
-        z, z_in, z_in_nhwc, _ = engine.latent_handoff(a, qmode, noise_z, torch.float32)
-        return y, y_in, y_in_nhwc, z, z_in, z_in_nhwc
-
-    def _layer_h_s_into(self, z_in_nhwc, B, hz, wz, out, c_total, c_offset):
-        """h_s with its last conv writing psi into channels [c_offset, c_offset + 2M) of `out` (NHWC f32, c_total channels)."""
-        a, h, w = z_in_nhwc, hz, wz
-        hs = self.hyper_decoder.ops
-        for i, op in enumerate(hs):
-            if i == len(hs) - 1:
-                self._layer(op, a, h, w, B, out=out, out_c_total=c_total, out_c_offset=c_offset)
-            else:
-                a = self._layer(op, a, h, w, B)
-            h, w = engine.conv_out_hw(op.conv, h, w)
-
-    def _layer_g_s(self, y_in_nhwc, B, hy, wy):
-        """g_s: NHWC f32 symbols -> x_hat NCHW f32."""
-        a, h, w = y_in_nhwc, hy, wy
-        dec = self.decoder.ops
-        for i, op in enumerate(dec):
-            last = i == len(dec) - 1
-            a = self._layer(op, a, h, w, B, out_layout=LAYOUT_NCHW if last else LAYOUT_NHWC)
-            h, w = engine.conv_out_hw(op.conv, h, w)
-        return a
 
     def compress(self, x: torch.Tensor) -> dict:
         """x [B, 3, H, W] (H, W multiples of 64) -> {"strings": [y1_strings, y2_strings, z_strings], "shape": (hz, wz)}: one bytes

@@ -14,8 +14,8 @@ import struct
 import numpy as np
 import torch
 
-from . import _lib, engine
-from ._lib import CODEC_FACTORIZED, CODEC_GM, Q_PASSTHRU, Q_ROUND, CodecHead, check, current_stream, ptr
+from . import _lib, engine, training
+from ._lib import CODEC_FACTORIZED, CODEC_GM, LAYOUT_NCHW, Q_PASSTHRU, Q_ROUND, CodecHead, check, current_stream, ptr
 from .codec import (ARMS, SYMBOL_LIMIT, Y_LANES, Z_LANES, _encode, _symbol_codes, checksums, lanes, max_step_pixels, pack_string,
                     parse_string, step_tables, z_tables)
 from .codec import FORMAT_VERSION as JAH_FORMAT_VERSION
@@ -33,8 +33,8 @@ def check_supported(model):
 
 
 def _heads(model, base_only=False):
-    """(m, context model, entropy parameters) of the heads a call runs."""
-    heads = [(model.M1, model.context_model_1, model.entropy_parameters_1), (model.M2, model.context_model_2, model.entropy_parameters_2)]
+    """The entropy heads (training.heads: context model, entropy parameters, c0, c1) a call runs."""
+    heads = training.heads(model)
     return heads[:1] if base_only else heads
 
 
@@ -69,7 +69,8 @@ class ParamHeads:
         npar = 2 if model.K == 1 else 3 * model.K
         self.raw, self._keep = [], []
         self.args = (CodecHead * len(sym_nhwc))()
-        for a, ((m, ctx, ep), sym) in zip(self.args, zip(_heads(model), sym_nhwc)):
+        for a, ((ctx, ep, c0, c1), sym) in zip(self.args, zip(_heads(model), sym_nhwc)):
+            m = c1 - c0
             w = packed_head(ctx, ep)
             raw = torch.empty((B, npar * m, hy, wy), dtype=torch.float32, device=psi.device)
             work = torch.empty(n * (2 * m + 2 * HIDDEN), dtype=torch.float32, device=psi.device)
@@ -98,18 +99,22 @@ def psi_nhwc(model, z_nhwc: torch.Tensor) -> torch.Tensor:
             fused_h_s_into(model, z_eng, 1, hz, wz, "bf16x3", pair, 2 * M, 0, None)
             torch.add(pair[..., :2 * M].float(), pair[..., 2 * M:].float(), out=psi[b:b + 1])
         else:
-            model._layer_h_s_into(z_eng, 1, hz, wz, psi[b:b + 1], 2 * M, 0)
+            model.hyper_decoder.run_nhwc(z_eng, 1, hz, wz, model.precision,
+                                         final_kw=dict(out=psi[b:b + 1], out_c_total=2 * M, out_c_offset=0))
     return psi
 
 
 def _analysis(model, x):
     """The eval forward's symbols (y_in, z_in), NCHW f32, through the route the forward takes."""
+    B, _, H, W = x.shape
     if model.fused_pipeline:
-        B, _, H, W = x.shape
         _, y_in, _, y_src = fused_g_a(model, x, False, None, "bf16x3", "bf16x3")
         _, z_in, _ = fused_h_a(model, y_src, B, H // 16, W // 16, False, None, "bf16x3", "bf16x3")
         return y_in, z_in
-    _, y_in, _, _, z_in, _ = model._layer_analysis(x, Q_ROUND, None, None)
+    y_nhwc, _, _ = model.encoder.run_nhwc(x, B, H, W, model.precision, in_layout=LAYOUT_NCHW)
+    _, y_in, _, _ = engine.latent_handoff(y_nhwc, Q_ROUND, None, torch.float32)
+    z_nhwc, _, _ = model.hyper_encoder.run_nhwc(y_nhwc, B, H // 16, W // 16, model.precision)
+    _, z_in, _, _ = engine.latent_handoff(z_nhwc, Q_ROUND, None, torch.float32)
     return y_in, z_in
 
 
@@ -124,7 +129,7 @@ def compress(model, x: torch.Tensor) -> dict:
     B, _, H, W = x.shape
     M, M1, K = model.M, model.M1, model.K
     hy, wy, hz, wz = H // 16, W // 16, H // 64, W // 64
-    ln = [lanes(Y_LANES, m) for m, _, _ in _heads(model)] + [lanes(Z_LANES, M)]
+    ln = [lanes(Y_LANES, c1 - c0) for _, _, c0, c1 in _heads(model)] + [lanes(Z_LANES, M)]
     with torch.cuda.device(x.device), torch.no_grad():
         y_in, z_in = _analysis(model, x.contiguous().float())
         big = torch.maximum(y_in.abs().amax(), z_in.abs().amax())
@@ -194,7 +199,7 @@ def _parse_all(model, strings, shape, base_only):
         raise ValueError(f"need as many strings per layer as images (>= 1); got {[len(s) for s in layers]}")
     if not isinstance(shape, (list, tuple)) or len(shape) != 2 or any(int(v) != v or v < 1 for v in shape):
         raise ValueError(f"shape must be (hz, wz) with positive ints, got {shape!r}")
-    ln = [lanes(Z_LANES, model.M)] + [lanes(Y_LANES, m) for m, _, _ in _heads(model, base_only)]
+    ln = [lanes(Z_LANES, model.M)] + [lanes(Y_LANES, c1 - c0) for _, _, c0, c1 in _heads(model, base_only)]
     lane_tabs, base, enh = [[] for _ in layers], [], []
     for b in range(len(zs)):
         hdr, offs, words = parse_z(zs[b], model, ln[0], b)
@@ -245,7 +250,7 @@ def decompress(model, strings, shape, base_only: bool = False) -> dict:
         z_hat = z_nhwc.permute(0, 3, 1, 2).contiguous()
         psi = psi_nhwc(model, z_nhwc)
         # y1 (and y2): one wavefront step at a time, both heads' parameters in one launch per layer; no host synchronisation
-        ms = [m for m, _, _ in _heads(model, base_only)]
+        ms = [c1 - c0 for _, _, c0, c1 in _heads(model, base_only)]
         y_nhwc = [torch.zeros((B, hy, wy, m), dtype=torch.float32, device=dev) for m in ms]
         heads = ParamHeads(model, y_nhwc, psi, all_pixels=False)
         tabs = [None] * len(ms)
@@ -264,7 +269,8 @@ def decompress(model, strings, shape, base_only: bool = False) -> dict:
             fused = model.fused_pipeline
             _, y_hat, y_eng, _ = engine.latent_handoff(torch.cat(y_nhwc, dim=-1).contiguous(), Q_PASSTHRU, None,
                                                        "bf16x2" if fused else torch.float32)
-            x_hat = fused_g_s(model, y_eng, B, hy, wy, "bf16x3") if fused else model._layer_g_s(y_eng, B, hy, wy)
+            x_hat = fused_g_s(model, y_eng, B, hy, wy, "bf16x3") if fused else \
+                model.decoder.run_nhwc(y_eng, B, hy, wy, model.precision, final_kw=dict(out_layout=LAYOUT_NCHW))[0]
             out = {"x_hat": x_hat, "y_hat": y_hat, "y1_hat": y_parts[0], "y2_hat": y_parts[1], "z_hat": z_hat}
         bad = (torch.cat(got) != want).cpu().numpy().reshape(len(got), B)
     for layer, flags in zip(("base layer (y1 and z)", "enhancement layer (y2)"), bad):

@@ -5,8 +5,9 @@ The reference has no backward code of its own: its gradients are what torch auto
 RateDistortionLoss.py:5-49.  Here the whole model is ONE autograd node (``_TrainForward``): its forward (``_forward_impl``) runs
 layer by layer with fp32 NHWC tensors in between, every transform (g_a, g_s, h_a, h_s; the 5x5 chains and the 3x3 residual
 graphs alike) recording its ops and their tensors on a ``Tape``; its backward (``_backward_impl``) walks each transform's tape in
-reverse (``Tape.backward``) around the hand-written entropy side, a hand-scheduled chain of C-ABI calls (include/nic.h,
-"training step" section):
+reverse (``Tape.backward``) around the hand-written entropy side (``head_forward`` / ``head_backward`` per entropy head of
+``heads``: one for JointAutoregressiveHierarchical and HierarchicalMixtureResidual, two for ScalableImageCoding, whose loss and
+autograd wrapping live in training_scalable.py), a hand-scheduled chain of C-ABI calls (include/nic.h, "training step" section):
 
     data gradient of a conv      nic_conv_fwd with the mirrored descriptor (Conv2d <-> ConvTranspose2d, same weight tensor)
     weight / bias gradients      nic_conv_wgrad_tc (tcgen05, MN-major operands) / nic_conv_wgrad (fp32) - all 25 taps of the masked
@@ -44,6 +45,7 @@ import torch.nn as nn
 
 from . import _lib, engine
 from ._lib import (ConvDesc, DT_F32, EPI_BIAS, EPI_LRELU, LAYOUT_NCHW, LAYOUT_NHWC, PREC_FP32, Q_NOISE, Q_PASSTHRU, Q_ROUND, check, current_stream, ptr)
+from .EntropyModels import gm_likelihood
 from .Models import draw_noise, mixture_params, single_head_outputs
 
 PREC = "fp32"
@@ -482,29 +484,110 @@ _FACT_SLICES = (("matrices", 0, 0, 3), ("biases", 0, 3, 6), ("factors", 0, 6, 9)
                 ("matrices", 3, 39, 42), ("biases", 3, 42, 43))
 
 
+# ---- the entropy side: one or more (context model, entropy parameters) heads over channel ranges of y, and the factorized prior
+
+def heads(model) -> list:
+    """[(context model, entropy parameters, c0, c1)]: the entropy heads of a model, each over the channels [c0, c1) of y and the
+    shared hyper features psi.  One head over all of y (JointAutoregressiveHierarchical, HierarchicalMixtureResidual); the base
+    [0, M1) and the enhancement [M1, M) head of ScalableImageCoding."""
+    if hasattr(model, "M1"):
+        return [(model.context_model_1, model.entropy_parameters_1, 0, model.M1),
+                (model.context_model_2, model.entropy_parameters_2, model.M1, model.M)]
+    return [(model.context_model, model.entropy_parameters, 0, model.M)]
+
+
+def gm_likelihood_bwd(y: torch.Tensor, raw: torch.Tensor, g_logp: torch.Tensor, m: int, K: int):
+    """(d y, d raw), NCHW f32, of logp = log p(y | raw) (nic_gm_likelihood_bwd) for the upstream gradient g_logp."""
+    b, _, h, w = y.shape
+    dy, draw = torch.empty_like(y), torch.empty_like(raw)
+    check(_lib.load().nic_gm_likelihood_bwd(ptr(y), ptr(raw), ptr(g_logp), 0.0, b, m, h * w, K, ptr(dy), ptr(draw), current_stream()),
+          "nic_gm_likelihood_bwd")
+    return dy, draw
+
+
+def head_forward(arm: str, head, K: int, y_i: torch.Tensor, y_i_nhwc: torch.Tensor, comb: torch.Tensor, lean: bool):
+    """One entropy head on its symbols y_i (NCHW) / y_i_nhwc: the context conv writes phi into channels [0, 2 m) of the concat
+    buffer `comb` (NHWC, psi already at [2 m, 2 m + 2 M)), then the 1x1 stack and the likelihood.  -> (likelihood dict, the
+    tensors head_backward reads)."""
+    ctx, ep, c0, c1 = head
+    B, hy, wy, _ = y_i_nhwc.shape
+    ctx.masked.apply_mask_()
+    conv_forward(arm, ctx.masked, EPI_BIAS, y_i_nhwc, B, hy, wy, out=comb, out_c_total=comb.shape[-1], out_c_offset=0, mask_a=True)
+    ops = ep.ops
+    e1 = conv_forward(arm, ops[0].conv, ops[0].epilogue, comb, B, hy, wy)
+    e2 = conv_forward(arm, ops[1].conv, ops[1].epilogue, e1, B, hy, wy)
+    raw = conv_forward(arm, ops[2].conv, ops[2].epilogue, e2, B, hy, wy, out_layout=LAYOUT_NCHW)
+    ly = gm_likelihood(y_i, raw, c1 - c0, K, Q_PASSTHRU, full=not lean, want_y_in=False)
+    return ly, dict(comb=comb, e1=e1, e2=e2, raw=raw, y_i=y_i, y_i_nhwc=y_i_nhwc)
+
+
+def head_backward(arm: str, head, K: int, st: dict, g_logp: torch.Tensor, put, wgrad):
+    """Backward of head_forward from the gradient of the head's logp: -> (gradient of y_i, NHWC; gradient of psi, NHWC).
+    Parameter gradients go to put(param, grad); wgrad = conv_wgrad or its side-stream form (as in Tape.backward)."""
+    ctx, ep, c0, c1 = head
+    m = c1 - c0
+    B, hy, wy, _ = st["y_i_nhwc"].shape
+    dy_lik, draw = gm_likelihood_bwd(st["y_i"], st["raw"], g_logp.contiguous().float(), m, K)
+    d_y = to_nhwc(dy_lik)
+    g = to_nhwc(draw)
+    ops = ep.ops
+    for i, (op, a) in reversed(list(enumerate(zip(ops, (st["comb"], st["e1"], st["e2"]))))):
+        dw, db = wgrad(op.conv, a, g, B, hy, wy, LAYOUT_NHWC, LAYOUT_NHWC, arm=arm)
+        put(op.conv.weight, dw); put(op.conv.bias, db)
+        if i > 0:
+            g = lrelu_bwd_(conv_dgrad(op.conv, g, B, hy, wy, arm=arm), a)
+    # the first 1x1 conv reads [phi | psi]: its data gradient splits along its input channels
+    w0 = ops[0].conv.weight.detach()
+    d_phi = conv_dgrad(ops[0].conv, g, B, hy, wy, weight=w0[:, :2 * m].contiguous(), c_in=2 * m, arm=arm)
+    d_psi = conv_dgrad(ops[0].conv, g, B, hy, wy, weight=w0[:, 2 * m:].contiguous(), c_in=w0.shape[1] - 2 * m, arm=arm)
+    dw, db = wgrad(ctx.masked, st["y_i_nhwc"], d_phi, B, hy, wy, LAYOUT_NHWC, LAYOUT_NHWC, arm=arm)
+    put(ctx.masked.weight, dw); put(ctx.masked.bias, db)
+    return add_(d_y, conv_dgrad(ctx.masked, d_phi, B, hy, wy, arm=arm)), d_psi
+
+
+def factorized_bwd(fe: nn.Module, z_in: torch.Tensor, fparams: torch.Tensor, g_logp: torch.Tensor, put) -> torch.Tensor:
+    """Gradient (NCHW) of z_in from the gradient of the factorized prior's logp; the parameter gradients go to put."""
+    b, m, h, w = z_in.shape
+    dz = torch.empty_like(z_in)
+    dpar = _f32((m, 43), z_in.device)
+    check(_lib.load().nic_factorized_likelihood_bwd(ptr(z_in), ptr(fparams), ptr(g_logp.contiguous().float()), 0.0, b, m, h * w,
+                                                    ptr(dz), ptr(dpar), current_stream()), "nic_factorized_likelihood_bwd")
+    for name, idx, lo, hi in _FACT_SLICES:
+        prm = getattr(fe, name)[idx]
+        put(prm, dpar[:, lo:hi].reshape(prm.shape).contiguous())
+    return dz
+
+
 # ---- the model as one autograd node ------------------------------------------------------------------------------
 
-def _forward_impl(model, x, noise_z, noise_y, lean, qmode: int = Q_NOISE, arm: Optional[str] = None):
-    """The layer-by-layer forward (fp32 NHWC tensors between layers, layer inputs kept): -> (outputs tuple, saved state S).
-    qmode = Q_NOISE is the training forward; Q_ROUND the evaluation forward of a model whose channel count the fused
-    pair-tensor pipeline is not built for (Models.py uses it for M != 128 on the bf16x3 arm)."""
+def _forward_impl(model, x, noise_z, noise_y, lean, qmode: int = Q_NOISE, arm: Optional[str] = None, record: bool = True):
+    """The layer-by-layer forward (fp32 NHWC tensors between layers) of a model with any number of entropy heads (`heads`)
+    -> (outputs, saved state S).  Outputs in the order single_head_outputs / two_head_outputs take them: x_hat, the heads' logp,
+    logp_z, y, y_in, z, z_in, p_z, the heads' p, the heads' partial sums, the partial sums of z, the heads' mixture_params.
+    qmode = Q_NOISE is the training forward; Q_ROUND the evaluation forward.
+    record=True (training, and JointAutoregressiveHierarchical's evaluation outside the fused pipeline's channel counts): every
+    transform records on a Tape and S keeps what _backward_impl reads; under a CUDA-graph capture g_s runs as a parallel branch.
+    record=False (evaluation of the residual family and of ScalableImageCoding outside its fused pipeline): no tapes, so the
+    transforms hand bf16 pairs between convs and drop their pair forms per layer; everything on the current stream (a per-layer
+    forget_pairs on one stream would free pair tensors another stream still reads); S is None."""
     engine.require_cuda(x, "x")
     dev = x.device
     B, _, H, W = x.shape
     M, K = model.M, model.K
     hy, wy, hz, wz = H // 16, W // 16, H // 64, W // 64
     arm = arm or train_precision(model)
-    S = {t: Tape(arm, B) for t in ("g_a", "g_s", "h_a", "h_s")}       # each transform's ops with the tensors its backward reads
+    hds = heads(model)
+    S = {t: Tape(arm, B) if record else None for t in ("g_a", "g_s", "h_a", "h_s")}    # each transform's ops and tensors
     with torch.cuda.device(dev):
         y_nhwc, _, _ = model.encoder.run_nhwc(x, B, H, W, arm, in_layout=LAYOUT_NCHW, tape=S["g_a"])
         y, y_in, y_in_nhwc, _ = engine.latent_handoff(y_nhwc, qmode, noise_y, torch.float32)
 
         def synthesis():
-            return model.decoder.run_nhwc(y_in_nhwc, B, hy, wy, arm, tape=S["g_s"])[0]        # the RGB layer writes NCHW
+            return model.decoder.run_nhwc(y_in_nhwc, B, hy, wy, arm, tape=S["g_s"], final_kw=dict(out_layout=LAYOUT_NCHW))[0]
         # g_s reads only y_in: it runs as its own branch (a second stream; a parallel branch of a captured graph) beside the
         # entropy path h_a -> h_s -> context -> entropy parameters -> likelihoods
         main = torch.cuda.current_stream(dev)
-        branch = _side_stream(dev, 1) if _overlap() else None
+        branch = _side_stream(dev, 1) if (record and _overlap()) else None
         if branch is not None:
             if arm == "bf16x3":
                 to_pair(y_in_nhwc)               # both branches consume the pair form: make it before the fork
@@ -514,41 +597,40 @@ def _forward_impl(model, x, noise_z, noise_y, lean, qmode: int = Q_NOISE, arm: O
         # h_a (reads the unquantised y)
         z_nhwc, _, _ = model.hyper_encoder.run_nhwc(y_nhwc, B, hy, wy, arm, tape=S["h_a"])
         z, z_in, z_in_nhwc, _ = engine.latent_handoff(z_nhwc, qmode, noise_z, torch.float32)
-        # h_s -> psi, context -> phi, both windows of `combined`
-        combined = _f32((B, hy, wy, 4 * M), dev)
+        # h_s writes psi into head 0's concat buffer [phi_0 (2 m_0) | psi (2 M)]; every other head's buffer gets a copy of it
+        combs = [_f32((B, hy, wy, 2 * (c1 - c0) + 2 * M), dev) for _, _, c0, c1 in hds]
+        m0 = hds[0][3] - hds[0][2]
         model.hyper_decoder.run_nhwc(z_in_nhwc, B, hz, wz, arm, tape=S["h_s"],
-                                     final_kw=dict(out=combined, out_c_total=4 * M, out_c_offset=2 * M))
-        masked = model.context_model.masked
-        masked.apply_mask_()
-        conv_forward(arm, masked, EPI_BIAS, y_in_nhwc, B, hy, wy, out=combined, out_c_total=4 * M, out_c_offset=0, mask_a=True)
-        ep = model.entropy_parameters.ops
-        e1 = conv_forward(arm, ep[0].conv, ep[0].epilogue, combined, B, hy, wy)
-        e2 = conv_forward(arm, ep[1].conv, ep[1].epilogue, e1, B, hy, wy)
-        raw = conv_forward(arm, ep[2].conv, ep[2].epilogue, e2, B, hy, wy, out_layout=LAYOUT_NCHW)
-        from .EntropyModels import gm_likelihood
-        ly = gm_likelihood(y_in, raw, M, K, Q_PASSTHRU, full=not lean, want_y_in=False)
+                                     final_kw=dict(out=combs[0], out_c_total=combs[0].shape[-1], out_c_offset=2 * m0))
+        for (_, _, c0, c1), comb in zip(hds[1:], combs[1:]):
+            comb[..., 2 * (c1 - c0):] = combs[0][..., 2 * m0:]
+        lys, states = [], []
+        for head, comb in zip(hds, combs):
+            c0, c1 = head[2], head[3]
+            ly, st = head_forward(arm, head, K, y_in[:, c0:c1].contiguous(), y_in_nhwc[..., c0:c1].contiguous(), comb, lean)
+            lys.append(ly)
+            states.append(st)
         _, p_z, logp_z, parts_z = model.factorized_entropy_model.likelihood(z_in, Q_PASSTHRU)
         if branch is not None:
             main.wait_stream(branch)
         else:
             x_hat = synthesis()
-    S["arm"] = arm
-    S.update(combined=combined, e1=e1, e2=e2, raw=raw, y_in=y_in, y_in_nhwc=y_in_nhwc, z_in=z_in, z_in_nhwc=z_in_nhwc, y_nhwc=y_nhwc,
+    outs = (x_hat, *[ly["logp"] for ly in lys], logp_z, y, y_in, z, z_in, p_z, *[ly["p"] for ly in lys],
+            *[ly["partials"] for ly in lys], parts_z, *[t for ly in lys for t in mixture_params(ly, K, lean)])
+    if not record:
+        return outs, None
+    S.update(arm=arm, heads=states, y_in_nhwc=y_in_nhwc, z_in=z_in, z_in_nhwc=z_in_nhwc, y_nhwc=y_nhwc,
              fparams=model.factorized_entropy_model.packed(), shape=(B, H, W))
-    nd = [y, y_in, z, z_in, p_z, ly["p"], ly["partials"], parts_z] + mixture_params(ly, K, lean)
-    return (x_hat, ly["logp"], logp_z, *nd), S
+    return outs, S
 
 
-def _backward_impl(model, S, g_xhat, g_logp_y, g_logp_z, partial_hook=None) -> Dict[int, torch.Tensor]:
-    """The hand-scheduled backward: {id(parameter): gradient} from the gradients of x_hat / logp_y / logp_z (any may be None).
+def _backward_impl(model, S, g_xhat, g_logp_heads, g_logp_z, partial_hook=None) -> Dict[int, torch.Tensor]:
+    """The hand-scheduled backward: {id(parameter): gradient} from the gradients of x_hat / of every head's logp (a list in
+    `heads` order) / of logp_z (x_hat's and logp_z's may be None; the entropy heads are skipped unless every head has one).
     partial_hook(grads, streams): called once, when every gradient except g_a's has been ENQUEUED (g_s, the entropy path and h_a
     are done, on `streams`) and only g_a's backward remains - the data-parallel trainer starts the all-reduce of those ~24 of the
     29 MB there, so that it overlaps g_a's backward; the hook may replace entries of `grads` (views of its reduced bucket)."""
-    lib = _lib.load()
-    B, H, W = S["shape"]
-    M, K = model.M, model.K
-    hy, wy, hz, wz = H // 16, W // 16, H // 64, W // 64
-    dev = S["raw"].device
+    dev = S["y_in_nhwc"].device
     arm = S["arm"]
     grads: Dict[int, torch.Tensor] = {}
 
@@ -583,43 +665,22 @@ def _backward_impl(model, S, g_xhat, g_logp_y, g_logp_z, partial_hook=None) -> D
             with (torch.cuda.stream(branch) if branch is not None else contextlib.nullcontext()):
                 d_yin_gs = S["g_s"].backward(g_xhat.contiguous().float(), LAYOUT_NCHW, put, conv_wgrad_async, root=S["y_in_nhwc"],
                                              side=side, keep=keep)
-        # ---- p_y: likelihood, entropy parameters, context model, h_s --------------------------------------------
+        # ---- p_y: every head's likelihood, entropy parameters and context model; h_s --------------------------------
+        # the y gradient of the entropy path is the channel concatenation of the heads', the psi gradient their sum
         d_zin = None
-        if g_logp_y is not None:
-            gl = g_logp_y.contiguous().float()
-            dy_lik = torch.empty_like(S["y_in"])
-            draw = torch.empty_like(S["raw"])
-            check(lib.nic_gm_likelihood_bwd(ptr(S["y_in"]), ptr(S["raw"]), ptr(gl), 0.0, B, M, hy * wy, K, ptr(dy_lik), ptr(draw),
-                                            current_stream()), "nic_gm_likelihood_bwd")
-            d_yin = to_nhwc(dy_lik, accumulate_into=d_yin)
-            g = to_nhwc(draw)
-            ep = model.entropy_parameters.ops
-            for i, (op, a) in reversed(list(enumerate(zip(ep, (S["combined"], S["e1"], S["e2"]))))):
-                dw, db = conv_wgrad_async(op.conv, a, g, B, hy, wy, LAYOUT_NHWC, LAYOUT_NHWC, arm=arm)
-                put(op.conv.weight, dw); put(op.conv.bias, db)
-                if i > 0:
-                    g = lrelu_bwd_(conv_dgrad(op.conv, g, B, hy, wy, arm=arm), a)
-            w0 = ep[0].conv.weight.detach()
-            d_phi = conv_dgrad(ep[0].conv, g, B, hy, wy, weight=w0[:, :2 * M].contiguous(), c_in=2 * M, arm=arm)
-            d_psi = conv_dgrad(ep[0].conv, g, B, hy, wy, weight=w0[:, 2 * M:].contiguous(), c_in=2 * M, arm=arm)
-            masked = model.context_model.masked
-            dw, db = conv_wgrad_async(masked, S["y_in_nhwc"], d_phi, B, hy, wy, LAYOUT_NHWC, LAYOUT_NHWC, arm=arm)
-            put(masked.weight, dw); put(masked.bias, db)
-            d_yin = add_(d_yin, conv_dgrad(masked, d_phi, B, hy, wy, arm=arm))
-            del g                                                # the concat buffer's gradient is consumed: free it before h_s's backward
+        if all(g is not None for g in g_logp_heads):
+            d_ys, d_psi = [], None
+            for head, st, gl in zip(heads(model), S["heads"], g_logp_heads):
+                d_y, d_psi_i = head_backward(arm, head, model.K, st, gl, put, conv_wgrad_async)
+                d_ys.append(d_y)
+                d_psi = d_psi_i if d_psi is None else add_(d_psi, d_psi_i)
+            d_yin = d_ys[0] if len(d_ys) == 1 else torch.cat(d_ys, dim=-1)
+            del d_ys
             d_zin = S["h_s"].backward(d_psi, LAYOUT_NHWC, put, conv_wgrad_async, root=S["z_in_nhwc"], side=side, keep=keep)
         # ---- p_z ----------------------------------------------------------------------------------------------------
         if g_logp_z is not None:
-            gl = g_logp_z.contiguous().float()
-            fe = model.factorized_entropy_model
-            dz_fac = torch.empty_like(S["z_in"])
-            dpar = _f32((M, 43), dev)
-            check(lib.nic_factorized_likelihood_bwd(ptr(S["z_in"]), ptr(S["fparams"]), ptr(gl), 0.0, B, M, hz * wz, ptr(dz_fac),
-                                                    ptr(dpar), current_stream()), "nic_factorized_likelihood_bwd")
-            for name, idx, lo, hi in _FACT_SLICES:
-                prm = getattr(fe, name)[idx]
-                put(prm, dpar[:, lo:hi].reshape(prm.shape).contiguous())
-            d_zin = to_nhwc(dz_fac, accumulate_into=d_zin)
+            dz = factorized_bwd(model.factorized_entropy_model, S["z_in"], S["fparams"], g_logp_z, put)
+            d_zin = to_nhwc(dz, accumulate_into=d_zin)
         # ---- h_a (z_in = z + noise: the gradient passes unchanged) --------------------------------------------------
         dy = d_yin
         if d_zin is not None:
@@ -659,7 +720,7 @@ class _TrainForward(torch.autograd.Function):
         if S is None:
             raise RuntimeError("the saved activations of this forward pass were released by its first backward(); run the forward "
                                "again (retain_graph=True is not supported by the hand-written backward)")
-        grads = _backward_impl(model, S, g_xhat, g_logp_y, g_logp_z)
+        grads = _backward_impl(model, S, g_xhat, [g_logp_y], g_logp_z)
         ctx.S = None
         params = [p for _, p in model.named_parameters()]
         return (None, None, None, None, None, *[grads.get(id(p)) for p in params])
@@ -686,7 +747,7 @@ def step_gradients(model, x: torch.Tensor, lambda_rd: float, noise=None, partial
     with torch.cuda.device(x.device):
         check(_lib.load().nic_sse_bwd(ptr(x_hat), ptr(x), x.numel(), float(lambda_rd) * 65025.0 * 2.0 / x.numel(), ptr(gx), current_stream()),
               "nic_sse_bwd")
-    grads = _backward_impl(model, S, gx, gl.expand(logp_y.shape), gl.expand(logp_z.shape), partial_hook=partial_hook)
+    grads = _backward_impl(model, S, gx, [gl.expand(logp_y.shape)], gl.expand(logp_z.shape), partial_hook=partial_hook)
     for p in model.parameters():
         g = grads.get(id(p))
         if g is not None:

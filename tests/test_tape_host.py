@@ -1,6 +1,7 @@
 """CPU (no GPU): the host logic of the training step's transforms - ``training.Tape`` and the ``tape=`` plumbing of Layers.py /
-Components._Transform (5x5) / Components._Chain (3x3) - with torch stand-ins for the C-ABI calls (conv forward / weight gradient /
-adjoint conv, GDN forward / backward, LeakyReLU backward, add).  What is checked is the BOOKKEEPING: every op of the transforms is
+Components._Transform (5x5) / Components._Chain (3x3) - and of its entropy heads (``training.head_forward`` / ``head_backward``),
+with torch stand-ins for the C-ABI calls (conv forward / weight gradient / adjoint conv, GDN forward / backward, LeakyReLU backward,
+add, layout conversion, Gaussian(-mixture) likelihood forward / backward).  What is checked is the BOOKKEEPING: every op of the transforms is
 recorded once, gradients of tensors with two consumers (the block input feeding the main path and the skip) are summed, the gradient
 of the transform's input comes back, and every parameter gets its gradient - against torch autograd over the oracle's restatement
 of the same transforms (oracle/forward.py: analysis / synthesis / hyper_* and their _3x3 forms, pinned to the reference's own
@@ -59,9 +60,10 @@ def torch_backend(monkeypatch):
             return torch.autograd.grad(y, (wt, b), go)
 
     def conv_dgrad(conv, g, n, h_in, w_in, g_layout=NHWC, weight=None, c_in=None, arm="fp32"):
-        x = torch.zeros(n, conv.in_channels, h_in, w_in, dtype=torch.float64, requires_grad=True)
+        # weight / c_in: a slice of the layer's input channels (the [phi | psi] split of the first entropy-parameter conv)
+        x = torch.zeros(n, c_in or conv.in_channels, h_in, w_in, dtype=torch.float64, requires_grad=True)
         with torch.enable_grad():
-            y = _fconv(conv, x, conv.weight.detach().double(), conv.bias.detach().double())
+            y = _fconv(conv, x, (conv.weight if weight is None else weight).detach().double(), None)
             return torch.autograd.grad(y, x, _nchw(g, g_layout).double())[0].permute(0, 2, 3, 1).contiguous()
 
     def gdn_forward(arm, gdn, u, n, h, w):
@@ -81,8 +83,12 @@ def torch_backend(monkeypatch):
 
     def add_(dst, src):
         return dst.add_(src)
+
+    def to_nhwc(t, accumulate_into=None):
+        t = t.permute(0, 2, 3, 1)
+        return t.contiguous() if accumulate_into is None else accumulate_into.add_(t)
     for name, fn in dict(conv_forward=conv_forward, conv_wgrad=conv_wgrad, conv_dgrad=conv_dgrad, gdn_forward=gdn_forward, gdn_bwd=gdn_bwd,
-                         lrelu_bwd_=lrelu_bwd_, add_=add_).items():
+                         lrelu_bwd_=lrelu_bwd_, add_=add_, to_nhwc=to_nhwc).items():
         monkeypatch.setattr(T, name, fn)
     return T
 
@@ -170,3 +176,77 @@ def test_chain_writes_its_last_conv_into_a_channel_window(torch_backend):
         g = torch.randn(n, ho, wo, 2 * M, dtype=torch.float64)
         gx = tape.backward(g, NHWC, lambda p, v: grads.__setitem__(id(p), v), T.conv_wgrad, root=x)
         assert gx.shape == x.shape and len(grads) == len(list(mod.parameters())), cls.__name__
+
+
+@pytest.mark.parametrize("K", [1, 3])
+@pytest.mark.parametrize("scalable", [False, True])
+def test_entropy_heads_route_gradients(torch_backend, monkeypatch, scalable, K):
+    """training.head_forward / head_backward over training.heads: one head over all of y (JointAutoregressiveHierarchical) or the
+    base + enhancement heads of ScalableImageCoding (M1 < M) over the shared psi.  Every context / entropy-parameter gradient, the
+    y gradient (the heads' channel concatenation) and the psi gradient (the heads' sum) against autograd over oracle.forward.context
+    -> entropy_parameters_raw -> conditional_likelihood."""
+    from neural_image_compression_b200 import Models
+    T = torch_backend
+
+    def lik(y, raw, m, K_):
+        return O.conditional_likelihood(y, O.split_parameters(raw, m, K_), K_)
+
+    def gm_likelihood(y, raw, m, K_, qmode, full=True, want_y_in=True):
+        with torch.no_grad():
+            p = lik(y, raw, m, K_)
+        return {"p": p, "logp": torch.log(p), "partials": None}
+
+    def gm_likelihood_bwd(y, raw, g_logp, m, K_):
+        y, raw = y.detach().requires_grad_(), raw.detach().requires_grad_()
+        with torch.enable_grad():
+            return torch.autograd.grad(torch.log(lik(y, raw, m, K_)), (y, raw), g_logp)
+    monkeypatch.setattr(T, "gm_likelihood", gm_likelihood)
+    monkeypatch.setattr(T, "gm_likelihood_bwd", gm_likelihood_bwd)
+    M, n, h, w = 8, 2, 5, 6
+    torch.manual_seed(11)
+    model = Models.ScalableImageCoding(M, 3, K, precision="fp32") if scalable else Models.JointAutoregressiveHierarchical(M, K, precision="fp32")
+    heads = T.heads(model)
+    assert [(c0, c1) for _, _, c0, c1 in heads] == ([(0, 3), (3, M)] if scalable else [(0, M)])
+    prefixes = [("context_model_1", "entropy_parameters_1"), ("context_model_2", "entropy_parameters_2")] if scalable else \
+        [("context_model", "entropy_parameters")]
+    gen = torch.Generator().manual_seed(12)
+    y = torch.randint(-3, 4, (n, M, h, w), generator=gen).double()
+    psi = torch.randn(n, 2 * M, h, w, generator=gen, dtype=torch.float64)
+    g_logp = [torch.randn(n, c1 - c0, h, w, generator=gen).double() for _, _, c0, c1 in heads]       # exact in f32 (head_backward's cast)
+    # oracle: autograd over the restated heads
+    sd = {k: v.detach().double().clone().requires_grad_() for k, v in model.state_dict().items() if not k.endswith("mask")}
+    yr, psir = y.clone().requires_grad_(), psi.clone().requires_grad_()
+    prev, O.DIFFERENTIABLE = O.DIFFERENTIABLE, True
+    try:
+        total = 0
+        for (_, _, c0, c1), (cm, ep), g in zip(heads, prefixes, g_logp):
+            yi = yr[:, c0:c1]
+            raw = O.entropy_parameters_raw(sd, torch.cat([O.context(sd, yi, torch.float64, cm), psir], dim=1), torch.float64, ep)
+            total = total + (g * torch.log(lik(yi, raw, c1 - c0, K))).sum()
+        total.backward()
+    finally:
+        O.DIFFERENTIABLE = prev
+    # the package's heads
+    grads = {}
+
+    def put(p, g):
+        grads[id(p)] = g if id(p) not in grads else grads[id(p)] + g
+    y_nhwc, psi_nhwc = y.permute(0, 2, 3, 1).contiguous(), psi.permute(0, 2, 3, 1)
+    d_y, d_psi = [], None
+    for head, g in zip(heads, g_logp):
+        c0, c1 = head[2], head[3]
+        comb = torch.full((n, h, w, 2 * (c1 - c0) + 2 * M), float("nan"), dtype=torch.float64)
+        comb[..., 2 * (c1 - c0):] = psi_nhwc
+        ly, st = T.head_forward("fp32", head, K, y[:, c0:c1].contiguous(), y_nhwc[..., c0:c1].contiguous(), comb, False)
+        assert torch.allclose(ly["logp"], torch.log(lik(y[:, c0:c1], st["raw"], c1 - c0, K)))
+        dy_i, dpsi_i = T.head_backward("fp32", head, K, st, g, put, T.conv_wgrad)
+        d_y.append(dy_i)
+        d_psi = dpsi_i if d_psi is None else d_psi + dpsi_i
+    names = {id(p): k for k, p in model.named_parameters()}
+    want = [k for k in sd if k.startswith(tuple(cm + "." for pre in prefixes for cm in pre))]
+    assert sorted(names[i] for i in grads) == sorted(want)
+    for i, g in grads.items():
+        ref = sd[names[i]].grad
+        assert torch.allclose(g, ref, rtol=1e-8, atol=1e-10 * float(ref.abs().max() + 1)), names[i]
+    assert torch.allclose(torch.cat(d_y, dim=-1).permute(0, 3, 1, 2), yr.grad, rtol=1e-8, atol=1e-12)
+    assert torch.allclose(d_psi.permute(0, 3, 1, 2), psir.grad, rtol=1e-8, atol=1e-12)
