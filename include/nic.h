@@ -491,6 +491,15 @@ int nic_codec_encode(int32_t kind, const uint64_t* code, const float* sym, int32
 int nic_codec_decode(int32_t kind, const uint8_t* blob, const int64_t* lane_off, const int32_t* lane_words, uint32_t* state, int32_t* pos,
                      int32_t init, const uint32_t* cdf, const int32_t* lo, const int32_t* nbins, int32_t b, int32_t m, int32_t h, int32_t w,
                      int32_t lanes, int32_t t, float* out, void* stream);
+/*
+ * One wavefront step t of y in one launch (DESIGN.md section 11): one CTA per (image, lane) builds the lane's table rows of the step
+ * in shared memory from params (raw entropy parameters [b, (3K | 2) m, h, w], NCHW f32, k = K; only the step's pixels are read) with
+ * the function nic_codec_tables uses, and decodes them as nic_codec_decode(GM) does with the tables of nic_codec_tables(TABLES):
+ * the same symbols, states and read positions.  blob, lane_off, lane_words, state, pos, init and out as nic_codec_decode.
+ */
+int nic_codec_decode_step(const uint8_t* blob, const int64_t* lane_off, const int32_t* lane_words, uint32_t* state, int32_t* pos,
+                          int32_t init, const float* params, int32_t b, int32_t m, int32_t k, int32_t h, int32_t w, int32_t lanes, int32_t t,
+                          float* out, void* stream);
 /* out [b] = per image sum over the symbols (y [b, y_per_image] then z [b, z_per_image], NCHW f32) of a 32-bit mix of (index, value),
  * mod 2^32 */
 int nic_codec_checksum(const float* y, int64_t y_per_image, const float* z, int64_t z_per_image, int32_t b, uint32_t* out, void* stream);

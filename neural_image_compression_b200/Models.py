@@ -369,6 +369,19 @@ class HierarchicalMixtureResidual(nn.Module):
                                       arm=self.precision, record=False)
         return single_head_outputs(*outs, K=self.K, training=training)
 
+    def compress(self, x: torch.Tensor) -> dict:
+        """x [B, 3, H, W] (H, W multiples of 64) -> {"strings": [y_strings, z_strings], "shape": (hz, wz)}: one bytes object per
+        image in each list, coded with the eval-mode symbols (the forward's y_in / z_in).  Format: DESIGN.md section 11."""
+        from . import residual_codec
+        return residual_codec.compress(self, x)
+
+    def decompress(self, strings, shape) -> dict:
+        """strings / shape as compress returned them (any subset of the images, in any order) -> {"x_hat", "y_hat", "z_hat"},
+        NCHW f32; x_hat = g_s(y_hat), not clamped.  Raises ValueError on a string of another model, precision arm, M or K, on a
+        malformed string, or when an image's symbol checksum does not match (corrupted bytes, other weights)."""
+        from . import residual_codec
+        return residual_codec.decompress(self, strings, shape)
+
 
 class ScalableImageCoding(nn.Module):
     """The scalable-coding variant of /root/reference/Models.py:208-338: the JointAutoregressiveHierarchical trunk at M

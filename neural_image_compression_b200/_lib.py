@@ -109,6 +109,7 @@ SIGNATURES = {
     "nic_codec_tables": (C.c_int, [_i32, _i32, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp]),
     "nic_codec_encode": (C.c_int, [_i32, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i64, _vp, _vp, _vp]),
     "nic_codec_decode": (C.c_int, [_i32, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp]),
+    "nic_codec_decode_step": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i32, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp]),
     "nic_codec_checksum": (C.c_int, [_vp, _i64, _vp, _i64, _i32, _vp, _vp]),
     "nic_codec_params": (C.c_int, [C.POINTER(CodecHead), _i32, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _vp]),
 }

@@ -3,6 +3,7 @@
 //   codec_table_kernel    the ONE place where floats become integer frequencies (encoder and decoder both call it)
 //   codec_encode_kernel   one thread per (image, lane): the lane's symbols in reverse decode order -> 16-bit words
 //   codec_decode_kernel   one thread per (image, lane): one wavefront step of y, or all of z
+//   codec_decode_step_kernel  one CTA per (image, lane): one wavefront step of y, its tables built in shared memory (section 11)
 //   codec_checksum_kernel per-image 32-bit checksum of the y and z symbols
 //
 // rANS: 32-bit state in [2^16, 2^32), 16-bit renormalisation words, 16-bit probability precision.  A table row of one
@@ -11,6 +12,7 @@
 #include "codec_step.cuh"
 #include "common.cuh"
 #include "entropy_math.cuh"
+#include "tc_host.cuh"
 
 namespace nic {
 
@@ -282,6 +284,88 @@ codec_decode_kernel(int kind, const uint8_t* __restrict__ blob, const int64_t* _
   pos[g] = rd.pos;
 }
 
+// One wavefront step of y for one (image, lane) per CTA, tables in shared memory.  The lane's rows of step t, in its decode order
+// (pixels with i ascending, then channels c = lane, lane + lanes, ...), are built by the builder warps with the same element_code as
+// codec_table_kernel, kStepChunk rows at a time into one of two buffers; thread 0 decodes chunk k from one buffer while the
+// builders fill the other with chunk k + 1.  The decode arithmetic is codec_decode_kernel's, so symbols, states and read positions
+// are the same bits.  Every loop count is fixed by the shapes: a corrupted string only changes the values decoded.
+constexpr int kStepChunk = 64;                                 // rows per chunk: one per builder thread
+constexpr int kStepThreads = 32 + kStepChunk;                  // warp 0 decodes, warps 1 .. 2 build
+constexpr size_t kStepSmem = 2ull * kStepChunk * (kRow * sizeof(uint32_t) + 2 * sizeof(int32_t));
+
+__global__ void __launch_bounds__(kStepThreads)
+codec_decode_step_kernel(const uint8_t* __restrict__ blob, const int64_t* __restrict__ lane_off, const int32_t* __restrict__ lane_words,
+                         uint32_t* __restrict__ state, int32_t* __restrict__ pos, int init, const float* __restrict__ params, int m,
+                         int K, int h, int w, int lanes, int t, int i0, int cnt, float* __restrict__ out) {
+  extern __shared__ __align__(16) uint32_t s_step[];
+  uint32_t* s_cdf = s_step;                                    // [2][kStepChunk][kRow]
+  int32_t* s_lo = reinterpret_cast<int32_t*>(s_step + 2 * kStepChunk * kRow);
+  int32_t* s_n = s_lo + 2 * kStepChunk;
+  const int g = blockIdx.x, img = g / lanes, lane = g % lanes;
+  const int nc = (m - 1 - lane) / lanes + 1;                   // channels of this lane
+  const int rows = cnt * nc, chunks = (rows + kStepChunk - 1) / kStepChunk;
+  const long hw = static_cast<long>(h) * w;
+  const int np = K == 1 ? 2 : 3 * K;
+
+  auto build = [&](int k) {                                    // builder thread: row k * kStepChunk + (tid - 32) into buffer k & 1
+    const int b = threadIdx.x - 32, r = k * kStepChunk + b;
+    if (r >= rows) return;
+    const int p = r / nc, c = lane + (r - p * nc) * lanes, i = i0 + p;
+    const float* src = params + (static_cast<long>(img) * np * m + c) * hw + static_cast<long>(i) * w + (t - 3 * i);
+    float q[15];
+    for (int j = 0; j < np; ++j) q[j] = __ldg(src + static_cast<long>(j) * m * hw);
+    const int e = (k & 1) * kStepChunk + b;
+    element_code(NIC_CODEC_GM, K, q, kNoSymbol, s_cdf + e * kRow, s_lo + e, s_n + e);
+  };
+
+  uint32_t x = 0;
+  LaneReader rd{nullptr, 0, 0};
+  if (threadIdx.x == 0) {
+    const uint8_t* seg = blob + lane_off[g];
+    rd = LaneReader{seg + 4, lane_words[g], 0};
+    if (init) x = seg[0] | (seg[1] << 8) | (seg[2] << 16) | (static_cast<uint32_t>(seg[3]) << 24);
+    else { x = state[g]; rd.pos = pos[g]; }
+  }
+  if (threadIdx.x >= 32) build(0);
+  __syncthreads();
+  for (int k = 0; k < chunks; ++k) {
+    if (threadIdx.x >= 32) {
+      if (k + 1 < chunks) build(k + 1);
+    } else if (threadIdx.x == 0) {
+      const int r1 = min(rows, (k + 1) * kStepChunk);
+      for (int r = k * kStepChunk; r < r1; ++r) {
+        const int e = (k & 1) * kStepChunk + (r - k * kStepChunk);
+        const uint32_t* row = s_cdf + e * kRow;
+        const int n = s_n[e];
+        const uint32_t slot = x & (kProbScale - 1u);
+        int a = 0, z = n + 1;                                  // largest a with row[a] <= slot
+        while (z - a > 1) {
+          const int mid = (a + z) >> 1;
+          if (row[mid] <= slot) a = mid; else z = mid;
+        }
+        const uint32_t start = row[a], freq = row[a + 1] - start;
+        x = freq * (x >> kProbBits) + slot - start;
+        if (x < kRansL) x = (x << 16) | rd.next();
+        float v;
+        if (a == n) {
+          const uint32_t zlo = rans_bypass(x, rd);
+          const uint32_t zhi = rans_bypass(x, rd);
+          v = unzigzag(zlo | (zhi << 16));
+        } else {
+          v = static_cast<float>(s_lo[e] + a);
+        }
+        const int p = r / nc, c = lane + (r - p * nc) * lanes, i = i0 + p;
+        out[(static_cast<long>(img) * hw + static_cast<long>(i) * w + (t - 3 * i)) * m + c] = v;
+      }
+    }
+    __syncthreads();                                           // chunk k decoded, chunk k + 1 built
+  }
+  if (threadIdx.x == 0) {
+    state[g] = x;
+    pos[g] = rd.pos;
+  }
+}
+
 __device__ __forceinline__ uint32_t mix32(uint32_t idx, uint32_t v) {
   uint32_t hsh = idx * 0x9E3779B1u ^ (v + 0x7F4A7C15u);
   hsh ^= hsh >> 16; hsh *= 0x85EBCA6Bu;
@@ -352,6 +436,22 @@ int nic_codec_decode(int32_t kind, const uint8_t* blob, const int64_t* lane_off,
   codec_decode_kernel<<<(b * lanes + 63) / 64, 64, 0, as_stream(stream)>>>(kind, blob, lane_off, lane_words, state, pos, init, cdf, lo, nbins,
                                                                            b, m, h, w, lanes, t, out);
   return check_launch("codec_decode_kernel");
+}
+
+int nic_codec_decode_step(const uint8_t* blob, const int64_t* lane_off, const int32_t* lane_words, uint32_t* state, int32_t* pos,
+                          int32_t init, const float* params, int32_t b, int32_t m, int32_t k, int32_t h, int32_t w, int32_t lanes, int32_t t,
+                          float* out, void* stream) {
+  if (int rc = nic_check_device()) return rc;
+  if (b < 1 || m < 1 || k < 1 || k > 5 || h < 1 || w < 3 || lanes < 1 || lanes > m)
+    return fail(NIC_E_BADSHAPE, "codec_decode_step: b=%d m=%d k=%d h=%d w=%d lanes=%d", b, m, k, h, w, lanes);
+  if (t < 0 || t >= 3 * h + w - 3) return fail(NIC_E_BADSHAPE, "codec_decode_step: step %d of %d", t, 3 * h + w - 3);
+  if (!blob || !lane_off || !lane_words || !state || !pos || !params || !out) return fail(NIC_E_BADSHAPE, "codec_decode_step: null pointer");
+  if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(codec_decode_step_kernel), static_cast<int>(kStepSmem))) return rc;
+  int i0, cnt;
+  step_rows(t, h, w, i0, cnt);
+  codec_decode_step_kernel<<<b * lanes, kStepThreads, kStepSmem, as_stream(stream)>>>(blob, lane_off, lane_words, state, pos, init, params,
+                                                                                      m, k, h, w, lanes, t, i0, cnt, out);
+  return check_launch("codec_decode_step_kernel");
 }
 
 int nic_codec_checksum(const float* y, int64_t y_per_image, const float* z, int64_t z_per_image, int32_t b, uint32_t* out, void* stream) {

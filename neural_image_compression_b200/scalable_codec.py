@@ -91,7 +91,7 @@ def psi_nhwc(model, z_nhwc: torch.Tensor) -> torch.Tensor:
     B, hz, wz, M = z_nhwc.shape
     hy, wy = 4 * hz, 4 * wz
     psi = torch.empty((B, hy, wy, 2 * M), dtype=torch.float32, device=z_nhwc.device)
-    fused = model.fused_pipeline
+    fused = _fused(model)
     pair = torch.empty((1, hy, wy, 4 * M), dtype=torch.bfloat16, device=z_nhwc.device) if fused else None
     for b in range(B):
         _, _, z_eng, _ = engine.latent_handoff(z_nhwc[b:b + 1], Q_PASSTHRU, None, "bf16x2" if fused else torch.float32)
@@ -104,10 +104,16 @@ def psi_nhwc(model, z_nhwc: torch.Tensor) -> torch.Tensor:
     return psi
 
 
+def _fused(model) -> bool:
+    """True when the model's eval forward runs the fused pair-tensor pipeline; a model without one (HierarchicalMixtureResidual)
+    takes the transforms' run_nhwc route."""
+    return getattr(model, "fused_pipeline", False)
+
+
 def _analysis(model, x):
     """The eval forward's symbols (y_in, z_in), NCHW f32, through the route the forward takes."""
     B, _, H, W = x.shape
-    if model.fused_pipeline:
+    if _fused(model):
         _, y_in, _, y_src = fused_g_a(model, x, False, None, "bf16x3", "bf16x3")
         _, z_in, _ = fused_h_a(model, y_src, B, H // 16, W // 16, False, None, "bf16x3", "bf16x3")
         return y_in, z_in
@@ -116,6 +122,16 @@ def _analysis(model, x):
     z_nhwc, _, _ = model.hyper_encoder.run_nhwc(y_nhwc, B, H // 16, W // 16, model.precision)
     _, z_in, _, _ = engine.latent_handoff(z_nhwc, Q_ROUND, None, torch.float32)
     return y_in, z_in
+
+
+def synthesis(model, y_nhwc):
+    """Decoded y symbols NHWC f32 -> (y_hat NCHW, x_hat NCHW): g_s reads them through the same hand-off as the forward's."""
+    B, hy, wy, _ = y_nhwc.shape
+    fused = _fused(model)
+    _, y_hat, y_eng, _ = engine.latent_handoff(y_nhwc, Q_PASSTHRU, None, "bf16x2" if fused else torch.float32)
+    x_hat = fused_g_s(model, y_eng, B, hy, wy, "bf16x3") if fused else \
+        model.decoder.run_nhwc(y_eng, B, hy, wy, model.precision, final_kw=dict(out_layout=LAYOUT_NCHW))[0]
+    return y_hat, x_hat
 
 
 def _segments(words, count, n, b):
@@ -265,12 +281,7 @@ def decompress(model, strings, shape, base_only: bool = False) -> dict:
         got = [checksums(y, z_hat) for y in y_parts]
         out = {"y1_hat": y_parts[0], "z_hat": z_hat}
         if not base_only:
-            # g_s reads the symbols through the same hand-off as the forward's
-            fused = model.fused_pipeline
-            _, y_hat, y_eng, _ = engine.latent_handoff(torch.cat(y_nhwc, dim=-1).contiguous(), Q_PASSTHRU, None,
-                                                       "bf16x2" if fused else torch.float32)
-            x_hat = fused_g_s(model, y_eng, B, hy, wy, "bf16x3") if fused else \
-                model.decoder.run_nhwc(y_eng, B, hy, wy, model.precision, final_kw=dict(out_layout=LAYOUT_NCHW))[0]
+            y_hat, x_hat = synthesis(model, torch.cat(y_nhwc, dim=-1).contiguous())
             out = {"x_hat": x_hat, "y_hat": y_hat, "y1_hat": y_parts[0], "y2_hat": y_parts[1], "z_hat": z_hat}
         bad = (torch.cat(got) != want).cpu().numpy().reshape(len(got), B)
     for layer, flags in zip(("base layer (y1 and z)", "enhancement layer (y2)"), bad):
