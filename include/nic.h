@@ -8,6 +8,7 @@
  * reference Python call (file:line under /root/reference) whose arithmetic it replaces.
  * The Python host in neural_image_compression_b200/ binds these with ctypes
  * (see INTEGRATION.md for the stub a maintainer of the reference would add).
+ * 61 entries (tests/test_abi.py checks that the library exports every one).
  *
  * Conventions
  *   - extern "C", plain pointers and sizes, no torch / C++ types.
@@ -534,6 +535,15 @@ typedef struct nic_codec_head {
 } nic_codec_head;
 int nic_codec_params(const nic_codec_head* heads, int32_t n_heads, const float* psi, int32_t b, int32_t M, int32_t k, int32_t h,
                      int32_t w, int32_t t, void* stream);
+
+/*
+ * Image window of the any-size coders (DESIGN.md section 12), on contiguous f32 planes (planes = B x 3):
+ *   dst[p, i, j] = src[p, min(i, h_src - 1), min(j, w_src - 1)],  p < planes, i < h_dst, j < w_dst
+ * A larger dst is the encoder's edge-replicating pad (down and to the right), a smaller one the decoder's crop.  An exact copy;
+ * 64-bit offsets.  Any size < 1 or a null pointer: NIC_E_BADSHAPE, nothing launched.
+ */
+int nic_image_window(const float* src, int32_t planes, int32_t h_src, int32_t w_src, float* dst, int32_t h_dst, int32_t w_dst,
+                     void* stream);
 
 #ifdef __cplusplus
 }

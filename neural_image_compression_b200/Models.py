@@ -309,15 +309,17 @@ class JointAutoregressiveHierarchical(nn.Module):
                                    *mixture_params(ly, K, lean), K=K, training=training)
 
     def compress(self, x: torch.Tensor) -> dict:
-        """x [B, 3, H, W] (H, W multiples of 64) -> {"strings": [y_strings, z_strings], "shape": (hz, wz)}: one bytes object per
-        image in each list, coded with the eval-mode symbols (the forward's y_in / z_in).  Format: DESIGN.md section 9."""
+        """x [B, 3, H, W] (any H, W >= 1) -> {"strings": [y_strings, z_strings], "shape": (hz, wz)}: one bytes object per
+        image in each list, coded with the eval-mode symbols (the forward's y_in / z_in) of x padded by edge replication to
+        multiples of 64 (shape is the padded one).  Format: DESIGN.md sections 9 and 12."""
         from . import codec
         return codec.compress(self, x)
 
     def decompress(self, strings, shape) -> dict:
-        """strings / shape as compress returned them (any subset of the images, in any order) -> {"x_hat", "y_hat", "z_hat"},
-        NCHW f32; x_hat = g_s(y_hat), not clamped.  Raises ValueError on a string of another precision arm / M / K, on a malformed
-        string, or when an image's symbol checksum does not match (corrupted bytes, other weights)."""
+        """strings / shape as compress returned them (any subset of the images, in any order) -> {"x_hat", "y_hat", "z_hat"}, NCHW f32;
+        x_hat = g_s(y_hat) cropped to the image's size, not clamped; y_hat / z_hat at the padded latent shape.  Raises ValueError on a
+        string of another precision arm / M / K, on a malformed string or image size, or when an image's symbol checksum does not match
+        (corrupted bytes, other weights)."""
         from . import codec
         return codec.decompress(self, strings, shape)
 
@@ -370,15 +372,17 @@ class HierarchicalMixtureResidual(nn.Module):
         return single_head_outputs(*outs, K=self.K, training=training)
 
     def compress(self, x: torch.Tensor) -> dict:
-        """x [B, 3, H, W] (H, W multiples of 64) -> {"strings": [y_strings, z_strings], "shape": (hz, wz)}: one bytes object per
-        image in each list, coded with the eval-mode symbols (the forward's y_in / z_in).  Format: DESIGN.md section 11."""
+        """x [B, 3, H, W] (any H, W >= 1) -> {"strings": [y_strings, z_strings], "shape": (hz, wz)}: one bytes object per
+        image in each list, coded with the eval-mode symbols (the forward's y_in / z_in) of x padded by edge replication to
+        multiples of 64 (shape is the padded one).  Format: DESIGN.md sections 11 and 12."""
         from . import residual_codec
         return residual_codec.compress(self, x)
 
     def decompress(self, strings, shape) -> dict:
-        """strings / shape as compress returned them (any subset of the images, in any order) -> {"x_hat", "y_hat", "z_hat"},
-        NCHW f32; x_hat = g_s(y_hat), not clamped.  Raises ValueError on a string of another model, precision arm, M or K, on a
-        malformed string, or when an image's symbol checksum does not match (corrupted bytes, other weights)."""
+        """strings / shape as compress returned them (any subset of the images, in any order) -> {"x_hat", "y_hat", "z_hat"}, NCHW f32;
+        x_hat = g_s(y_hat) cropped to the image's size, not clamped; y_hat / z_hat at the padded latent shape.  Raises ValueError on a
+        string of another model, precision arm, M or K, on a malformed string or image size, or when an image's symbol checksum does not
+        match (corrupted bytes, other weights)."""
         from . import residual_codec
         return residual_codec.decompress(self, strings, shape)
 
@@ -502,16 +506,16 @@ class ScalableImageCoding(nn.Module):
         return self.precision == "bf16x3" and self.M in (128, 192) and self.M1 % 64 == 0 and self.M2 % 64 == 0
 
     def compress(self, x: torch.Tensor) -> dict:
-        """x [B, 3, H, W] (H, W multiples of 64) -> {"strings": [y1_strings, y2_strings, z_strings], "shape": (hz, wz)}: one bytes
-        object per image in each list, coded with the eval-mode symbols.  The base layer (y1 + z) decodes without the y2 strings.
-        Format: DESIGN.md section 10."""
+        """x [B, 3, H, W] (any H, W >= 1) -> {"strings": [y1_strings, y2_strings, z_strings], "shape": (hz, wz)}: one bytes
+        object per image in each list, coded with the eval-mode symbols of x padded by edge replication to multiples of 64 (shape
+        is the padded one).  The base layer (y1 + z) decodes without the y2 strings.  Format: DESIGN.md sections 10 and 12."""
         from . import scalable_codec
         return scalable_codec.compress(self, x)
 
     def decompress(self, strings, shape, base_only: bool = False) -> dict:
-        """strings / shape as compress returned them (any subset of the images, in any order) -> {"x_hat", "y_hat", "y1_hat",
-        "y2_hat", "z_hat"}, NCHW f32; x_hat = g_s(y_hat), not clamped.  base_only=True decodes z and y1 alone (strings[1] may be
-        None) and returns {"y1_hat", "z_hat"}.  Raises ValueError on a malformed string, a string of another model configuration,
-        or a checksum mismatch of a decoded layer (corrupted bytes, other weights)."""
+        """strings / shape as compress returned them (any subset of the images, in any order) -> {"x_hat", "y_hat", "y1_hat", "y2_hat",
+        "z_hat"}, NCHW f32; x_hat = g_s(y_hat) cropped to the image's size, not clamped; the latents at the padded shape.  base_only=True
+        decodes z and y1 alone (strings[1] may be None) and returns {"y1_hat", "z_hat"}.  Raises ValueError on a malformed string, a
+        string of another model configuration, or a checksum mismatch of a decoded layer (corrupted bytes, other weights)."""
         from . import scalable_codec
         return scalable_codec.decompress(self, strings, shape, base_only=base_only)

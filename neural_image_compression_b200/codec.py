@@ -17,7 +17,7 @@ import torch
 from . import _lib, engine
 from ._lib import (CODEC_FACTORIZED, CODEC_GM, CODEC_SYMBOL, CODEC_TABLES, CODEC_WINDOW, Q_PASSTHRU, check, current_stream,
                    ptr)
-from .Models import check_input, fused_g_a, fused_g_s, fused_h_a, fused_h_s_into, precision_arms
+from .Models import fused_g_a, fused_g_s, fused_h_a, fused_h_s_into, precision_arms
 
 FORMAT_VERSION = 1
 ARMS = ("fp32", "bf16", "mixed", "bf16x3")          # header byte 1
@@ -84,6 +84,112 @@ def parse_string(data: bytes, n_lanes: int, with_header: bool):
     if pos != len(data):
         raise ValueError(f"corrupt string: the lane lengths account for {pos} bytes, the string has {len(data)}")
     return hdr, offs, words
+
+
+# ---- images of any size (DESIGN.md section 12): the size extension the three formats share -------------------------------------
+
+SIZED = 0x80                                        # version-byte flag: the z string carries the image size
+SIZE = struct.Struct("<HH")                         # H, W, right after the model's header
+MAX_SIDE = 0xFFFF
+
+
+def mix32(idx: int, v: int) -> int:
+    """codec_checksum_kernel's 32-bit mix of (index, value) (csrc/codec.cu)."""
+    h = ((idx * 0x9E3779B1) & 0xFFFFFFFF) ^ ((v + 0x7F4A7C15) & 0xFFFFFFFF)
+    h ^= h >> 16
+    h = (h * 0x85EBCA6B) & 0xFFFFFFFF
+    h ^= h >> 13
+    h = (h * 0xC2B2AE35) & 0xFFFFFFFF
+    return h ^ (h >> 16)
+
+
+def salted(csum: int, size, sign: int = 1) -> int:
+    """A checksum field of a sized header: the symbol checksum plus mix32(0xFFFFFFFF, H << 16 | W), mod 2^32, so that a corrupted
+    size fails the decode even when it rounds up to the same latent shape.  size None: the checksum itself; sign -1 undoes it."""
+    if size is None:
+        return csum
+    return (csum + sign * mix32(0xFFFFFFFF, (size[0] << 16) | size[1])) & 0xFFFFFFFF
+
+
+def sized_header(header: bytes, size) -> bytes:
+    """The model's packed header as written for an image of `size` (None: an image whose sides are multiples of 64, today's
+    header): version byte | SIZED, then H, W."""
+    return header if size is None else bytes([header[0] | SIZED]) + header[1:] + SIZE.pack(*size)
+
+
+def version_name(v: int) -> str:
+    return f"{v & 0x7F}" + (" (sized)" if v & SIZED else "")
+
+
+def read_z_header(data, header: struct.Struct, version: int, shape, b: int):
+    """The header of one z string of any of the three formats -> (header tuple, image size (H, W), byte offset of the lane table).
+    An unsized string has size (64 hz, 64 wz).  ValueError, naming the image, on a header cut short, another version or a size that
+    is not the one spelling of an image of `shape`."""
+    if not isinstance(data, (bytes, bytearray)):
+        raise ValueError(f"image {b}: strings must be bytes, got {type(data).__name__}")
+    if len(data) < header.size:
+        raise ValueError(f"image {b}: truncated string: {len(data)} bytes, the header alone is {header.size}")
+    hdr = header.unpack_from(data, 0)
+    if hdr[0] & 0x7F != version:
+        raise ValueError(f"image {b}: unknown format version {version_name(hdr[0])} (this build reads version {version})")
+    hz, wz = int(shape[0]), int(shape[1])
+    if not hdr[0] & SIZED:
+        return hdr, (64 * hz, 64 * wz), header.size
+    if len(data) < header.size + SIZE.size:
+        raise ValueError(f"image {b}: truncated string: the size field is cut short ({len(data)} bytes)")
+    size = SIZE.unpack_from(data, header.size)
+    H, W = size
+    if H == 0 or W == 0:
+        raise ValueError(f"image {b}: the string gives an image size of {H}x{W}")
+    if H % 64 == 0 and W % 64 == 0:
+        raise ValueError(f"image {b}: a sized string for a {H}x{W} image (sides that are multiples of 64 are written unsized)")
+    if (-(-H // 64), -(-W // 64)) != (hz, wz):
+        raise ValueError(f"image {b}: a {H}x{W} image has a z latent of {-(-H // 64)}x{-(-W // 64)}, not shape {(hz, wz)}")
+    return hdr, size, header.size + SIZE.size
+
+
+def common_size(sizes):
+    """The image size of every string in one call -> (H, W); ValueError naming the first image whose size differs."""
+    for b, s in enumerate(sizes):
+        if s != sizes[0]:
+            raise ValueError(f"image {b}: a {s[0]}x{s[1]} image in a call that starts with a {sizes[0][0]}x{sizes[0][1]} one "
+                             f"(decode images of different sizes in separate calls)")
+    return sizes[0]
+
+
+def window(x: torch.Tensor, h: int, w: int) -> torch.Tensor:
+    """nic_image_window: [B, 3, h, w] f32 from the contiguous f32 x [B, 3, H, W] - its edge-replicating pad or its crop, launched on
+    x's device and that device's current stream whatever device is current."""
+    B, C, H, W = x.shape
+    with torch.cuda.device(x.device):
+        out = torch.empty((B, C, h, w), dtype=torch.float32, device=x.device)
+        check(_lib.load().nic_image_window(ptr(x), B * C, H, W, ptr(out), h, w, current_stream()), "nic_image_window")
+    return out
+
+
+def any_size_input(x: torch.Tensor):
+    """compress()'s input check: a CUDA tensor [B, 3, H, W] with H, W >= 1 -> (the image the model codes, (H, W) when the strings
+    carry the size, else None).  Sides that are multiples of 64 pass through untouched; others are padded by repeating the last row
+    and column up to the next multiples of 64."""
+    engine.require_cuda(x, "x")
+    if x.dim() != 4 or x.shape[1] != 3:
+        raise ValueError(f"expected x of shape [B, 3, H, W], got {tuple(x.shape)}")
+    H, W = x.shape[2:]
+    if H < 1 or W < 1:
+        raise ValueError(f"expected an image of at least 1x1 pixels, got {H}x{W}")
+    if H % 64 == 0 and W % 64 == 0:
+        return x, None
+    if H > MAX_SIDE or W > MAX_SIDE:
+        raise ValueError(f"an image whose sides are not multiples of 64 must be at most {MAX_SIDE} pixels high and wide; "
+                         f"got {H}x{W}")
+    return window(x.contiguous().float(), 64 * (-(-H // 64)), 64 * (-(-W // 64))), (H, W)
+
+
+def crop(x_hat: torch.Tensor, size) -> torch.Tensor:
+    """x_hat at the padded size -> the image's (H, W) (no launch when they are equal)."""
+    if tuple(x_hat.shape[2:]) == tuple(size):
+        return x_hat
+    return window(x_hat.contiguous(), *size)
 
 
 # ---- the shared parameter path ---------------------------------------------------------------------------------------
@@ -189,7 +295,7 @@ def checksums(y: torch.Tensor, z: torch.Tensor) -> torch.Tensor:
 # ---- compress / decompress -------------------------------------------------------------------------------------------
 
 def compress(model, x: torch.Tensor) -> dict:
-    check_input(x)
+    x, size = any_size_input(x)
     B, _, H, W = x.shape
     check_supported(model)
     M, K = model.M, model.K
@@ -220,12 +326,14 @@ def compress(model, x: torch.Tensor) -> dict:
         cap = words.shape[1]
         return [words[g, cap - count[g]:].tobytes() for g in range(b * n, (b + 1) * n)]
     y_strings = [pack_string(b"", segments(y_words, y_count, ly, b)) for b in range(B)]
-    z_strings = [pack_string(HEADER.pack(FORMAT_VERSION, arm, M, K, int(csum[b])), segments(z_words, z_count, lz, b)) for b in range(B)]
+    z_strings = [pack_string(sized_header(HEADER.pack(FORMAT_VERSION, arm, M, K, salted(int(csum[b]), size)), size),
+                             segments(z_words, z_count, lz, b)) for b in range(B)]
     return {"strings": [y_strings, z_strings], "shape": (hz, wz)}
 
 
-def _parse_all(model, strings, shape):
-    """Host-side validation of everything decompress reads: ValueError before any launch."""
+def _parse_sized(model, strings, shape):
+    """Host-side validation of everything decompress reads: ValueError before any launch.  -> (y strings, z strings, symbol
+    checksums, y lane (offsets, words) per image, z lane (offsets, words) per image, image size (H, W))."""
     if not isinstance(strings, (list, tuple)) or len(strings) != 2:
         raise ValueError("strings must be [y_strings, z_strings]")
     y_strings, z_strings = strings
@@ -235,23 +343,25 @@ def _parse_all(model, strings, shape):
         raise ValueError(f"shape must be (hz, wz) with positive ints, got {shape!r}")
     M, K = model.M, model.K
     ly, lz = lanes(Y_LANES, M), lanes(Z_LANES, M)
-    csum, y_lanes, z_lanes = [], [], []
+    csum, sizes, y_lanes, z_lanes = [], [], [], []
     for b, (ys, zs) in enumerate(zip(y_strings, z_strings)):
-        hdr, zoff, zwords = parse_string(zs, lz, True)
-        _, arm, m, k, cs = hdr
+        hdr, size, start = read_z_header(zs, HEADER, FORMAT_VERSION, shape, b)
+        v, arm, m, k, cs = hdr
         if arm >= len(ARMS) or ARMS[arm] != model.precision or m != M or k != K:
             got = ARMS[arm] if arm < len(ARMS) else f"arm #{arm}"
             raise ValueError(f"image {b}: the string was written by a model with precision={got!r}, M={m}, K={k}; this model has "
                              f"precision={model.precision!r}, M={M}, K={K}")
+        _, zoff, zwords = parse_string(bytes(zs[start:]), lz, False)
         _, yoff, ywords = parse_string(ys, ly, False)
-        csum.append(cs)
+        csum.append(salted(cs, size if v & SIZED else None, -1))
+        sizes.append(size)
         y_lanes.append((yoff, ywords))
-        z_lanes.append((zoff, zwords))
-    return y_strings, z_strings, csum, y_lanes, z_lanes
+        z_lanes.append(([start + o for o in zoff], zwords))
+    return y_strings, z_strings, csum, y_lanes, z_lanes, common_size(sizes)
 
 
 def decompress(model, strings, shape) -> dict:
-    y_strings, z_strings, csum, y_lanes, z_lanes = _parse_all(model, strings, shape)
+    y_strings, z_strings, csum, y_lanes, z_lanes, size = _parse_sized(model, strings, shape)
     check_supported(model)
     w0 = model.encoder.ops[0].conv.weight
     engine.require_cuda(w0, "model parameters")
@@ -294,7 +404,7 @@ def decompress(model, strings, shape) -> dict:
                                        ptr(tabs[0]), ptr(tabs[1]), ptr(tabs[2]), B, M, hy, wy, ly, t, ptr(y_nhwc), st), "nic_codec_decode")
         # g_s reads the symbols through the same hand-off as the forward's (same engine copy, same lo-half flag)
         _, y_hat, y_eng, _ = engine.latent_handoff(y_nhwc, Q_PASSTHRU, None, path.hdt)
-        x_hat = fused_g_s(model, y_eng, B, hy, wy, path.prec)
+        x_hat = crop(fused_g_s(model, y_eng, B, hy, wy, path.prec), size)
         bad = (checksums(y_hat, z_hat) != want).cpu().numpy()
     if bad.any():
         raise ValueError(f"checksum mismatch in image(s) {np.flatnonzero(bad).tolist()}: the strings are corrupted or were written "

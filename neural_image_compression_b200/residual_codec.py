@@ -14,10 +14,9 @@ import torch
 
 from . import _lib, engine
 from ._lib import CODEC_FACTORIZED, CODEC_GM, check, current_stream, ptr
-from .codec import (ARMS, HEADER, SYMBOL_LIMIT, Y_LANES, Z_LANES, _encode, _symbol_codes, checksums, lanes, pack_string,
-                    parse_string, z_tables)
+from .codec import (ARMS, HEADER, SIZED, SYMBOL_LIMIT, Y_LANES, Z_LANES, _encode, _symbol_codes, any_size_input, checksums,
+                    common_size, crop, lanes, pack_string, parse_string, read_z_header, salted, sized_header, z_tables)
 from .codec import FORMAT_VERSION as JAH_FORMAT_VERSION
-from .Models import check_input
 from .scalable_codec import FORMAT_VERSION as SCALABLE_FORMAT_VERSION
 from .scalable_codec import ParamHeads, _analysis, _segments, check_supported, psi_nhwc, synthesis
 
@@ -26,7 +25,7 @@ OTHER_FORMATS = {JAH_FORMAT_VERSION: "JointAutoregressiveHierarchical", SCALABLE
 
 
 def compress(model, x: torch.Tensor) -> dict:
-    check_input(x)
+    x, size = any_size_input(x)
     check_supported(model)
     B, _, H, W = x.shape
     M, K = model.M, model.K
@@ -50,37 +49,34 @@ def compress(model, x: torch.Tensor) -> dict:
     csum = small[B * (ly + lz):].view(np.uint32)
     arm = ARMS.index(model.precision)
     y_strings = [pack_string(b"", _segments(y_words, y_count, ly, b)) for b in range(B)]
-    z_strings = [pack_string(HEADER.pack(FORMAT_VERSION, arm, M, K, int(csum[b])), _segments(z_words, z_count, lz, b)) for b in range(B)]
+    z_strings = [pack_string(sized_header(HEADER.pack(FORMAT_VERSION, arm, M, K, salted(int(csum[b]), size)), size),
+                             _segments(z_words, z_count, lz, b)) for b in range(B)]
     return {"strings": [y_strings, z_strings], "shape": (hz, wz)}
 
 
-def parse_z(data, model, n_lanes: int, b: int):
-    """-> (header tuple, lane offsets, lane words) of a z string; ValueError on anything that is not one of this model's."""
-    if not isinstance(data, (bytes, bytearray)):
-        raise ValueError(f"image {b}: strings must be bytes, got {type(data).__name__}")
-    if len(data) and data[0] in OTHER_FORMATS:
-        raise ValueError(f"image {b}: a {OTHER_FORMATS[data[0]]} string (format {data[0]}), not a HierarchicalMixtureResidual one "
+def parse_z(data, model, n_lanes: int, b: int, shape):
+    """-> (header tuple with the symbol checksum, image size, lane offsets, lane words) of a z string; ValueError on anything that
+    is not one of this model's."""
+    if isinstance(data, (bytes, bytearray)) and len(data) and data[0] & 0x7F in OTHER_FORMATS:
+        v = data[0] & 0x7F
+        raise ValueError(f"image {b}: a {OTHER_FORMATS[v]} string (format {v}), not a HierarchicalMixtureResidual one "
                          f"(format {FORMAT_VERSION})")
-    if len(data) < HEADER.size:
-        raise ValueError(f"image {b}: truncated string: {len(data)} bytes, the header alone is {HEADER.size}")
-    hdr = HEADER.unpack_from(data, 0)
-    if hdr[0] != FORMAT_VERSION:
-        raise ValueError(f"image {b}: unknown format version {hdr[0]} (this build reads version {FORMAT_VERSION})")
-    _, arm, m, k, _ = hdr
+    hdr, size, start = read_z_header(data, HEADER, FORMAT_VERSION, shape, b)
+    _, arm, m, k, csum = hdr
     if arm >= len(ARMS) or ARMS[arm] != model.precision or (m, k) != (model.M, model.K):
         got = ARMS[arm] if arm < len(ARMS) else f"arm #{arm}"
         raise ValueError(f"image {b}: the string was written by a model with precision={got!r}, M={m}, K={k}; this model has "
                          f"precision={model.precision!r}, M={model.M}, K={model.K}")
     try:
-        _, offs, words = parse_string(bytes(data[HEADER.size:]), n_lanes, False)
+        _, offs, words = parse_string(bytes(data[start:]), n_lanes, False)
     except ValueError as e:
         raise ValueError(f"image {b}, z: {e}") from None
-    return hdr, [HEADER.size + o for o in offs], words
+    return hdr[:4] + (salted(csum, size if hdr[0] & SIZED else None, -1),), size, [start + o for o in offs], words
 
 
-def _parse_all(model, strings, shape):
-    """Host-side validation of everything decompress reads: ValueError before any launch.  -> (y strings, z strings, checksums,
-    y lane (offsets, words) per image, z lane (offsets, words) per image)."""
+def _parse_sized(model, strings, shape):
+    """Host-side validation of everything decompress reads: ValueError before any launch.  -> (y strings, z strings, symbol
+    checksums, y lane (offsets, words) per image, z lane (offsets, words) per image, image size (H, W))."""
     if not isinstance(strings, (list, tuple)) or len(strings) != 2:
         raise ValueError("strings must be [y_strings, z_strings]")
     y_strings, z_strings = strings
@@ -91,9 +87,10 @@ def _parse_all(model, strings, shape):
     if not isinstance(shape, (list, tuple)) or len(shape) != 2 or any(int(v) != v or v < 1 for v in shape):
         raise ValueError(f"shape must be (hz, wz) with positive ints, got {shape!r}")
     ly, lz = lanes(Y_LANES, model.M), lanes(Z_LANES, model.M)
-    csum, y_lanes, z_lanes = [], [], []
+    csum, sizes, y_lanes, z_lanes = [], [], [], []
     for b, (ys, zs) in enumerate(zip(y_strings, z_strings)):
-        hdr, zoff, zwords = parse_z(zs, model, lz, b)
+        hdr, size, zoff, zwords = parse_z(zs, model, lz, b, shape)
+        sizes.append(size)
         if not isinstance(ys, (bytes, bytearray)):
             raise ValueError(f"image {b}: strings must be bytes, got {type(ys).__name__}")
         try:
@@ -103,11 +100,16 @@ def _parse_all(model, strings, shape):
         csum.append(hdr[4])
         y_lanes.append((yoff, ywords))
         z_lanes.append((zoff, zwords))
-    return [bytes(s) for s in y_strings], [bytes(s) for s in z_strings], csum, y_lanes, z_lanes
+    return [bytes(s) for s in y_strings], [bytes(s) for s in z_strings], csum, y_lanes, z_lanes, common_size(sizes)
+
+
+def _parse_all(model, strings, shape):
+    """_parse_sized without the image size: the five values the host tests and tools/residual_codec_bench.py read."""
+    return _parse_sized(model, strings, shape)[:-1]
 
 
 def decompress(model, strings, shape) -> dict:
-    y_strings, z_strings, csum, y_lanes, z_lanes = _parse_all(model, strings, shape)
+    y_strings, z_strings, csum, y_lanes, z_lanes, size = _parse_sized(model, strings, shape)
     check_supported(model)
     w0 = model.entropy_parameters.net[0].weight
     engine.require_cuda(w0, "model parameters")
@@ -147,6 +149,7 @@ def decompress(model, strings, shape) -> dict:
             check(lib.nic_codec_decode_step(ptr(blob), ptr(y_off_d), ptr(y_nw_d), ptr(ys_state), ptr(ys_pos), int(t == 0), ptr(heads.raw[0]),
                                             B, M, K, hy, wy, ly, t, ptr(y_nhwc), st), "nic_codec_decode_step")
         y_hat, x_hat = synthesis(model, y_nhwc)
+        x_hat = crop(x_hat, size)
         bad = (checksums(y_hat, z_hat) != want).cpu().numpy()
     if bad.any():
         raise ValueError(f"checksum mismatch in image(s) {np.flatnonzero(bad).tolist()}: the strings are corrupted or were written "

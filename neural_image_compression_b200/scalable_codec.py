@@ -16,10 +16,10 @@ import torch
 
 from . import _lib, engine, training
 from ._lib import CODEC_FACTORIZED, CODEC_GM, LAYOUT_NCHW, Q_PASSTHRU, Q_ROUND, CodecHead, check, current_stream, ptr
-from .codec import (ARMS, SYMBOL_LIMIT, Y_LANES, Z_LANES, _encode, _symbol_codes, checksums, lanes, max_step_pixels, pack_string,
-                    parse_string, step_tables, z_tables)
+from .codec import (ARMS, SIZED, SYMBOL_LIMIT, Y_LANES, Z_LANES, _encode, _symbol_codes, any_size_input, checksums, common_size,
+                    crop, lanes, max_step_pixels, pack_string, parse_string, read_z_header, salted, sized_header, step_tables, z_tables)
 from .codec import FORMAT_VERSION as JAH_FORMAT_VERSION
-from .Models import check_input, fused_g_a, fused_g_s, fused_h_a, fused_h_s_into
+from .Models import fused_g_a, fused_g_s, fused_h_a, fused_h_s_into
 
 FORMAT_VERSION = 2
 HEADER = struct.Struct("<BBHHBII")      # version, arm, M, M1, K, base checksum (y1 and z), enhancement checksum (y2 and z)
@@ -140,7 +140,7 @@ def _segments(words, count, n, b):
 
 
 def compress(model, x: torch.Tensor) -> dict:
-    check_input(x)
+    x, size = any_size_input(x)
     check_supported(model)
     B, _, H, W = x.shape
     M, M1, K = model.M, model.M1, model.K
@@ -174,35 +174,32 @@ def compress(model, x: torch.Tensor) -> dict:
     arm = ARMS.index(model.precision)
     y1_strings = [pack_string(b"", _segments(words[0], counts[0], ln[0], b)) for b in range(B)]
     y2_strings = [pack_string(b"", _segments(words[1], counts[1], ln[1], b)) for b in range(B)]
-    z_strings = [pack_string(HEADER.pack(FORMAT_VERSION, arm, M, M1, K, int(base[b]), int(enh[b])), _segments(words[2], counts[2], ln[2], b))
-                 for b in range(B)]
+    z_strings = [pack_string(sized_header(HEADER.pack(FORMAT_VERSION, arm, M, M1, K, salted(int(base[b]), size), salted(int(enh[b]), size)),
+                                          size), _segments(words[2], counts[2], ln[2], b)) for b in range(B)]
     return {"strings": [y1_strings, y2_strings, z_strings], "shape": (hz, wz)}
 
 
-def parse_z(data, model, n_lanes: int, b: int):
-    """-> (header tuple, lane offsets, lane words) of a scalable z string; ValueError on anything that is not one of this model's."""
-    if not isinstance(data, (bytes, bytearray)):
-        raise ValueError(f"image {b}: strings must be bytes, got {type(data).__name__}")
-    if len(data) and data[0] == JAH_FORMAT_VERSION:
+def parse_z(data, model, n_lanes: int, b: int, shape):
+    """-> (header tuple with the symbol checksums, image size, lane offsets, lane words) of a scalable z string; ValueError on
+    anything that is not one of this model's."""
+    if isinstance(data, (bytes, bytearray)) and len(data) and data[0] & 0x7F == JAH_FORMAT_VERSION:
         raise ValueError(f"image {b}: a JointAutoregressiveHierarchical string (format {JAH_FORMAT_VERSION}), not a scalable one "
                          f"(format {FORMAT_VERSION})")
-    if len(data) < HEADER.size:
-        raise ValueError(f"image {b}: truncated string: {len(data)} bytes, the header alone is {HEADER.size}")
-    hdr = HEADER.unpack_from(data, 0)
-    if hdr[0] != FORMAT_VERSION:
-        raise ValueError(f"image {b}: unknown format version {hdr[0]} (this build reads version {FORMAT_VERSION})")
-    _, arm, m, m1, k, _, _ = hdr
+    hdr, size, start = read_z_header(data, HEADER, FORMAT_VERSION, shape, b)
+    _, arm, m, m1, k, base, enh = hdr
     if arm >= len(ARMS) or ARMS[arm] != model.precision or (m, m1, k) != (model.M, model.M1, model.K):
         got = ARMS[arm] if arm < len(ARMS) else f"arm #{arm}"
         raise ValueError(f"image {b}: the string was written by a model with precision={got!r}, M={m}, M1={m1}, K={k}; this model "
                          f"has precision={model.precision!r}, M={model.M}, M1={model.M1}, K={model.K}")
-    _, offs, words = parse_string(bytes(data[HEADER.size:]), n_lanes, False)
-    return hdr, [HEADER.size + o for o in offs], words
+    _, offs, words = parse_string(bytes(data[start:]), n_lanes, False)
+    salt = size if hdr[0] & SIZED else None
+    return hdr[:5] + (salted(base, salt, -1), salted(enh, salt, -1)), size, [start + o for o in offs], words
 
 
-def _parse_all(model, strings, shape, base_only):
+def _parse_sized(model, strings, shape, base_only):
     """Host-side validation of everything decompress reads: ValueError before any launch.  -> (strings of the layers it decodes
-    [z, y1(, y2)], their lane (offsets, words) per image, base checksums, enhancement checksums)."""
+    [z, y1(, y2)], their lane (offsets, words) per image, lane counts, base symbol checksums, enhancement symbol checksums, image
+    size (H, W))."""
     if not isinstance(strings, (list, tuple)) or len(strings) != 3:
         raise ValueError("strings must be [y1_strings, y2_strings, z_strings]")
     y1s, y2s, zs = strings
@@ -216,9 +213,10 @@ def _parse_all(model, strings, shape, base_only):
     if not isinstance(shape, (list, tuple)) or len(shape) != 2 or any(int(v) != v or v < 1 for v in shape):
         raise ValueError(f"shape must be (hz, wz) with positive ints, got {shape!r}")
     ln = [lanes(Z_LANES, model.M)] + [lanes(Y_LANES, c1 - c0) for _, _, c0, c1 in _heads(model, base_only)]
-    lane_tabs, base, enh = [[] for _ in layers], [], []
+    lane_tabs, base, enh, sizes = [[] for _ in layers], [], [], []
     for b in range(len(zs)):
-        hdr, offs, words = parse_z(zs[b], model, ln[0], b)
+        hdr, size, offs, words = parse_z(zs[b], model, ln[0], b, shape)
+        sizes.append(size)
         base.append(hdr[5])
         enh.append(hdr[6])
         lane_tabs[0].append((offs, words))
@@ -231,11 +229,16 @@ def _parse_all(model, strings, shape, base_only):
             except ValueError as e:
                 raise ValueError(f"image {b}, layer y{li}: {e}") from None
             lane_tabs[li].append((offs, words))
-    return [[bytes(s) for s in layer] for layer in layers], lane_tabs, ln, base, enh
+    return [[bytes(s) for s in layer] for layer in layers], lane_tabs, ln, base, enh, common_size(sizes)
+
+
+def _parse_all(model, strings, shape, base_only):
+    """_parse_sized without the image size: the five values the host tests read."""
+    return _parse_sized(model, strings, shape, base_only)[:-1]
 
 
 def decompress(model, strings, shape, base_only: bool = False) -> dict:
-    layers, lane_tabs, ln, base, enh = _parse_all(model, strings, shape, base_only)
+    layers, lane_tabs, ln, base, enh, size = _parse_sized(model, strings, shape, base_only)
     check_supported(model)
     w0 = model.encoder.ops[0].conv.weight
     engine.require_cuda(w0, "model parameters")
@@ -282,7 +285,7 @@ def decompress(model, strings, shape, base_only: bool = False) -> dict:
         out = {"y1_hat": y_parts[0], "z_hat": z_hat}
         if not base_only:
             y_hat, x_hat = synthesis(model, torch.cat(y_nhwc, dim=-1).contiguous())
-            out = {"x_hat": x_hat, "y_hat": y_hat, "y1_hat": y_parts[0], "y2_hat": y_parts[1], "z_hat": z_hat}
+            out = {"x_hat": crop(x_hat, size), "y_hat": y_hat, "y1_hat": y_parts[0], "y2_hat": y_parts[1], "z_hat": z_hat}
         bad = (torch.cat(got) != want).cpu().numpy().reshape(len(got), B)
     for layer, flags in zip(("base layer (y1 and z)", "enhancement layer (y2)"), bad):
         if flags.any():
