@@ -450,6 +450,17 @@ int nic_luma(const float* rgb, float* y, int32_t b, int32_t h, int32_t w, int32_
 size_t nic_ms_ssim_workspace_bytes(int32_t planes, int32_t h, int32_t w);
 int nic_ms_ssim_levels(const float* x, const float* y, int32_t planes, int32_t h, int32_t w, float data_range, int32_t clamp_y,
                        float* level_means, void* workspace, size_t workspace_bytes, void* stream);
+/*
+ * Backward of the level means with respect to the FIRST image (the MS-SSIM loss, DESIGN.md section 13):
+ * g_x [planes][h][w] = sum over (level, plane) of g_level[level][plane] * d level_mean / d x, where level_mean is the mean cs of
+ * levels 0-3 and the mean ssim of level 4.  `workspace` (>= nic_ms_ssim_bwd_workspace_bytes) must hold what
+ * nic_ms_ssim_levels(x, y, planes, h, w, data_range, clamp_y = 0, ...) left in it: the pooled pyramids are read back from there.
+ * No atomics: every element of g_x is written by one thread in a fixed order (bit-identical across calls and batch sizes).
+ * The first call on a device (as the first nic_ms_ssim_levels call) uploads the window and must run outside a stream capture.
+ */
+size_t nic_ms_ssim_bwd_workspace_bytes(int32_t planes, int32_t h, int32_t w);
+int nic_ms_ssim_bwd(const float* x, const float* y, int32_t planes, int32_t h, int32_t w, float data_range, const float* g_level,
+                    float* g_x, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- entropy coder (DESIGN.md section 9): byte strings for JointAutoregressiveHierarchical ------------------------------------
  * rANS with a 32-bit state in [2^16, 2^32), 16-bit renormalisation words and 16-bit probabilities.  A table row of one element is

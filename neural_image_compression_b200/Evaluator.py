@@ -22,9 +22,50 @@ from ._lib import check, current_stream, ptr
 MS_SSIM_WEIGHTS = (0.0448, 0.2856, 0.3001, 0.2363, 0.1333)
 
 
+def ms_ssim_levels(x: torch.Tensor, y: torch.Tensor, data_range: float = 1.0, clamp_y: bool = False,
+                   workspace: torch.Tensor = None) -> torch.Tensor:
+    """[5, planes, 2] = (mean ssim, mean cs) of every scale of the NCHW f32 planes of x and y (nic_ms_ssim_levels).  `workspace`
+    (uint8, default: a fresh one) keeps the pooled pyramids, which nic_ms_ssim_bwd reads back."""
+    lib = _lib.load()
+    b, c, h, w = x.shape
+    planes = b * c
+    lev = torch.empty((5, planes, 2), dtype=torch.float32, device=x.device)
+    ws = workspace if workspace is not None else torch.empty(lib.nic_ms_ssim_workspace_bytes(planes, h, w), dtype=torch.uint8, device=x.device)
+    with torch.cuda.device(x.device):
+        check(lib.nic_ms_ssim_levels(ptr(x), ptr(y), planes, h, w, float(data_range), int(clamp_y), ptr(lev), ptr(ws), ws.numel(),
+                                     current_stream()), "nic_ms_ssim_levels")
+    return lev
+
+
+_WEIGHTS = {}
+
+
+def _weights(device) -> torch.Tensor:
+    """The MS-SSIM weights on `device`, uploaded once: the training step's first (warm-up) call makes them, so a CUDA-graph
+    capture of the step never copies from the host."""
+    if device not in _WEIGHTS:
+        _WEIGHTS[device] = torch.tensor(MS_SSIM_WEIGHTS, dtype=torch.float32, device=device)
+    return _WEIGHTS[device]
+
+
+def combine_levels(lev: torch.Tensor):
+    """(terms [5, planes], value [planes]): the terms are the cs of scales 0-3 and the ssim of scale 4; the value of a plane is
+    prod relu(term)^w (pytorch_msssim's per-channel MS-SSIM)."""
+    wts = _weights(lev.device)
+    terms = torch.cat([lev[:4, :, 1], lev[4:, :, 0]], dim=0)
+    return terms, torch.prod(torch.relu(terms) ** wts.view(-1, 1), dim=0)
+
+
+def term_grads(terms: torch.Tensor, value: torch.Tensor) -> torch.Tensor:
+    """d value / d term [5, planes]: w_l value / term_l where term_l > 0, else 0 - the relu rule autograd applies to
+    combine_levels (a channel with any term <= 0 has value 0 and no gradient at all)."""
+    wts = _weights(terms.device).view(-1, 1)
+    pos = terms > 0
+    return torch.where(pos, wts * value / torch.where(pos, terms, torch.ones_like(terms)), torch.zeros_like(terms))
+
+
 def ms_ssim(x: torch.Tensor, y: torch.Tensor, data_range: float = 1.0, size_average: bool = True, clamp_y: bool = False) -> torch.Tensor:
     """pytorch_msssim.ms_ssim(x, y, data_range, size_average) for NCHW f32 batches on the device (Evaluator.py:38, 45)."""
-    lib = _lib.load()
     engine.require_cuda(x, "x")
     x, y = x.contiguous().float(), y.contiguous().float()
     if x.shape != y.shape or x.dim() != 4:
@@ -32,16 +73,8 @@ def ms_ssim(x: torch.Tensor, y: torch.Tensor, data_range: float = 1.0, size_aver
     b, c, h, w = x.shape
     if min(h, w) <= (11 - 1) * 2 ** 4:
         raise AssertionError("Image size should be larger than 160 due to the 4 downsamplings in ms-ssim")
-    planes = b * c
-    lev = torch.empty((5, planes, 2), dtype=torch.float32, device=x.device)
-    nbytes = lib.nic_ms_ssim_workspace_bytes(planes, h, w)
-    ws = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
-    with torch.cuda.device(x.device):
-        check(lib.nic_ms_ssim_levels(ptr(x), ptr(y), planes, h, w, float(data_range), int(clamp_y), ptr(lev), ptr(ws), nbytes,
-                                     current_stream()), "nic_ms_ssim_levels")
-    wts = torch.tensor(MS_SSIM_WEIGHTS, dtype=torch.float32, device=x.device)
-    terms = torch.cat([torch.relu(lev[:4, :, 1]), torch.relu(lev[4:, :, 0])], dim=0)        # cs of scales 0-3, ssim of scale 4
-    val = torch.prod(terms ** wts.view(-1, 1), dim=0).view(b, c)
+    _, val = combine_levels(ms_ssim_levels(x, y, data_range, clamp_y))
+    val = val.view(b, c)
     return val.mean() if size_average else val.mean(1)
 
 

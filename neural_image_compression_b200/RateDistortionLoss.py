@@ -83,6 +83,59 @@ def rd_loss(model_out: dict, x: torch.Tensor, lambda_rd: float):
     }
 
 
+MS_SSIM_MIN_SIDE = (11 - 1) * 2 ** 4        # five scales of an 11-tap VALID window: the smaller side must exceed 160
+
+
+def check_ms_ssim_shape(shape):
+    """ValueError (before any launch) for images whose smaller side is 160 pixels or less."""
+    if len(shape) != 4 or min(shape[2], shape[3]) <= MS_SSIM_MIN_SIDE:
+        raise ValueError(f"the MS-SSIM loss needs NCHW images whose smaller side exceeds {MS_SSIM_MIN_SIDE} pixels, got {tuple(shape)}")
+
+
+def ms_ssim_terms(model_out: dict, x: torch.Tensor, lambda_rd: float):
+    """Device-resident terms of the MS-SSIM loss, no host sync: (per_image [3, B], scalars [9], ms_ssim_per_image [B], state).
+    scalars = nic_rd_finalize's 8 with entry 5 replaced by loss = bpp_total + lambda * (1 - mean_b ms_ssim_b), then the batch
+    MS-SSIM.  x_hat is not clamped.  state = (x_hat, x, terms, value, workspace): what ms_ssim_x_hat_grad reads."""
+    from .Evaluator import combine_levels, ms_ssim_levels
+    check_ms_ssim_shape(tuple(model_out["x_hat"].shape))
+    per_image, scalars = rd_terms(model_out, x, lambda_rd)
+    x_hat = model_out["x_hat"].detach().contiguous().float()
+    x = x.to(x_hat.device).contiguous().float()
+    b, c, h, w = x.shape
+    ws = torch.empty(_lib.load().nic_ms_ssim_bwd_workspace_bytes(b * c, h, w), dtype=torch.uint8, device=x.device)
+    terms, value = combine_levels(ms_ssim_levels(x_hat, x, 1.0, False, workspace=ws))
+    per_img = value.view(b, c).mean(1)
+    ms = per_img.mean()
+    loss = scalars[2] + float(lambda_rd) * (1.0 - ms)
+    scalars = torch.cat([scalars[:5], loss.view(1), scalars[6:], ms.view(1)])
+    return per_image, scalars, per_img, (x_hat, x, terms, value, ws)
+
+
+def ms_ssim_rd_loss(model_out: dict, x: torch.Tensor, lambda_rd: float):
+    """CompressAI's RateDistortionLoss(metric="ms-ssim"): loss = bpp_total + lambda * (1 - ms_ssim(x_hat, x, data_range=1)), the
+    MS-SSIM of pytorch_msssim averaged over the batch, x_hat unclamped.  rd_loss's keys ('mse' / 'psnr' still reported) plus
+    'ms_ssim' (float) and 'ms_ssim_per_image' (device tensor [B]); one host synchronisation.  'loss' is differentiable when the
+    model output is (training._MSSSIMRDLoss: nic_ms_ssim_bwd for x_hat, the rate gradient for logp_y / logp_z)."""
+    with torch.no_grad():
+        per_image, scalars, per_img, state = ms_ssim_terms(model_out, x, lambda_rd)
+    loss = scalars[5]
+    diff = [model_out[k] for k in ("logp_y", "logp_z", "x_hat")]
+    if torch.is_grad_enabled() and any(t.requires_grad for t in diff):
+        from .training import _MSSSIMRDLoss
+        loss = _MSSSIMRDLoss.apply(diff[0], diff[1], diff[2], float(lambda_rd), scalars, state)
+    s = scalars.tolist()                                   # the one host synchronisation
+    _check_pipeline()
+    mse_per_image = per_image[2]
+    return {
+        "loss": loss,
+        "bpp_y": s[0], "bpp_z": s[1], "bpp_total": s[2], "mse": s[3], "psnr": s[4],
+        "mse_per_image": mse_per_image,
+        "psnr_per_image": -10 * torch.log10(mse_per_image + 1e-8),
+        "bits_y": s[6], "bits_z": s[7], "bits_total": s[6] + s[7],
+        "ms_ssim": s[8], "ms_ssim_per_image": per_img,
+    }
+
+
 def vision_rd_loss(model_out: dict, x: torch.Tensor, lambda_rd: float, gamma: float = 0.0, frozen_activation=None, V=None):
     """``vision_rd_loss`` of /root/reference/RateDistortionLoss.py:52-121 for ScalableImageCoding outputs: rate terms of the
     two latent parts and of z, reconstruction MSE / PSNR, ``loss = bpp_total + lambda_rd * mse`` (:98, no 255^2 here).

@@ -92,6 +92,8 @@ SIGNATURES = {
     "nic_luma": (C.c_int, [_vp, _vp, _i32, _i32, _i32, _i32, _vp]),
     "nic_ms_ssim_workspace_bytes": (_sz, [_i32, _i32, _i32]),
     "nic_ms_ssim_levels": (C.c_int, [_vp, _vp, _i32, _i32, _i32, _f32, _i32, _vp, _vp, _sz, _vp]),
+    "nic_ms_ssim_bwd_workspace_bytes": (_sz, [_i32, _i32, _i32]),
+    "nic_ms_ssim_bwd": (C.c_int, [_vp, _vp, _i32, _i32, _i32, _f32, _vp, _vp, _vp, _sz, _vp]),
     "nic_adam_multi_step": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i32, _f32, _f32, _f32, _f32, _i32, _vp, _vp]),
     "nic_adam_multi_step_ex": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i32, _f32, _vp, _f32, _f32, _f32, _f32, _i32, _vp, _vp]),
     "nic_counter_increment": (C.c_int, [_vp, _vp]),

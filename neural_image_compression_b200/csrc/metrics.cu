@@ -8,7 +8,7 @@
 //   C1 = (0.01 L)^2, C2 = (0.03 L)^2; five scales with 2x2 average pooling (padding = size % 2, zeros counted) between them;
 //   result = prod_i relu(cs_i)^w_i * relu(ssim_5)^w_5 per (image, channel), weights (0.0448, 0.2856, 0.3001, 0.2363, 0.1333).
 // Reductions are per-block partial sums folded in a fixed order (deterministic).
-#include "common.cuh"
+#include "tc_host.cuh"
 
 namespace nic {
 
@@ -175,7 +175,121 @@ __global__ void eval_sse_fold_kernel(const float* __restrict__ partials, int par
   }
 }
 
-static int ensure_gauss() {                       // the constant-memory window is per device: upload once on each
+// ---- backward of the per-level means (the MS-SSIM loss, DESIGN.md section 13; oracle/ms_ssim_bwd.py restates it) ----------------
+constexpr int kBT = 32;                         // level-input pixels per tile edge (one CTA)
+constexpr int kBO = kBT + kWin - 1;             // 42: VALID output pixels whose window touches the tile
+constexpr int kBI = kBO + kWin - 1;             // 52: input pixels those outputs read
+constexpr int kBwdSmemFloats = 2 * kBI * (kBI + 1) + 6 * kBI * kBO + 3 * kBO * (kBO + 1);
+constexpr int kBwdSmemBytes = kBwdSmemFloats * 4;
+
+/*
+ * One 32 x 32 tile of level l's input gradient of one plane:
+ *   g[i][j] = (G^T a + 2 x (G^T b) + 2 (x - y) (G^T e))[i][j] + g_coarse[(i + ph) / 2][(j + pw) / 2] / 4
+ * with a, b, e the derivatives of the level's cs map (ssim map at the last level) with respect to m1 = G x, exx = G x^2 and
+ * euu = G (x - y)^2 at every VALID output pixel, times g_level[plane] / (ho wo), and zero outside the VALID output.
+ * The CTA stages 52 x 52 of x and y, recomputes the six moment maps over the 42 x 42 output pixels that touch the tile, forms
+ * a / b / e there and applies the transposed filter.  Every output element is written by one thread, from sums in a fixed order.
+ */
+__global__ void __launch_bounds__(256)
+ms_ssim_bwd_tile_kernel(const float* __restrict__ xs, const float* __restrict__ ys, int h, int w, float c1, float c2, int last,
+                        const float* __restrict__ g_level, const float* __restrict__ g_coarse, int hc, int wc, int ph, int pw,
+                        float* __restrict__ g_out) {
+  extern __shared__ float smem[];
+  float (*sx)[kBI + 1] = reinterpret_cast<float (*)[kBI + 1]>(smem);
+  float (*sy)[kBI + 1] = reinterpret_cast<float (*)[kBI + 1]>(smem + kBI * (kBI + 1));
+  float* hb = smem + 2 * kBI * (kBI + 1);                       // [6][kBI][kBO] moment rows; later [3][kBO][kBT] filtered rows
+  float* ab = hb + 6 * kBI * kBO;                               // [3][kBO][kBO + 1]: a, b, e
+  const int plane = blockIdx.z;
+  const int ho = h - kWin + 1, wo = w - kWin + 1;
+  const int ty0 = blockIdx.y * kBT, tx0 = blockIdx.x * kBT;
+  const int oy0 = ty0 - (kWin - 1), ox0 = tx0 - (kWin - 1);     // first output row / column (and first staged input row / column)
+  const long plane_off = static_cast<long>(plane) * h * w;
+  const float* xp = xs + plane_off;
+  const float* yp = ys + plane_off;
+  for (int i = threadIdx.x; i < kBI * kBI; i += 256) {
+    const int r = i / kBI, c = i % kBI;
+    const int gy = oy0 + r, gx = ox0 + c;
+    float a = 0.f, b = 0.f;
+    if (gy >= 0 && gy < h && gx >= 0 && gx < w) { a = xp[static_cast<long>(gy) * w + gx]; b = yp[static_cast<long>(gy) * w + gx]; }
+    sx[r][c] = a; sy[r][c] = b;
+  }
+  __syncthreads();
+  // moments along the rows: 52 rows x 42 output columns, six maps
+  for (int i = threadIdx.x; i < kBI * kBO; i += 256) {
+    const int r = i / kBO, c = i % kBO;
+    float m1 = 0.f, m2 = 0.f, xx = 0.f, yy = 0.f, mu = 0.f, uu = 0.f;
+#pragma unroll
+    for (int k = 0; k < kWin; ++k) {
+      const float g = c_gauss[k], a = sx[r][c + k], b = sy[r][c + k], u = a - b;
+      m1 += g * a; m2 += g * b; xx += g * a * a; yy += g * b * b; mu += g * u; uu += g * u * u;
+    }
+    hb[0 * kBI * kBO + i] = m1; hb[1 * kBI * kBO + i] = m2; hb[2 * kBI * kBO + i] = xx;
+    hb[3 * kBI * kBO + i] = yy; hb[4 * kBI * kBO + i] = mu; hb[5 * kBI * kBO + i] = uu;
+  }
+  __syncthreads();
+  const float scale = g_level[plane] / (static_cast<float>(ho) * static_cast<float>(wo));
+  for (int i = threadIdx.x; i < kBO * kBO; i += 256) {
+    const int r = i / kBO, c = i % kBO;
+    const int p = oy0 + r, q = ox0 + c;
+    float a = 0.f, b = 0.f, e = 0.f;
+    if (p >= 0 && p < ho && q >= 0 && q < wo) {
+      float mom[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+      for (int k = 0; k < kWin; ++k) {
+        const float g = c_gauss[k];
+#pragma unroll
+        for (int m = 0; m < 6; ++m) mom[m] += g * hb[m * kBI * kBO + (r + k) * kBO + c];
+      }
+      const float m1 = mom[0], m2 = mom[1], mu = mom[4];
+      const float d = mom[2] - m1 * m1 + mom[3] - m2 * m2 + c2;
+      const float v = mom[5] - mu * mu;
+      const float inv_d = 1.f / d, vd = v * inv_d;
+      a = 2.f * (mu - m1 * vd) * inv_d;
+      b = vd * inv_d;
+      e = -inv_d;
+      if (last) {
+        const float inv_b = 1.f / (m1 * m1 + m2 * m2 + c1);
+        const float mu2b = mu * mu * inv_b;
+        const float lum = 1.f - mu2b, cs = 1.f - vd;
+        a = 2.f * (m1 * mu2b - mu) * inv_b * cs + lum * a;
+        b *= lum; e *= lum;
+      }
+      a *= scale; b *= scale; e *= scale;
+    }
+    ab[(0 * kBO + r) * (kBO + 1) + c] = a; ab[(1 * kBO + r) * (kBO + 1) + c] = b; ab[(2 * kBO + r) * (kBO + 1) + c] = e;
+  }
+  __syncthreads();
+  // transposed filter along the rows: output column c = jj + 10 - k feeds input column jj with tap k
+  for (int i = threadIdx.x; i < 3 * kBO * kBT; i += 256) {
+    const int m = i / (kBO * kBT), r = (i / kBT) % kBO, jj = i % kBT;
+    float t = 0.f;
+#pragma unroll
+    for (int k = 0; k < kWin; ++k) t += c_gauss[k] * ab[(m * kBO + r) * (kBO + 1) + jj + (kWin - 1) - k];
+    hb[i] = t;
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < kBT * kBT; i += 256) {
+    const int ii = i / kBT, jj = i % kBT;
+    const int gi = ty0 + ii, gj = tx0 + jj;
+    if (gi >= h || gj >= w) continue;
+    float t0 = 0.f, t1 = 0.f, t2 = 0.f;
+#pragma unroll
+    for (int k = 0; k < kWin; ++k) {
+      const float g = c_gauss[k];
+      const int r = ii + (kWin - 1) - k;
+      t0 += g * hb[(0 * kBO + r) * kBT + jj]; t1 += g * hb[(1 * kBO + r) * kBT + jj]; t2 += g * hb[(2 * kBO + r) * kBT + jj];
+    }
+    const float xv = sx[ii + kWin - 1][jj + kWin - 1], uv = xv - sy[ii + kWin - 1][jj + kWin - 1];
+    float gv = t0 + 2.f * xv * t1 + 2.f * uv * t2;
+    if (g_coarse) gv += 0.25f * g_coarse[(static_cast<long>(plane) * hc + (gi + ph) / 2) * wc + (gj + pw) / 2];
+    g_out[plane_off + static_cast<long>(gi) * w + gj] = gv;
+  }
+}
+
+// The constant-memory window is per device: uploaded once on each by the first nic_ms_ssim_levels / nic_ms_ssim_bwd call there
+// (cudaMemcpyToSymbol, which a CUDA-graph capture cannot record), so that first call must run outside any capture - as the
+// warm-up step of parallel.ShardedTrainer(graph=True) does before it captures.
+static int ensure_gauss() {
   static bool done_dev[64] = {};
   int dev = 0;
   if (int rc = check_cuda(cudaGetDevice(&dev), "cudaGetDevice")) return rc;
@@ -234,6 +348,15 @@ size_t nic_ms_ssim_workspace_bytes(int32_t planes, int32_t h, int32_t w) {
   return (2 * pooled * planes + tiles * planes * 2 + static_cast<size_t>(planes) * 5 * 2 + 64) * sizeof(float) + 1024;
 }
 
+size_t nic_ms_ssim_bwd_workspace_bytes(int32_t planes, int32_t h, int32_t w) {
+  if (planes < 1 || h < 1 || w < 1) return 0;
+  // the forward's workspace (its pooled pyramids are read back) + the gradients of the pooled levels 1-4
+  size_t pooled = 0;
+  int hh = h, ww = w;
+  for (int l = 1; l < 5; ++l) { hh = (hh + 2 * (hh % 2) - 2) / 2 + 1; ww = (ww + 2 * (ww % 2) - 2) / 2 + 1; pooled += static_cast<size_t>(hh) * ww; }
+  return nic_ms_ssim_workspace_bytes(planes, h, w) + pooled * planes * sizeof(float);
+}
+
 /*
  * level_means [5][planes][2] = (mean ssim, mean cs) of every scale; the caller combines them (prod relu(.)^w, mean over channels).
  */
@@ -273,6 +396,48 @@ int nic_ms_ssim_levels(const float* x, const float* y, int32_t planes, int32_t h
     avgpool2_kernel<<<static_cast<int>(blocks), 256, 0, st>>>(cy, ny, planes, ch, cw, ph, pw, nh, nw, clamp);
     if (int rc = check_launch("avgpool2_kernel")) return rc;
     cx = nx; cy = ny; ch = nh; cw = nw; clamp = 0;
+  }
+  return NIC_OK;
+}
+
+/*
+ * g_x [planes][h][w] = d loss / d x from g_level [5][planes] = d loss / d (mean cs of levels 0-3 | mean ssim of level 4).  The
+ * workspace is the one nic_ms_ssim_levels(x, y, ..., clamp_y = 0) filled (same x, y, sizes, data_range), at least
+ * nic_ms_ssim_bwd_workspace_bytes long: its pooled pyramids are read back, the level gradients go behind them.
+ */
+int nic_ms_ssim_bwd(const float* x, const float* y, int32_t planes, int32_t h, int32_t w, float data_range, const float* g_level,
+                    float* g_x, void* workspace, size_t workspace_bytes, void* stream) {
+  if (int rc = nic_check_device()) return rc;
+  if (planes < 1 || h < 1 || w < 1) return fail(NIC_E_BADSHAPE, "ms_ssim_bwd: planes=%d h=%d w=%d", planes, h, w);
+  if ((h < w ? h : w) <= (kWin - 1) * 16) return fail(NIC_E_BADSHAPE, "ms_ssim_bwd: the smaller side must exceed %d pixels (five scales of an 11-tap window)", (kWin - 1) * 16);
+  if (!x || !y || !g_level || !g_x) return fail(NIC_E_BADSHAPE, "ms_ssim_bwd: null pointer");
+  const size_t need = nic_ms_ssim_bwd_workspace_bytes(planes, h, w);
+  if (!workspace || workspace_bytes < need) return fail(NIC_E_WORKSPACE, "ms_ssim_bwd: workspace %zu < %zu bytes", workspace_bytes, need);
+  if (int rc = ensure_gauss()) return rc;
+  if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(ms_ssim_bwd_tile_kernel), kBwdSmemBytes)) return rc;
+  cudaStream_t st = as_stream(stream);
+  const float c1 = (0.01f * data_range) * (0.01f * data_range), c2 = (0.03f * data_range) * (0.03f * data_range);
+  // the forward's layout: tile partials, then (x_l, y_l) for l = 1..4; the level gradients start at the forward's size
+  float* ws = static_cast<float*>(workspace);
+  const size_t tiles0 = static_cast<size_t>((h + kTile - 1) / kTile) * ((w + kTile - 1) / kTile);
+  const float* lx[5] = {x}; const float* ly[5] = {y};
+  int lh[5] = {h}, lw[5] = {w};
+  float* lg[5] = {g_x};
+  float* pyr = ws + tiles0 * planes * 2;
+  float* grad = reinterpret_cast<float*>(static_cast<char*>(workspace) + nic_ms_ssim_workspace_bytes(planes, h, w));
+  for (int l = 1; l < 5; ++l) {
+    lh[l] = (lh[l - 1] + 2 * (lh[l - 1] % 2) - 2) / 2 + 1; lw[l] = (lw[l - 1] + 2 * (lw[l - 1] % 2) - 2) / 2 + 1;
+    const size_t n = static_cast<size_t>(planes) * lh[l] * lw[l];
+    lx[l] = pyr; ly[l] = pyr + n; pyr += 2 * n;
+    lg[l] = grad; grad += n;
+  }
+  for (int l = 4; l >= 0; --l) {
+    dim3 grid((lw[l] + kBT - 1) / kBT, (lh[l] + kBT - 1) / kBT, planes);
+    const float* gc = l < 4 ? lg[l + 1] : nullptr;
+    const int hc = l < 4 ? lh[l + 1] : 0, wc = l < 4 ? lw[l + 1] : 0;
+    ms_ssim_bwd_tile_kernel<<<grid, 256, kBwdSmemBytes, st>>>(lx[l], ly[l], lh[l], lw[l], c1, c2, l == 4, g_level + static_cast<long>(l) * planes,
+                                                              gc, hc, wc, lh[l] % 2, lw[l] % 2, lg[l]);
+    if (int rc = check_launch("ms_ssim_bwd_tile_kernel")) return rc;
   }
   return NIC_OK;
 }

@@ -314,14 +314,22 @@ class ShardedTrainer:
     shape and replays it: the ~380 kernel launches of a step, their tensor-map encodes and the Python around them are paid
     once.  The noise comes from torch's graph-safe Philox state (a fresh draw every replay).  The returned dict then holds
     device tensors only ('loss', 'scalars' = the 8 rd scalars of nic_rd_finalize); read them when needed.  Steps with injected
-    noise run eagerly."""
+    noise run eagerly.
+
+    distortion="ms-ssim" trains for MS-SSIM (RateDistortionLoss.ms_ssim_rd_loss: loss = bpp + lambda * (1 - MS-SSIM), no 255^2);
+    'scalars' then has a 9th entry, the batch MS-SSIM.  The all-reduce is the same: with equal shards the average of the per-rank
+    gradients of a batch-mean loss is the global gradient.  Not built for ScalableImageCoding (vision_rd_loss is its loss)."""
 
     def __init__(self, model, lambda_rd: float, lr: float = 1e-4, group=None, bucket_bytes: int = 32 << 20, optimizer=None,
-                 graph: bool = False):
-        from .training import Adam
-        self.model, self.lambda_rd, self.group, self.graph = model, lambda_rd, group, graph
-        self.optimizer = optimizer if optimizer is not None else Adam(model.parameters(), lr=lr)
+                 graph: bool = False, distortion: str = "mse"):
+        from .training import DISTORTIONS, Adam
         self._scalable = type(model).__name__ == "ScalableImageCoding"
+        if distortion not in DISTORTIONS:
+            raise ValueError(f"distortion must be one of {DISTORTIONS}, got {distortion!r}")
+        if self._scalable and distortion != "mse":
+            raise ValueError("ScalableImageCoding trains with vision_rd_loss (MSE); distortion='ms-ssim' is not built for it")
+        self.model, self.lambda_rd, self.group, self.graph, self.distortion = model, lambda_rd, group, graph, distortion
+        self.optimizer = optimizer if optimizer is not None else Adam(model.parameters(), lr=lr)
         self.buckets = grad_buckets(model.parameters(), bucket_bytes)
         self._flats = [None] * len(self.buckets)
         self._graphs = {}
@@ -346,7 +354,7 @@ class ShardedTrainer:
             loss, terms = scalable_step(self.model, x_local, self.lambda_rd, noise=noise)
             return loss, None, torch.stack([terms[k] for k in ("bpp_y1", "bpp_y2", "bpp_z", "mse", "psnr", "loss")])
         from .training import step_gradients
-        return step_gradients(self.model, x_local, self.lambda_rd, noise=noise, partial_hook=partial_hook)
+        return step_gradients(self.model, x_local, self.lambda_rd, noise=noise, partial_hook=partial_hook, distortion=self.distortion)
 
     # ---- gradient all-reduce INSIDE the captured step, overlapped with g_a's backward -------------------------------------------
     def _comm_setup(self, device):
@@ -470,12 +478,15 @@ class ShardedTrainer:
             if not adam_done:
                 self.optimizer.step()
             self.step_count += 1
-            # scalars: the 8 rd scalars of nic_rd_finalize; ScalableImageCoding: (bpp_y1, bpp_y2, bpp_z, mse, psnr, loss)
+            # scalars: the 8 rd scalars of nic_rd_finalize (+ the batch MS-SSIM with distortion='ms-ssim'); ScalableImageCoding: (bpp_y1, bpp_y2, bpp_z, mse, psnr, loss)
             return {"loss": loss, "scalars": scalars, "mse_per_image": None if per_image is None else per_image[2]}
-        from .RateDistortionLoss import rd_loss
+        from .RateDistortionLoss import ms_ssim_rd_loss, rd_loss
+        if self.distortion == "ms-ssim":
+            from .RateDistortionLoss import check_ms_ssim_shape
+            check_ms_ssim_shape(tuple(x_local.shape))
         self.optimizer.zero_grad()
         out = self.model(x_local, training=True, noise=noise, lean=True)
-        rd = rd_loss(out, x_local, self.lambda_rd)
+        rd = (ms_ssim_rd_loss if self.distortion == "ms-ssim" else rd_loss)(out, x_local, self.lambda_rd)
         rd["loss"].backward()
         self._allreduce()
         self.optimizer.step()

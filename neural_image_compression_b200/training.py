@@ -16,7 +16,8 @@ autograd wrapping live in training_scalable.py), a hand-scheduled chain of C-ABI
                                  (incl. compressai's LowerBound gradient rule on the stored parameters)
     LeakyReLU                    nic_lrelu_bwd
     likelihoods                  nic_gm_likelihood_bwd, nic_factorized_likelihood_bwd
-    distortion                   nic_sse_bwd (``_RDLoss`` below is rd_loss's autograd node)
+    distortion                   nic_sse_bwd (``_RDLoss`` below is rd_loss's autograd node); nic_ms_ssim_bwd for the MS-SSIM
+                                 loss (``_MSSSIMRDLoss``, ms_ssim_rd_loss's node)
     optimizer                    nic_adam_multi_step (``Adam`` below: torch.optim.Adam semantics, Main.ipynb:133; one launch)
 
 ``step_gradients`` runs the same forward + loss + backward WITHOUT the autograd engine (calling thread, current stream): the form
@@ -726,12 +727,20 @@ class _TrainForward(torch.autograd.Function):
         return (None, None, None, None, None, *[grads.get(id(p)) for p in params])
 
 
+DISTORTIONS = ("mse", "ms-ssim")
+
+
 @torch.no_grad()
-def step_gradients(model, x: torch.Tensor, lambda_rd: float, noise=None, partial_hook=None):
+def step_gradients(model, x: torch.Tensor, lambda_rd: float, noise=None, partial_hook=None, distortion: str = "mse"):
     """forward + rd_loss + backward of one step WITHOUT the autograd engine (everything on the calling thread and its current
     stream - what a CUDA-graph capture needs): accumulates into .grad like loss.backward() and returns
-    (loss [device scalar], per_image [3, B], scalars [8])."""
-    from .RateDistortionLoss import rd_terms
+    (loss [device scalar], per_image [3, B], scalars [8]).  distortion="ms-ssim": the loss of ms_ssim_rd_loss, whose x_hat
+    gradient comes from nic_ms_ssim_bwd; scalars then has a 9th entry, the batch MS-SSIM, and entry 5 is that loss."""
+    from .RateDistortionLoss import check_ms_ssim_shape, ms_ssim_terms, rd_terms
+    if distortion not in DISTORTIONS:
+        raise ValueError(f"distortion must be one of {DISTORTIONS}, got {distortion!r}")
+    if distortion == "ms-ssim":
+        check_ms_ssim_shape(tuple(x.shape))
     B, _, H, W = x.shape
     noise_z, noise_y = draw_noise(model.M, x, noise)
     forget_pairs()
@@ -740,13 +749,17 @@ def step_gradients(model, x: torch.Tensor, lambda_rd: float, noise=None, partial
     x_hat, logp_y, logp_z = outs[:3]
     engine.attach_partials(logp_y, outs[9])
     engine.attach_partials(logp_z, outs[10])
-    per_image, scalars = rd_terms({"x_hat": x_hat, "logp_y": logp_y, "logp_z": logp_z}, x, lambda_rd)
-    # d loss / d logp = -1 / (ln 2 * H * W * B); d loss / d x_hat = lambda * 255^2 * 2 (x_hat - x) / numel  (RateDistortionLoss.py:13-34)
-    gl = torch.full((1,), -1.0 / (math.log(2.0) * H * W * B), dtype=torch.float32, device=x.device)
-    gx = torch.empty_like(x_hat)
-    with torch.cuda.device(x.device):
-        check(_lib.load().nic_sse_bwd(ptr(x_hat), ptr(x), x.numel(), float(lambda_rd) * 65025.0 * 2.0 / x.numel(), ptr(gx), current_stream()),
-              "nic_sse_bwd")
+    if distortion == "ms-ssim":
+        per_image, scalars, _, state = ms_ssim_terms({"x_hat": x_hat, "logp_y": logp_y, "logp_z": logp_z}, x, lambda_rd)
+        gx = ms_ssim_x_hat_grad(state, lambda_rd)
+    else:
+        per_image, scalars = rd_terms({"x_hat": x_hat, "logp_y": logp_y, "logp_z": logp_z}, x, lambda_rd)
+        # d loss / d x_hat = lambda * 255^2 * 2 (x_hat - x) / numel  (RateDistortionLoss.py:13-34)
+        gx = torch.empty_like(x_hat)
+        with torch.cuda.device(x.device):
+            check(_lib.load().nic_sse_bwd(ptr(x_hat), ptr(x), x.numel(), float(lambda_rd) * 65025.0 * 2.0 / x.numel(), ptr(gx), current_stream()),
+                  "nic_sse_bwd")
+    gl = torch.full((1,), -1.0 / (math.log(2.0) * H * W * B), dtype=torch.float32, device=x.device)     # d loss / d logp, both losses
     grads = _backward_impl(model, S, gx, [gl.expand(logp_y.shape)], gl.expand(logp_z.shape), partial_hook=partial_hook)
     for p in model.parameters():
         g = grads.get(id(p))
@@ -784,6 +797,40 @@ class _RDLoss(torch.autograd.Function):
         with torch.cuda.device(x_hat.device):
             check(_lib.load().nic_sse_bwd(ptr(x_hat), ptr(x), x.numel(), coef, ptr(gx), current_stream()), "nic_sse_bwd")
         gx.mul_(g.float())
+        return gl.expand(ctx.shapes[0]), gl.expand(ctx.shapes[1]), gx, None, None, None
+
+
+def ms_ssim_x_hat_grad(state, lambda_rd: float, g: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """d loss / d x_hat of loss = bpp + lambda * (1 - mean ms_ssim) (times the upstream scalar g) through nic_ms_ssim_bwd, from the
+    state ms_ssim_terms returned: the level coefficients are d loss / d term = -lambda / planes * d value / d term."""
+    from .Evaluator import term_grads
+    x_hat, x, terms, value, ws = state
+    b, c, h, w = x.shape
+    coef = term_grads(terms, value) * (-float(lambda_rd) / (b * c))
+    if g is not None:
+        coef = coef * g.float()
+    gx = torch.empty_like(x_hat)
+    with torch.cuda.device(x_hat.device):
+        check(_lib.load().nic_ms_ssim_bwd(ptr(x_hat), ptr(x), b * c, h, w, 1.0, ptr(coef), ptr(gx), ptr(ws), ws.numel(), current_stream()),
+              "nic_ms_ssim_bwd")
+    return gx
+
+
+class _MSSSIMRDLoss(torch.autograd.Function):
+    """loss = bpp_total + lambda * (1 - mean_b ms_ssim_b) (RateDistortionLoss.ms_ssim_rd_loss) as one node: the value comes from
+    ms_ssim_terms, the gradients are d loss / d logp = -1 / (ln 2 * H * W * B) and the x_hat gradient of nic_ms_ssim_bwd."""
+
+    @staticmethod
+    def forward(ctx, logp_y, logp_z, x_hat, lambda_rd, scalars, state):
+        ctx.state, ctx.lambda_rd, ctx.shapes = state, float(lambda_rd), (logp_y.shape, logp_z.shape)
+        return scalars[5].clone()
+
+    @staticmethod
+    def backward(ctx, g):
+        B, _, H, W = ctx.state[1].shape
+        gl = g.float() * (-1.0 / (math.log(2.0) * H * W * B))
+        gx = ms_ssim_x_hat_grad(ctx.state, ctx.lambda_rd, g)
+        ctx.state = None
         return gl.expand(ctx.shapes[0]), gl.expand(ctx.shapes[1]), gx, None, None, None
 
 
