@@ -93,7 +93,8 @@ typedef struct nic_conv_desc {
   int32_t kh, kw, stride, pad;      /* kernel, stride (1|2), padding                            */
   int32_t transposed;               /* 0: Conv2d, 1: ConvTranspose2d                            */
   int32_t output_padding;           /* ConvTranspose2d only                                     */
-  int32_t mask_a;                   /* 1: PixelCNN mask 'A', 2: mask 'B' (ContextModels.py:13-16) */
+  int32_t mask_a;                   /* 1: PixelCNN mask 'A', 2: mask 'B' (ContextModels.py:13-16),
+                                       NIC_MASK_CHECKERBOARD: checkerboard context (see below)  */
   int32_t epilogue;                 /* NIC_EPI_*                                                */
   int32_t precision;                /* NIC_PREC_*                                               */
   int32_t in_layout, out_layout;    /* NIC_LAYOUT_*                                             */
@@ -102,6 +103,14 @@ typedef struct nic_conv_desc {
                                        channels [out_c_offset, out_c_offset + c_out) (makes the
                                        torch.cat of Models.py:73 free); 0,0 = plain             */
 } nic_conv_desc;
+
+/*
+ * Checkerboard context (He et al., CVPR 2021; DESIGN.md section 14).  Anchors are the pixels (i, j) with i + j even, non-anchors
+ * those with i + j odd.  A conv with mask_a = NIC_MASK_CHECKERBOARD keeps only the taps (kh, kw) with kh + kw odd (12 of 25 for
+ * 5x5, no centre tap; the others are dropped, never multiplied), so a non-anchor reads anchors only; nic_conv_fwd then writes 0
+ * into its output channel window at every anchor (nic_checkerboard_zero), bias included.
+ */
+#define NIC_MASK_CHECKERBOARD 3
 
 int nic_version(void);
 const char* nic_last_error(void);
@@ -512,6 +521,33 @@ int nic_codec_decode(int32_t kind, const uint8_t* blob, const int64_t* lane_off,
 int nic_codec_decode_step(const uint8_t* blob, const int64_t* lane_off, const int32_t* lane_words, uint32_t* state, int32_t* pos,
                           int32_t init, const float* params, int32_t b, int32_t m, int32_t k, int32_t h, int32_t w, int32_t lanes, int32_t t,
                           float* out, void* stream);
+/*
+ * Checkerboard coder (DESIGN.md section 14, format 4).  Lanes: lanes_c channel classes x ceil(h / band_rows) row bands; lane
+ * g = img * lanes + r * lanes_c + l (lanes = lanes_c * ceil(h / band_rows)) holds the channels c = l (mod lanes_c) of the latent rows
+ * [r band_rows, (r + 1) band_rows).  Its decode order: pass 0 = the anchors (i + j even) of the band in raster order, each pixel's
+ * channels ascending; pass 1 = the non-anchors likewise.  One rANS stream per lane runs through both passes.
+ *
+ * Encode: as nic_codec_encode(GM) in that order; cap >= 3 * ceil(m / lanes_c) * band_rows * w + 2.
+ */
+int nic_codec_encode_checkerboard(const uint64_t* code, const float* sym, int32_t b, int32_t m, int32_t h, int32_t w, int32_t lanes_c,
+                                  int32_t band_rows, int64_t cap, uint16_t* words, int32_t* count, void* stream);
+/*
+ * Decode pass s (0: anchors, 1: non-anchors) of every lane in one launch: nic_codec_decode_step's kernel (one CTA per (image, lane),
+ * table rows built in shared memory from params by the encoder's function, chunks of 64, one thread decoding) walking the lane's
+ * pixels of the pass instead of a wavefront step.  Pass 0 starts every lane from its segment; pass 1 continues from state / pos
+ * [b * lanes].  params: raw entropy parameters [b, (3K | 2) m, h, w], NCHW f32, exact at the pass's pixels.
+ */
+int nic_codec_decode_pass(const uint8_t* blob, const int64_t* lane_off, const int32_t* lane_words, uint32_t* state, int32_t* pos,
+                          const float* params, int32_t b, int32_t m, int32_t k, int32_t h, int32_t w, int32_t lanes_c, int32_t band_rows,
+                          int32_t pass, float* out, void* stream);
+/*
+ * Writes 0 into channels [c_offset, c_offset + c) of a tensor with c_total channels at every anchor pixel (i + j even) of [n, h, w]:
+ * the anchor zeroing of a checkerboard context conv's output (nic_conv_fwd enqueues it after the conv), and of the gradient of that
+ * output in the training step.  dtype NIC_DT_F32 / NIC_DT_BF16 in NIC_LAYOUT_NHWC or NIC_LAYOUT_NCHW; NIC_DT_BF16X2 (hi / lo pair,
+ * 2 c_total channels [hi | lo]) in NHWC, both halves zeroed.
+ */
+int nic_checkerboard_zero(void* y, int32_t dtype, int32_t layout, int32_t n, int32_t h, int32_t w, int32_t c, int32_t c_total,
+                          int32_t c_offset, void* stream);
 /* out [b] = per image sum over the symbols (y [b, y_per_image] then z [b, z_per_image], NCHW f32) of a 32-bit mix of (index, value),
  * mod 2^32 */
 int nic_codec_checksum(const float* y, int64_t y_per_image, const float* z, int64_t z_per_image, int32_t b, uint32_t* out, void* stream);

@@ -28,7 +28,7 @@ import torch.nn as nn
 from . import engine
 from ._lib import LAYOUT_NCHW, LAYOUT_NHWC, MODEL_PRECISIONS, Q_NOISE, Q_PASSTHRU, Q_ROUND
 from .Components import Decoder5x5, Encoder5x5, HyperDecoder5x5, HyperEncoder5x5
-from .ContextModels import ContextModel
+from .ContextModels import CheckerboardContextModel, ContextModel
 from .EntropyModels import FactorizedEntropyBottleneck, GaussianConditional, GaussianMixtureConditional, gm_likelihood
 from .ParametersModels import EntropyParameters
 
@@ -193,6 +193,7 @@ class JointAutoregressiveHierarchical(nn.Module):
                 (~1e-5 relative; 3x the MMA work), activations carried between layers as bf16 hi/lo pairs - the
                 parity-grade tensor-core arm.
     """
+    context_model_class = ContextModel
 
     def __init__(self, latent_channels: int = 192, K: int = 1, *, precision: Optional[str] = None):
         super().__init__()
@@ -208,7 +209,7 @@ class JointAutoregressiveHierarchical(nn.Module):
         self.hyper_encoder = HyperEncoder5x5(latent_channels=self.M)
         self.hyper_decoder = HyperDecoder5x5(latent_channels=self.M)
         self.factorized_entropy_model = FactorizedEntropyBottleneck(self.M)
-        self.context_model = ContextModel(latent_channels=self.M)
+        self.context_model = self.context_model_class(latent_channels=self.M)
         self.entropy_parameters = EntropyParameters(latent_channels=self.M, hyper_latent_channels=self.H, K=self.K)
         self.precision = engine.resolve_precision(precision, latent_channels)
         if self.precision not in MODEL_PRECISIONS:
@@ -322,6 +323,31 @@ class JointAutoregressiveHierarchical(nn.Module):
         (corrupted bytes, other weights)."""
         from . import codec
         return codec.decompress(self, strings, shape)
+
+
+class JointCheckerboardHierarchical(JointAutoregressiveHierarchical):
+    """JointAutoregressiveHierarchical with the checkerboard context model (He et al., CVPR 2021; convention in ContextModels.py
+    and DESIGN.md section 14): same constructor, attributes, precision arms, output dict and ``state_dict`` keys, modules built in
+    the same order (a seeded build draws the same weights); ``context_model`` is a CheckerboardContextModel.  Anchors (i + j even)
+    are coded from the hyperprior alone, non-anchors from the hyperprior and the anchors, so ``decompress`` runs two parameter passes
+    and two rANS passes at any image size instead of one wavefront step per 3 hy + wy - 3.  Every forward route (eager, graph
+    branches, CtxEpPlan, the layer-by-layer and training forms) gets the anchor zeroing from the conv call itself."""
+    context_model_class = CheckerboardContextModel
+
+    def compress(self, x: torch.Tensor) -> dict:
+        """x [B, 3, H, W] (any H, W >= 1) -> {"strings": [y_strings, z_strings], "shape": (hz, wz)}: one bytes object per
+        image in each list, coded with the eval-mode symbols of x padded by edge replication to multiples of 64 (shape is the
+        padded one).  Format 4: DESIGN.md sections 12 and 14."""
+        from . import checkerboard_codec
+        return checkerboard_codec.compress(self, x)
+
+    def decompress(self, strings, shape) -> dict:
+        """strings / shape as compress returned them (any subset of the images, in any order) -> {"x_hat", "y_hat", "z_hat"}, NCHW f32;
+        x_hat = g_s(y_hat) cropped to the image's size, not clamped; y_hat / z_hat at the padded latent shape.  Raises ValueError on a
+        string of another model, precision arm, M or K, on a malformed string or image size, or when an image's symbol checksum does not
+        match (corrupted bytes, other weights)."""
+        from . import checkerboard_codec
+        return checkerboard_codec.decompress(self, strings, shape)
 
 
 class HierarchicalMixtureResidual(nn.Module):

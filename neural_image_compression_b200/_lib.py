@@ -19,6 +19,7 @@ DT_F32, DT_BF16, DT_BF16X2 = 0, 1, 2
 PREC_FP32, PREC_BF16, PREC_BF16X3 = 0, 1, 2
 EPI_BIAS, EPI_LRELU, EPI_GDN, EPI_IGDN = 0, 1, 2, 3
 Q_ROUND, Q_NOISE, Q_PASSTHRU = 0, 1, 2
+MASK_A, MASK_B, MASK_CHECKERBOARD = 1, 2, 3        # nic_conv_desc.mask_a
 PRECISIONS = {"fp32": PREC_FP32, "bf16": PREC_BF16, "bf16x3": PREC_BF16X3}
 # model-level modes: "mixed" = g_a and h_a (everything upstream of the rounding) in fp32, the rest in bf16
 #                     "bf16x3" = every transform on the tensor cores with hi/lo-split operands (fp32 grade)
@@ -113,6 +114,9 @@ SIGNATURES = {
     "nic_codec_decode": (C.c_int, [_i32, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp]),
     "nic_codec_decode_step": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i32, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp]),
     "nic_codec_checksum": (C.c_int, [_vp, _i64, _vp, _i64, _i32, _vp, _vp]),
+    "nic_codec_encode_checkerboard": (C.c_int, [_vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _i64, _vp, _vp, _vp]),
+    "nic_codec_decode_pass": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp]),
+    "nic_checkerboard_zero": (C.c_int, [_vp, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _vp]),
     "nic_codec_params": (C.c_int, [C.POINTER(CodecHead), _i32, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _vp]),
     "nic_image_window": (C.c_int, [_vp, _i32, _i32, _i32, _vp, _i32, _i32, _vp]),
 }

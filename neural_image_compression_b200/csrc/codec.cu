@@ -1,9 +1,11 @@
 // Entropy coder of JointAutoregressiveHierarchical (DESIGN.md section 9): quantised CDF tables, rANS encode, rANS decode.
 //
 //   codec_table_kernel    the ONE place where floats become integer frequencies (encoder and decoder both call it)
-//   codec_encode_kernel   one thread per (image, lane): the lane's symbols in reverse decode order -> 16-bit words
+//   codec_encode_kernel   one thread per (image, lane): the lane's symbols in reverse decode order (wavefront, raster or
+//                         checkerboard walk) -> 16-bit words
 //   codec_decode_kernel   one thread per (image, lane): one wavefront step of y, or all of z
-//   codec_decode_step_kernel  one CTA per (image, lane): one wavefront step of y, its tables built in shared memory (section 11)
+//   codec_decode_step_kernel  one CTA per (image, lane): one wavefront step of y (section 11) or one checkerboard pass (section 14),
+//                         its tables built in shared memory
 //   codec_checksum_kernel per-image 32-bit checksum of the y and z symbols
 //
 // rANS: 32-bit state in [2^16, 2^32), 16-bit renormalisation words, 16-bit probability precision.  A table row of one
@@ -161,18 +163,51 @@ codec_table_kernel(int kind, int mode, const float* __restrict__ params, const f
   }
 }
 
-// The lane's symbols in DECODE order: kind GM (y) = steps t ascending, pixels of the step with i ascending, channels c = lane,
-// lane + lanes, ... ascending; kind FACTORIZED (z) = pixels in raster order, channels likewise.  The encoder walks it backwards.
+// The lane's symbols in DECODE order, as a sequence of steps, each a run of pixels with the lane's channels per pixel (c = c0,
+// c0 + cl, ... ascending; c0 = lane % cl):
+//   kind GM (y, wavefront)   steps t ascending, pixels of the step with i ascending; cl = lanes
+//   kind FACTORIZED (z)      pixels in raster order, one per step; cl = lanes
+//   kWalkCheckerboard (y)    lane = r * cl + l covers the rows [r band, r band + band): step t = pass s * nb + row i - r band
+//                            (nb = the band's rows), pixels of row i with (i + j + s) even, j ascending - pass 0 the anchors, pass 1
+//                            the non-anchors (DESIGN.md section 14)
+// The encoder walks it backwards.
+constexpr int kWalkCheckerboard = 2;
+
 struct LaneWalk {
-  int kind, m, h, w, lane, lanes;
-  __device__ int steps() const { return kind == NIC_CODEC_GM ? 3 * h + w - 3 : h * w; }
+  int kind, m, h, w, lane, lanes, cl, band;
+  __device__ int c0() const { return lane % cl; }
+  __device__ int row0() const { return (lane / cl) * band; }
+  __device__ int band_rows() const { return min(band, h - row0()); }
+  __device__ int steps() const {
+    return kind == NIC_CODEC_GM ? 3 * h + w - 3 : (kind == kWalkCheckerboard ? 2 * band_rows() : h * w);
+  }
   __device__ void rows(int t, int& i0, int& cnt) const {
     if (kind == NIC_CODEC_GM) step_rows(t, h, w, i0, cnt);
-    else { i0 = t; cnt = 1; }
+    else if (kind == kWalkCheckerboard) {
+      const int nb = band_rows(), s = t / nb;
+      i0 = row0() + t - s * nb;
+      cnt = (w - ((i0 + s) & 1) + 1) / 2;
+    } else { i0 = t; cnt = 1; }
   }
   __device__ long pix(int t, int i0, int p) const {            // pixel index i * w + j of the p-th pixel of step t
     if (kind == NIC_CODEC_GM) { const int i = i0 + p; return static_cast<long>(i) * w + (t - 3 * i); }
+    if (kind == kWalkCheckerboard) return static_cast<long>(i0) * w + ((i0 + t / band_rows()) & 1) + 2 * p;
     return t;
+  }
+  // the steps [t0, t1) as one run: its pixel count and its p-th pixel (<= 16 steps: a checkerboard pass of one band)
+  __device__ int span_count(int t0, int t1) const {
+    int n = 0;
+    for (int t = t0; t < t1; ++t) { int i0, cnt; rows(t, i0, cnt); n += cnt; }
+    return n;
+  }
+  __device__ long span_pix(int t0, int t1, int p) const {
+    for (int t = t0; t < t1; ++t) {
+      int i0, cnt;
+      rows(t, i0, cnt);
+      if (p < cnt) return pix(t, i0, p);
+      p -= cnt;
+    }
+    return 0;                                                  // not reached: p < span_count(t0, t1)
   }
 };
 
@@ -183,22 +218,22 @@ __device__ __forceinline__ void rans_put(uint32_t& x, uint32_t start, uint32_t f
 
 __global__ void __launch_bounds__(64)
 codec_encode_kernel(int kind, const uint64_t* __restrict__ code, const float* __restrict__ sym, int b, int m, int h, int w, int lanes,
-                    long cap, uint16_t* __restrict__ words, int32_t* __restrict__ count) {
+                    int cl, int band, long cap, uint16_t* __restrict__ words, int32_t* __restrict__ count) {
   const int g = blockIdx.x * blockDim.x + threadIdx.x;
   if (g >= b * lanes) return;
   const int img = g / lanes;
-  const LaneWalk lw{kind, m, h, w, g % lanes, lanes};
+  const LaneWalk lw{kind, m, h, w, g % lanes, lanes, cl, band};
   const long hw = static_cast<long>(h) * w;
   uint16_t* row = words + g * cap;
   long wp = cap;
   uint32_t x = kRansL;
-  const int c_last = lw.lane + ((m - 1 - lw.lane) / lanes) * lanes;
+  const int c_last = lw.c0() + ((m - 1 - lw.c0()) / cl) * cl;
   for (int t = lw.steps() - 1; t >= 0; --t) {
     int i0, cnt;
     lw.rows(t, i0, cnt);
     for (int p = cnt - 1; p >= 0; --p) {
       const long pix = lw.pix(t, i0, p);
-      for (int c = c_last; c >= 0; c -= lanes) {
+      for (int c = c_last; c >= 0; c -= cl) {
         const long e = (static_cast<long>(img) * m + c) * hw + pix;
         const uint64_t cd = code[e];
         if (cd >> 32) {                                        // escape: the raw value words first (they decode after the bin)
@@ -243,7 +278,7 @@ codec_decode_kernel(int kind, const uint8_t* __restrict__ blob, const int64_t* _
   const int g = blockIdx.x * blockDim.x + threadIdx.x;
   if (g >= b * lanes) return;
   const int img = g / lanes;
-  const LaneWalk lw{kind, m, h, w, g % lanes, lanes};
+  const LaneWalk lw{kind, m, h, w, g % lanes, lanes, lanes, 0};
   const uint8_t* seg = blob + lane_off[g];
   LaneReader rd{seg + 4, lane_words[g], 0};
   uint32_t x;
@@ -284,37 +319,45 @@ codec_decode_kernel(int kind, const uint8_t* __restrict__ blob, const int64_t* _
   pos[g] = rd.pos;
 }
 
-// One wavefront step of y for one (image, lane) per CTA, tables in shared memory.  The lane's rows of step t, in its decode order
-// (pixels with i ascending, then channels c = lane, lane + lanes, ...), are built by the builder warps with the same element_code as
-// codec_table_kernel, kStepChunk rows at a time into one of two buffers; thread 0 decodes chunk k from one buffer while the
-// builders fill the other with chunk k + 1.  The decode arithmetic is codec_decode_kernel's, so symbols, states and read positions
-// are the same bits.  Every loop count is fixed by the shapes: a corrupted string only changes the values decoded.
+// The steps [t0, t1) of the lane walk of y for one (image, lane) per CTA, tables in shared memory: one wavefront step (section 11)
+// or one checkerboard pass (section 14; t0, t1 = pass * nb, (pass + 1) * nb with the lane's band of nb rows).  The lane's rows
+// in its decode order are built by the builder warps with the same element_code as codec_table_kernel, kStepChunk rows at a time
+// into one of two buffers; thread 0 decodes chunk k from one buffer while the builders fill the other with chunk k + 1.  The
+// decode arithmetic is codec_decode_kernel's, so symbols, states and read positions are the same bits.  Every loop count is fixed
+// by the shapes: a corrupted string only changes the values decoded.
 constexpr int kStepChunk = 64;                                 // rows per chunk: one per builder thread
 constexpr int kStepThreads = 32 + kStepChunk;                  // warp 0 decodes, warps 1 .. 2 build
-constexpr size_t kStepSmem = 2ull * kStepChunk * (kRow * sizeof(uint32_t) + 2 * sizeof(int32_t));
+constexpr size_t kStepSmem = 2ull * kStepChunk * (kRow * sizeof(uint32_t) + 3 * sizeof(int32_t));
 
 __global__ void __launch_bounds__(kStepThreads)
 codec_decode_step_kernel(const uint8_t* __restrict__ blob, const int64_t* __restrict__ lane_off, const int32_t* __restrict__ lane_words,
                          uint32_t* __restrict__ state, int32_t* __restrict__ pos, int init, const float* __restrict__ params, int m,
-                         int K, int h, int w, int lanes, int t, int i0, int cnt, float* __restrict__ out) {
+                         int K, int kind, int h, int w, int lanes, int cl, int band, int t, float* __restrict__ out) {
   extern __shared__ __align__(16) uint32_t s_step[];
   uint32_t* s_cdf = s_step;                                    // [2][kStepChunk][kRow]
   int32_t* s_lo = reinterpret_cast<int32_t*>(s_step + 2 * kStepChunk * kRow);
   int32_t* s_n = s_lo + 2 * kStepChunk;
-  const int g = blockIdx.x, img = g / lanes, lane = g % lanes;
-  const int nc = (m - 1 - lane) / lanes + 1;                   // channels of this lane
-  const int rows = cnt * nc, chunks = (rows + kStepChunk - 1) / kStepChunk;
+  int32_t* s_pix = s_n + 2 * kStepChunk;                       // the row's pixel i * w + j
+  const int g = blockIdx.x, img = g / lanes;
+  const LaneWalk lw{kind, m, h, w, g % lanes, lanes, cl, band};
+  const int c0 = lw.c0();
+  // t: the wavefront step, or the checkerboard pass
+  const int t0 = kind == kWalkCheckerboard ? t * lw.band_rows() : t, t1 = kind == kWalkCheckerboard ? t0 + lw.band_rows() : t + 1;
+  const int nc = (m - 1 - c0) / cl + 1;                        // channels of this lane
+  const int rows = lw.span_count(t0, t1) * nc, chunks = (rows + kStepChunk - 1) / kStepChunk;
   const long hw = static_cast<long>(h) * w;
   const int np = K == 1 ? 2 : 3 * K;
 
   auto build = [&](int k) {                                    // builder thread: row k * kStepChunk + (tid - 32) into buffer k & 1
     const int b = threadIdx.x - 32, r = k * kStepChunk + b;
     if (r >= rows) return;
-    const int p = r / nc, c = lane + (r - p * nc) * lanes, i = i0 + p;
-    const float* src = params + (static_cast<long>(img) * np * m + c) * hw + static_cast<long>(i) * w + (t - 3 * i);
+    const int p = r / nc, c = c0 + (r - p * nc) * cl;
+    const long pix = lw.span_pix(t0, t1, p);
+    const float* src = params + (static_cast<long>(img) * np * m + c) * hw + pix;
     float q[15];
     for (int j = 0; j < np; ++j) q[j] = __ldg(src + static_cast<long>(j) * m * hw);
     const int e = (k & 1) * kStepChunk + b;
+    s_pix[e] = static_cast<int32_t>(pix);
     element_code(NIC_CODEC_GM, K, q, kNoSymbol, s_cdf + e * kRow, s_lo + e, s_n + e);
   };
 
@@ -354,8 +397,8 @@ codec_decode_step_kernel(const uint8_t* __restrict__ blob, const int64_t* __rest
         } else {
           v = static_cast<float>(s_lo[e] + a);
         }
-        const int p = r / nc, c = lane + (r - p * nc) * lanes, i = i0 + p;
-        out[(static_cast<long>(img) * hw + static_cast<long>(i) * w + (t - 3 * i)) * m + c] = v;
+        const int p = r / nc, c = c0 + (r - p * nc) * cl;
+        out[(static_cast<long>(img) * hw + s_pix[e]) * m + c] = v;
       }
     }
     __syncthreads();                                           // chunk k decoded, chunk k + 1 built
@@ -421,7 +464,7 @@ int nic_codec_encode(int32_t kind, const uint64_t* code, const float* sym, int32
     return fail(NIC_E_BADSHAPE, "codec_encode: b=%d m=%d h=%d w=%d lanes=%d", b, m, h, w, lanes);
   if (cap < 3L * ((m + lanes - 1) / lanes) * h * w + 2) return fail(NIC_E_WORKSPACE, "codec_encode: lane capacity %lld words", static_cast<long long>(cap));
   if (!code || !sym || !words || !count) return fail(NIC_E_BADSHAPE, "codec_encode: null pointer");
-  codec_encode_kernel<<<(b * lanes + 63) / 64, 64, 0, as_stream(stream)>>>(kind, code, sym, b, m, h, w, lanes, cap, words, count);
+  codec_encode_kernel<<<(b * lanes + 63) / 64, 64, 0, as_stream(stream)>>>(kind, code, sym, b, m, h, w, lanes, lanes, 0, cap, words, count);
   return check_launch("codec_encode_kernel");
 }
 
@@ -447,10 +490,43 @@ int nic_codec_decode_step(const uint8_t* blob, const int64_t* lane_off, const in
   if (t < 0 || t >= 3 * h + w - 3) return fail(NIC_E_BADSHAPE, "codec_decode_step: step %d of %d", t, 3 * h + w - 3);
   if (!blob || !lane_off || !lane_words || !state || !pos || !params || !out) return fail(NIC_E_BADSHAPE, "codec_decode_step: null pointer");
   if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(codec_decode_step_kernel), static_cast<int>(kStepSmem))) return rc;
-  int i0, cnt;
-  step_rows(t, h, w, i0, cnt);
   codec_decode_step_kernel<<<b * lanes, kStepThreads, kStepSmem, as_stream(stream)>>>(blob, lane_off, lane_words, state, pos, init, params,
-                                                                                      m, k, h, w, lanes, t, i0, cnt, out);
+                                                                                      m, k, NIC_CODEC_GM, h, w, lanes, lanes, 0, t, out);
+  return check_launch("codec_decode_step_kernel");
+}
+
+static int checkerboard_lanes(const char* what, int32_t b, int32_t m, int32_t h, int32_t w, int32_t lanes_c, int32_t band_rows, int* lanes) {
+  if (b < 1 || m < 1 || h < 1 || w < 1 || lanes_c < 1 || lanes_c > m || band_rows < 1)
+    return fail(NIC_E_BADSHAPE, "%s: b=%d m=%d h=%d w=%d lanes_c=%d band_rows=%d", what, b, m, h, w, lanes_c, band_rows);
+  *lanes = lanes_c * ((h + band_rows - 1) / band_rows);
+  return NIC_OK;
+}
+
+int nic_codec_encode_checkerboard(const uint64_t* code, const float* sym, int32_t b, int32_t m, int32_t h, int32_t w, int32_t lanes_c,
+                                  int32_t band_rows, int64_t cap, uint16_t* words, int32_t* count, void* stream) {
+  if (int rc = nic_check_device()) return rc;
+  int lanes;
+  if (int rc = checkerboard_lanes("codec_encode_checkerboard", b, m, h, w, lanes_c, band_rows, &lanes)) return rc;
+  if (cap < 3L * ((m + lanes_c - 1) / lanes_c) * band_rows * w + 2)
+    return fail(NIC_E_WORKSPACE, "codec_encode_checkerboard: lane capacity %lld words", static_cast<long long>(cap));
+  if (!code || !sym || !words || !count) return fail(NIC_E_BADSHAPE, "codec_encode_checkerboard: null pointer");
+  codec_encode_kernel<<<(b * lanes + 63) / 64, 64, 0, as_stream(stream)>>>(kWalkCheckerboard, code, sym, b, m, h, w, lanes, lanes_c, band_rows,
+                                                                           cap, words, count);
+  return check_launch("codec_encode_kernel");
+}
+
+int nic_codec_decode_pass(const uint8_t* blob, const int64_t* lane_off, const int32_t* lane_words, uint32_t* state, int32_t* pos,
+                          const float* params, int32_t b, int32_t m, int32_t k, int32_t h, int32_t w, int32_t lanes_c, int32_t band_rows,
+                          int32_t pass, float* out, void* stream) {
+  if (int rc = nic_check_device()) return rc;
+  int lanes;
+  if (int rc = checkerboard_lanes("codec_decode_pass", b, m, h, w, lanes_c, band_rows, &lanes)) return rc;
+  if (k < 1 || k > 5 || (pass != 0 && pass != 1)) return fail(NIC_E_BADSHAPE, "codec_decode_pass: k=%d pass=%d", k, pass);
+  if (!blob || !lane_off || !lane_words || !state || !pos || !params || !out) return fail(NIC_E_BADSHAPE, "codec_decode_pass: null pointer");
+  if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(codec_decode_step_kernel), static_cast<int>(kStepSmem))) return rc;
+  codec_decode_step_kernel<<<b * lanes, kStepThreads, kStepSmem, as_stream(stream)>>>(blob, lane_off, lane_words, state, pos, pass == 0,
+                                                                                      params, m, k, kWalkCheckerboard, h, w, lanes, lanes_c,
+                                                                                      band_rows, pass, out);
   return check_launch("codec_decode_step_kernel");
 }
 

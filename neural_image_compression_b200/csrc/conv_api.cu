@@ -13,6 +13,30 @@ int pack_weight_tc(const nic_conv_desc*, const TapTable&, const float*, void*, c
 int pack_gdn_tc(int32_t, float, const float*, const float*, float*, void*, int32_t, cudaStream_t);
 size_t packed_weight_elems_tc(const nic_conv_desc*, const TapTable&);
 size_t conv_workspace_bytes_tc(const nic_conv_desc*);
+
+// Anchor zeroing of the checkerboard context (include/nic.h, NIC_MASK_CHECKERBOARD): one thread per (anchor pixel, channel of the
+// window); `elem` = bytes per element (4: f32, 2: bf16), `halves` = 2 for a hi / lo pair (the lo half c_total channels further on).
+__global__ void __launch_bounds__(256)
+checkerboard_zero_kernel(char* __restrict__ y, int elem, int nchw, int halves, int n, int h, int w, int c, int c_total, int c_offset) {
+  const int wa = (w + 1) / 2;                                    // anchors of a row (at most)
+  const long total = static_cast<long>(n) * h * wa * c;
+  for (long e = static_cast<long>(blockIdx.x) * blockDim.x + threadIdx.x; e < total; e += static_cast<long>(gridDim.x) * blockDim.x) {
+    const int ch = static_cast<int>(e % c);
+    const long pr = e / c;
+    const int k = static_cast<int>(pr % wa), i = static_cast<int>((pr / wa) % h);
+    const long img = pr / (static_cast<long>(wa) * h);
+    const int j = (i & 1) + 2 * k;
+    if (j >= w) continue;
+    for (int half = 0; half < halves; ++half) {
+      const long cc = c_offset + ch + static_cast<long>(half) * c_total;
+      const long idx = nchw ? ((img * c_total + cc) * h + i) * w + j
+                            : ((img * h + i) * w + j) * (static_cast<long>(halves) * c_total) + cc;
+      if (elem == 4) reinterpret_cast<float*>(y)[idx] = 0.f;
+      else reinterpret_cast<unsigned short*>(y)[idx] = 0;
+    }
+  }
+}
+
 }  // namespace nic
 
 using namespace nic;
@@ -80,15 +104,39 @@ int nic_conv_fwd_ex(const nic_conv_desc* d, const void* x, const void* w_packed,
   if (int rc = validate_conv_desc(d)) return rc;
   if (d->n == 0) return NIC_OK;
   if (!x || !w_packed || !bias || !y) return fail(NIC_E_BADSHAPE, "conv: null pointer");
+  int rc;
   switch (d->precision) {
     case NIC_PREC_FP32:
-      return conv_fwd_fp32(d, x, w_packed, bias, gdn_gamma, gdn_beta, y, workspace, workspace_bytes, as_stream(stream));
+      rc = conv_fwd_fp32(d, x, w_packed, bias, gdn_gamma, gdn_beta, y, workspace, workspace_bytes, as_stream(stream));
+      break;
     case NIC_PREC_BF16:
     case NIC_PREC_BF16X3:
-      return conv_fwd_tc(d, x, w_packed, bias, gdn_gamma, gdn_beta, y, workspace, workspace_bytes, as_stream(stream), in_lo_nonzero);
+      rc = conv_fwd_tc(d, x, w_packed, bias, gdn_gamma, gdn_beta, y, workspace, workspace_bytes, as_stream(stream), in_lo_nonzero);
+      break;
     default:
       return fail(NIC_E_BADSHAPE, "conv: precision %d", d->precision);
   }
+  if (rc || d->mask_a != NIC_MASK_CHECKERBOARD) return rc;
+  // checkerboard context: phi = 0 at the anchors (bias included), a separate launch after the conv
+  return nic_checkerboard_zero(y, d->out_dtype, d->out_layout, d->n, d->h_out, d->w_out, d->c_out, d->out_c_total ? d->out_c_total : d->c_out,
+                               d->out_c_offset, stream);
+}
+
+int nic_checkerboard_zero(void* y, int32_t dtype, int32_t layout, int32_t n, int32_t h, int32_t w, int32_t c, int32_t c_total,
+                          int32_t c_offset, void* stream) {
+  if (n < 0 || h < 1 || w < 1 || c < 1 || c_offset < 0 || c_offset + c > c_total)
+    return fail(NIC_E_BADSHAPE, "checkerboard_zero: n=%d h=%d w=%d window [%d,+%d) of %d channels", n, h, w, c_offset, c, c_total);
+  if (dtype != NIC_DT_F32 && dtype != NIC_DT_BF16 && dtype != NIC_DT_BF16X2) return fail(NIC_E_BADSHAPE, "checkerboard_zero: dtype %d", dtype);
+  if (layout != NIC_LAYOUT_NHWC && (layout != NIC_LAYOUT_NCHW || dtype == NIC_DT_BF16X2))
+    return fail(NIC_E_BADSHAPE, "checkerboard_zero: layout %d with dtype %d", layout, dtype);
+  if (!y) return fail(NIC_E_BADSHAPE, "checkerboard_zero: null pointer");
+  if (n == 0) return NIC_OK;
+  const long total = static_cast<long>(n) * h * ((w + 1) / 2) * c;
+  const long blocks = (total + 255) / 256 < 4096 ? (total + 255) / 256 : 4096;
+  checkerboard_zero_kernel<<<static_cast<unsigned>(blocks), 256, 0, as_stream(stream)>>>(
+      static_cast<char*>(y), dtype == NIC_DT_F32 ? 4 : 2, layout == NIC_LAYOUT_NCHW, dtype == NIC_DT_BF16X2 ? 2 : 1, n, h, w, c, c_total,
+      c_offset);
+  return check_launch("checkerboard_zero_kernel");
 }
 
 int nic_ctx_ep_fwd(const nic_ctx_ep_args* a, void* stream) {

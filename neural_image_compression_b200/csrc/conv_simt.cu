@@ -36,6 +36,8 @@ int validate_conv_desc(const nic_conv_desc* d) {
   if (d->out_c_total != 0 && (d->out_c_offset < 0 || d->out_c_offset + d->c_out > d->out_c_total))
     return fail(NIC_E_BADSHAPE, "conv: channel window [%d,+%d) outside %d", d->out_c_offset, d->c_out, d->out_c_total);
   if (d->epilogue < NIC_EPI_BIAS || d->epilogue > NIC_EPI_IGDN) return fail(NIC_E_BADSHAPE, "conv: epilogue %d", d->epilogue);
+  if (d->mask_a == NIC_MASK_CHECKERBOARD && (d->stride != 1 || d->epilogue != NIC_EPI_BIAS))
+    return fail(NIC_E_UNSUPPORTED, "conv: the checkerboard context needs stride 1 and the bias epilogue");
   return NIC_OK;
 }
 
@@ -48,7 +50,11 @@ int build_tap_table(const nic_conv_desc* d, TapTable* t) {
     t->py[0] = t->px[0] = 0; t->phase_begin[0] = 0;
     for (int kh = 0; kh < d->kh; ++kh)
       for (int kw = 0; kw < d->kw; ++kw) {
-        if (d->mask_a && !(kh < d->kh / 2 || (kh == d->kh / 2 && kw < d->kw / 2 + (d->mask_a == 2 ? 1 : 0)))) continue;   // 'A'; 2 = 'B': centre tap kept
+        if (d->mask_a == NIC_MASK_CHECKERBOARD) {
+          if (!((kh + kw) & 1)) continue;                      // checkerboard: only the odd-parity taps, which read anchors
+        } else if (d->mask_a && !(kh < d->kh / 2 || (kh == d->kh / 2 && kw < d->kw / 2 + (d->mask_a == 2 ? 1 : 0)))) {
+          continue;                                            // 'A'; 2 = 'B': centre tap kept
+        }
         t->dy[q] = kh - d->pad; t->dx[q] = kw - d->pad; t->kh[q] = kh; t->kw[q] = kw; ++q;
       }
     t->phase_begin[1] = q;

@@ -279,6 +279,13 @@ def latent_handoff(v_nhwc: torch.Tensor, qmode: int, noise: Optional[torch.Tenso
     return v, v_in, v_in_nhwc, v_lowp
 
 
+def checkerboard_zero_(t: torch.Tensor) -> torch.Tensor:
+    """In place: 0 at the anchors (i + j even) of a contiguous NHWC f32 tensor [n, h, w, c] (nic_checkerboard_zero)."""
+    n, h, w, c = t.shape
+    check(_lib.load().nic_checkerboard_zero(ptr(t), DT_F32, LAYOUT_NHWC, n, h, w, c, c, 0, current_stream()), "nic_checkerboard_zero")
+    return t
+
+
 def attach_partials(logp: torch.Tensor, parts: torch.Tensor) -> None:
     """Let the per-image partial sums the likelihood kernel produced ride along with `logp` for rd_loss (RateDistortionLoss.py:
     13-14), together with logp's version: a caller that modifies logp in place invalidates them (rd_loss then re-sums)."""

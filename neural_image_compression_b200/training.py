@@ -45,7 +45,9 @@ import torch
 import torch.nn as nn
 
 from . import _lib, engine
-from ._lib import (ConvDesc, DT_F32, EPI_BIAS, EPI_LRELU, LAYOUT_NCHW, LAYOUT_NHWC, PREC_FP32, Q_NOISE, Q_PASSTHRU, Q_ROUND, check, current_stream, ptr)
+from .engine import checkerboard_zero_
+from ._lib import (ConvDesc, DT_F32, EPI_BIAS, EPI_LRELU, LAYOUT_NCHW, LAYOUT_NHWC, MASK_CHECKERBOARD, PREC_FP32, Q_NOISE, Q_PASSTHRU, Q_ROUND,
+                   check, current_stream, ptr)
 from .EntropyModels import gm_likelihood
 from .Models import draw_noise, mixture_params, single_head_outputs
 
@@ -150,7 +152,7 @@ def forget_pairs():
     _PAIRS.clear()
 
 
-def _train_op(conv: nn.Module, epilogue: int, mask_a: bool = False) -> engine.ConvOp:
+def _train_op(conv: nn.Module, epilogue: int, mask_a: int = 0) -> engine.ConvOp:
     """ConvOp of a layer WITHOUT its GDN (the training step keeps the pre-GDN tensor), cached on the module."""
     cache = conv.__dict__.setdefault("_nic_train_ops", {})
     key = (epilogue, mask_a)
@@ -166,8 +168,9 @@ def _is_first_layer_shape(conv: nn.Module) -> bool:
 
 def conv_forward(arm: str, conv: nn.Module, epilogue: int, x: torch.Tensor, n: int, h: int, w: int, in_layout: int = LAYOUT_NHWC,
                  out_layout: int = LAYOUT_NHWC, out: Optional[torch.Tensor] = None, out_c_total: int = 0, out_c_offset: int = 0,
-                 mask_a: bool = False, pair_out: bool = False) -> torch.Tensor:
+                 mask_a: int = 0, pair_out: bool = False) -> torch.Tensor:
     """One conv (+ bias / LeakyReLU) with f32 tensors at both ends; the contraction on the tensor cores in the bf16x3 arm.
+    mask_a: the nic_conv_desc mask code of a context conv (its module's `_op.mask_a`), 0 for a plain conv.
     pair_out (evaluation chains of the residual family): where the tensor-core kernel runs, leave the result as the bf16 hi/lo
     pair the next conv consumes (no f32 round trip, no nic_to_pair launch); x may itself be such a pair."""
     op = _train_op(conv, epilogue, mask_a)
@@ -513,7 +516,8 @@ def head_forward(arm: str, head, K: int, y_i: torch.Tensor, y_i_nhwc: torch.Tens
     ctx, ep, c0, c1 = head
     B, hy, wy, _ = y_i_nhwc.shape
     ctx.masked.apply_mask_()
-    conv_forward(arm, ctx.masked, EPI_BIAS, y_i_nhwc, B, hy, wy, out=comb, out_c_total=comb.shape[-1], out_c_offset=0, mask_a=True)
+    conv_forward(arm, ctx.masked, EPI_BIAS, y_i_nhwc, B, hy, wy, out=comb, out_c_total=comb.shape[-1], out_c_offset=0,
+                 mask_a=ctx.masked._op.mask_a)
     ops = ep.ops
     e1 = conv_forward(arm, ops[0].conv, ops[0].epilogue, comb, B, hy, wy)
     e2 = conv_forward(arm, ops[1].conv, ops[1].epilogue, e1, B, hy, wy)
@@ -541,6 +545,8 @@ def head_backward(arm: str, head, K: int, st: dict, g_logp: torch.Tensor, put, w
     w0 = ops[0].conv.weight.detach()
     d_phi = conv_dgrad(ops[0].conv, g, B, hy, wy, weight=w0[:, :2 * m].contiguous(), c_in=2 * m, arm=arm)
     d_psi = conv_dgrad(ops[0].conv, g, B, hy, wy, weight=w0[:, 2 * m:].contiguous(), c_in=w0.shape[1] - 2 * m, arm=arm)
+    if ctx.masked._op.mask_a == MASK_CHECKERBOARD:
+        checkerboard_zero_(d_phi)                                # phi is the constant 0 at the anchors
     dw, db = wgrad(ctx.masked, st["y_i_nhwc"], d_phi, B, hy, wy, LAYOUT_NHWC, LAYOUT_NHWC, arm=arm)
     put(ctx.masked.weight, dw); put(ctx.masked.bias, db)
     return add_(d_y, conv_dgrad(ctx.masked, d_phi, B, hy, wy, arm=arm)), d_psi
