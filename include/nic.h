@@ -409,6 +409,10 @@ int nic_factorized_likelihood_bwd(const float* z_in, const float* fparams, const
 
 /* g_x_hat = coef * (x_hat - x): backward of the MSE term (RateDistortionLoss.py:26-34; coef = g_loss * lambda * 255^2 * 2 / (B*C*H*W)) */
 int nic_sse_bwd(const float* x_hat, const float* x, int64_t n, float coef, float* g_x_hat, void* stream);
+/* The same with one coefficient per image: g_x_hat[i] = coef[i / per_image] * (x_hat[i] - x[i]) over b images (coef: device [b]) -
+ * the MSE backward of a batch trained at per-image lambdas (gain units, DESIGN.md section 15) */
+int nic_sse_bwd_per_image(const float* x_hat, const float* x, int32_t b, int64_t per_image, const float* coef, float* g_x_hat,
+                          void* stream);
 
 /* dst += src */
 int nic_add_inplace(float* dst, const float* src, int64_t n, void* stream);
@@ -591,6 +595,45 @@ int nic_codec_params(const nic_codec_head* heads, int32_t n_heads, const float* 
  */
 int nic_image_window(const float* src, int32_t planes, int32_t h_src, int32_t w_src, float* dst, int32_t h_dst, int32_t w_dst,
                      void* stream);
+
+/* ---- gain units (GainedCheckerboardHierarchical, DESIGN.md section 15) -------------------------------------------------- */
+
+/*
+ * Per-image gain vectors out [4, B, M] = (g_y, ginv_y, g_z, ginv_z) from the four log-gain tables [L, M] and the quality codes
+ * q_code [B] (device int32, q = q_code / 1024 in [0, L - 1]): l = floor(q), t = q - l, out = expf((1 - t) log[l] + t log[min(l + 1,
+ * L - 1)]).  The forward, the encoder and the decoder all use it, so the gains are the same bits in every direction.  No host
+ * synchronisation (graph-capturable).
+ */
+int nic_gain_vectors(const float* y_log_gain, const float* y_log_inv_gain, const float* z_log_gain, const float* z_log_inv_gain,
+                     int32_t L, int32_t M, const int32_t* q_code, int32_t B, float* out, void* stream);
+
+/*
+ * nic_latent_handoff_ex with gain units: v_g = gain (.) v (gain [n, c] per image and channel, NULL = 1) is the tensor that is
+ * quantised (qmode) and written to v_nchw; v_src_nhwc (optional) receives v_g NHWC in src_dtype (f32, bf16 or bf16 pair: h_a's
+ * input).  The symbols go to v_in_nchw / v_in_nhwc (out_dtype, with the lo-half flag in_lo_nonzero) as in nic_latent_handoff_ex.
+ * scaled_nhwc (optional) receives inv_gain (.) v_in (inv_gain [n, c], NULL = 1) NHWC in scaled_dtype: g_s's or h_s's input.  It
+ * never sets the flag (it is not integer).  Any output may be NULL.
+ */
+int nic_latent_handoff_gain(const float* v_nhwc, int32_t n, int32_t c, int32_t h, int32_t w, int32_t qmode, const float* noise_nchw,
+                            const float* gain, float* v_nchw, float* v_in_nchw, void* v_in_nhwc, int32_t out_dtype,
+                            int32_t* in_lo_nonzero, void* v_src_nhwc, int32_t src_dtype, const float* inv_gain, void* scaled_nhwc,
+                            int32_t scaled_dtype, void* stream);
+
+/*
+ * Gain backward over NHWC f32 tensors [n, hw, c]: dst = factor (.) grad (accumulate = 1: dst += factor (.) grad; dst may be grad
+ * itself) and dgain [n, c] = sum over the pixels of grad (.) other.  dst or dgain may be NULL.  Fixed-order double reduction, no
+ * atomics: bitwise repeatable and independent of the batch.
+ */
+int nic_gain_bwd(const float* grad, const float* factor, const float* other, int32_t n, int32_t c, int64_t hw, float* dst,
+                 int32_t accumulate, float* dgain, void* stream);
+
+/*
+ * Fold of the per-image gain-vector gradients d_gains [4, B, M] (with the gains [4, B, M] of nic_gain_vectors) into the gradients of
+ * the four log-gain tables d_tables [4, L, M] (overwritten): d log[l] += (1 - t_b) g_b dg_b, d log[l + 1] += t_b g_b dg_b, images in
+ * order.
+ */
+int nic_gain_fold(const float* gains, const float* d_gains, const int32_t* q_code, int32_t B, int32_t L, int32_t M, float* d_tables,
+                  void* stream);
 
 #ifdef __cplusplus
 }

@@ -19,13 +19,14 @@ the host):
 from __future__ import annotations
 
 import contextlib
+import math
 import os
 from typing import Optional, Tuple
 
 import torch
 import torch.nn as nn
 
-from . import engine
+from . import _lib, engine
 from ._lib import LAYOUT_NCHW, LAYOUT_NHWC, MODEL_PRECISIONS, Q_NOISE, Q_PASSTHRU, Q_ROUND
 from .Components import Decoder5x5, Encoder5x5, HyperDecoder5x5, HyperEncoder5x5
 from .ContextModels import CheckerboardContextModel, ContextModel
@@ -104,12 +105,9 @@ def two_head_outputs(x_hat, logp_y1, logp_y2, logp_z, y, y_in, z, z_in, p_z, p_y
 
 # ---- stages of the fused pair-tensor pipeline (JointAutoregressiveHierarchical, ScalableImageCoding's bf16x3 arm, the codec) ----
 
-def fused_g_a(model, x, training, noise_y, prec_up, prec):
-    """g_a -> y hand-off of the fused pipeline (Models.py:52, 57-64): activations NHWC between layers (bf16 hi/lo pairs in the bf16x3
-    arm).  Returns (y, y_in, y_in_nhwc, y_src) with y_src = the unquantised y in the engine's layout for h_a (Models.py:53)."""
+def _g_a_nhwc(model, x, prec_up):
+    """g_a of the fused pipeline: activations NHWC between layers (bf16 hi/lo pairs in the bf16x3 arm) -> y f32 [B, hy, wy, M]."""
     B, _, H, W = x.shape
-    adt = engine.act_dtype(prec)
-    pair = prec == "bf16x3"
     a, h, w, layout = x, H, W, LAYOUT_NCHW
     enc = model.encoder.ops
     for i, op in enumerate(enc):
@@ -117,23 +115,58 @@ def fused_g_a(model, x, training, noise_y, prec_up, prec):
                    out_dtype=torch.float32 if i == len(enc) - 1 else None)
         h, w = engine.conv_out_hw(op.conv, h, w)
         layout = LAYOUT_NHWC
-    y_nhwc = a                                                     # f32 [B, hy, wy, M]
+    return a
+
+
+def fused_g_a(model, x, training, noise_y, prec_up, prec):
+    """g_a -> y hand-off of the fused pipeline (Models.py:52, 57-64).  Returns (y, y_in, y_in_nhwc, y_src) with y_src = the
+    unquantised y in the engine's layout for h_a (Models.py:53)."""
+    adt = engine.act_dtype(prec)
+    pair = prec == "bf16x3"
+    y_nhwc = _g_a_nhwc(model, x, prec_up)
     lowp = prec_up != "fp32"
     y, y_in, y_in_nhwc, y_lowp = engine.latent_handoff(y_nhwc, Q_NOISE if training else Q_ROUND, noise_y, "bf16x2" if pair else adt,
                                                        want_lowp=lowp, lowp_pair=prec_up == "bf16x3")
     return y, y_in, y_in_nhwc, (y_lowp if lowp else y_nhwc)
 
 
-def fused_h_a(model, y_src, B, hy, wy, training, noise_z, prec_up, prec):
-    """h_a -> z hand-off (Models.py:53, 57-64).  Returns (z, z_in, z_in_nhwc)."""
-    adt = engine.act_dtype(prec)
+def _h_a_nhwc(model, y_src, B, hy, wy, prec_up):
     a, h, w = y_src, hy, wy
     ha = model.hyper_encoder.ops
     for i, op in enumerate(ha):
         a = op.run(a, B, h, w, prec_up, out_dtype=torch.float32 if i == len(ha) - 1 else None)
         h, w = engine.conv_out_hw(op.conv, h, w)
-    z, z_in, z_in_nhwc, _ = engine.latent_handoff(a, Q_NOISE if training else Q_ROUND, noise_z, "bf16x2" if prec == "bf16x3" else adt)
+    return a
+
+
+def fused_h_a(model, y_src, B, hy, wy, training, noise_z, prec_up, prec):
+    """h_a -> z hand-off (Models.py:53, 57-64).  Returns (z, z_in, z_in_nhwc)."""
+    adt = engine.act_dtype(prec)
+    z, z_in, z_in_nhwc, _ = engine.latent_handoff(_h_a_nhwc(model, y_src, B, hy, wy, prec_up), Q_NOISE if training else Q_ROUND,
+                                                  noise_z, "bf16x2" if prec == "bf16x3" else adt)
     return z, z_in, z_in_nhwc
+
+
+def engine_dtype(prec: str):
+    """The hand-off dtype of the activations a transform of arm `prec` reads (latent_handoff's in_dtype)."""
+    return "bf16x2" if prec == "bf16x3" else engine.act_dtype(prec)
+
+
+def fused_g_a_gained(model, x, training, noise_y, prec_up, prec, gains: "Gains"):
+    """fused_g_a with gain units: y = g_y (.) g_a(x) is the tensor that is quantised.  Returns (y, y_in, y_in_nhwc, y_src, gs_in):
+    the symbols y_in_nhwc (with their lo-half flag) for the context conv, y_src = y for h_a, gs_in = ginv_y (.) y_in for g_s,
+    all written by one nic_latent_handoff_gain pass."""
+    src = torch.float32 if prec_up == "fp32" else ("bf16x2" if prec_up == "bf16x3" else torch.bfloat16)
+    return engine.latent_handoff_gain(_g_a_nhwc(model, x, prec_up), Q_NOISE if training else Q_ROUND, noise_y, gains.g_y, gains.ginv_y,
+                                      engine_dtype(prec), src, engine_dtype(prec))
+
+
+def fused_h_a_gained(model, y_src, B, hy, wy, training, noise_z, prec_up, prec, gains: "Gains"):
+    """fused_h_a with gain units: z = g_z (.) h_a(y) is quantised.  Returns (z, z_in, hs_in) with hs_in = ginv_z (.) z_in, h_s's
+    input (no lo-half flag: it is not integer)."""
+    z, z_in, _, _, hs_in = engine.latent_handoff_gain(_h_a_nhwc(model, y_src, B, hy, wy, prec_up), Q_NOISE if training else Q_ROUND,
+                                                      noise_z, gains.g_z, gains.ginv_z, None, None, engine_dtype(prec))
+    return z, z_in, hs_in
 
 
 def fused_h_s_into(model, z_in_nhwc, B, hz, wz, prec, combined, c_total, c_offset, lo_flag):
@@ -224,13 +257,17 @@ class JointAutoregressiveHierarchical(nn.Module):
         lean  : skip materialising weights/mus/sigmas (mu/sigma); those keys are then absent.
         """
         check_input(x)
+        return self._forward(x, training, noise, lean, None)
+
+    def _forward(self, x, training, noise, lean, gains: Optional["Gains"]):
+        """forward with the gain units' per-image vectors (GainedCheckerboardHierarchical), or None for the model without them."""
         B, _, H, W = x.shape
         if training and torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
             # the reference's training call (Trainer.py:82): autograd is on, so the step must be differentiable.  One autograd
             # node over the fp32 arm with hand-written backward kernels (training.py); under torch.no_grad() the call below
             # runs the forward-only path of self.precision instead.
             from . import training as _training
-            return _training.train_forward(self, x, noise=noise, lean=lean)
+            return _training.train_forward(self, x, noise=noise, lean=lean, gains=gains)
         if self.precision == "bf16x3" and self.M not in (128, 192):
             # the fused pair-tensor pipeline (GDN kernels, first layer) is built for 128 and 192 channels (the reference's default);
             # other channel counts that are multiples of 64 run layer by layer: every conv and both GDN contractions on the
@@ -242,7 +279,7 @@ class JointAutoregressiveHierarchical(nn.Module):
                 nz, ny = draw_noise(self.M, x, noise) if training else (None, None)
                 _training.forget_pairs()
                 res, _ = _training._forward_impl(self, x.contiguous().float(), nz, ny, lean, qmode=Q_NOISE if training else Q_ROUND,
-                                                 arm="bf16x3")
+                                                 arm="bf16x3", gains=gains)
                 _training.forget_pairs()
             return single_head_outputs(*res, K=self.K, training=training)
         prec_up, prec = precision_arms(self.precision)
@@ -254,7 +291,11 @@ class JointAutoregressiveHierarchical(nn.Module):
         hy, wy, hz, wz = H // 16, W // 16, H // 64, W // 64
         with torch.cuda.device(x.device), torch.no_grad():
             noise_z, noise_y = draw_noise(M, x, noise) if training else (None, None)
-            y, y_in, y_in_nhwc, y_src = fused_g_a(self, x, training, noise_y, prec_up, prec)
+            if gains is None:
+                y, y_in, y_in_nhwc, y_src = fused_g_a(self, x, training, noise_y, prec_up, prec)
+                gs_in = y_in_nhwc
+            else:
+                y, y_in, y_in_nhwc, y_src, gs_in = fused_g_a_gained(self, x, training, noise_y, prec_up, prec, gains)
 
             # ---- two parallel branches while the pass is captured in a CUDA graph: g_s (needs y_in only) and the context conv
             # (y_in only) run beside h_a -> h_s; the context conv joins before the 1x1 stack, g_s at the end
@@ -262,7 +303,7 @@ class JointAutoregressiveHierarchical(nn.Module):
             if branch is not None:
                 branch.wait_stream(main_stream)
                 with torch.cuda.stream(branch):
-                    x_hat = fused_g_s(self, y_in_nhwc, B, hy, wy, prec)
+                    x_hat = fused_g_s(self, gs_in, B, hy, wy, prec)
             # phi = combined[..., 0:2M] (context), psi = combined[..., 2M:4M] (h_s): torch.cat([phi, psi]) never happens.
             # (the quantised symbols split into bf16 pairs with an all-zero lo half - the hand-off kernel checks and flags it on the
             #  device: their first consumers - h_s layer 1, the context conv, g_s layer 1 - run 2 of the 3 MMA passes)
@@ -279,8 +320,11 @@ class JointAutoregressiveHierarchical(nn.Module):
                 with (torch.cuda.stream(branch2) if branch2 is not None else contextlib.nullcontext()):
                     self.context_model.masked._op.run(y_in_nhwc, B, hy, wy, prec, out=combined, out_c_total=4 * M, out_c_offset=0,
                                                       in_lo_flag=y_flag)
-            z, z_in, z_in_nhwc = fused_h_a(self, y_src, B, hy, wy, training, noise_z, prec_up, prec)
-            fused_h_s_into(self, z_in_nhwc, B, hz, wz, prec, combined, 4 * M, 2 * M, getattr(z_in_nhwc, "_nic_lo_flag", None))
+            if gains is None:
+                z, z_in, hs_in = fused_h_a(self, y_src, B, hy, wy, training, noise_z, prec_up, prec)
+            else:
+                z, z_in, hs_in = fused_h_a_gained(self, y_src, B, hy, wy, training, noise_z, prec_up, prec, gains)
+            fused_h_s_into(self, hs_in, B, hz, wz, prec, combined, 4 * M, 2 * M, getattr(hs_in, "_nic_lo_flag", None))
             if branch2 is not None:
                 main_stream.wait_stream(branch2)
 
@@ -305,7 +349,7 @@ class JointAutoregressiveHierarchical(nn.Module):
             if branch is not None:
                 main_stream.wait_stream(branch)                 # join
             else:
-                x_hat = fused_g_s(self, y_in_nhwc, B, hy, wy, prec)
+                x_hat = fused_g_s(self, gs_in, B, hy, wy, prec)
         return single_head_outputs(x_hat, ly["logp"], logp_z, y, y_in, z, z_in, p_z, ly["p"], ly["partials"], parts_z,
                                    *mixture_params(ly, K, lean), K=K, training=training)
 
@@ -348,6 +392,120 @@ class JointCheckerboardHierarchical(JointAutoregressiveHierarchical):
         match (corrupted bytes, other weights)."""
         from . import checkerboard_codec
         return checkerboard_codec.decompress(self, strings, shape)
+
+
+QUALITY_QUANTUM = 1024                               # every route snaps quality q to q_code / 1024, q_code = round(1024 q)
+
+
+class GainUnits(nn.Module):
+    """The gain units of Cui et al. (CVPR 2021): L learned rows of per-channel gains on y and z and of their inverse gains, stored as
+    natural logs (initialised to 0, i.e. gains of 1), each parameter [L, M]."""
+
+    def __init__(self, levels: int, channels: int):
+        super().__init__()
+        for name in ("y_log_gain", "y_log_inv_gain", "z_log_gain", "z_log_inv_gain"):
+            setattr(self, name, nn.Parameter(torch.zeros(levels, channels)))
+
+    def tables(self):
+        return self.y_log_gain, self.y_log_inv_gain, self.z_log_gain, self.z_log_inv_gain
+
+
+class Gains:
+    """The per-image gain vectors of one call: vec [4, B, M] = (g_y, ginv_y, g_z, ginv_z) from nic_gain_vectors, q_code int32 [B]."""
+
+    def __init__(self, vec: torch.Tensor, q_code: torch.Tensor):
+        self.vec, self.q_code = vec, q_code
+        self.g_y, self.ginv_y, self.g_z, self.ginv_z = vec.unbind(0)
+
+    @property
+    def quality(self) -> torch.Tensor:
+        return self.q_code.float() / QUALITY_QUANTUM
+
+
+def quality_codes(levels: int, quality, B: int, device) -> torch.Tensor:
+    """quality (None = levels - 1, a float, a sequence or tensor of 1 or B values in [0, levels - 1]) -> q_code int32 [B] on `device`,
+    q_code = floor(1024 q + 0.5).  Host values are checked (ValueError); a CUDA tensor (the trainer's draws) is snapped and clamped
+    on the device without a host synchronisation."""
+    top = QUALITY_QUANTUM * (levels - 1)
+    if isinstance(quality, torch.Tensor) and quality.is_cuda:
+        q = quality.detach().reshape(-1).float()
+        if q.numel() not in (1, B):
+            raise ValueError(f"quality: expected 1 or {B} values, got {q.numel()}")
+        return torch.floor(q * QUALITY_QUANTUM + 0.5).clamp_(0, top).to(torch.int32).expand(B).contiguous()
+    if quality is None:
+        vals = [float(levels - 1)]
+    elif isinstance(quality, torch.Tensor):
+        vals = [float(v) for v in quality.reshape(-1).tolist()]
+    elif isinstance(quality, (int, float)):
+        vals = [float(quality)]
+    else:
+        vals = [float(v) for v in quality]
+    if len(vals) not in (1, B):
+        raise ValueError(f"quality: expected 1 or {B} values, got {len(vals)}")
+    for v in vals:
+        if not (0.0 <= v <= levels - 1):
+            raise ValueError(f"quality must lie in [0, {levels - 1}], got {v}")
+    codes = [min(int(math.floor(v * QUALITY_QUANTUM + 0.5)), top) for v in vals]
+    return torch.tensor(codes * (B // len(codes)) if len(codes) == 1 else codes, dtype=torch.int32).to(device)
+
+
+def gain_vectors(model, q_code: torch.Tensor) -> Gains:
+    """nic_gain_vectors: the per-image gains of the quality codes q_code (device int32 [B]) - the one kernel the forward, the encoder
+    and the decoder share."""
+    gu = model.gain_units
+    tabs = [t.detach().float().contiguous() for t in gu.tables()]
+    engine.require_cuda(tabs[0], "gain tables")
+    B = q_code.numel()
+    L, M = tabs[0].shape
+    vec = torch.empty((4, B, M), dtype=torch.float32, device=tabs[0].device)
+    with torch.cuda.device(vec.device):
+        _lib.check(_lib.load().nic_gain_vectors(*[_lib.ptr(t) for t in tabs], L, M, _lib.ptr(q_code), B, _lib.ptr(vec),
+                                                _lib.current_stream()), "nic_gain_vectors")
+    return Gains(vec, q_code)
+
+
+class GainedCheckerboardHierarchical(JointCheckerboardHierarchical):
+    """JointCheckerboardHierarchical that codes at any quality q in [0, levels - 1] with gain units (Cui et al., CVPR 2021; DESIGN.md
+    section 15).  ``gain_units`` holds four [levels, M] log-gain tables; for image b, l = floor(q), t = q - l and each gain is
+    expf((1 - t) log[l] + t log[min(l + 1, levels - 1)]).  y = g_y (.) g_a(x) is quantised; the context conv, the 1x1 stack and the
+    likelihood read y_in, h_a reads y, g_s reads ginv_y (.) y_in; z = g_z (.) h_a(y) is quantised, the factorized prior reads z_in
+    and h_s reads ginv_z (.) z_in.  With every log-gain 0 it computes exactly JointCheckerboardHierarchical.
+
+    The modules are built in the parent's order with ``gain_units`` last: a seeded build draws the parent's weights, and a parent
+    checkpoint loads with ``load_state_dict(..., strict=False)`` (the fine-tuning path from a single-rate model)."""
+
+    def __init__(self, latent_channels: int = 192, K: int = 1, levels: int = 6, *, precision: Optional[str] = None):
+        if not isinstance(levels, int) or isinstance(levels, bool) or not 2 <= levels <= 64:
+            raise ValueError(f"levels must be an int in [2, 64], got {levels!r}")
+        super().__init__(latent_channels, K, precision=precision)
+        self.levels = levels
+        self.gain_units = GainUnits(levels, self.M)
+
+    def gains(self, quality, B: int, device) -> Gains:
+        return gain_vectors(self, quality_codes(self.levels, quality, B, device))
+
+    def forward(self, x: torch.Tensor, training: bool = True, *, quality=None,
+                noise: Optional[Tuple[torch.Tensor, torch.Tensor]] = None, lean: bool = False):
+        """The parent's dict at quality `quality` (None = levels - 1; a float, or one value per image), plus 'quality': the snapped
+        per-image values [B] (round(1024 q) / 1024), which every route (forward, training, compress, decompress) uses."""
+        check_input(x)
+        gains = self.gains(quality, x.shape[0], x.device)
+        out = self._forward(x, training, noise, lean, gains)
+        out["quality"] = gains.quality
+        return out
+
+    def compress(self, x: torch.Tensor, quality=None) -> dict:
+        """x [B, 3, H, W] (any H, W >= 1) at quality `quality` (a float or one value per image) -> {"strings": [y_strings, z_strings],
+        "shape": (hz, wz)}.  Format 5: DESIGN.md section 15."""
+        from . import gained_codec
+        return gained_codec.compress(self, x, quality)
+
+    def decompress(self, strings, shape) -> dict:
+        """strings / shape as compress returned them (any subset of the images, in any order) -> {"x_hat", "y_hat", "z_hat",
+        "quality"}; each image at the quality its string carries.  Raises ValueError on a string of another model, precision arm, M,
+        K or number of levels, on a malformed string, quality or image size, or on a checksum mismatch."""
+        from . import gained_codec
+        return gained_codec.decompress(self, strings, shape)
 
 
 class HierarchicalMixtureResidual(nn.Module):

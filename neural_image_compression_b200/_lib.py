@@ -87,6 +87,7 @@ SIGNATURES = {
     "nic_gm_likelihood_bwd": (C.c_int, [_vp, _vp, _vp, _f32, _i32, _i32, _i32, _i32, _vp, _vp, _vp]),
     "nic_factorized_likelihood_bwd": (C.c_int, [_vp, _vp, _vp, _f32, _i32, _i32, _i32, _vp, _vp, _vp]),
     "nic_sse_bwd": (C.c_int, [_vp, _vp, _i64, _f32, _vp, _vp]),
+    "nic_sse_bwd_per_image": (C.c_int, [_vp, _vp, _i32, _i64, _vp, _vp, _vp]),
     "nic_add_inplace": (C.c_int, [_vp, _vp, _i64, _vp]),
     "nic_layout_convert": (C.c_int, [_vp, _vp, _i32, _i32, _i32, _i32, _i32, _vp]),
     "nic_eval_mse": (C.c_int, [_vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp]),
@@ -119,6 +120,12 @@ SIGNATURES = {
     "nic_checkerboard_zero": (C.c_int, [_vp, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _vp]),
     "nic_codec_params": (C.c_int, [C.POINTER(CodecHead), _i32, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _vp]),
     "nic_image_window": (C.c_int, [_vp, _i32, _i32, _i32, _vp, _i32, _i32, _vp]),
+    # gain units
+    "nic_gain_vectors": (C.c_int, [_vp, _vp, _vp, _vp, _i32, _i32, _vp, _i32, _vp, _vp]),
+    "nic_latent_handoff_gain": (C.c_int, [_vp, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _i32, _vp, _vp,
+                                          _i32, _vp]),
+    "nic_gain_bwd": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i64, _vp, _i32, _vp, _vp]),
+    "nic_gain_fold": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, _vp, _vp]),
 }
 
 # entropy coder constants of include/nic.h

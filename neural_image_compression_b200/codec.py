@@ -216,11 +216,15 @@ class ParamPath:
         self.plan = engine.CtxEpPlan(model.context_model.masked._op, model.entropy_parameters.ops, B, hy, wy, self.prec, M, K, device,
                                      full=False)
 
-    def hyper(self, z_nhwc: torch.Tensor):
-        """z symbols NHWC f32 -> (z_hat NCHW f32, combined: psi in its channels [2M, 4M))."""
+    def hyper(self, z_nhwc: torch.Tensor, inv_gain=None):
+        """z symbols NHWC f32 -> (z_hat NCHW f32, combined: psi in its channels [2M, 4M)).  inv_gain [B, M] (gain units): h_s reads
+        inv_gain (.) z_hat, from the gained hand-off."""
         M, B, prec = self.model.M, self.B, self.prec
         hz, wz = z_nhwc.shape[1:3]
-        _, z_hat, z_eng, _ = engine.latent_handoff(z_nhwc, Q_PASSTHRU, None, self.hdt)
+        if inv_gain is None:
+            _, z_hat, z_eng, _ = engine.latent_handoff(z_nhwc, Q_PASSTHRU, None, self.hdt)
+        else:
+            _, z_hat, _, _, z_eng = engine.latent_handoff_gain(z_nhwc, Q_PASSTHRU, None, None, inv_gain, None, None, self.hdt)
         combined = torch.empty((B, self.hy, self.wy, (2 if prec == "bf16x3" else 1) * 4 * M), dtype=engine.act_dtype(prec),
                                device=self.device)
         fused_h_s_into(self.model, z_eng, B, hz, wz, prec, combined, 4 * M, 2 * M, None)          # no lo-half hint (module docstring)

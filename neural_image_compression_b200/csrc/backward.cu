@@ -312,6 +312,11 @@ __global__ void sse_bwd_kernel(const float* __restrict__ x_hat, const float* __r
   for (long i = static_cast<long>(blockIdx.x) * blockDim.x + threadIdx.x; i < n; i += static_cast<long>(gridDim.x) * blockDim.x)
     g[i] = coef * (x_hat[i] - x[i]);
 }
+__global__ void sse_bwd_per_image_kernel(const float* __restrict__ x_hat, const float* __restrict__ x, const float* __restrict__ coef,
+                                         long per_image, float* __restrict__ g, long n) {
+  for (long i = static_cast<long>(blockIdx.x) * blockDim.x + threadIdx.x; i < n; i += static_cast<long>(gridDim.x) * blockDim.x)
+    g[i] = coef[i / per_image] * (x_hat[i] - x[i]);
+}
 __global__ void add_inplace_kernel(float* __restrict__ dst, const float* __restrict__ src, long n) {
   for (long i = static_cast<long>(blockIdx.x) * blockDim.x + threadIdx.x; i < n; i += static_cast<long>(gridDim.x) * blockDim.x)
     dst[i] += src[i];
@@ -789,6 +794,16 @@ int nic_sse_bwd(const float* x_hat, const float* x, int64_t n, float coef, float
   if (n == 0) return NIC_OK;
   sse_bwd_kernel<<<ew_blocks(n), 256, 0, as_stream(stream)>>>(x_hat, x, coef, g_x_hat, n);
   return check_launch("sse_bwd_kernel");
+}
+
+int nic_sse_bwd_per_image(const float* x_hat, const float* x, int32_t b, int64_t per_image, const float* coef, float* g_x_hat,
+                          void* stream) {
+  if (int rc = nic_check_device()) return rc;
+  if (b < 0 || per_image < 1 || (b > 0 && (!x_hat || !x || !coef || !g_x_hat))) return fail(NIC_E_BADSHAPE, "sse_bwd_per_image: bad arguments");
+  if (b == 0) return NIC_OK;
+  const long n = static_cast<long>(b) * per_image;
+  sse_bwd_per_image_kernel<<<ew_blocks(n), 256, 0, as_stream(stream)>>>(x_hat, x, coef, per_image, g_x_hat, n);
+  return check_launch("sse_bwd_per_image_kernel");
 }
 
 int nic_add_inplace(float* dst, const float* src, int64_t n, void* stream) {

@@ -279,6 +279,38 @@ def latent_handoff(v_nhwc: torch.Tensor, qmode: int, noise: Optional[torch.Tenso
     return v, v_in, v_in_nhwc, v_lowp
 
 
+def _nhwc_out(n, h, w, c, dtype, device):
+    """(tensor, NIC_DT_*) of an NHWC hand-off output; dtype torch.float32, torch.bfloat16 or "bf16x2" (hi/lo pair, 2c channels)."""
+    if dtype == "bf16x2":
+        return torch.empty((n, h, w, 2 * c), dtype=torch.bfloat16, device=device), DT_BF16X2
+    return torch.empty((n, h, w, c), dtype=dtype, device=device), (DT_BF16 if dtype == torch.bfloat16 else DT_F32)
+
+
+def latent_handoff_gain(v_nhwc: torch.Tensor, qmode: int, noise: Optional[torch.Tensor], gain: Optional[torch.Tensor],
+                        inv_gain: Optional[torch.Tensor], sym_dtype=None, src_dtype=None, scaled_dtype=None):
+    """The hand-off with gain units (nic_latent_handoff_gain): v_g = gain (.) v is quantised.  gain / inv_gain: [n, c] f32 per
+    image and channel, or None for 1.  Returns (v_g NCHW, v_in NCHW, symbols NHWC in sym_dtype | None, v_g NHWC in src_dtype | None,
+    inv_gain (.) v_in NHWC in scaled_dtype | None); dtypes as latent_handoff's in_dtype.  A pair-format symbol tensor carries
+    `_nic_lo_flag`; the scaled one never does."""
+    lib = _lib.load()
+    n, h, w, c = v_nhwc.shape
+    dev = v_nhwc.device
+    v = torch.empty((n, c, h, w), dtype=torch.float32, device=dev)
+    v_in = torch.empty_like(v)
+    sym, sym_dt = _nhwc_out(n, h, w, c, sym_dtype, dev) if sym_dtype is not None else (None, DT_F32)
+    src, src_dt = _nhwc_out(n, h, w, c, src_dtype, dev) if src_dtype is not None else (None, DT_F32)
+    scaled, sc_dt = _nhwc_out(n, h, w, c, scaled_dtype, dev) if scaled_dtype is not None else (None, DT_F32)
+    if noise is not None:
+        noise = noise.contiguous().float()
+    flag = torch.empty(1, dtype=torch.int32, device=dev) if sym_dt == DT_BF16X2 else None
+    check(lib.nic_latent_handoff_gain(ptr(v_nhwc), n, c, h, w, qmode, ptr(noise), ptr(gain), ptr(v), ptr(v_in), ptr(sym), sym_dt,
+                                      ptr(flag), ptr(src), src_dt, ptr(inv_gain), ptr(scaled), sc_dt, current_stream()),
+          "nic_latent_handoff_gain")
+    if flag is not None:
+        sym._nic_lo_flag = flag
+    return v, v_in, sym, src, scaled
+
+
 def checkerboard_zero_(t: torch.Tensor) -> torch.Tensor:
     """In place: 0 at the anchors (i + j even) of a contiguous NHWC f32 tensor [n, h, w, c] (nic_checkerboard_zero)."""
     n, h, w, c = t.shape

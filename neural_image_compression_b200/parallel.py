@@ -11,7 +11,7 @@ from __future__ import annotations
 
 import math
 import os
-from typing import Optional
+from typing import Optional, Sequence
 
 import torch
 import torch.distributed as dist
@@ -318,11 +318,27 @@ class ShardedTrainer:
 
     distortion="ms-ssim" trains for MS-SSIM (RateDistortionLoss.ms_ssim_rd_loss: loss = bpp + lambda * (1 - MS-SSIM), no 255^2);
     'scalars' then has a 9th entry, the batch MS-SSIM.  The all-reduce is the same: with equal shards the average of the per-rank
-    gradients of a batch-mean loss is the global gradient.  Not built for ScalableImageCoding (vision_rd_loss is its loss)."""
+    gradients of a batch-mean loss is the global gradient.  Not built for ScalableImageCoding (vision_rd_loss is its loss).
 
-    def __init__(self, model, lambda_rd: float, lr: float = 1e-4, group=None, bucket_bytes: int = 32 << 20, optimizer=None,
-                 graph: bool = False, distortion: str = "mse"):
+    lambdas=[lambda_0 ... lambda_{L-1}] (instead of lambda_rd; models with gain units, L = model.levels) trains every quality at once:
+    each step draws an integer level per local image on the device (torch.randint on the CUDA generator, so a graph replay draws
+    fresh levels), codes the image at that quality and weighs its distortion by lambdas[level] (training.step_gradients with a
+    per-image lambda).  Such steps always run through step_gradients, eagerly or from the graph."""
+
+    def __init__(self, model, lambda_rd: Optional[float] = None, lr: float = 1e-4, group=None, bucket_bytes: int = 32 << 20,
+                 optimizer=None, graph: bool = False, distortion: str = "mse", lambdas: Optional[Sequence[float]] = None):
         from .training import DISTORTIONS, Adam
+        if lambdas is not None:
+            if not hasattr(model, "gain_units"):
+                raise ValueError(f"lambdas: {type(model).__name__} has no gain units (train it with one lambda_rd)")
+            lambdas = [float(v) for v in lambdas]
+            if len(lambdas) != model.levels:
+                raise ValueError(f"lambdas: the model has {model.levels} levels, got {len(lambdas)} lambdas")
+            if lambda_rd is not None:
+                raise ValueError("pass lambda_rd or lambdas, not both")
+        elif lambda_rd is None:
+            raise ValueError("ShardedTrainer needs lambda_rd (or lambdas for a model with gain units)")
+        self.lambdas, self._lambdas_dev = lambdas, None
         self._scalable = type(model).__name__ == "ScalableImageCoding"
         if distortion not in DISTORTIONS:
             raise ValueError(f"distortion must be one of {DISTORTIONS}, got {distortion!r}")
@@ -354,6 +370,12 @@ class ShardedTrainer:
             loss, terms = scalable_step(self.model, x_local, self.lambda_rd, noise=noise)
             return loss, None, torch.stack([terms[k] for k in ("bpp_y1", "bpp_y2", "bpp_z", "mse", "psnr", "loss")])
         from .training import step_gradients
+        if self.lambdas is not None:
+            if self._lambdas_dev is None or self._lambdas_dev.device != x_local.device:
+                self._lambdas_dev = torch.tensor(self.lambdas, dtype=torch.float32, device=x_local.device)
+            level = torch.randint(0, len(self.lambdas), (x_local.shape[0],), device=x_local.device)
+            return step_gradients(self.model, x_local, self._lambdas_dev[level], noise=noise, partial_hook=partial_hook,
+                                  distortion=self.distortion, quality=level.float())
         return step_gradients(self.model, x_local, self.lambda_rd, noise=noise, partial_hook=partial_hook, distortion=self.distortion)
 
     # ---- gradient all-reduce INSIDE the captured step, overlapped with g_a's backward -------------------------------------------
@@ -467,7 +489,7 @@ class ShardedTrainer:
         return res, fuse_adam, comm_in_graph
 
     def step(self, x_local: torch.Tensor, noise=None) -> dict:
-        if (self.graph and noise is None) or self._scalable:
+        if (self.graph and noise is None) or self._scalable or self.lambdas is not None:
             reduced = False
             if self.graph and noise is None:
                 (loss, per_image, scalars), adam_done, reduced = self._graphed(x_local)

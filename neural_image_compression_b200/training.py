@@ -406,6 +406,13 @@ def to_nhwc(t_nchw: torch.Tensor, accumulate_into: Optional[torch.Tensor] = None
     return out
 
 
+def gain_bwd(grad: torch.Tensor, factor: torch.Tensor, other: torch.Tensor, n: int, c: int, hw: int, dst: Optional[torch.Tensor],
+             accumulate: bool, dgain: Optional[torch.Tensor]):
+    """nic_gain_bwd over NHWC f32 [n, hw, c]: dst (= or +=) factor (.) grad, dgain [n, c] = sum over the pixels of grad (.) other."""
+    check(_lib.load().nic_gain_bwd(ptr(grad), ptr(factor), ptr(other), n, c, hw, ptr(dst), int(accumulate), ptr(dgain),
+                                   current_stream()), "nic_gain_bwd")
+
+
 def add_(dst: torch.Tensor, src: torch.Tensor) -> torch.Tensor:
     check(_lib.load().nic_add_inplace(ptr(dst), ptr(src), dst.numel(), current_stream()), "nic_add_inplace")
     return dst
@@ -567,7 +574,8 @@ def factorized_bwd(fe: nn.Module, z_in: torch.Tensor, fparams: torch.Tensor, g_l
 
 # ---- the model as one autograd node ------------------------------------------------------------------------------
 
-def _forward_impl(model, x, noise_z, noise_y, lean, qmode: int = Q_NOISE, arm: Optional[str] = None, record: bool = True):
+def _forward_impl(model, x, noise_z, noise_y, lean, qmode: int = Q_NOISE, arm: Optional[str] = None, record: bool = True,
+                  gains=None):
     """The layer-by-layer forward (fp32 NHWC tensors between layers) of a model with any number of entropy heads (`heads`)
     -> (outputs, saved state S).  Outputs in the order single_head_outputs / two_head_outputs take them: x_hat, the heads' logp,
     logp_z, y, y_in, z, z_in, p_z, the heads' p, the heads' partial sums, the partial sums of z, the heads' mixture_params.
@@ -576,7 +584,9 @@ def _forward_impl(model, x, noise_z, noise_y, lean, qmode: int = Q_NOISE, arm: O
     transform records on a Tape and S keeps what _backward_impl reads; under a CUDA-graph capture g_s runs as a parallel branch.
     record=False (evaluation of the residual family and of ScalableImageCoding outside its fused pipeline): no tapes, so the
     transforms hand bf16 pairs between convs and drop their pair forms per layer; everything on the current stream (a per-layer
-    forget_pairs on one stream would free pair tensors another stream still reads); S is None."""
+    forget_pairs on one stream would free pair tensors another stream still reads); S is None.
+    gains (GainedCheckerboardHierarchical: Models.Gains): both hand-offs go through nic_latent_handoff_gain; h_a reads g_y (.) y,
+    g_s reads ginv_y (.) y_in and h_s ginv_z (.) z_in.  None: the hand-offs of the models without gain units."""
     engine.require_cuda(x, "x")
     dev = x.device
     B, _, H, W = x.shape
@@ -587,27 +597,37 @@ def _forward_impl(model, x, noise_z, noise_y, lean, qmode: int = Q_NOISE, arm: O
     S = {t: Tape(arm, B) if record else None for t in ("g_a", "g_s", "h_a", "h_s")}    # each transform's ops and tensors
     with torch.cuda.device(dev):
         y_nhwc, _, _ = model.encoder.run_nhwc(x, B, H, W, arm, in_layout=LAYOUT_NCHW, tape=S["g_a"])
-        y, y_in, y_in_nhwc, _ = engine.latent_handoff(y_nhwc, qmode, noise_y, torch.float32)
+        if gains is None:
+            y, y_in, y_in_nhwc, _ = engine.latent_handoff(y_nhwc, qmode, noise_y, torch.float32)
+            ha_in, gs_in = y_nhwc, y_in_nhwc
+        else:
+            f32 = torch.float32
+            y, y_in, y_in_nhwc, ha_in, gs_in = engine.latent_handoff_gain(y_nhwc, qmode, noise_y, gains.g_y, gains.ginv_y, f32, f32, f32)
 
         def synthesis():
-            return model.decoder.run_nhwc(y_in_nhwc, B, hy, wy, arm, tape=S["g_s"], final_kw=dict(out_layout=LAYOUT_NCHW))[0]
+            return model.decoder.run_nhwc(gs_in, B, hy, wy, arm, tape=S["g_s"], final_kw=dict(out_layout=LAYOUT_NCHW))[0]
         # g_s reads only y_in: it runs as its own branch (a second stream; a parallel branch of a captured graph) beside the
         # entropy path h_a -> h_s -> context -> entropy parameters -> likelihoods
         main = torch.cuda.current_stream(dev)
         branch = _side_stream(dev, 1) if (record and _overlap()) else None
         if branch is not None:
             if arm == "bf16x3":
-                to_pair(y_in_nhwc)               # both branches consume the pair form: make it before the fork
+                to_pair(gs_in)                   # both branches consume the pair form: make it before the fork
             branch.wait_stream(main)
             with torch.cuda.stream(branch):
                 x_hat = synthesis()
         # h_a (reads the unquantised y)
-        z_nhwc, _, _ = model.hyper_encoder.run_nhwc(y_nhwc, B, hy, wy, arm, tape=S["h_a"])
-        z, z_in, z_in_nhwc, _ = engine.latent_handoff(z_nhwc, qmode, noise_z, torch.float32)
+        z_nhwc, _, _ = model.hyper_encoder.run_nhwc(ha_in, B, hy, wy, arm, tape=S["h_a"])
+        if gains is None:
+            z, z_in, z_in_nhwc, _ = engine.latent_handoff(z_nhwc, qmode, noise_z, torch.float32)
+            hs_in = z_in_nhwc
+        else:
+            z, z_in, z_in_nhwc, _, hs_in = engine.latent_handoff_gain(z_nhwc, qmode, noise_z, gains.g_z, gains.ginv_z, torch.float32,
+                                                                      None, torch.float32)
         # h_s writes psi into head 0's concat buffer [phi_0 (2 m_0) | psi (2 M)]; every other head's buffer gets a copy of it
         combs = [_f32((B, hy, wy, 2 * (c1 - c0) + 2 * M), dev) for _, _, c0, c1 in hds]
         m0 = hds[0][3] - hds[0][2]
-        model.hyper_decoder.run_nhwc(z_in_nhwc, B, hz, wz, arm, tape=S["h_s"],
+        model.hyper_decoder.run_nhwc(hs_in, B, hz, wz, arm, tape=S["h_s"],
                                      final_kw=dict(out=combs[0], out_c_total=combs[0].shape[-1], out_c_offset=2 * m0))
         for (_, _, c0, c1), comb in zip(hds[1:], combs[1:]):
             comb[..., 2 * (c1 - c0):] = combs[0][..., 2 * m0:]
@@ -626,8 +646,11 @@ def _forward_impl(model, x, noise_z, noise_y, lean, qmode: int = Q_NOISE, arm: O
             *[ly["partials"] for ly in lys], parts_z, *[t for ly in lys for t in mixture_params(ly, K, lean)])
     if not record:
         return outs, None
-    S.update(arm=arm, heads=states, y_in_nhwc=y_in_nhwc, z_in=z_in, z_in_nhwc=z_in_nhwc, y_nhwc=y_nhwc,
+    # the roots of the g_s, h_s and h_a tapes (the symbols and y itself without gain units)
+    S.update(arm=arm, heads=states, y_in_nhwc=gs_in, z_in=z_in, z_in_nhwc=hs_in, y_nhwc=ha_in,
              fparams=model.factorized_entropy_model.packed(), shape=(B, H, W))
+    if gains is not None:
+        S["gain"] = dict(gains=gains, y=y_nhwc, y_sym=y_in_nhwc, z=z_nhwc, z_sym=z_in_nhwc)
     return outs, S
 
 
@@ -660,6 +683,13 @@ def _backward_impl(model, S, g_xhat, g_logp_heads, g_logp_z, partial_hook=None) 
         keep.extend((a, g, pairs))
         return out
 
+    G = S.get("gain")                                            # gain units: gradients of the four gain vectors, per image
+    if G is not None:
+        gains = G["gains"]
+        d_gain = torch.zeros_like(gains.vec)
+        B_, hy_, wy_, M_ = G["y"].shape
+        hz_, wz_ = G["z"].shape[1:3]
+
     with torch.cuda.device(dev), torch.no_grad():
         d_yin = None                                             # NHWC gradient w.r.t. y_in from the entropy path (likelihood, context)
         d_yin_gs = None                                          # ... and from g_s, whose backward runs as its own branch
@@ -684,6 +714,8 @@ def _backward_impl(model, S, g_xhat, g_logp_heads, g_logp_z, partial_hook=None) 
             d_yin = d_ys[0] if len(d_ys) == 1 else torch.cat(d_ys, dim=-1)
             del d_ys
             d_zin = S["h_s"].backward(d_psi, LAYOUT_NHWC, put, conv_wgrad_async, root=S["z_in_nhwc"], side=side, keep=keep)
+            if G is not None:                                    # h_s read ginv_z (.) z_in
+                gain_bwd(d_zin, gains.ginv_z, G["z_sym"], B_, M_, hz_ * wz_, d_zin, False, d_gain[3])
         # ---- p_z ----------------------------------------------------------------------------------------------------
         if g_logp_z is not None:
             dz = factorized_bwd(model.factorized_entropy_model, S["z_in"], S["fparams"], g_logp_z, put)
@@ -691,14 +723,28 @@ def _backward_impl(model, S, g_xhat, g_logp_heads, g_logp_z, partial_hook=None) 
         # ---- h_a (z_in = z + noise: the gradient passes unchanged) --------------------------------------------------
         dy = d_yin
         if d_zin is not None:
+            if G is not None:                                    # z_in = g_z (.) z + noise
+                gain_bwd(d_zin, gains.g_z, G["z"], B_, M_, hz_ * wz_, d_zin, False, d_gain[2])
             g = S["h_a"].backward(d_zin, LAYOUT_NHWC, put, conv_wgrad_async, root=S["y_nhwc"], side=side, keep=keep)
             dy = g if dy is None else add_(dy, g)
             del g                                                # summed into dy: free it before g_a's backward
         # ---- merge the branches: dy = d(entropy path) + d(h_a) + d(g_s) ---------------------------------------------------------
         if branch is not None:
             main.wait_stream(branch)
-        if d_yin_gs is not None:
+        if d_yin_gs is not None and G is not None:               # g_s read ginv_y (.) y_in
+            gain_bwd(d_yin_gs, gains.ginv_y, G["y_sym"], B_, M_, hy_ * wy_, d_yin_gs if dy is None else dy, dy is not None, d_gain[1])
+            dy = d_yin_gs if dy is None else dy
+        elif d_yin_gs is not None:
             dy = d_yin_gs if dy is None else add_(dy, d_yin_gs)
+        if G is not None:
+            if dy is not None:                                   # y_in = g_y (.) y + noise
+                gain_bwd(dy, gains.g_y, G["y"], B_, M_, hy_ * wy_, dy, False, d_gain[0])
+            tables = model.gain_units.tables()
+            d_tab = _f32((4,) + tuple(tables[0].shape), dev)
+            check(_lib.load().nic_gain_fold(ptr(gains.vec), ptr(d_gain), ptr(gains.q_code), B_, tables[0].shape[0], M_, ptr(d_tab),
+                                            current_stream()), "nic_gain_fold")
+            for t, d in zip(tables, d_tab.unbind(0)):
+                put(t, d)
         if partial_hook is not None:
             partial_hook(grads, [st for st in (main, side) if st is not None])
         # ---- g_a (y_in = y + noise) ---------------------------------------------------------------------------------
@@ -715,8 +761,8 @@ class _TrainForward(torch.autograd.Function):
     """The whole model as ONE autograd node (what makes the reference trainer's loss.backward() work, Trainer.py:85)."""
 
     @staticmethod
-    def forward(ctx, model, x, noise_z, noise_y, lean, *params):
-        outs, S = _forward_impl(model, x, noise_z, noise_y, lean)
+    def forward(ctx, model, x, noise_z, noise_y, lean, gains, *params):
+        outs, S = _forward_impl(model, x, noise_z, noise_y, lean, gains=gains)
         ctx.model, ctx.S = model, S
         ctx.mark_non_differentiable(*outs[3:])
         return outs
@@ -730,32 +776,59 @@ class _TrainForward(torch.autograd.Function):
         grads = _backward_impl(model, S, g_xhat, [g_logp_y], g_logp_z)
         ctx.S = None
         params = [p for _, p in model.named_parameters()]
-        return (None, None, None, None, None, *[grads.get(id(p)) for p in params])
+        return (None, None, None, None, None, None, *[grads.get(id(p)) for p in params])
 
 
 DISTORTIONS = ("mse", "ms-ssim")
 
 
 @torch.no_grad()
-def step_gradients(model, x: torch.Tensor, lambda_rd: float, noise=None, partial_hook=None, distortion: str = "mse"):
+def step_gradients(model, x: torch.Tensor, lambda_rd, noise=None, partial_hook=None, distortion: str = "mse", quality=None):
     """forward + rd_loss + backward of one step WITHOUT the autograd engine (everything on the calling thread and its current
     stream - what a CUDA-graph capture needs): accumulates into .grad like loss.backward() and returns
     (loss [device scalar], per_image [3, B], scalars [8]).  distortion="ms-ssim": the loss of ms_ssim_rd_loss, whose x_hat
-    gradient comes from nic_ms_ssim_bwd; scalars then has a 9th entry, the batch MS-SSIM, and entry 5 is that loss."""
+    gradient comes from nic_ms_ssim_bwd; scalars then has a 9th entry, the batch MS-SSIM, and entry 5 is that loss.
+    Models with gain units: quality as the model's forward takes it (a CUDA tensor is snapped on the device), and lambda_rd may be a
+    device tensor [B] of per-image lambdas: loss = bpp_total + mean_b(lambda_b 255^2 mse_b) (MS-SSIM: mean_b(lambda_b (1 - ms_ssim_b)))."""
     from .RateDistortionLoss import check_ms_ssim_shape, ms_ssim_terms, rd_terms
     if distortion not in DISTORTIONS:
         raise ValueError(f"distortion must be one of {DISTORTIONS}, got {distortion!r}")
     if distortion == "ms-ssim":
         check_ms_ssim_shape(tuple(x.shape))
     B, _, H, W = x.shape
+    gains = None
+    if hasattr(model, "gain_units"):
+        gains = model.gains(quality, B, x.device)
+    elif quality is not None:
+        raise ValueError(f"quality: {type(model).__name__} has no gain units")
+    per_lambda = isinstance(lambda_rd, torch.Tensor)
+    if per_lambda and (gains is None or lambda_rd.numel() != B):
+        raise ValueError("a tensor lambda_rd holds one lambda per image of a model with gain units")
     noise_z, noise_y = draw_noise(model.M, x, noise)
     forget_pairs()
     x = x.contiguous().float()
-    outs, S = _forward_impl(model, x, noise_z, noise_y, True)
+    outs, S = _forward_impl(model, x, noise_z, noise_y, True, gains=gains)
     x_hat, logp_y, logp_z = outs[:3]
     engine.attach_partials(logp_y, outs[9])
     engine.attach_partials(logp_z, outs[10])
-    if distortion == "ms-ssim":
+    if per_lambda:
+        # per-image lambdas: the terms at lambda 0 (scalars[5] = bpp_total), the distortion term from the per-image values
+        lam = lambda_rd.detach().reshape(B).float()
+        terms = {"x_hat": x_hat, "logp_y": logp_y, "logp_z": logp_z}
+        if distortion == "ms-ssim":
+            per_image, scalars, ms_img, state = ms_ssim_terms(terms, x, 0.0)
+            loss = scalars[2] + (lam * (1.0 - ms_img)).mean()
+            gx = ms_ssim_x_hat_grad(state, lam)
+        else:
+            per_image, scalars = rd_terms(terms, x, 0.0)
+            loss = scalars[2] + (lam * 65025.0 * per_image[2]).mean()
+            gx = torch.empty_like(x_hat)
+            coef = lam * (65025.0 * 2.0 / x.numel())
+            with torch.cuda.device(x.device):
+                check(_lib.load().nic_sse_bwd_per_image(ptr(x_hat), ptr(x), B, x[0].numel(), ptr(coef), ptr(gx), current_stream()),
+                      "nic_sse_bwd_per_image")
+        scalars = torch.cat([scalars[:5], loss.view(1), scalars[6:]])
+    elif distortion == "ms-ssim":
         per_image, scalars, _, state = ms_ssim_terms({"x_hat": x_hat, "logp_y": logp_y, "logp_z": logp_z}, x, lambda_rd)
         gx = ms_ssim_x_hat_grad(state, lambda_rd)
     else:
@@ -774,12 +847,13 @@ def step_gradients(model, x: torch.Tensor, lambda_rd: float, noise=None, partial
     return scalars[5], per_image, scalars
 
 
-def train_forward(model, x: torch.Tensor, noise=None, lean: bool = False) -> dict:
-    """``model(x, training=True)`` as a differentiable call (used by JointAutoregressiveHierarchical.forward when autograd is on)."""
+def train_forward(model, x: torch.Tensor, noise=None, lean: bool = False, gains=None) -> dict:
+    """``model(x, training=True)`` as a differentiable call (used by JointAutoregressiveHierarchical.forward when autograd is on);
+    gains: the per-image gain vectors of GainedCheckerboardHierarchical."""
     noise_z, noise_y = draw_noise(model.M, x, noise)
     forget_pairs()
     params = [p for _, p in model.named_parameters()]
-    res = _TrainForward.apply(model, x.contiguous().float(), noise_z, noise_y, lean, *params)
+    res = _TrainForward.apply(model, x.contiguous().float(), noise_z, noise_y, lean, gains, *params)
     return single_head_outputs(*res, K=model.K, training=True)
 
 
@@ -806,13 +880,17 @@ class _RDLoss(torch.autograd.Function):
         return gl.expand(ctx.shapes[0]), gl.expand(ctx.shapes[1]), gx, None, None, None
 
 
-def ms_ssim_x_hat_grad(state, lambda_rd: float, g: Optional[torch.Tensor] = None) -> torch.Tensor:
+def ms_ssim_x_hat_grad(state, lambda_rd, g: Optional[torch.Tensor] = None) -> torch.Tensor:
     """d loss / d x_hat of loss = bpp + lambda * (1 - mean ms_ssim) (times the upstream scalar g) through nic_ms_ssim_bwd, from the
-    state ms_ssim_terms returned: the level coefficients are d loss / d term = -lambda / planes * d value / d term."""
+    state ms_ssim_terms returned: the level coefficients are d loss / d term = -lambda / planes * d value / d term.  lambda_rd may
+    be a device tensor [B] of per-image lambdas (each image's planes get its own)."""
     from .Evaluator import term_grads
     x_hat, x, terms, value, ws = state
     b, c, h, w = x.shape
-    coef = term_grads(terms, value) * (-float(lambda_rd) / (b * c))
+    if isinstance(lambda_rd, torch.Tensor):
+        coef = term_grads(terms, value) * (-lambda_rd.float().repeat_interleave(c) / (b * c))
+    else:
+        coef = term_grads(terms, value) * (-float(lambda_rd) / (b * c))
     if g is not None:
         coef = coef * g.float()
     gx = torch.empty_like(x_hat)
