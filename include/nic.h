@@ -545,6 +545,19 @@ int nic_codec_decode_pass(const uint8_t* blob, const int64_t* lane_off, const in
                           const float* params, int32_t b, int32_t m, int32_t k, int32_t h, int32_t w, int32_t lanes_c, int32_t band_rows,
                           int32_t pass, float* out, void* stream);
 /*
+ * Channel-slice forms of the two entries above (DESIGN.md section 16, format 6): the walk of one slice of m channels that occupies
+ * the channels [c_off, c_off + m) of a latent with c_total channels (c_off + m <= c_total).  Lanes, their order and cap are those
+ * of a latent of m channels.  Encode: code and sym are the full NCHW [b, c_total, h, w] tensors.  Decode: params are the slice's
+ * raw entropy parameters [b, (3K | 2) m, h, w] and the symbols go to the channels [c_off, c_off + m) of out, NHWC f32
+ * [b, h, w, c_total].  With c_off = 0 and c_total = m they are nic_codec_encode_checkerboard / nic_codec_decode_pass.
+ */
+int nic_codec_encode_checkerboard_slice(const uint64_t* code, const float* sym, int32_t b, int32_t c_total, int32_t c_off, int32_t m,
+                                        int32_t h, int32_t w, int32_t lanes_c, int32_t band_rows, int64_t cap, uint16_t* words, int32_t* count,
+                                        void* stream);
+int nic_codec_decode_pass_slice(const uint8_t* blob, const int64_t* lane_off, const int32_t* lane_words, uint32_t* state, int32_t* pos,
+                                const float* params, int32_t b, int32_t c_total, int32_t c_off, int32_t m, int32_t k, int32_t h, int32_t w,
+                                int32_t lanes_c, int32_t band_rows, int32_t pass, float* out, void* stream);
+/*
  * Writes 0 into channels [c_offset, c_offset + c) of a tensor with c_total channels at every anchor pixel (i + j even) of [n, h, w]:
  * the anchor zeroing of a checkerboard context conv's output (nic_conv_fwd enqueues it after the conv), and of the gradient of that
  * output in the training step.  dtype NIC_DT_F32 / NIC_DT_BF16 in NIC_LAYOUT_NHWC or NIC_LAYOUT_NCHW; NIC_DT_BF16X2 (hi / lo pair,

@@ -1,4 +1,5 @@
-"""Masked autoregressive context model (/root/reference/ContextModels.py) and the checkerboard context model.
+"""Masked autoregressive context model (/root/reference/ContextModels.py), the checkerboard context model and the channel context
+model of the channel slices.
 
 ``MaskedConv2d`` keeps the reference's ``weight`` / ``bias`` parameters and ``mask`` buffer
 (:12-16).  The engine packs only the live taps of mask 'A' (12 of 25 for 5x5), so the masked
@@ -101,3 +102,19 @@ class CheckerboardContextModel(nn.Module):
 
     def forward(self, x: torch.Tensor) -> torch.Tensor:
         return self.masked(x)
+
+
+# ---- channel context (ELIC, He et al., CVPR 2022; Minnen & Singh, ICIP 2020): DESIGN.md section 16 ----------------------------
+# Slice s of y (channels [o_s, o_s + m_s)) also reads the slices before it, y[:, :o_s], through one unmasked 5x5 conv.  Those slices
+# are fully decoded before slice s starts, so its output phi_ch is NOT zeroed at the anchors.
+
+class ChannelContextModel(nn.Module):
+    """``.conv``: an unmasked 5x5 conv with bias, o_s -> 2 m_s, padding 2, over the channels [0, o_s) of y."""
+
+    def __init__(self, in_channels: int, latent_channels: int):
+        super().__init__()
+        self.conv = nn.Conv2d(in_channels, 2 * latent_channels, kernel_size=5, stride=1, padding=2)
+        self._op = engine.ConvOp(self.conv, EPI_BIAS)
+
+    def forward(self, y_prev: torch.Tensor) -> torch.Tensor:
+        return engine.run_sequential_nchw([self._op], y_prev, "fp32")

@@ -29,7 +29,7 @@ import torch.nn as nn
 from . import _lib, engine
 from ._lib import LAYOUT_NCHW, LAYOUT_NHWC, MODEL_PRECISIONS, Q_NOISE, Q_PASSTHRU, Q_ROUND
 from .Components import Decoder5x5, Encoder5x5, HyperDecoder5x5, HyperEncoder5x5
-from .ContextModels import CheckerboardContextModel, ContextModel
+from .ContextModels import ChannelContextModel, CheckerboardContextModel, ContextModel
 from .EntropyModels import FactorizedEntropyBottleneck, GaussianConditional, GaussianMixtureConditional, gm_likelihood
 from .ParametersModels import EntropyParameters
 
@@ -506,6 +506,200 @@ class GainedCheckerboardHierarchical(JointCheckerboardHierarchical):
         K or number of levels, on a malformed string, quality or image size, or on a checksum mismatch."""
         from . import gained_codec
         return gained_codec.decompress(self, strings, shape)
+
+
+def default_slices(M: int) -> Tuple[int, ...]:
+    """64-channel slices with any remainder as the last one: (64, 64) at M = 128, (64, 64, 64) at 192, (M,) below 64."""
+    n, r = divmod(M, 64)
+    return (64,) * n + ((r,) if r else ()) if n else (M,)
+
+
+def check_slices(slices, M: int) -> Tuple[int, ...]:
+    """slices (None = default_slices) -> a tuple of positive ints that sum to M; ValueError otherwise."""
+    if slices is None:
+        return default_slices(M)
+    if not isinstance(slices, (tuple, list)) or not slices or \
+            any(not isinstance(m, int) or isinstance(m, bool) or m < 1 for m in slices) or sum(slices) != M:
+        raise ValueError(f"slices must be a non-empty tuple of positive ints that sum to latent_channels={M}, got {slices!r}")
+    return tuple(slices)
+
+
+def merge_slices(lys: list, K: int, lean: bool):
+    """The likelihood dicts of the channel slices -> (logp, p, per-image partial sums of logp, *mixture params) over all M channels
+    in channel order.  One slice: its own tensors (so slices=(M,) returns what JointCheckerboardHierarchical returns)."""
+    if len(lys) == 1:
+        return (lys[0]["logp"], lys[0]["p"], lys[0]["partials"], *mixture_params(lys[0], K, lean))
+    logp = torch.cat([ly["logp"] for ly in lys], dim=1)
+    p = torch.cat([ly["p"] for ly in lys], dim=1)
+    parts = engine.partials(logp.shape[0], logp.device)
+    with torch.cuda.device(logp.device):
+        _lib.check(_lib.load().nic_sum_fwd(_lib.ptr(logp), logp.shape[0], logp[0].numel(), _lib.ptr(parts), _lib.current_stream()),
+                   "nic_sum_fwd")
+    params = [] if lean else [torch.cat([ly[k] for ly in lys], dim=1 if K == 1 else 2) for k in _param_names(K)]
+    return (logp, p, parts, *params)
+
+
+def _channel_window(t: torch.Tensor, c0: int, c1: int, M: int, pair: bool) -> torch.Tensor:
+    """Channels [c0, c1) of NHWC symbols with M channels (pairs: [hi(M) | lo(M)] -> [hi | lo] of the window), contiguous."""
+    if c0 == 0 and c1 == M:
+        return t
+    if pair:
+        return torch.cat([t[..., c0:c1], t[..., M + c0:M + c1]], dim=-1).contiguous()
+    return t[..., c0:c1].contiguous()
+
+
+def slice_buffers(model, B: int, hy: int, wy: int, prec: str, device) -> list:
+    """One NHWC concat buffer per slice, [phi_sp (2 m_s) | phi_ch (2 m_s, s >= 1) | psi (2 M)] (bf16x3: [hi | lo] pairs)."""
+    pair = prec == "bf16x3"
+    return [torch.empty((B, hy, wy, (2 if pair else 1) * ep.net[0].in_channels), dtype=engine.act_dtype(prec), device=device)
+            for ep in model.entropy_parameters]
+
+
+def slice_psi_into(model, z_eng, B: int, hz: int, wz: int, prec: str, combs: list, lo_flag):
+    """h_s writes psi into slice 0's buffer; every other slice's buffer gets a copy (both halves of a pair)."""
+    M, pair = model.M, prec == "bf16x3"
+    c0 = combs[0].shape[-1] // (2 if pair else 1)
+    fused_h_s_into(model, z_eng, B, hz, wz, prec, combs[0], c0, c0 - 2 * M, lo_flag)
+    for comb in combs[1:]:
+        c = comb.shape[-1] // (2 if pair else 1)
+        comb[..., c - 2 * M:c] = combs[0][..., c0 - 2 * M:c0]
+        if pair:
+            comb[..., 2 * c - 2 * M:] = combs[0][..., 2 * c0 - 2 * M:]
+
+
+def slice_raw(model, s: int, y_eng: torch.Tensor, comb: torch.Tensor, B: int, hy: int, wy: int, prec: str, lo_flag=None) -> torch.Tensor:
+    """The raw entropy parameters [B, (3K | 2) m_s, hy, wy] of slice s from the engine-layout symbols y_eng (all M channels) and
+    the slice's buffer with psi in place: checkerboard conv over the slice, channel conv over the slices before it, 1x1 stack.  The
+    eval forward and both directions of the coder call this."""
+    M, pair = model.M, prec == "bf16x3"
+    o, m = model.offsets[s], model.slices[s]
+    c = comb.shape[-1] // (2 if pair else 1)
+    ctx = model.context_models[s].masked
+    ctx.apply_mask_()
+    ctx._op.run(_channel_window(y_eng, o, o + m, M, pair), B, hy, wy, prec, out=comb, out_c_total=c, out_c_offset=0, in_lo_flag=lo_flag)
+    if s > 0:
+        model.channel_contexts[s - 1]._op.run(_channel_window(y_eng, 0, o, M, pair), B, hy, wy, prec, out=comb, out_c_total=c,
+                                              out_c_offset=2 * m, in_lo_flag=lo_flag)
+    ops = model.entropy_parameters[s].ops
+    a = ops[0].run(comb, B, hy, wy, prec)
+    a = ops[1].run(a, B, hy, wy, prec)
+    return ops[2].run(a, B, hy, wy, prec, out_layout=LAYOUT_NCHW, out_dtype=torch.float32)
+
+
+class ChannelCheckerboardHierarchical(nn.Module):
+    """The space-channel context model (ELIC, He et al., CVPR 2022, after the channel-wise autoregression of Minnen & Singh, ICIP
+    2020; DESIGN.md section 16): JointCheckerboardHierarchical's trunk (g_a, g_s, h_a, h_s, factorized prior) with y split into the
+    channel slices `slices` (default 64-channel slices, any remainder last).  Slice s, channels [o_s, o_s + m_s), is coded from
+    [phi_sp | phi_ch | psi]:
+      * phi_sp = context_models[s] (CheckerboardContextModel(m_s)) over the slice: 0 at the anchors;
+      * phi_ch = channel_contexts[s - 1] (ChannelContextModel(o_s, m_s), s >= 1) over the slices before it: not zeroed, they are
+        fully decoded before slice s starts;
+      * psi = h_s(z_hat), shared by every slice;
+    through entropy_parameters[s] (1x1 stack, cin = 2 m_s (+ 2 m_s) + 2 M -> 640 -> 640 -> (2 | 3K) m_s).  Training reads the noisy
+    y_in of the earlier slices (teacher forcing).  decompress runs two parameter and two rANS passes per slice.
+
+    The trunk is built first and in the parent's order (a seeded build draws the parent's trunk; a parent checkpoint loads its trunk
+    with ``load_state_dict(..., strict=False)``), then the slice modules slice by slice.  With slices=(M,) and the parent's weights
+    under context_models.0 / entropy_parameters.0 the model computes exactly JointCheckerboardHierarchical.
+
+    precision: "bf16x3" (default when M and every slice width are multiples of 64) or "fp32".  The eval forward runs the fused
+    pipeline in fp32 and in bf16x3 at M = 128 / 192, else training._forward_impl without tapes."""
+
+    def __init__(self, latent_channels: int = 192, K: int = 1, slices=None, *, precision: Optional[str] = None):
+        super().__init__()
+        check_channels(latent_channels, K)
+        self.M, self.K, self.H = latent_channels, K, latent_channels
+        self.slices = check_slices(slices, latent_channels)
+        self.offsets = tuple(sum(self.slices[:s]) for s in range(len(self.slices)))
+        tc_ok = all(c % 64 == 0 for c in (self.M,) + self.slices)
+        precision = precision or engine.DEFAULT_PRECISION
+        self.precision = ("bf16x3" if tc_ok else "fp32") if precision == "auto" else precision
+        if self.precision not in ("fp32", "bf16x3") or (self.precision == "bf16x3" and not tc_ok):
+            raise ValueError("ChannelCheckerboardHierarchical: precision must be 'fp32', or 'bf16x3' with latent_channels and every "
+                             f"slice width multiples of 64; got precision={self.precision!r}, slices={self.slices}")
+        self.distribution = "Mean-Scale Gaussian" if K == 1 else "Mixture of Gaussians"
+        self.conditional = GaussianConditional() if K == 1 else GaussianMixtureConditional()
+        # the trunk in JointCheckerboardHierarchical's order, then the slice modules slice by slice
+        self.encoder = Encoder5x5(latent_channels=self.M)
+        self.decoder = Decoder5x5(latent_channels=self.M)
+        self.hyper_encoder = HyperEncoder5x5(latent_channels=self.M)
+        self.hyper_decoder = HyperDecoder5x5(latent_channels=self.M)
+        self.factorized_entropy_model = FactorizedEntropyBottleneck(self.M)
+        self.context_models, self.channel_contexts, self.entropy_parameters = nn.ModuleList(), nn.ModuleList(), nn.ModuleList()
+        for s, (o, m) in enumerate(zip(self.offsets, self.slices)):
+            self.context_models.append(CheckerboardContextModel(latent_channels=m))
+            if s > 0:
+                self.channel_contexts.append(ChannelContextModel(o, m))
+            self.entropy_parameters.append(EntropyParameters(latent_channels=m, hyper_latent_channels=self.H, K=K,
+                                                             context_channels=2 * m if s > 0 else 0))
+
+    @property
+    def fused_pipeline(self) -> bool:
+        """True when the eval forward runs the fused pipeline (fp32, or bf16x3 at M = 128 / 192), else training._forward_impl."""
+        return self.precision == "fp32" or self.M in (128, 192)
+
+    def forward(self, x: torch.Tensor, training: bool = True, *, noise: Optional[Tuple[torch.Tensor, torch.Tensor]] = None,
+                lean: bool = False):
+        """JointCheckerboardHierarchical's dict: p_y / logp_y and mu / sigma (weights / mus / sigmas) over all M channels in channel
+        order; logp_y carries the per-image partial sums for rd_loss."""
+        check_input(x)
+        from . import training as T
+        if training and torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
+            return T.train_forward(self, x, noise=noise, lean=lean)
+        if self.fused_pipeline:
+            return self._forward_fused(x, training, noise, lean)
+        with torch.no_grad():
+            noise_z, noise_y = draw_noise(self.M, x, noise) if training else (None, None)
+            T.forget_pairs()
+            outs, _ = T._forward_impl(self, x.contiguous().float(), noise_z, noise_y, lean, qmode=Q_NOISE if training else Q_ROUND,
+                                      arm=self.precision, record=False)
+            T.forget_pairs()
+        return single_head_outputs(*outs, K=self.K, training=training)
+
+    def _forward_fused(self, x, training, noise, lean):
+        """The trunk on the fused pipeline (g_s a parallel branch of a captured graph), the slices on slice_raw + the likelihood."""
+        B, _, H, W = x.shape
+        M, K, prec = self.M, self.K, self.precision
+        x = x.contiguous().float()
+        hy, wy, hz, wz = H // 16, W // 16, H // 64, W // 64
+        with torch.cuda.device(x.device), torch.no_grad():
+            noise_z, noise_y = draw_noise(M, x, noise) if training else (None, None)
+            y, y_in, y_in_nhwc, y_src = fused_g_a(self, x, training, noise_y, prec, prec)
+            branch, main_stream = _branch_stream(x.device), torch.cuda.current_stream(x.device)
+            if branch is not None:
+                branch.wait_stream(main_stream)
+                with torch.cuda.stream(branch):
+                    x_hat = fused_g_s(self, y_in_nhwc, B, hy, wy, prec)
+            z, z_in, z_in_nhwc = fused_h_a(self, y_src, B, hy, wy, training, noise_z, prec, prec)
+            combs = slice_buffers(self, B, hy, wy, prec, x.device)
+            slice_psi_into(self, z_in_nhwc, B, hz, wz, prec, combs, getattr(z_in_nhwc, "_nic_lo_flag", None))
+            y_flag = getattr(y_in_nhwc, "_nic_lo_flag", None)
+            lys = []
+            for s, (o, m) in enumerate(zip(self.offsets, self.slices)):
+                raw = slice_raw(self, s, y_in_nhwc, combs[s], B, hy, wy, prec, y_flag)
+                y_s = y_in if m == M else y_in[:, o:o + m].contiguous()
+                lys.append(gm_likelihood(y_s, raw, m, K, Q_PASSTHRU, full=not lean, want_y_in=False))
+            logp_y, p_y, parts_y, *params = merge_slices(lys, K, lean)
+            _, p_z, logp_z, parts_z = self.factorized_entropy_model.likelihood(z_in, Q_PASSTHRU)
+            if branch is not None:
+                main_stream.wait_stream(branch)
+            else:
+                x_hat = fused_g_s(self, y_in_nhwc, B, hy, wy, prec)
+        return single_head_outputs(x_hat, logp_y, logp_z, y, y_in, z, z_in, p_z, p_y, parts_y, parts_z, *params, K=K, training=training)
+
+    def compress(self, x: torch.Tensor) -> dict:
+        """x [B, 3, H, W] (any H, W >= 1) -> {"strings": [y_strings, z_strings], "shape": (hz, wz)}: one bytes object per image in
+        each list, coded with the eval-mode symbols of x padded by edge replication to multiples of 64 (shape is the padded one).
+        Format 6: DESIGN.md sections 12 and 16."""
+        from . import channel_codec
+        return channel_codec.compress(self, x)
+
+    def decompress(self, strings, shape) -> dict:
+        """strings / shape as compress returned them (any subset of the images, in any order) -> {"x_hat", "y_hat", "z_hat"}, NCHW f32;
+        x_hat = g_s(y_hat) cropped to the image's size, not clamped.  Raises ValueError on a string of another model, precision arm,
+        M, K or slices, on a malformed string or image size, or when an image's symbol checksum does not match."""
+        from . import channel_codec
+        return channel_codec.decompress(self, strings, shape)
 
 
 class HierarchicalMixtureResidual(nn.Module):

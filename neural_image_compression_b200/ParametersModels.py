@@ -18,7 +18,9 @@ from ._lib import EPI_BIAS, EPI_LRELU
 
 
 class EntropyParameters(nn.Module):
-    def __init__(self, latent_channels: int = 192, hyper_latent_channels: int = 192, K: int = 1):
+    def __init__(self, latent_channels: int = 192, hyper_latent_channels: int = 192, K: int = 1, *, context_channels: int = 0):
+        """context_channels: extra input channels between phi and psi (the channel context of ChannelCheckerboardHierarchical's
+        slices: [phi (2M) | phi_ch (context_channels) | psi (2H)]); 0 is the reference's stack."""
         super().__init__()
         if not isinstance(K, int) or K < 1:
             raise ValueError(f"K must be int >= 1, got {K}")
@@ -26,7 +28,7 @@ class EntropyParameters(nn.Module):
         self.distribution = "Mean-Scale Gaussian" if K == 1 else "Mixture of Gaussians"
         self.latent_channels = latent_channels
         self.hyper_latent_channels = hyper_latent_channels
-        cin = 2 * latent_channels + 2 * hyper_latent_channels
+        cin = 2 * latent_channels + context_channels + 2 * hyper_latent_channels
         cout = 2 * latent_channels if K == 1 else 3 * K * latent_channels
         self.net = nn.Sequential(nn.Conv2d(cin, 640, kernel_size=1), nn.LeakyReLU(),
                                  nn.Conv2d(640, 640, kernel_size=1), nn.LeakyReLU(),

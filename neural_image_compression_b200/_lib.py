@@ -117,6 +117,9 @@ SIGNATURES = {
     "nic_codec_checksum": (C.c_int, [_vp, _i64, _vp, _i64, _i32, _vp, _vp]),
     "nic_codec_encode_checkerboard": (C.c_int, [_vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _i64, _vp, _vp, _vp]),
     "nic_codec_decode_pass": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp]),
+    "nic_codec_encode_checkerboard_slice": (C.c_int, [_vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _i64, _vp, _vp, _vp]),
+    "nic_codec_decode_pass_slice": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _i32,
+                                              _vp, _vp]),
     "nic_checkerboard_zero": (C.c_int, [_vp, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _vp]),
     "nic_codec_params": (C.c_int, [C.POINTER(CodecHead), _i32, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _vp]),
     "nic_image_window": (C.c_int, [_vp, _i32, _i32, _i32, _vp, _i32, _i32, _vp]),

@@ -2,10 +2,11 @@
 //
 //   codec_table_kernel    the ONE place where floats become integer frequencies (encoder and decoder both call it)
 //   codec_encode_kernel   one thread per (image, lane): the lane's symbols in reverse decode order (wavefront, raster or
-//                         checkerboard walk) -> 16-bit words
+//                         checkerboard walk; the checkerboard walk over a channel window [c_off, c_off + m) of c_total channels
+//                         for the channel slices of section 16) -> 16-bit words
 //   codec_decode_kernel   one thread per (image, lane): one wavefront step of y, or all of z
-//   codec_decode_step_kernel  one CTA per (image, lane): one wavefront step of y (section 11) or one checkerboard pass (section 14),
-//                         its tables built in shared memory
+//   codec_decode_step_kernel  one CTA per (image, lane): one wavefront step of y (section 11) or one checkerboard pass (section 14;
+//                         of one channel slice, section 16), its tables built in shared memory
 //   codec_checksum_kernel per-image 32-bit checksum of the y and z symbols
 //
 // rANS: 32-bit state in [2^16, 2^32), 16-bit renormalisation words, 16-bit probability precision.  A table row of one
@@ -217,8 +218,8 @@ __device__ __forceinline__ void rans_put(uint32_t& x, uint32_t start, uint32_t f
 }
 
 __global__ void __launch_bounds__(64)
-codec_encode_kernel(int kind, const uint64_t* __restrict__ code, const float* __restrict__ sym, int b, int m, int h, int w, int lanes,
-                    int cl, int band, long cap, uint16_t* __restrict__ words, int32_t* __restrict__ count) {
+codec_encode_kernel(int kind, const uint64_t* __restrict__ code, const float* __restrict__ sym, int b, int c_total, int c_off, int m, int h,
+                    int w, int lanes, int cl, int band, long cap, uint16_t* __restrict__ words, int32_t* __restrict__ count) {
   const int g = blockIdx.x * blockDim.x + threadIdx.x;
   if (g >= b * lanes) return;
   const int img = g / lanes;
@@ -234,7 +235,7 @@ codec_encode_kernel(int kind, const uint64_t* __restrict__ code, const float* __
     for (int p = cnt - 1; p >= 0; --p) {
       const long pix = lw.pix(t, i0, p);
       for (int c = c_last; c >= 0; c -= cl) {
-        const long e = (static_cast<long>(img) * m + c) * hw + pix;
+        const long e = (static_cast<long>(img) * c_total + c_off + c) * hw + pix;
         const uint64_t cd = code[e];
         if (cd >> 32) {                                        // escape: the raw value words first (they decode after the bin)
           const uint32_t z = zigzag(static_cast<int>(sym[e]));
@@ -332,7 +333,8 @@ constexpr size_t kStepSmem = 2ull * kStepChunk * (kRow * sizeof(uint32_t) + 3 * 
 __global__ void __launch_bounds__(kStepThreads)
 codec_decode_step_kernel(const uint8_t* __restrict__ blob, const int64_t* __restrict__ lane_off, const int32_t* __restrict__ lane_words,
                          uint32_t* __restrict__ state, int32_t* __restrict__ pos, int init, const float* __restrict__ params, int m,
-                         int K, int kind, int h, int w, int lanes, int cl, int band, int t, float* __restrict__ out) {
+                         int K, int kind, int h, int w, int lanes, int cl, int band, int t, int c_total, int c_off,
+                         float* __restrict__ out) {
   extern __shared__ __align__(16) uint32_t s_step[];
   uint32_t* s_cdf = s_step;                                    // [2][kStepChunk][kRow]
   int32_t* s_lo = reinterpret_cast<int32_t*>(s_step + 2 * kStepChunk * kRow);
@@ -398,7 +400,7 @@ codec_decode_step_kernel(const uint8_t* __restrict__ blob, const int64_t* __rest
           v = static_cast<float>(s_lo[e] + a);
         }
         const int p = r / nc, c = c0 + (r - p * nc) * cl;
-        out[(static_cast<long>(img) * hw + s_pix[e]) * m + c] = v;
+        out[(static_cast<long>(img) * hw + s_pix[e]) * c_total + c_off + c] = v;
       }
     }
     __syncthreads();                                           // chunk k decoded, chunk k + 1 built
@@ -464,7 +466,8 @@ int nic_codec_encode(int32_t kind, const uint64_t* code, const float* sym, int32
     return fail(NIC_E_BADSHAPE, "codec_encode: b=%d m=%d h=%d w=%d lanes=%d", b, m, h, w, lanes);
   if (cap < 3L * ((m + lanes - 1) / lanes) * h * w + 2) return fail(NIC_E_WORKSPACE, "codec_encode: lane capacity %lld words", static_cast<long long>(cap));
   if (!code || !sym || !words || !count) return fail(NIC_E_BADSHAPE, "codec_encode: null pointer");
-  codec_encode_kernel<<<(b * lanes + 63) / 64, 64, 0, as_stream(stream)>>>(kind, code, sym, b, m, h, w, lanes, lanes, 0, cap, words, count);
+  codec_encode_kernel<<<(b * lanes + 63) / 64, 64, 0, as_stream(stream)>>>(kind, code, sym, b, m, 0, m, h, w, lanes, lanes, 0, cap, words,
+                                                                           count);
   return check_launch("codec_encode_kernel");
 }
 
@@ -491,7 +494,7 @@ int nic_codec_decode_step(const uint8_t* blob, const int64_t* lane_off, const in
   if (!blob || !lane_off || !lane_words || !state || !pos || !params || !out) return fail(NIC_E_BADSHAPE, "codec_decode_step: null pointer");
   if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(codec_decode_step_kernel), static_cast<int>(kStepSmem))) return rc;
   codec_decode_step_kernel<<<b * lanes, kStepThreads, kStepSmem, as_stream(stream)>>>(blob, lane_off, lane_words, state, pos, init, params,
-                                                                                      m, k, NIC_CODEC_GM, h, w, lanes, lanes, 0, t, out);
+                                                                                      m, k, NIC_CODEC_GM, h, w, lanes, lanes, 0, t, m, 0, out);
   return check_launch("codec_decode_step_kernel");
 }
 
@@ -502,32 +505,49 @@ static int checkerboard_lanes(const char* what, int32_t b, int32_t m, int32_t h,
   return NIC_OK;
 }
 
-int nic_codec_encode_checkerboard(const uint64_t* code, const float* sym, int32_t b, int32_t m, int32_t h, int32_t w, int32_t lanes_c,
-                                  int32_t band_rows, int64_t cap, uint16_t* words, int32_t* count, void* stream) {
+int nic_codec_encode_checkerboard_slice(const uint64_t* code, const float* sym, int32_t b, int32_t c_total, int32_t c_off, int32_t m,
+                                        int32_t h, int32_t w, int32_t lanes_c, int32_t band_rows, int64_t cap, uint16_t* words, int32_t* count,
+                                        void* stream) {
   if (int rc = nic_check_device()) return rc;
   int lanes;
   if (int rc = checkerboard_lanes("codec_encode_checkerboard", b, m, h, w, lanes_c, band_rows, &lanes)) return rc;
+  if (c_off < 0 || c_total < c_off + m)
+    return fail(NIC_E_BADSHAPE, "codec_encode_checkerboard: channels [%d, %d) of %d", c_off, c_off + m, c_total);
   if (cap < 3L * ((m + lanes_c - 1) / lanes_c) * band_rows * w + 2)
     return fail(NIC_E_WORKSPACE, "codec_encode_checkerboard: lane capacity %lld words", static_cast<long long>(cap));
   if (!code || !sym || !words || !count) return fail(NIC_E_BADSHAPE, "codec_encode_checkerboard: null pointer");
-  codec_encode_kernel<<<(b * lanes + 63) / 64, 64, 0, as_stream(stream)>>>(kWalkCheckerboard, code, sym, b, m, h, w, lanes, lanes_c, band_rows,
-                                                                           cap, words, count);
+  codec_encode_kernel<<<(b * lanes + 63) / 64, 64, 0, as_stream(stream)>>>(kWalkCheckerboard, code, sym, b, c_total, c_off, m, h, w, lanes,
+                                                                           lanes_c, band_rows, cap, words, count);
   return check_launch("codec_encode_kernel");
+}
+
+int nic_codec_encode_checkerboard(const uint64_t* code, const float* sym, int32_t b, int32_t m, int32_t h, int32_t w, int32_t lanes_c,
+                                  int32_t band_rows, int64_t cap, uint16_t* words, int32_t* count, void* stream) {
+  return nic_codec_encode_checkerboard_slice(code, sym, b, m, 0, m, h, w, lanes_c, band_rows, cap, words, count, stream);
+}
+
+int nic_codec_decode_pass_slice(const uint8_t* blob, const int64_t* lane_off, const int32_t* lane_words, uint32_t* state, int32_t* pos,
+                                const float* params, int32_t b, int32_t c_total, int32_t c_off, int32_t m, int32_t k, int32_t h, int32_t w,
+                                int32_t lanes_c, int32_t band_rows, int32_t pass, float* out, void* stream) {
+  if (int rc = nic_check_device()) return rc;
+  int lanes;
+  if (int rc = checkerboard_lanes("codec_decode_pass", b, m, h, w, lanes_c, band_rows, &lanes)) return rc;
+  if (k < 1 || k > 5 || (pass != 0 && pass != 1)) return fail(NIC_E_BADSHAPE, "codec_decode_pass: k=%d pass=%d", k, pass);
+  if (c_off < 0 || c_total < c_off + m)
+    return fail(NIC_E_BADSHAPE, "codec_decode_pass: channels [%d, %d) of %d", c_off, c_off + m, c_total);
+  if (!blob || !lane_off || !lane_words || !state || !pos || !params || !out) return fail(NIC_E_BADSHAPE, "codec_decode_pass: null pointer");
+  if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(codec_decode_step_kernel), static_cast<int>(kStepSmem))) return rc;
+  codec_decode_step_kernel<<<b * lanes, kStepThreads, kStepSmem, as_stream(stream)>>>(blob, lane_off, lane_words, state, pos, pass == 0,
+                                                                                      params, m, k, kWalkCheckerboard, h, w, lanes, lanes_c,
+                                                                                      band_rows, pass, c_total, c_off, out);
+  return check_launch("codec_decode_step_kernel");
 }
 
 int nic_codec_decode_pass(const uint8_t* blob, const int64_t* lane_off, const int32_t* lane_words, uint32_t* state, int32_t* pos,
                           const float* params, int32_t b, int32_t m, int32_t k, int32_t h, int32_t w, int32_t lanes_c, int32_t band_rows,
                           int32_t pass, float* out, void* stream) {
-  if (int rc = nic_check_device()) return rc;
-  int lanes;
-  if (int rc = checkerboard_lanes("codec_decode_pass", b, m, h, w, lanes_c, band_rows, &lanes)) return rc;
-  if (k < 1 || k > 5 || (pass != 0 && pass != 1)) return fail(NIC_E_BADSHAPE, "codec_decode_pass: k=%d pass=%d", k, pass);
-  if (!blob || !lane_off || !lane_words || !state || !pos || !params || !out) return fail(NIC_E_BADSHAPE, "codec_decode_pass: null pointer");
-  if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(codec_decode_step_kernel), static_cast<int>(kStepSmem))) return rc;
-  codec_decode_step_kernel<<<b * lanes, kStepThreads, kStepSmem, as_stream(stream)>>>(blob, lane_off, lane_words, state, pos, pass == 0,
-                                                                                      params, m, k, kWalkCheckerboard, h, w, lanes, lanes_c,
-                                                                                      band_rows, pass, out);
-  return check_launch("codec_decode_step_kernel");
+  return nic_codec_decode_pass_slice(blob, lane_off, lane_words, state, pos, params, b, m, 0, m, k, h, w, lanes_c, band_rows, pass, out,
+                                     stream);
 }
 
 int nic_codec_checksum(const float* y, int64_t y_per_image, const float* z, int64_t z_per_image, int32_t b, uint32_t* out, void* stream) {

@@ -49,7 +49,7 @@ from .engine import checkerboard_zero_
 from ._lib import (ConvDesc, DT_F32, EPI_BIAS, EPI_LRELU, LAYOUT_NCHW, LAYOUT_NHWC, MASK_CHECKERBOARD, PREC_FP32, Q_NOISE, Q_PASSTHRU, Q_ROUND,
                    check, current_stream, ptr)
 from .EntropyModels import gm_likelihood
-from .Models import draw_noise, mixture_params, single_head_outputs
+from .Models import draw_noise, merge_slices, mixture_params, single_head_outputs
 
 PREC = "fp32"
 WGRAD_TC = os.environ.get("NIC_WGRAD_TC", "1") != "0"      # tensor-core weight gradients in the bf16x3 arm (0: fp32 kernel everywhere)
@@ -500,7 +500,11 @@ _FACT_SLICES = (("matrices", 0, 0, 3), ("biases", 0, 3, 6), ("factors", 0, 6, 9)
 def heads(model) -> list:
     """[(context model, entropy parameters, c0, c1)]: the entropy heads of a model, each over the channels [c0, c1) of y and the
     shared hyper features psi.  One head over all of y (JointAutoregressiveHierarchical, HierarchicalMixtureResidual); the base
-    [0, M1) and the enhancement [M1, M) head of ScalableImageCoding."""
+    [0, M1) and the enhancement [M1, M) head of ScalableImageCoding.  ChannelCheckerboardHierarchical: one head per channel slice,
+    each with a fifth entry, its channel context model over y[:, :c0] (None for the first slice)."""
+    if hasattr(model, "slices"):
+        return [(model.context_models[s], model.entropy_parameters[s], o, o + m, model.channel_contexts[s - 1] if s else None)
+                for s, (o, m) in enumerate(zip(model.offsets, model.slices))]
     if hasattr(model, "M1"):
         return [(model.context_model_1, model.entropy_parameters_1, 0, model.M1),
                 (model.context_model_2, model.entropy_parameters_2, model.M1, model.M)]
@@ -516,27 +520,34 @@ def gm_likelihood_bwd(y: torch.Tensor, raw: torch.Tensor, g_logp: torch.Tensor, 
     return dy, draw
 
 
-def head_forward(arm: str, head, K: int, y_i: torch.Tensor, y_i_nhwc: torch.Tensor, comb: torch.Tensor, lean: bool):
+def head_forward(arm: str, head, K: int, y_i: torch.Tensor, y_i_nhwc: torch.Tensor, comb: torch.Tensor, lean: bool,
+                 y_prev_nhwc: Optional[torch.Tensor] = None):
     """One entropy head on its symbols y_i (NCHW) / y_i_nhwc: the context conv writes phi into channels [0, 2 m) of the concat
-    buffer `comb` (NHWC, psi already at [2 m, 2 m + 2 M)), then the 1x1 stack and the likelihood.  -> (likelihood dict, the
-    tensors head_backward reads)."""
-    ctx, ep, c0, c1 = head
+    buffer `comb` (NHWC, psi already in its last 2 M channels), a channel context conv (fifth entry of the head) phi_ch of
+    y_prev_nhwc = y_in[..., :c0] into [2 m, 4 m), then the 1x1 stack and the likelihood.  -> (likelihood dict, the tensors
+    head_backward reads)."""
+    ctx, ep, c0, c1 = head[:4]
+    chan = head[4] if len(head) > 4 else None
     B, hy, wy, _ = y_i_nhwc.shape
     ctx.masked.apply_mask_()
     conv_forward(arm, ctx.masked, EPI_BIAS, y_i_nhwc, B, hy, wy, out=comb, out_c_total=comb.shape[-1], out_c_offset=0,
                  mask_a=ctx.masked._op.mask_a)
+    if chan is not None:
+        conv_forward(arm, chan.conv, EPI_BIAS, y_prev_nhwc, B, hy, wy, out=comb, out_c_total=comb.shape[-1], out_c_offset=2 * (c1 - c0))
     ops = ep.ops
     e1 = conv_forward(arm, ops[0].conv, ops[0].epilogue, comb, B, hy, wy)
     e2 = conv_forward(arm, ops[1].conv, ops[1].epilogue, e1, B, hy, wy)
     raw = conv_forward(arm, ops[2].conv, ops[2].epilogue, e2, B, hy, wy, out_layout=LAYOUT_NCHW)
     ly = gm_likelihood(y_i, raw, c1 - c0, K, Q_PASSTHRU, full=not lean, want_y_in=False)
-    return ly, dict(comb=comb, e1=e1, e2=e2, raw=raw, y_i=y_i, y_i_nhwc=y_i_nhwc)
+    return ly, dict(comb=comb, e1=e1, e2=e2, raw=raw, y_i=y_i, y_i_nhwc=y_i_nhwc, y_prev_nhwc=y_prev_nhwc)
 
 
-def head_backward(arm: str, head, K: int, st: dict, g_logp: torch.Tensor, put, wgrad):
+def head_backward(arm: str, head, K: int, st: dict, g_logp: torch.Tensor, put, wgrad, prev=(), d_prev: Optional[list] = None):
     """Backward of head_forward from the gradient of the head's logp: -> (gradient of y_i, NHWC; gradient of psi, NHWC).
-    Parameter gradients go to put(param, grad); wgrad = conv_wgrad or its side-stream form (as in Tape.backward)."""
-    ctx, ep, c0, c1 = head
+    Parameter gradients go to put(param, grad); wgrad = conv_wgrad or its side-stream form (as in Tape.backward).  A head with a
+    channel context appends to d_prev the gradients (NHWC) of the channel ranges `prev` of y_prev, one per range."""
+    ctx, ep, c0, c1 = head[:4]
+    chan = head[4] if len(head) > 4 else None
     m = c1 - c0
     B, hy, wy, _ = st["y_i_nhwc"].shape
     dy_lik, draw = gm_likelihood_bwd(st["y_i"], st["raw"], g_logp.contiguous().float(), m, K)
@@ -548,10 +559,18 @@ def head_backward(arm: str, head, K: int, st: dict, g_logp: torch.Tensor, put, w
         put(op.conv.weight, dw); put(op.conv.bias, db)
         if i > 0:
             g = lrelu_bwd_(conv_dgrad(op.conv, g, B, hy, wy, arm=arm), a)
-    # the first 1x1 conv reads [phi | psi]: its data gradient splits along its input channels
+    # the first 1x1 conv reads [phi | psi] ([phi | phi_ch | psi] with a channel context): its data gradient splits along its input
+    # channels
     w0 = ops[0].conv.weight.detach()
+    cp = 4 * m if chan is not None else 2 * m
     d_phi = conv_dgrad(ops[0].conv, g, B, hy, wy, weight=w0[:, :2 * m].contiguous(), c_in=2 * m, arm=arm)
-    d_psi = conv_dgrad(ops[0].conv, g, B, hy, wy, weight=w0[:, 2 * m:].contiguous(), c_in=w0.shape[1] - 2 * m, arm=arm)
+    d_psi = conv_dgrad(ops[0].conv, g, B, hy, wy, weight=w0[:, cp:].contiguous(), c_in=w0.shape[1] - cp, arm=arm)
+    if chan is not None:
+        d_ch = conv_dgrad(ops[0].conv, g, B, hy, wy, weight=w0[:, 2 * m:cp].contiguous(), c_in=2 * m, arm=arm)
+        dw, db = wgrad(chan.conv, st["y_prev_nhwc"], d_ch, B, hy, wy, LAYOUT_NHWC, LAYOUT_NHWC, arm=arm)
+        put(chan.conv.weight, dw); put(chan.conv.bias, db)
+        wc = chan.conv.weight.detach()
+        d_prev.extend(conv_dgrad(chan.conv, d_ch, B, hy, wy, weight=wc[:, a:b].contiguous(), c_in=b - a, arm=arm) for a, b in prev)
     if ctx.masked._op.mask_a == MASK_CHECKERBOARD:
         checkerboard_zero_(d_phi)                                # phi is the constant 0 at the anchors
     dw, db = wgrad(ctx.masked, st["y_i_nhwc"], d_phi, B, hy, wy, LAYOUT_NHWC, LAYOUT_NHWC, arm=arm)
@@ -624,17 +643,19 @@ def _forward_impl(model, x, noise_z, noise_y, lean, qmode: int = Q_NOISE, arm: O
         else:
             z, z_in, z_in_nhwc, _, hs_in = engine.latent_handoff_gain(z_nhwc, qmode, noise_z, gains.g_z, gains.ginv_z, torch.float32,
                                                                       None, torch.float32)
-        # h_s writes psi into head 0's concat buffer [phi_0 (2 m_0) | psi (2 M)]; every other head's buffer gets a copy of it
-        combs = [_f32((B, hy, wy, 2 * (c1 - c0) + 2 * M), dev) for _, _, c0, c1 in hds]
-        m0 = hds[0][3] - hds[0][2]
+        # h_s writes psi into the last 2 M channels of head 0's concat buffer [phi_0 (2 m_0) | (phi_ch) | psi (2 M)]; every other
+        # head's buffer gets a copy of it
+        combs = [_f32((B, hy, wy, head[1].net[0].in_channels), dev) for head in hds]
+        p0 = combs[0].shape[-1] - 2 * M
         model.hyper_decoder.run_nhwc(hs_in, B, hz, wz, arm, tape=S["h_s"],
-                                     final_kw=dict(out=combs[0], out_c_total=combs[0].shape[-1], out_c_offset=2 * m0))
-        for (_, _, c0, c1), comb in zip(hds[1:], combs[1:]):
-            comb[..., 2 * (c1 - c0):] = combs[0][..., 2 * m0:]
+                                     final_kw=dict(out=combs[0], out_c_total=combs[0].shape[-1], out_c_offset=p0))
+        for comb in combs[1:]:
+            comb[..., comb.shape[-1] - 2 * M:] = combs[0][..., p0:]
         lys, states = [], []
         for head, comb in zip(hds, combs):
             c0, c1 = head[2], head[3]
-            ly, st = head_forward(arm, head, K, y_in[:, c0:c1].contiguous(), y_in_nhwc[..., c0:c1].contiguous(), comb, lean)
+            prev = y_in_nhwc[..., :c0].contiguous() if len(head) > 4 and head[4] is not None else None
+            ly, st = head_forward(arm, head, K, y_in[:, c0:c1].contiguous(), y_in_nhwc[..., c0:c1].contiguous(), comb, lean, prev)
             lys.append(ly)
             states.append(st)
         _, p_z, logp_z, parts_z = model.factorized_entropy_model.likelihood(z_in, Q_PASSTHRU)
@@ -642,8 +663,12 @@ def _forward_impl(model, x, noise_z, noise_y, lean, qmode: int = Q_NOISE, arm: O
             main.wait_stream(branch)
         else:
             x_hat = synthesis()
-    outs = (x_hat, *[ly["logp"] for ly in lys], logp_z, y, y_in, z, z_in, p_z, *[ly["p"] for ly in lys],
-            *[ly["partials"] for ly in lys], parts_z, *[t for ly in lys for t in mixture_params(ly, K, lean)])
+    if hasattr(model, "slices"):                 # channel slices: one p_y / logp_y over all M channels (single_head_outputs' order)
+        logp_y, p_y, parts_y, *params = merge_slices(lys, K, lean)
+        outs = (x_hat, logp_y, logp_z, y, y_in, z, z_in, p_z, p_y, parts_y, parts_z, *params)
+    else:
+        outs = (x_hat, *[ly["logp"] for ly in lys], logp_z, y, y_in, z, z_in, p_z, *[ly["p"] for ly in lys],
+                *[ly["partials"] for ly in lys], parts_z, *[t for ly in lys for t in mixture_params(ly, K, lean)])
     if not record:
         return outs, None
     # the roots of the g_s, h_s and h_a tapes (the symbols and y itself without gain units)
@@ -703,13 +728,21 @@ def _backward_impl(model, S, g_xhat, g_logp_heads, g_logp_z, partial_hook=None) 
                 d_yin_gs = S["g_s"].backward(g_xhat.contiguous().float(), LAYOUT_NCHW, put, conv_wgrad_async, root=S["y_in_nhwc"],
                                              side=side, keep=keep)
         # ---- p_y: every head's likelihood, entropy parameters and context model; h_s --------------------------------
-        # the y gradient of the entropy path is the channel concatenation of the heads', the psi gradient their sum
+        # the y gradient of the entropy path is the channel concatenation of the heads', the psi gradient their sum; a head's channel
+        # context adds its gradient of y[:, :c0] into the heads before it, head by head in order
         d_zin = None
+        hds = heads(model)
+        if len(g_logp_heads) == 1 and len(hds) > 1 and g_logp_heads[0] is not None:      # channel slices: one logp_y over all of y
+            g_logp_heads = [g_logp_heads[0][:, h[2]:h[3]] for h in hds]
         if all(g is not None for g in g_logp_heads):
             d_ys, d_psi = [], None
-            for head, st, gl in zip(heads(model), S["heads"], g_logp_heads):
-                d_y, d_psi_i = head_backward(arm, head, model.K, st, gl, put, conv_wgrad_async)
+            for i, (head, st, gl) in enumerate(zip(hds, S["heads"], g_logp_heads)):
+                prev = [(h[2], h[3]) for h in hds[:i]]
+                d_prev = []
+                d_y, d_psi_i = head_backward(arm, head, model.K, st, gl, put, conv_wgrad_async, prev, d_prev)
                 d_ys.append(d_y)
+                for d_j, g_j in zip(d_ys, d_prev):
+                    add_(d_j, g_j)
                 d_psi = d_psi_i if d_psi is None else add_(d_psi, d_psi_i)
             d_yin = d_ys[0] if len(d_ys) == 1 else torch.cat(d_ys, dim=-1)
             del d_ys
